@@ -3,13 +3,24 @@
 AC254-150-AB doublet spot diagram, 2^20 collimated rays (Fibonacci disc, 20 mm), sequential SDF
 lens-surface path, Spotdetector at the vendor back focus.  Metric: ray-surface interactions/s.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One "step" = one full solve_system! of the ray bundle (all waves).  `value` is measured with the rays
 resident in HBM (device pointers into the C ABI, spot output left on the device); `e2e` goes through
 the same C ABI with pinned HOST buffers, host->device and device->host copies inside the timed
 region.  Rank r of an N-GPU run traces its own 2^20-ray shard (weak scaling, no data-path
 collective: rays are independent, outputs are disjoint slices).
+
+--dump-outputs DIR writes what the last timed step of each leg returned to its caller as DIR/<name>.npy
+(rank 0's shard), so that two builds can be compared output for output; the inputs are fixed, so the same
+arguments give the same inputs on every run:
+    spot_xz, spot_object, nseg, interactions   resident leg: Spotdetector (x, z) per ray (NaN: no detector
+                                               reached), detector object id (-1: none), segments per ray
+    e2e_spot_xz, e2e_interactions              the same from the host-buffer leg
+    detector_field, detector_pixel_index       C3 Photodetector field (re, im) at a fixed seeded sample of
+                                               its pixels (column-major pixel index)
+    ray_index                                  only with --rays above 2^20: the fixed seeded sample of rays
+                                               the per-ray arrays hold
 """
 import argparse
 import json
@@ -36,6 +47,8 @@ FLOP_SDF, FLOP_TRI, FLOP_INT = 45.0, 40.0, 60.0
 K1_DRAM_BYTES_PER_LAUNCH = 91.1e6
 K1_TRAFFIC_SOURCE = ("profiles/r02l_ncu_k1_lean.txt (mean of the 4 waves, 2^20 rays per launch: 67.2 MB read + 23.9 MB written; algorithmic = 64 B ray "
                      "state read + 36 B hit record written per ray -- part of the hit records is still in the 126 MB L2 when the kernel ends)")
+# --dump-outputs: at most this many bytes in all; per-ray arrays keep at most DUMP_RAYS rows, the detector field DUMP_PIXELS pixels
+DUMP_BYTES, DUMP_RAYS, DUMP_PIXELS = 64 << 20, 1 << 20, 1 << 18
 
 
 def rays_for_rank(rank, n=N_RAYS):
@@ -48,6 +61,24 @@ def rays_for_rank(rank, n=N_RAYS):
         x, z = pos[:, 0].copy(), pos[:, 2].copy()
         pos[:, 0], pos[:, 2] = c * x - s * z, s * x + c * z
     return np.ascontiguousarray(pos), np.ascontiguousarray(d)
+
+
+def sample_index(n, cap, seed):
+    """Rows kept by --dump-outputs: all n, or a fixed seeded sample of `cap` of them in ascending order."""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, cap, replace=False))
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as <path>/<name>.npy; all are float32 / float64 and DUMP_BYTES at most together."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes, more than {DUMP_BYTES}")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def bind_to_gpu_numa(local_rank):
@@ -191,7 +222,10 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary retrace (a4) and PSFDetector (N2) measurements")
     ap.add_argument("--no-numa", action="store_true", help="leave the CPU affinity of the rank alone")
     ap.add_argument("--full-inputs", action="store_true", help="e2e ships a direction and a wavelength id per ray (52 B/ray) instead of one of each per bundle")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of each leg as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -241,12 +275,15 @@ def main():
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")   # > 126 MB L2
     torch.cuda.synchronize()
 
+    kept = []      # the newest resident result: freed when the next step starts, so the last one is still there for --dump-outputs
+
     def step_device():
+        while kept:
+            kept.pop().free()
         res = m.trace_rays(dsys, (pos_d.data_ptr(), n), dir_d.data_ptr(), lam_d.data_ptr(), None, None, 100,
                            keep_segments=False, device_inputs=True)
-        inter = res.interactions
-        res.free()
-        return inter
+        kept.append(res)
+        return res.interactions
 
     import ctypes as C
     if args.full_inputs:
@@ -296,6 +333,16 @@ def main():
         sampler.start()
     times, inter = timed(step_device, args.steps, args.warmup, "trace_resident")
     c = L.counters(dev)
+    dump = {} if args.dump_outputs and rank == 0 else None
+    last = kept.pop()
+    if dump is not None:
+        rows = sample_index(n, DUMP_RAYS, seed=1)
+        obj, xz = last.spots()
+        dump.update(spot_xz=xz[rows], spot_object=obj[rows].astype(np.float32),
+                    nseg=last.beams()["nseg"][rows].astype(np.float32), interactions=np.array([last.interactions], np.float64))
+        if len(rows) < n:
+            dump["ray_index"] = rows.astype(np.float64)
+    last.free()
     n_total_steps = args.steps
     solo_ms = None
     if world > 1:
@@ -305,6 +352,8 @@ def main():
             solo_ms = sum(t_solo) / len(t_solo)
         dist.barrier()
     times_e, inter_e = timed(step_e2e, args.steps, args.warmup, "trace_e2e")
+    if dump is not None:
+        dump.update(e2e_spot_xz=spot_xz_p.numpy()[rows], e2e_interactions=np.array([inter_e], np.float64))
 
     def agg(times):
         t = torch.tensor([sum(times)], dtype=torch.float64, device="cuda")
@@ -327,7 +376,7 @@ def main():
     det = None
     if not args.no_detector:
         sampler.mark("detector", True)
-        det = bench_detector(m, L, dev, stream, args.c3_side, args.c3_pixels, 2, 1, flush, peak, rank, world, comm)
+        det = bench_detector(m, L, dev, stream, args.c3_side, args.c3_pixels, 2, 1, flush, peak, rank, world, comm, dump)
         sampler.mark("detector", False)
     if extras is not None:
         extras["psf"] = bench_psf(m, L, dev, stream, flush, peak)
@@ -380,6 +429,8 @@ def main():
             out.update(extras)
         if not args.no_cpu_baseline:
             out["cpu_baseline"] = cpu_baseline()
+        if dump is not None:
+            dump_outputs(args.dump_outputs, dump)
         print(json.dumps(out), file=json_out)
         json_out.flush()
     if comm is not None:
@@ -430,11 +481,12 @@ FLOP_PAIR = 226.0       # the same weights (add/mul 1, sqrt/div 8, transcendenta
                         # pd_field_fast, counted op by op in DESIGN.md "K4" -- the work the kernel actually has to do
 
 
-def bench_detector(m, L, dev, stream, k_side, pd_n, steps, warmup, flush, peak_tflops, rank=0, world=1, comm=None):
+def bench_detector(m, L, dev, stream, k_side, pd_n, steps, warmup, flush, peak_tflops, rank=0, world=1, comm=None, dump=None):
     """Metric 2 (Photodetector px-beamlets/s) on the C3 workload: Keplerian expander + Photodetector(40 mm, pd_n), the
     k_side x k_side beamlet lattice (pitch 8 mm / 256, w0 = 1.5 pitch, lambda = 1 um; k_side = 256 is BASELINE's 65536-beamlet
     config).  STRONG scaling: the lattice is cut into `world` bands of rows, rank r traces and accumulates band r onto a full
-    partial field, and the partial fields are summed by bmo_pd_allreduce (NCCL inside libbmo.so) inside the timed region."""
+    partial field, and the partial fields are summed by bmo_pd_allreduce (NCCL inside libbmo.so) inside the timed region.
+    `dump` (a dict, --dump-outputs) receives a fixed sample of the field the last timed step left on the device."""
     import ctypes as C
     import torch
     from tests import scenes2 as s2
@@ -495,6 +547,9 @@ def bench_detector(m, L, dev, stream, k_side, pd_n, steps, warmup, flush, peak_t
     pairs = out["device"]["pairs"]
     ach = FLOP_PAIR * out["device"]["pairs_rank"] / (out["device"]["k4_ms"] * 1e-3) / 1e12
     res.free()
+    if dump is not None:
+        px = sample_index(pd_n * pd_n, DUMP_PIXELS, seed=2)
+        dump.update(detector_field=field_d.view(-1, 2).cpu().numpy()[px], detector_pixel_index=px.astype(np.float64))
     nbytes = int(field_h.numel() * 8)
     return {
         "metric": "Photodetector px-beamlets/s", "unit": "px-beamlets/s",
