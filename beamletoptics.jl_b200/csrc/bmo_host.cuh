@@ -32,7 +32,9 @@ struct NvtxRange {
     NvtxRange& operator=(const NvtxRange&) = delete;
 };
 
-struct DevCounters { unsigned long long interactions, sdf, tri, bad_ids; };   // bad_ids: rays whose lambda_id / pose_id was out of range (init_queue)
+// bad_ids: rays whose lambda_id / pose_id was out of range (init_queue, solve_rays_persistent).
+// tiles, most_nseg: per-call words of solve_rays_persistent (zeroed by every such call): next tile of rays, largest nseg of a ray.
+struct DevCounters { unsigned long long interactions, sdf, tri, bad_ids, tiles, most_nseg; };
 
 }  // namespace bmo
 
@@ -46,12 +48,16 @@ struct bmo_ctx {
     int64_t k1_launches = 0, interactions_seen = 0, bad_ids_seen = 0;
     bmo::DevCounters* d_counters = nullptr;
     long long* d_totals = nullptr;   // [4] scratch for scans
-    long long* h_totals = nullptr;   // pinned, 8 entries for the scans + 8 per sub-batch slot
+    long long* h_totals = nullptr;   // pinned, 8 entries for the scans + 8 per sub-batch slot + the device counters (72..77)
     int64_t waves = 0, launches = 0, px_beamlets = 0, psf_pairs = 0;
     double psf_ms = 0;
     double trace_ms = 0, pd_ms = 0;
     int64_t pool_slack = 0;   // bytes by which bmo_retrace has grown the stream-ordered pool beyond its own needs (see there)
     int sm_count = 148;
+    // solve_rays_persistent (bmo_trace.cu: persistent_blocks): the variant and table size last sized, its resident blocks per SM
+    const void* persist_fn = nullptr;
+    size_t persist_smem = 0;
+    int persist_blocks = 0;
 };
 
 struct bmo_sys {

@@ -14,6 +14,8 @@
 //                         number them deterministically and append the reflected ones to the queue.
 //   K1+K2 fused_wave0     plain rays through a splitter-free system, all waves of a chunk in one launch (used by
 //                         pipelined host-input calls, where the number of launches is what limits).
+// Plain rays through a splitter-free LEAN system whose segments are not kept need no waves at all: solve_rays_persistent
+// carries every ray from the caller's inputs to its last interaction in one launch.
 //   K1r retrace_intersect_wave   K1 of a retrace call (stored path re-validated per beam).
 //   K3 compact_fused      queue compaction in one cooperative launch once the dead slots are the majority
 //                         (compact_count + scan_counts + compact_scatter as the fallback).
@@ -109,6 +111,24 @@ BMO_D V3 shfl3(V3 v, int l) {
 
 // ---- K1: intersect ------------------------------------------------------------------------------
 constexpr int IBLOCK = 128;
+// Copies the small system tables into shared memory with the NT threads of the block: prims | parts | bounds, and for the LEAN
+// kernels one packed word per part (lean_part_info).  The caller synchronises the block.
+template <int NT, bool LEAN>
+BMO_D void stage_tables(const SysView& S, unsigned char* smem) {
+    const int nw = S.n_prims * (int)(sizeof(bmo_prim) / 8), nq = S.n_parts * (int)(sizeof(bmo_part) / 8);
+    const double* src = reinterpret_cast<const double*>(S.prims);
+    double* dst = reinterpret_cast<double*>(smem);
+    for (int k = threadIdx.x; k < nw; k += NT) dst[k] = src[k];
+    src = reinterpret_cast<const double*>(S.parts);
+    dst = reinterpret_cast<double*>(smem + (size_t)S.n_prims * sizeof(bmo_prim));
+    for (int k = threadIdx.x; k < nq; k += NT) dst[k] = src[k];
+    double* s_bounds = reinterpret_cast<double*>(smem + (size_t)S.n_prims * sizeof(bmo_prim) + (size_t)S.n_parts * sizeof(bmo_part));
+    for (int k = threadIdx.x; k < NBOUND * S.n_parts; k += NT) s_bounds[k] = S.bounds[k];
+    if (LEAN) {
+        unsigned long long* s_pinfo = reinterpret_cast<unsigned long long*>(s_bounds + NBOUND * S.n_parts);
+        for (int k = threadIdx.x; k < S.n_parts; k += NT) s_pinfo[k] = lean_part_info(S.parts[k], S.objects[S.parts[k].object]);
+    }
+}
 // STAGED: the small system tables (prims, parts, bounds) live in shared memory -- a compile-time fact,
 // so that the marching loop reads them with LDS instead of generic loads.
 // LEAN: every SDF part is a union of at most 4 plain primitives and every mesh is small (bmo_sys::all_lean): the union loop keeps
@@ -134,18 +154,7 @@ __global__ void __launch_bounds__(IBLOCK, MINB) intersect_wave(const IntersectPa
     bmo_part* s_parts = reinterpret_cast<bmo_part*>(smem_raw + (size_t)S.n_prims * sizeof(bmo_prim));
     double* s_bounds = reinterpret_cast<double*>(smem_raw + (size_t)S.n_prims * sizeof(bmo_prim) + (size_t)S.n_parts * sizeof(bmo_part));
     if (STAGED) {
-        const int nw = S.n_prims * (int)(sizeof(bmo_prim) / 8), nq = S.n_parts * (int)(sizeof(bmo_part) / 8);
-        const double* src = reinterpret_cast<const double*>(S.prims);
-        double* dst = reinterpret_cast<double*>(s_prims);
-        for (int k = threadIdx.x; k < nw; k += IBLOCK) dst[k] = src[k];
-        src = reinterpret_cast<const double*>(S.parts);
-        dst = reinterpret_cast<double*>(s_parts);
-        for (int k = threadIdx.x; k < nq; k += IBLOCK) dst[k] = src[k];
-        for (int k = threadIdx.x; k < NBOUND * S.n_parts; k += IBLOCK) s_bounds[k] = S.bounds[k];
-        if (LEAN) {
-            unsigned long long* s_pinfo = reinterpret_cast<unsigned long long*>(s_bounds + NBOUND * S.n_parts);
-            for (int k = threadIdx.x; k < S.n_parts; k += IBLOCK) s_pinfo[k] = lean_part_info(S.parts[k], S.objects[S.parts[k].object]);
-        }
+        stage_tables<IBLOCK, LEAN>(S, smem_raw);
         __syncthreads();
     }
 
@@ -215,18 +224,7 @@ __global__ void __launch_bounds__(Cfg<MODE>::BLOCK, 6) retrace_intersect_wave(co
     bmo_part* s_parts = reinterpret_cast<bmo_part*>(smem_raw + (size_t)S.n_prims * sizeof(bmo_prim));
     double* s_bounds = reinterpret_cast<double*>(smem_raw + (size_t)S.n_prims * sizeof(bmo_prim) + (size_t)S.n_parts * sizeof(bmo_part));
     if (STAGED) {
-        const int nw = S.n_prims * (int)(sizeof(bmo_prim) / 8), nq = S.n_parts * (int)(sizeof(bmo_part) / 8);
-        const double* src = reinterpret_cast<const double*>(S.prims);
-        double* dst = reinterpret_cast<double*>(s_prims);
-        for (int k = threadIdx.x; k < nw; k += Cfg<MODE>::BLOCK) dst[k] = src[k];
-        src = reinterpret_cast<const double*>(S.parts);
-        dst = reinterpret_cast<double*>(s_parts);
-        for (int k = threadIdx.x; k < nq; k += Cfg<MODE>::BLOCK) dst[k] = src[k];
-        for (int k = threadIdx.x; k < NBOUND * S.n_parts; k += Cfg<MODE>::BLOCK) s_bounds[k] = S.bounds[k];
-        if (LEAN) {
-            unsigned long long* s_pinfo = reinterpret_cast<unsigned long long*>(s_bounds + NBOUND * S.n_parts);
-            for (int k = threadIdx.x; k < S.n_parts; k += Cfg<MODE>::BLOCK) s_pinfo[k] = lean_part_info(S.parts[k], S.objects[S.parts[k].object]);
-        }
+        stage_tables<Cfg<MODE>::BLOCK, LEAN>(S, smem_raw);
         __syncthreads();
     }
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -318,6 +316,59 @@ __global__ void __launch_bounds__(Cfg<MODE>::BLOCK, 6) retrace_intersect_wave(co
     if (lane == 0) {
         if (sd) atomicAdd(&P.counters->sdf, (unsigned long long)sd);
         if (tr) atomicAdd(&P.counters->tri, (unsigned long long)tr);
+    }
+}
+
+// ---- interact3d without polarisation -------------------------------------------------------------------
+// Spotdetector.jl:50-61: where the ray meets the detector plane, in the detector's (x, z)
+struct SpotHit { int obj; double x, z; };
+BMO_D void spot_hit(const SysView& S, int object, int pose, V3 pos, V3 dir, double t, SpotHit& sp) {
+    const double* dp = S.det_pose + 12 * ((int64_t)pose * S.n_objects + object);
+    V3 hp = pos + t * dir;
+    V3 loc = hp - mk3(dp[0], dp[1], dp[2]);
+    sp.obj = object;
+    sp.x = dot(loc, mk3(dp[3], dp[6], dp[9]));     // orientation[:,1]
+    sp.z = dot(loc, mk3(dp[5], dp[8], dp[11]));    // orientation[:,3]
+}
+// interact3d of a plain ray, or of one ray of a Gaussian triple, with part hit_part (pt of object ob) at distance t, normal nrm:
+// the continuing ray goes to o (o.valid stays false when interact3d returns nothing), a Spotdetector hit to sp, and split is set
+// when the part is a beamsplitter coating (the children are made by the caller).  The state is passed by value so that the
+// wavefront kernels (interact_body) and the whole-solve kernel (solve_rays_persistent) run the same code on it.
+BMO_D void interact_plain(const SysView& S, const bmo_part& pt, const bmo_object& ob, int hit_part, V3 pos, V3 dir, double rn, double t,
+                          V3 nrm, int lam, int pose, RayOut& o, bool& split, SpotHit& sp) {
+    const auto n_of_hit = [&]() { return S.n_table[pt.n_row * S.n_lambda + lam]; };   // only refractive parts have a row
+    switch (ob.kind) {
+        case BMO_OBJ_REFRACTIVE:
+            interact_refractive_plain(pos, dir, rn, t, nrm, n_of_hit(), S.n_system, hit_part, o);
+            break;
+        case BMO_OBJ_DOUBLET:      // DoubletLenses.jl:66-76
+            interact_refractive_plain(pos, dir, rn, t, nrm, n_of_hit(), S.n_system, hit_part, o);
+            o.hint = ob.first_part + (1 - (hit_part - ob.first_part));
+            break;
+        case BMO_OBJ_MIRROR:
+            interact_mirror_plain(pos, dir, rn, t, nrm, o);
+            break;
+        case BMO_OBJ_CUBE_BS:      // CubeBeamsplitter.jl:63-121
+            if (pt.role == BMO_ROLE_COATING) split = true;
+            else {
+                interact_refractive_plain(pos, dir, rn, t, nrm, n_of_hit(), S.n_system, hit_part, o);
+                o.hint = ob.first_part + 2;
+            }
+            break;
+        case BMO_OBJ_PLATE_BS:     // PlateBeamsplitter.jl:189-275
+            if (pt.role == BMO_ROLE_COATING) split = true;
+            else {
+                interact_refractive_plain(pos, dir, rn, t, nrm, n_of_hit(), S.n_system, hit_part, o);
+                o.hint = ob.first_part + 1;
+            }
+            break;
+        case BMO_OBJ_THIN_BS:
+            split = true;
+            break;
+        case BMO_OBJ_SPOTDETECTOR:
+            spot_hit(S, pt.object, pose, pos, dir, t, sp);
+            break;
+        default: break;  // PolarizationFilter (PolarizedRay only: no method -> nothing), Photodetector, IntersectableObject
     }
 }
 
@@ -437,58 +488,51 @@ BMO_D void interact_body(const StepParams& P, const Hit& h_reg, const int wave_o
         RayOut ta, tb;
         ta.valid = tb.valid = false; ta.err = tb.err = false; ta.warn = tb.warn = false; ta.hint = tb.hint = -1;
         Cx Et[3];
-        if (pol) { Et[0] = E0[0]; Et[1] = E0[1]; Et[2] = E0[2]; }
-        switch (ob.kind) {
-            case BMO_OBJ_REFRACTIVE:
-                if (pol) { interact_refractive(pos, dir, rn, Et, true, t, h.n, n_of_hit(), S.n_system, hit_part, ta); o1 = ta; }
-                else interact_refractive_plain(pos, dir, rn, t, h.n, n_of_hit(), S.n_system, hit_part, o1);
-                break;
-            case BMO_OBJ_DOUBLET:      // DoubletLenses.jl:66-76 (Ray only; a PolarizedRay has no method -> nothing)
-                if (pol) break;
-                interact_refractive_plain(pos, dir, rn, t, h.n, n_of_hit(), S.n_system, hit_part, o1);
-                o1.hint = ob.first_part + (1 - (hit_part - ob.first_part));
-                break;
-            case BMO_OBJ_MIRROR:
-                if (pol) { interact_mirror(pos, dir, rn, Et, true, t, h.n, ta); o1 = ta; }
-                else interact_mirror_plain(pos, dir, rn, t, h.n, o1);
-                break;
-            case BMO_OBJ_CUBE_BS:      // CubeBeamsplitter.jl:63-121
-                if (pt.role == BMO_ROLE_COATING) split = true;
-                else {
-                    if (pol) { interact_refractive(pos, dir, rn, Et, true, t, h.n, n_of_hit(), S.n_system, hit_part, ta); o1 = ta; }
-                    else interact_refractive_plain(pos, dir, rn, t, h.n, n_of_hit(), S.n_system, hit_part, o1);
-                    o1.hint = ob.first_part + 2;
+        SpotHit sp; sp.obj = -1;
+        if (!pol) interact_plain(S, pt, ob, hit_part, pos, dir, rn, t, h.n, lam, pose, o1, split, sp);
+        else {
+            Et[0] = E0[0]; Et[1] = E0[1]; Et[2] = E0[2];
+            switch (ob.kind) {
+                case BMO_OBJ_REFRACTIVE:
+                    interact_refractive(pos, dir, rn, Et, true, t, h.n, n_of_hit(), S.n_system, hit_part, ta); o1 = ta;
+                    break;
+                case BMO_OBJ_MIRROR:
+                    interact_mirror(pos, dir, rn, Et, true, t, h.n, ta); o1 = ta;
+                    break;
+                case BMO_OBJ_CUBE_BS:      // CubeBeamsplitter.jl:63-121
+                    if (pt.role == BMO_ROLE_COATING) split = true;
+                    else {
+                        interact_refractive(pos, dir, rn, Et, true, t, h.n, n_of_hit(), S.n_system, hit_part, ta); o1 = ta;
+                        o1.hint = ob.first_part + 2;
+                    }
+                    break;
+                case BMO_OBJ_PLATE_BS:     // PlateBeamsplitter.jl:189-275
+                    if (pt.role == BMO_ROLE_COATING) split = true;
+                    else {
+                        interact_refractive(pos, dir, rn, Et, true, t, h.n, n_of_hit(), S.n_system, hit_part, ta); o1 = ta;
+                        o1.hint = ob.first_part + 1;
+                    }
+                    break;
+                case BMO_OBJ_THIN_BS:
+                    split = true;
+                    break;
+                case BMO_OBJ_POLFILTER: {   // PolarizationFilter.jl:31-47
+                    const double* dp = S.det_pose + 12 * ((int64_t)pose * S.n_objects + pt.object);
+                    interact_polfilter(pos, dir, rn, Et, t, dp + 3, S.jones + 10 * (int64_t)ob.pd_n, ta);
+                    o1 = ta;
+                    break;
                 }
-                break;
-            case BMO_OBJ_PLATE_BS:     // PlateBeamsplitter.jl:189-275
-                if (pt.role == BMO_ROLE_COATING) split = true;
-                else {
-                    if (pol) { interact_refractive(pos, dir, rn, Et, true, t, h.n, n_of_hit(), S.n_system, hit_part, ta); o1 = ta; }
-                    else interact_refractive_plain(pos, dir, rn, t, h.n, n_of_hit(), S.n_system, hit_part, o1);
-                    o1.hint = ob.first_part + 1;
-                }
-                break;
-            case BMO_OBJ_THIN_BS:
-                split = true;
-                break;
-            case BMO_OBJ_POLFILTER: {   // PolarizationFilter.jl:31-47 (PolarizedRay only; other beams: no method -> nothing)
-                if (!pol) break;
-                const double* dp = S.det_pose + 12 * ((int64_t)pose * S.n_objects + pt.object);
-                interact_polfilter(pos, dir, rn, Et, t, dp + 3, S.jones + 10 * (int64_t)ob.pd_n, ta);
-                o1 = ta;
-                break;
+                case BMO_OBJ_SPOTDETECTOR:
+                    spot_hit(S, pt.object, pose, pos, dir, t, sp);
+                    break;
+                default: break;  // Doublet (Ray only; a PolarizedRay has no method -> nothing), Photodetector, IntersectableObject
             }
-            case BMO_OBJ_SPOTDETECTOR: {  // Spotdetector.jl:50-61
-                const double* dp = S.det_pose + 12 * ((int64_t)pose * S.n_objects + pt.object);
-                V3 hp = pos + t * dir;
-                V3 loc = hp - mk3(dp[0], dp[1], dp[2]);
-                const int64_t bi = (int64_t)beam * R + r;
-                P.B.spot_obj[bi] = pt.object;
-                P.B.spot_xz[2 * bi] = dot(loc, mk3(dp[3], dp[6], dp[9]));        // orientation[:,1]
-                P.B.spot_xz[2 * bi + 1] = dot(loc, mk3(dp[5], dp[8], dp[11]));   // orientation[:,3]
-                break;
-            }
-            default: break;  // Photodetector (field added by bmo_pd_accumulate), IntersectableObject
+        }
+        if (sp.obj >= 0) {
+            const int64_t bi = (int64_t)beam * R + r;
+            P.B.spot_obj[bi] = sp.obj;
+            P.B.spot_xz[2 * bi] = sp.x;
+            P.B.spot_xz[2 * bi + 1] = sp.z;
         }
         if (!NS && split) {
             bs_children(pos, dir, Et, pol, t, h.n, pt.reflectance, pt.transmittance, ta, tb);
@@ -716,18 +760,7 @@ __global__ void __launch_bounds__(IBLOCK, MINB) fused_wave0(const StepParams P) 
     bmo_part* s_parts = reinterpret_cast<bmo_part*>(smem_raw + (size_t)S.n_prims * sizeof(bmo_prim));
     double* s_bounds = reinterpret_cast<double*>(smem_raw + (size_t)S.n_prims * sizeof(bmo_prim) + (size_t)S.n_parts * sizeof(bmo_part));
     if (STAGED) {
-        const int nw = S.n_prims * (int)(sizeof(bmo_prim) / 8), nq = S.n_parts * (int)(sizeof(bmo_part) / 8);
-        const double* src = reinterpret_cast<const double*>(S.prims);
-        double* dst = reinterpret_cast<double*>(s_prims);
-        for (int k = threadIdx.x; k < nw; k += IBLOCK) dst[k] = src[k];
-        src = reinterpret_cast<const double*>(S.parts);
-        dst = reinterpret_cast<double*>(s_parts);
-        for (int k = threadIdx.x; k < nq; k += IBLOCK) dst[k] = src[k];
-        for (int k = threadIdx.x; k < NBOUND * S.n_parts; k += IBLOCK) s_bounds[k] = S.bounds[k];
-        if (LEAN) {
-            unsigned long long* s_pinfo = reinterpret_cast<unsigned long long*>(s_bounds + NBOUND * S.n_parts);
-            for (int k = threadIdx.x; k < S.n_parts; k += IBLOCK) s_pinfo[k] = lean_part_info(S.parts[k], S.objects[S.parts[k].object]);
-        }
+        stage_tables<IBLOCK, LEAN>(S, smem_raw);
         __syncthreads();
     }
     const int64_t ri = (int64_t)blockIdx.x * IBLOCK + threadIdx.x;
@@ -777,6 +810,129 @@ __global__ void __launch_bounds__(IBLOCK, MINB) fused_wave0(const StepParams P) 
     if ((threadIdx.x & 31) == 0) {
         if (sd) atomicAdd(&P.counters->sdf, (unsigned long long)sd);
         if (tr) atomicAdd(&P.counters->tri, (unsigned long long)tr);
+    }
+}
+
+// ---- whole solve of plain rays through a splitter-free LEAN system in one launch ---------------------------
+// Without beamsplitters no ray ever makes or meets another one, so the wave structure (queue, hit records, one launch per wave,
+// compaction) has nothing to coordinate: each thread carries its ray from the caller's inputs through tracing_step! and
+// interact3d until it dies, misses, reaches a detector or has r_max rays, and writes its beam-table entry once.  As many
+// blocks as are resident at once stage the tables once; each warp takes tiles of 32 rays from a global counter, so rays
+// with more interactions than others do not leave a tail.  The march and interact_plain are the device functions the wave
+// kernels run, in the same order, so every per-ray result and counter is the wave path's bit for bit.
+struct SolveParams {
+    SysView S;
+    const double *pos, *dir;        // [n][3]; dir [3] with dir_uniform (BMO_UNIFORM_DIR)
+    const int32_t *lam, *pose;      // [n] or NULL (0 for every ray)
+    int64_t n;
+    int32_t r_max, dir_uniform;
+    BeamTab B;
+    DevCounters* counters;          // tiles and most_nseg zeroed by the caller
+};
+// Per-thread scratch columns besides the march's (s_ls): the ray's refractive index (s_pn), wavelength id and segment index
+// (s_pi rows 0 / 1) are not needed by the march and would otherwise hold registers through it.  2 KB on top of the 22 KB of
+// intersect_wave's static scratch: with the LEAN gate's 24 KB of tables (staged_smem) a block stays within the 48 KB it gets
+// without opting in (checked at launch, persistent_blocks).
+template <int MINB>
+__global__ void __launch_bounds__(IBLOCK, MINB) solve_rays_persistent(const SolveParams P) {
+    __shared__ float s_lb[LB_ROWS * LB_STRIDE];
+    __shared__ double s_ls[LS_SLOTS * LB_STRIDE];
+    __shared__ double s_pn[LB_STRIDE];
+    __shared__ int s_pi[2 * LB_STRIDE];
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const SysView& S = P.S;
+    bmo_prim* s_prims = reinterpret_cast<bmo_prim*>(smem_raw);
+    bmo_part* s_parts = reinterpret_cast<bmo_part*>(smem_raw + (size_t)S.n_prims * sizeof(bmo_prim));
+    double* s_bounds = reinterpret_cast<double*>(smem_raw + (size_t)S.n_prims * sizeof(bmo_prim) + (size_t)S.n_parts * sizeof(bmo_part));
+    stage_tables<IBLOCK, true>(S, smem_raw);
+    __syncthreads();
+    TraceCtx C;
+    C.M.meshes = S.meshes; C.M.vertices = S.vertices; C.M.faces = S.faces; C.M.nodes = S.nodes; C.M.bvh_faces = S.bvh_faces;
+    C.M.n_vertices = S.n_vertices; C.M.n_poses = S.n_poses; C.M.bvh_ok = S.bvh_ok;
+    C.objects = S.objects; C.n_parts = S.n_parts; C.zr = S.zr;
+    C.pose = 0;   // the tables are staged: one pose (a ray with another pose_id is rejected below)
+    C.prims = s_prims; C.parts = s_parts; C.bounds = s_bounds;
+    C.lb_addr = smem_u32(s_lb + threadIdx.x);
+    const unsigned sc = smem_u32(s_ls + threadIdx.x), pinfo = smem_u32(s_bounds + NBOUND * S.n_parts);
+    const unsigned a_n = smem_u32(s_pn + threadIdx.x), a_lam = smem_u32(s_pi + threadIdx.x), a_seg = a_lam + 4u * LB_STRIDE;
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31;
+    const long long n_tiles = (P.n + 31) / 32;
+    Stats st; st.sdf = 0; st.tri = 0;
+    unsigned n_int = 0, n_bad = 0, most = 0;
+#pragma unroll 1
+    for (;;) {
+        long long tile = 0;
+        if (lane == 0) tile = (long long)atomicAdd(&P.counters->tiles, 1ull);
+        tile = __shfl_sync(full, tile, 0);
+        if (tile >= n_tiles) break;
+        const int64_t ri = tile * 32 + lane;
+        if (ri < P.n) {
+            // the ray as init_queue makes it: Ray(pos, dir, lambda) has n = 1 (Rays.jl:32-42)
+            const int64_t di = P.dir_uniform ? 0 : ri;
+            V3 pos = mk3(P.pos[3 * ri], P.pos[3 * ri + 1], P.pos[3 * ri + 2]);
+            V3 dir = mk3(P.dir[3 * di], P.dir[3 * di + 1], P.dir[3 * di + 2]);
+            int lam = P.lam ? P.lam[ri] : 0, pose = P.pose ? P.pose[ri] : 0;
+            // an id outside the tables is parked (status ERROR, no segment) and counted; the call then returns BMO_EINVAL
+            const bool bad = (unsigned)lam >= (unsigned)S.n_lambda || (unsigned)pose >= (unsigned)S.n_poses;
+            if (bad) { lam = 0; pose = 0; n_bad++; }
+            int hint = -1, nseg = 0, status = BMO_ST_ERROR;
+            bool warn = false;
+            SpotHit sp; sp.obj = -1; sp.x = sp.z = __longlong_as_double(0x7ff8000000000000ll);   // NaN until a Spotdetector is hit
+            sts_f64(a_n, 1.0);
+            sts_f32(a_lam, __int_as_float(lam));
+            sts_f32(a_seg, __int_as_float(0));
+    #pragma unroll 1
+            while (!bad) {
+                // one wave: tracing_step! (intersect_wave), then the outcome and interact3d (interact_body<0, *, true>)
+                const int seg = __float_as_int(lds_f32(a_seg));
+                Hit h; h.part = -1; h.t = INFINITY; h.n = mk3(0, 0, 0);
+                const bool budget = seg + 1 < P.r_max;   // `while length(rays) < r_max` (System.jl:133)
+                if (budget) h = tracing_step_lean(C, sc, C.lb_addr, pinfo, pos, dir, hint, st);
+                int s = budget ? (h.part < 0 ? BMO_ST_MISS : BMO_ST_ACTIVE) : BMO_ST_RMAX;
+                RayOut o;
+                o.valid = false; o.err = false; o.warn = false; o.hint = -1;
+                if (s == BMO_ST_ACTIVE) {
+                    n_int++;
+                    // the ray as the march left it in its scratch column (not carried through the march in registers)
+                    pos = ls_load3(sc, LS_POS); dir = ls_load3(sc, LS_DIR);
+                    const double rn = lds_f64(a_n);
+                    const int lm = __float_as_int(lds_f32(a_lam));
+                    const bmo_part& pt = s_parts[h.part];
+                    const bmo_object& ob = S.objects[pt.object];
+                    bool split = false;   // never set: the system has no beamsplitter
+                    interact_plain(S, pt, ob, h.part, pos, dir, rn, h.t, h.n, lm, 0, o, split, sp);
+                    if (!o.valid) s = BMO_ST_ABSORBED;
+                    if (o.valid && o.err) s = BMO_ST_ERROR;
+                    warn |= o.valid && o.warn;
+                }
+                if (s != BMO_ST_ACTIVE) { nseg = seg + 1; status = s; break; }
+                pos = o.pos; dir = o.dir; hint = o.hint;
+                sts_f64(a_n, o.n);
+                sts_f32(a_seg, __int_as_float(seg + 1));
+            }
+            // the beam-table entry init_queue and the waves would have left (bit 8 of status: see interact_body)
+            P.B.parent[ri] = -1; P.B.slot[ri] = -1; P.B.nseg[ri] = nseg; P.B.status[ri] = status | (warn ? 0x100 : 0);
+            P.B.lam[ri] = lam; P.B.pose[ri] = pose;
+            P.B.spot_obj[ri] = sp.obj; P.B.spot_xz[2 * ri] = sp.x; P.B.spot_xz[2 * ri + 1] = sp.z;
+            most = max(most, (unsigned)nseg);
+        }
+    }
+    unsigned sd = st.sdf, tr = st.tri;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        sd += __shfl_xor_sync(full, sd, o);
+        tr += __shfl_xor_sync(full, tr, o);
+        n_int += __shfl_xor_sync(full, n_int, o);
+        n_bad += __shfl_xor_sync(full, n_bad, o);
+        most = max(most, __shfl_xor_sync(full, most, o));
+    }
+    if (lane == 0) {
+        if (sd) atomicAdd(&P.counters->sdf, (unsigned long long)sd);
+        if (tr) atomicAdd(&P.counters->tri, (unsigned long long)tr);
+        if (n_int) atomicAdd(&P.counters->interactions, (unsigned long long)n_int);
+        if (n_bad) atomicAdd(&P.counters->bad_ids, (unsigned long long)n_bad);
+        if (most) atomicMax(&P.counters->most_nseg, (unsigned long long)most);
     }
 }
 
@@ -1678,6 +1834,17 @@ int32_t SubTrace::begin(const TraceInputs& in_h) {
     return BMO_OK;
 }
 
+// Dynamic shared memory of the trace kernels (0 unless the tables are staged); lean: the LEAN builds apply (bmo_lean.cuh).
+static size_t staged_smem(const bmo_sys* sys, bool staged, bool& lean) {
+    const SysView& V = sys->view;
+    static const bool lean_ok = !(getenv("BMO_LEAN") && atoi(getenv("BMO_LEAN")) == 0);   // tuning knob: BMO_LEAN=0 uses the general kernels everywhere
+    const size_t tab_bytes = (size_t)V.n_prims * sizeof(bmo_prim) + (size_t)V.n_parts * (sizeof(bmo_part) + NBOUND * sizeof(double));
+    // kernels compiled for lean unions + small meshes only; their tables live in shared memory next to 22 KB of per-thread
+    // scratch (static), so the tables + part words have to fit in what is left of the 48 KB a block gets without opting in
+    lean = lean_ok && sys->all_lean && !sys->has_rare && staged && tab_bytes + (size_t)V.n_parts * 8 <= 24 * 1024;
+    return staged ? tab_bytes + (lean ? (size_t)V.n_parts * 8 : 0) : 0;
+}
+
 // enqueue the next waves on this sub-batch's stream and the read-back of their totals
 int32_t SubTrace::enqueue_chunk() {
     int32_t rc;
@@ -1730,14 +1897,9 @@ int32_t SubTrace::enqueue_chunk() {
         // wave), so it only pays where the number of launches is what limits the call.
         static const int fuse_policy = getenv("BMO_FUSE") ? atoi(getenv("BMO_FUSE")) : 1;
         const bool allow_fused = !rt.on && (fuse_policy == 2 || (fuse_policy == 1 && pipelined));
-        const SysView& V = sys->view;
         const bool rk = sys->has_rare;     // kernels compiled with the cylindrical / aspheric primitives
-        static const bool lean_ok = !(getenv("BMO_LEAN") && atoi(getenv("BMO_LEAN")) == 0);   // tuning knob: BMO_LEAN=0 uses the general kernels everywhere
-        const size_t tab_bytes = (size_t)V.n_prims * sizeof(bmo_prim) + (size_t)V.n_parts * (sizeof(bmo_part) + NBOUND * sizeof(double));
-        // kernels compiled for lean unions + small meshes only; their tables live in shared memory next to 22 KB of per-thread
-        // scratch (static), so the tables + part words have to fit in what is left of the 48 KB a block gets without opting in
-        const bool lean = lean_ok && sys->all_lean && !rk && staged && tab_bytes + (size_t)V.n_parts * 8 <= 24 * 1024;
-        const size_t smem = staged ? tab_bytes + (lean ? (size_t)V.n_parts * 8 : 0) : 0;
+        bool lean;
+        const size_t smem = staged_smem(sys, staged, lean);
         BMO_CUDA(cudaEventRecord(ev[2 * c], st));
         if (mode == 0 && !has_splitter && allow_fused) {
             // sequential lens-stack path: intersect + interact in one kernel, hit records stay in registers; without a
@@ -1929,6 +2091,60 @@ void SubTrace::release() {
     ev.clear();
 }
 
+// The variant of solve_rays_persistent this process runs (tuning knob BMO_PMINB: resident blocks per SM it is compiled for, 4 - 8)
+static const void* persistent_kernel() {
+    static const int pminb = std::min(8, std::max(4, getenv("BMO_PMINB") ? atoi(getenv("BMO_PMINB")) : 6));
+    const void* fns[] = {(const void*)solve_rays_persistent<4>, (const void*)solve_rays_persistent<5>, (const void*)solve_rays_persistent<6>,
+                         (const void*)solve_rays_persistent<7>, (const void*)solve_rays_persistent<8>};
+    return fns[pminb - 4];
+}
+// Resident blocks per SM of persistent_kernel() with smem bytes of tables, 0 if a block would not fit the 48 KB of shared memory
+// it gets without opting in (static scratch + tables): such a call keeps the waves.  Cached per context.
+static int32_t persistent_blocks(bmo_ctx* ctx, size_t smem, int* blocks) {
+    const void* fn = persistent_kernel();
+    if (ctx->persist_fn != fn || ctx->persist_smem != smem) {
+        cudaFuncAttributes fa;
+        BMO_CUDA(cudaFuncGetAttributes(&fa, fn));
+        int b = 0;
+        if (fa.sharedSizeBytes + smem <= (size_t)48 * 1024) BMO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, fn, IBLOCK, smem));
+        ctx->persist_fn = fn; ctx->persist_smem = smem; ctx->persist_blocks = b;
+    }
+    *blocks = ctx->persist_blocks;
+    return BMO_OK;
+}
+
+// The whole solve of a `persistent` call (trace_common) on the caller's stream: the result tables are written by the kernel, the
+// counters (with the largest nseg, from which the caller derives the wave count) come back with one copy into h_totals.
+// blocks: resident blocks per SM (persistent_blocks).
+static int32_t solve_persistent(bmo_sys* sys, const TraceInputs& in_h, int32_t r_max, bool on_dev, size_t smem, int blocks, bmo_result* res,
+                                int32_t* spot_obj_out, double* spot_xz_out) {
+    bmo_ctx* ctx = sys->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = in_h.n;
+    int32_t rc;
+    std::vector<void*> tmp;
+    SolveParams sp{};
+    sp.S = sys->view; sp.n = n; sp.r_max = r_max; sp.dir_uniform = in_h.dir_uniform; sp.B = beamtab(res); sp.counters = ctx->d_counters;
+    if ((rc = stage_in(in_h.pos, (size_t)n * 3, on_dev, st, &sp.pos, tmp))) return rc;
+    if ((rc = stage_in(in_h.dir, in_h.dir_uniform ? 3 : (size_t)n * 3, on_dev, st, &sp.dir, tmp))) return rc;
+    if ((rc = stage_in(in_h.lam, (size_t)n, on_dev, st, &sp.lam, tmp))) return rc;
+    if ((rc = stage_in(in_h.pose, (size_t)n, on_dev, st, &sp.pose, tmp))) return rc;
+    BMO_CUDA(cudaMemsetAsync(&ctx->d_counters->tiles, 0, 2 * sizeof(unsigned long long), st));   // tiles, most_nseg
+    const int64_t grid = std::min<int64_t>((int64_t)blocks * ctx->sm_count, (n + IBLOCK - 1) / IBLOCK);
+    BMO_CUDA(cudaEventRecord(ctx->evk0, st));
+    void* args[] = {&sp};
+    BMO_CUDA(cudaLaunchKernel(persistent_kernel(), dim3((unsigned)grid), dim3(IBLOCK), args, smem, st));
+    BMO_LAUNCH(ctx, "solve_rays_persistent");
+    BMO_CUDA(cudaEventRecord(ctx->evk1, st));
+    BMO_CUDA(cudaMemcpyAsync(ctx->h_totals + 72, ctx->d_counters, sizeof(DevCounters), cudaMemcpyDeviceToHost, st));
+    if (spot_xz_out) {
+        if (spot_obj_out) BMO_CUDA(cudaMemcpyAsync(spot_obj_out, res->spot_obj, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        BMO_CUDA(cudaMemcpyAsync(spot_xz_out, res->spot_xz, (size_t)2 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    }
+    for (void* p : tmp) dev_free(p, st);
+    return BMO_OK;
+}
+
 static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int32_t r_max, uint32_t flags, bmo_result** out,
                             int32_t* spot_obj_out = nullptr, double* spot_xz_out = nullptr, const RetraceView* prev_rt = nullptr) {
     NvtxRange nvtx_("bmo_trace");
@@ -1963,83 +2179,103 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
     static const int max_sub = getenv("BMO_SUBBATCHES") ? std::min(8, std::max(1, atoi(getenv("BMO_SUBBATCHES")))) : 4;
     int n_sub = 1;
     if (!on_dev && !has_splitter && !res->keep) n_sub = (int)std::min<int64_t>(max_sub, std::max<int64_t>(1, n / (128 * 1024)));
-    while ((int)ctx->aux_streams.size() < n_sub - 1) {
-        cudaStream_t s2;
-        BMO_CUDA(cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
-        ctx->aux_streams.push_back(s2);
+    // Plain rays through a splitter-free LEAN system whose segments are not kept, in one stream: one launch solves them all
+    // (solve_rays_persistent); BMO_PERSIST=0 runs them through the waves instead (A/B timing).
+    static const bool persist_ok = !(getenv("BMO_PERSIST") && atoi(getenv("BMO_PERSIST")) == 0);
+    bool lean;
+    const size_t smem = staged_smem(sys, staged, lean);
+    int pblocks = 0;
+    if (persist_ok && mode == 0 && !has_splitter && !prev_rt && !res->keep && lean && n_sub == 1 && (rc = persistent_blocks(ctx, smem, &pblocks))) {
+        bmo_result_free(res);
+        return rc;
     }
-    cudaEvent_t ev_fork = nullptr;
-    if (n_sub > 1) {   // the auxiliary streams start after everything already queued on the caller's stream (result tables included)
-        BMO_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
-        BMO_CUDA(cudaEventRecord(ev_fork, st));
-    }
-    std::vector<SubTrace> subs((size_t)n_sub);
-    for (int k = 0; k < n_sub; k++) {
-        SubTrace& s = subs[k];
-        s.sys = sys; s.ctx = ctx; s.res = res; s.st = k == 0 ? st : ctx->aux_streams[k - 1]; s.slot = k;
-        s.mode = mode; s.R = R; s.nfq = nf_queue(mode); s.nfs = nf_scratch(mode); s.nsd = res->nsd;
-        s.units = mode == 2 ? Cfg<2>::UNITS : Cfg<0>::UNITS;
-        s.r_max = r_max; s.has_splitter = has_splitter; s.staged = staged; s.on_dev = on_dev; s.pipelined = n_sub > 1;
-        s.beam0 = n * k / n_sub; s.n = n * (k + 1) / n_sub - s.beam0;
-        s.spot_obj_out = spot_obj_out; s.spot_xz_out = spot_xz_out;
-        if (prev_rt) s.rt = *prev_rt;
-        if (k > 0) BMO_CUDA(cudaStreamWaitEvent(s.st, ev_fork, 0));
-        if (!has_splitter && n_sub == 1 && !prev_rt) {
-            auto it = sys->hints.find({mode, n});
-            if (it != sys->hints.end()) s.first_chunk = it->second.first_chunk;
-        }
-        if ((rc = s.begin(in_h))) return rc;
-        s.n_beams = n;
-        if (has_splitter) {     // sizes the previous call of this shape ended with (see bmo_sys::hints)
-            auto it = sys->hints.find({mode, n});
-            if (it != sys->hints.end()) {
-                const bmo_sys::TraceHint& hh = it->second;
-                if (hh.slots * R > s.cur.cap && (rc = grow_queue(s.cur, hh.slots * R, s.nfq, NI_Q, s.st))) return rc;
-                if (hh.scr > s.scr.cap) { free_queue(s.scr, s.st); if ((rc = alloc_queue(s.scr, hh.scr, s.nfs, NI_S, s.st))) return rc; }
-                if ((rc = ensure_beams(res, hh.beams, s.st))) return rc;
-            }
-        }
-        if ((rc = s.enqueue_chunk())) return rc;     // the first sub-batch is already copying / tracing while the others are set up
-    }
-    const double tp1 = tnow_ms();
-    // Every sub-batch always has its next chunk of waves in flight: as soon as the host has looked at
-    // the totals of one chunk it enqueues the next one on that stream, before it waits for the
-    // following sub-batch (they finish roughly in order: their input copies are serialised on the link).
-    for (bool any = true; any;) {
-        any = false;
-        for (auto& s : subs) {
-            if (s.launched == 0) continue;
-            if ((rc = s.finish_chunk())) return rc;
-            s.launched = 0;
-            if (prof) fprintf(stderr, "[bmo]   sub-batch %d: chunk done at %.3f ms (waited %.3f), alive %lld\n", s.slot, tnow_ms() - tp0, s.host_wait_ms, (long long)s.alive);
-            if (s.alive > 0) {
-                if (s.wave > s.max_waves()) return fail(BMO_ESTATE, "trace: wave loop did not terminate (more than 64 generations of r_max rays)");
-                if ((rc = s.enqueue_chunk())) return rc;
-                any = true;
-            }
-        }
-    }
-    const double tp2 = tnow_ms();
+    const bool persistent = pblocks > 0;
     int wave = 0;
-    double tp_wave_sync = 0;
-    for (auto& s : subs) { wave = std::max(wave, s.waves_done); tp_wave_sync += s.host_wait_ms; }
-    ctx->waves += wave;
-    res->n_beams = has_splitter ? subs[0].n_beams : n;
-    res->waves = wave;
-    if (!has_splitter && n_sub == 1 && !prev_rt && subs[0].alive_after_w0 >= 0)   // would the look after wave 0 have compacted?
-        sys->hints[{mode, n}].first_chunk = (2 * subs[0].alive_after_w0 > n || n < 4096) ? 4 : 1;
-    if (has_splitter) {
-        bmo_sys::TraceHint& hh = sys->hints[{mode, n}];
-        hh.slots = std::max(hh.slots, subs[0].cur.cap / R); hh.scr = std::max(hh.scr, subs[0].scr.cap); hh.beams = std::max(hh.beams, res->cap_beams);
+    double tp1 = tp0, tp2 = tp0, tp_wave_sync = 0;   // host timeline (BMO_HOST_PROFILE)
+    if (persistent) {
+        if ((rc = solve_persistent(sys, in_h, r_max, on_dev, smem, pblocks, res, spot_obj_out, spot_xz_out))) {
+            bmo_result_free(res);
+            return rc;
+        }
+        res->n_beams = n;
+        tp1 = tp2 = tnow_ms();
+    } else {
+        while ((int)ctx->aux_streams.size() < n_sub - 1) {
+            cudaStream_t s2;
+            BMO_CUDA(cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
+            ctx->aux_streams.push_back(s2);
+        }
+        cudaEvent_t ev_fork = nullptr;
+        if (n_sub > 1) {   // the auxiliary streams start after everything already queued on the caller's stream (result tables included)
+            BMO_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
+            BMO_CUDA(cudaEventRecord(ev_fork, st));
+        }
+        std::vector<SubTrace> subs((size_t)n_sub);
+        for (int k = 0; k < n_sub; k++) {
+            SubTrace& s = subs[k];
+            s.sys = sys; s.ctx = ctx; s.res = res; s.st = k == 0 ? st : ctx->aux_streams[k - 1]; s.slot = k;
+            s.mode = mode; s.R = R; s.nfq = nf_queue(mode); s.nfs = nf_scratch(mode); s.nsd = res->nsd;
+            s.units = mode == 2 ? Cfg<2>::UNITS : Cfg<0>::UNITS;
+            s.r_max = r_max; s.has_splitter = has_splitter; s.staged = staged; s.on_dev = on_dev; s.pipelined = n_sub > 1;
+            s.beam0 = n * k / n_sub; s.n = n * (k + 1) / n_sub - s.beam0;
+            s.spot_obj_out = spot_obj_out; s.spot_xz_out = spot_xz_out;
+            if (prev_rt) s.rt = *prev_rt;
+            if (k > 0) BMO_CUDA(cudaStreamWaitEvent(s.st, ev_fork, 0));
+            if (!has_splitter && n_sub == 1 && !prev_rt) {
+                auto it = sys->hints.find({mode, n});
+                if (it != sys->hints.end()) s.first_chunk = it->second.first_chunk;
+            }
+            if ((rc = s.begin(in_h))) return rc;
+            s.n_beams = n;
+            if (has_splitter) {     // sizes the previous call of this shape ended with (see bmo_sys::hints)
+                auto it = sys->hints.find({mode, n});
+                if (it != sys->hints.end()) {
+                    const bmo_sys::TraceHint& hh = it->second;
+                    if (hh.slots * R > s.cur.cap && (rc = grow_queue(s.cur, hh.slots * R, s.nfq, NI_Q, s.st))) return rc;
+                    if (hh.scr > s.scr.cap) { free_queue(s.scr, s.st); if ((rc = alloc_queue(s.scr, hh.scr, s.nfs, NI_S, s.st))) return rc; }
+                    if ((rc = ensure_beams(res, hh.beams, s.st))) return rc;
+                }
+            }
+            if ((rc = s.enqueue_chunk())) return rc;     // the first sub-batch is already copying / tracing while the others are set up
+        }
+        tp1 = tnow_ms();
+        // Every sub-batch always has its next chunk of waves in flight: as soon as the host has looked at
+        // the totals of one chunk it enqueues the next one on that stream, before it waits for the
+        // following sub-batch (they finish roughly in order: their input copies are serialised on the link).
+        for (bool any = true; any;) {
+            any = false;
+            for (auto& s : subs) {
+                if (s.launched == 0) continue;
+                if ((rc = s.finish_chunk())) return rc;
+                s.launched = 0;
+                if (prof) fprintf(stderr, "[bmo]   sub-batch %d: chunk done at %.3f ms (waited %.3f), alive %lld\n", s.slot, tnow_ms() - tp0, s.host_wait_ms, (long long)s.alive);
+                if (s.alive > 0) {
+                    if (s.wave > s.max_waves()) return fail(BMO_ESTATE, "trace: wave loop did not terminate (more than 64 generations of r_max rays)");
+                    if ((rc = s.enqueue_chunk())) return rc;
+                    any = true;
+                }
+            }
+        }
+        tp2 = tnow_ms();
+        for (auto& s : subs) { wave = std::max(wave, s.waves_done); tp_wave_sync += s.host_wait_ms; }
+        ctx->waves += wave;
+        res->n_beams = has_splitter ? subs[0].n_beams : n;
+        res->waves = wave;
+        if (!has_splitter && n_sub == 1 && !prev_rt && subs[0].alive_after_w0 >= 0)   // would the look after wave 0 have compacted?
+            sys->hints[{mode, n}].first_chunk = (2 * subs[0].alive_after_w0 > n || n < 4096) ? 4 : 1;
+        if (has_splitter) {
+            bmo_sys::TraceHint& hh = sys->hints[{mode, n}];
+            hh.slots = std::max(hh.slots, subs[0].cur.cap / R); hh.scr = std::max(hh.scr, subs[0].scr.cap); hh.beams = std::max(hh.beams, res->cap_beams);
+        }
+        // join: the caller's stream continues after every sub-batch (copies of the Spotdetector hits included)
+        for (int k = 1; k < n_sub; k++) {
+            BMO_CUDA(cudaEventRecord(ev_fork, subs[k].st));
+            BMO_CUDA(cudaStreamWaitEvent(st, ev_fork, 0));
+            BMO_CUDA(cudaStreamSynchronize(subs[k].st));
+        }
+        for (auto& s : subs) s.release();
+        if (ev_fork) cudaEventDestroy(ev_fork);
     }
-    // join: the caller's stream continues after every sub-batch (copies of the Spotdetector hits included)
-    for (int k = 1; k < n_sub; k++) {
-        BMO_CUDA(cudaEventRecord(ev_fork, subs[k].st));
-        BMO_CUDA(cudaStreamWaitEvent(st, ev_fork, 0));
-        BMO_CUDA(cudaStreamSynchronize(subs[k].st));
-    }
-    for (auto& s : subs) s.release();
-    if (ev_fork) cudaEventDestroy(ev_fork);
     const int nsd = res->nsd;
     // segment table: first_seg = exclusive scan of nseg, then gather wave-major -> beam-major
     // (spot-only traces compute first_seg lazily, see ensure_first_seg)
@@ -2067,8 +2303,17 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
     ctx->trace_ms = ms;
     {
         DevCounters h;
-        if (n_sub == 1) memcpy(&h, ctx->h_totals + 72, sizeof(h));   // copied behind the last chunk of waves (enqueue_chunk), stream synchronised since
+        if (n_sub == 1) memcpy(&h, ctx->h_totals + 72, sizeof(h));   // copied behind the last chunk of waves or the solve, stream synchronised since
         else BMO_CUDA(cudaMemcpy(&h, ctx->d_counters, sizeof(h), cudaMemcpyDeviceToHost));
+        if (persistent) {
+            // the waves the wave loop would have counted: one per segment of the longest beam, at least one
+            wave = (int)std::max<unsigned long long>(1, h.most_nseg);
+            ctx->waves += wave;
+            res->waves = wave;
+            float kms = 0;
+            BMO_CUDA(cudaEventElapsedTime(&kms, ctx->evk0, ctx->evk1));
+            ctx->k1_ms += kms; ctx->k1_launches++;
+        }
         res->interactions = (int64_t)h.interactions - ctx->interactions_seen;  // the counter is cumulative since the last reset
         ctx->interactions_seen = (int64_t)h.interactions;
         const int64_t bad = (int64_t)h.bad_ids - ctx->bad_ids_seen;
