@@ -7,7 +7,7 @@ is spelled `f_` here.  There is no CPU fallback.
 """
 from . import linalg
 from ._lib import BmoError, counters, counters_reset, measure_fp64_peak
-from .beams import (Beam, BeamletBundle, CollimatedSource, GaussianBeamlet, Intersection, PointSource, PolarizedRay, Ray,
+from .beams import (Beam, BeamletBundle, CollimatedSource, DeviceSource, GaussianBeamlet, Intersection, PointSource, PolarizedRay, Ray,
                     RayBundle, UniformDiscSource)
 from .components import (AcylindricalSurface, CircularFlatSurface, ConcaveSphericalMirror, CubeBeamsplitter, EvenAsphericalSurface, LensFromSurfaces, SphericalSurface, CylindricalLens, CylindricalSurface, RectangularFlatSurface, DiscreteRefractiveIndex, DoubletLens, IntersectableObject, Lens,
                          MeshDummy, Mirror, NonInteractableObject, ObjectGroup, PSFDetector, Photodetector, PolarizationFilter, Prism, RectangularCompensatorPlate,
@@ -18,7 +18,7 @@ from .components import (AcylindricalSurface, CircularFlatSurface, ConcaveSpheri
 from .shapes import (AcylindricalSurfaceSDF, AsphericalSurfaceSDF, BoxSDF, CircularFlatMesh, ConcaveAsphericalSurfaceSDF, ConvexAsphericalSurfaceSDF, ConcaveCylinderSDF, ConcaveSphericalSurfaceSDF, ConvexCylinderSDF, ConvexSphericalSurfaceSDF, CubeMesh, CuboidMesh, CutSphereSDF,
                      CylinderSDF, Mesh, MeniscusLensSDF, PlanoSurfaceSDF, QuadraticFlatMesh, RectangularFlatMesh, RetroMesh,
                      RightAnglePrismSDF, RingSDF, SphereSDF, ThinLensSDF, UnionSDF, load_stl)
-from .solver import DeviceSystem, TraceResult, pd_accumulate, retrace, solve_system_, trace_beamlets, trace_rays, trace_rays_spots, upload_system
+from .solver import DeviceSystem, TraceResult, pd_accumulate, retrace, solve_system_, spot_stats, trace_beamlets, trace_rays, trace_rays_spots, upload_system
 from .sweep import flatten_poses, solve_pose_sweep, KinProgram, get_pose_tables, solve_pose_sweep_device
 from . import parallel
 from .parallel import solve_system_sharded

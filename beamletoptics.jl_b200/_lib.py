@@ -17,6 +17,7 @@ PD_REFERENCE_ORDER = 4
 UNIFORM_DIR = 8
 COMM_SYNC = 16
 COMM_ID_BYTES = 128
+SRC_DISC, SRC_COLLIMATED, SRC_POINT = 0, 1, 2     # bmo_source_kind
 
 STATUS_NAMES = ["ACTIVE", "MISS", "ABSORBED", "RMAX", "SPLIT", "CLIPPED", "TORN", "ERROR"]
 
@@ -82,6 +83,21 @@ class bmo_result_info(C.Structure):
                 ("rays_per_beam", C.c_int32), ("polarized", C.c_int32), ("waves", C.c_int32), ("reserved", C.c_int32)]
 
 
+class bmo_source_ring(C.Structure):
+    _fields_ = [("first", C.c_int64), ("count", C.c_int64), ("start", C.c_double * 3), ("rot", C.c_double * 9)]
+
+
+class bmo_source_desc(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("reserved", C.c_int32), ("n_rays", C.c_int64), ("n_rings", C.c_int64),
+                ("rings", C.POINTER(bmo_source_ring)), ("pos", C.c_double * 3), ("dir", C.c_double * 3), ("e1", C.c_double * 3),
+                ("e2", C.c_double * 3), ("radius", C.c_double), ("phi0", C.c_double)]
+
+
+class bmo_spot_info(C.Structure):
+    _fields_ = [("hits", C.c_int64), ("outside", C.c_int64), ("centroid", C.c_double * 2), ("rms", C.c_double), ("max_r", C.c_double),
+                ("lo", C.c_double * 2), ("hi", C.c_double * 2)]
+
+
 # every symbol include/bmo.h declares (checked by tests/test_abi.py)
 EXPORTS = [
     "bmo_init", "bmo_shutdown", "bmo_last_error", "bmo_set_stream", "bmo_counters_get", "bmo_counters_reset",
@@ -91,6 +107,7 @@ EXPORTS = [
     "bmo_result_free", "bmo_pd_accumulate", "bmo_pd_accumulate_poses", "bmo_pd_power", "bmo_pd_sweep", "bmo_measure_fp64_peak",
     "bmo_system_set_kinematics", "bmo_system_apply_poses", "bmo_system_get_pose",
     "bmo_debug_normals", "bmo_trim",
+    "bmo_source_create", "bmo_source_device", "bmo_source_rays", "bmo_source_free", "bmo_spot_stats",
     "bmo_comm_unique_id", "bmo_comm_init", "bmo_comm_init_local", "bmo_comm_info", "bmo_pd_allreduce", "bmo_pd_allreduce_local", "bmo_comm_free",
 ]
 
@@ -139,6 +156,11 @@ def lib():
         L.bmo_system_set_kinematics.argtypes = [_vp, C.c_int32, _vp, _vp]
         L.bmo_system_apply_poses.argtypes = [_vp, C.c_int32, C.c_int32, _vp, C.c_int32, _vp]
         L.bmo_system_get_pose.argtypes = [_vp, C.c_int32, _vp, _vp, _vp, _vp]
+        L.bmo_source_create.argtypes = [_vp, C.POINTER(bmo_source_desc), C.POINTER(_vp)]
+        L.bmo_source_device.argtypes = [_vp, C.POINTER(C.c_int64), C.POINTER(_vp), C.POINTER(_vp), _ip]
+        L.bmo_source_rays.argtypes = [_vp, _vp, _vp]
+        L.bmo_source_free.argtypes = [_vp]
+        L.bmo_spot_stats.argtypes = [_vp, C.c_int32, _vp, C.c_int32, C.c_int32, C.POINTER(bmo_spot_info), _vp, C.c_uint32]
         L.bmo_comm_unique_id.argtypes = [_vp]
         L.bmo_comm_init.argtypes = [_vp, C.c_int32, C.c_int32, _vp, C.POINTER(_vp)]
         L.bmo_comm_init_local.argtypes = [C.c_int32, C.POINTER(_vp), C.POINTER(_vp)]

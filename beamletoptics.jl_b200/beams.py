@@ -5,6 +5,7 @@ Single beams mirror the reference's objects (`Ray`, `Beam`, `GaussianBeamlet`); 
 `CollimatedSource` of a million rays is one bundle, not a million Python objects.
 Citations: /root/reference/src.
 """
+import ctypes as C
 import math
 
 import numpy as np
@@ -219,12 +220,137 @@ def _basis(dir, b1):
     return d, la.v3(b1)
 
 
-def UniformDiscSource(pos, dir, diameter, lam=1e-6, num_rays=1000, e1=None):
-    """BeamGroups.jl:222-245 (Fibonacci disc); `e1` fixes the reference's random in-plane basis."""
+def _bundle_dir(d):
+    """The direction RayBundle stores for the unit vector `d` (it normalises once more)."""
+    return tuple(float(x) for x in RayBundle(np.zeros(3), np.array(d)).dir[0])
+
+
+def source_rings(kind, d, b1, size, num_rings, num_rays):
+    """Ring layout of CollimatedSource (kind "collimated", size = diameter) and PointSource ("point", size = theta):
+    [(first, count, start, rot)] for rings 1 .. num_rings - 1.  Ray 0 is the centre / axis; ring rays
+    [first, first + count) are start, rot * start, rot * (rot * start), ... with rot = rotate3d(d, 2 pi / count); start is
+    the ring's first offset r * b1 (collimated) or first direction (point).  A ring of count 0 is skipped (rot = identity).
+    The host constructors expand this table and the device descriptor (DeviceSource) carries it, so both use one layout."""
+    m = num_rays - 1
+    if kind == "collimated":
+        radii = [(size / 2) * i / (num_rings - 1) for i in range(1, num_rings)]
+        starts = [la.scale(r, b1) for r in radii]
+        circm = [r * 2 * math.pi for r in radii]
+    else:
+        b2 = la.normalize(la.cross(d, b1))
+        step = size / (num_rings - 1)
+        starts = [la.matvec(la.rotate3d(b2, step * i), d) for i in range(1, num_rings)]
+        circm = [la.norm(la.sub(nd, la.scale(la.dot(nd, d), d))) * 2 * math.pi for nd in starts]
+    ds = sum(circm) / m
+    counts = [int(round(c / ds)) for c in circm]
+    counts[-1] += m - sum(counts)
+    rings, first = [], 1
+    for start, count in zip(starts, counts):
+        rings.append((first, count, start, la.rotate3d(d, 2 * math.pi / count) if count else la.IDENTITY))
+        first += count
+    return rings
+
+
+def _expand_rings(rings, emit):
+    """Host expansion of a ring table: emit(v) for every ring ray in ray order (serial recurrence v <- rot v)."""
+    for _, count, v, rot in rings:
+        for _ in range(count):
+            emit(v)
+            v = la.matvec(rot, v)
+
+
+class DeviceSource:
+    """A source whose rays are generated on the GPU (bmo_source_create) from a descriptor: the basis, the ring table and
+    every transcendental are computed here by the code that builds the host bundles.  One bmo_source is created per
+    device on first use; `pos` / `dir` download the rays (device 0) for inspection.  solve_system_ traces it from the
+    device pointers, so no per-ray data crosses the bus.  The handles belong to the per-process contexts of _lib.context,
+    which live until the process ends, so freeing them from __del__ never outlives the context."""
+
+    def __init__(self, kind, n, pos, dir, lam, rings=(), e1=(0.0, 0.0, 0.0), e2=(0.0, 0.0, 0.0), radius=0.0, phi0=0.0):
+        from . import _lib as L
+        self.kind, self.n, self.lam = kind, int(n), float(lam)
+        self.uniform_dir = kind != L.SRC_POINT
+        self.E0 = None
+        self._rings = (L.bmo_source_ring * max(1, len(rings)))()
+        for i, (first, count, start, rot) in enumerate(rings):
+            self._rings[i].first, self._rings[i].count = int(first), int(count)
+            self._rings[i].start[:] = [float(x) for x in start]
+            self._rings[i].rot[:] = [float(rot[r][c]) for r in range(3) for c in range(3)]
+        desc = L.bmo_source_desc()
+        desc.kind, desc.n_rays, desc.n_rings = kind, self.n, len(rings)
+        desc.pos[:], desc.dir[:], desc.e1[:], desc.e2[:] = la.v3(pos), la.v3(dir), la.v3(e1), la.v3(e2)
+        desc.radius, desc.phi0 = float(radius), float(phi0)
+        # what the rays depend on, without the pointer: the root signature of a retrace
+        self._sig = bytes(desc) + bytes(memoryview(self._rings))[:len(rings) * C.sizeof(L.bmo_source_ring)] + np.float64(self.lam).tobytes()
+        desc.rings = self._rings
+        self.desc = desc
+        self._handles = {}
+        self._host = None
+        self.result = None
+
+    def __len__(self): return self.n
+
+    def signature(self): return self._sig
+
+    def handle(self, device=0):
+        """The bmo_source of this descriptor on `device` (created on first use)."""
+        from . import _lib as L
+        if device not in self._handles:
+            h = C.c_void_p()
+            L.check(L.lib().bmo_source_create(L.context(device), C.byref(self.desc), C.byref(h)))
+            self._handles[device] = h
+        return self._handles[device]
+
+    def device_arrays(self, device=0):
+        """(n, pos, dir, uniform_dir): device pointers for bmo_trace_rays with BMO_INPUT_DEVICE."""
+        from . import _lib as L
+        n, p, d, u = C.c_int64(), C.c_void_p(), C.c_void_p(), C.c_int32()
+        L.check(L.lib().bmo_source_device(self.handle(device), C.byref(n), C.byref(p), C.byref(d), C.byref(u)))
+        return int(n.value), p.value, d.value, bool(u.value)
+
+    def rays(self, device=0):
+        """Host copies (pos (n, 3), dir (n, 3)) of the rays generated on `device` (bmo_source_rays)."""
+        from . import _lib as L
+        pos, dir = np.zeros((self.n, 3)), np.zeros((self.n, 3))
+        L.check(L.lib().bmo_source_rays(self.handle(device), L.ptr(pos), L.ptr(dir)))
+        return pos, dir
+
+    def _download(self):
+        if self._host is None:
+            self._host = self.rays(next(iter(self._handles), 0))
+        return self._host
+
+    @property
+    def pos(self): return self._download()[0]
+
+    @property
+    def dir(self): return self._download()[1]
+
+    def free(self):
+        from . import _lib as L
+        for h in self._handles.values():
+            L.lib().bmo_source_free(h)
+        self._handles = {}
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
+def UniformDiscSource(pos, dir, diameter, lam=1e-6, num_rays=1000, e1=None, on_device=False):
+    """BeamGroups.jl:222-245 (Fibonacci disc); `e1` fixes the reference's random in-plane basis.  on_device=True returns a
+    DeviceSource whose positions are computed on the GPU (within a few ulp of these: CUDA's sin / cos)."""
     d, e1 = _basis(dir, e1)
     e2 = la.normalize(la.cross(d, e1))
     R = diameter / 2
     phi0 = 2 * math.pi / (1 + math.sqrt(5))
+    if on_device:
+        from . import _lib as L
+        b = DeviceSource(L.SRC_DISC, num_rays, pos, _bundle_dir(d), lam, e1=e1, e2=e2, radius=R, phi0=phi0)
+        b.diameter = float(diameter)
+        return b
     k = np.arange(num_rays, dtype=np.float64)
     rho = np.sqrt((k + 0.5) / num_rays)
     phi = k * phi0
@@ -236,36 +362,28 @@ def UniformDiscSource(pos, dir, diameter, lam=1e-6, num_rays=1000, e1=None):
     return b
 
 
-def CollimatedSource(pos, dir, diameter, lam=1e-6, num_rings=10, num_rays=None, b1=None):
-    """BeamGroups.jl:152-195 (concentric rings)."""
+def CollimatedSource(pos, dir, diameter, lam=1e-6, num_rings=10, num_rays=None, b1=None, on_device=False):
+    """BeamGroups.jl:152-195 (concentric rings).  on_device=True returns a DeviceSource with bit-identical rays."""
     if num_rays is None:
         num_rays = 100 * num_rings
     if num_rays < num_rings * 20:
         raise ValueError("No. of rays should be atleast 20x no. of rings")
     d, b1 = _basis(dir, b1)
     p0 = la.v3(pos)
-    pts = [p0]
-    num_rays -= 1
-    radii = [(diameter / 2) * i / (num_rings - 1) for i in range(1, num_rings)]
-    circm = [r * 2 * math.pi for r in radii]
-    ds = sum(circm) / num_rays
-    n_rays = [int(round(c / ds)) for c in circm]
-    n_rays[-1] += num_rays - sum(n_rays)
-    for r, numEl in zip(radii, n_rays):
-        if numEl == 0:
-            continue
-        Rm = la.rotate3d(d, 2 * math.pi / numEl)
-        helper = la.scale(r, b1)
-        for _ in range(numEl):
-            pts.append(la.add(p0, helper))
-            helper = la.matvec(Rm, helper)
-    b = RayBundle(np.array(pts), np.array(d), lam)
+    rings = source_rings("collimated", d, b1, diameter, num_rings, num_rays)
+    if on_device:
+        from . import _lib as L
+        b = DeviceSource(L.SRC_COLLIMATED, num_rays, p0, _bundle_dir(d), lam, rings=rings)
+    else:
+        pts = [p0]
+        _expand_rings(rings, lambda v: pts.append(la.add(p0, v)))
+        b = RayBundle(np.array(pts), np.array(d), lam)
     b.diameter = float(diameter)
     return b
 
 
-def PointSource(pos, dir, theta, lam=1e-6, num_rings=10, num_rays=None, b1=None):
-    """BeamGroups.jl:51-100 (cone of concentric fans)."""
+def PointSource(pos, dir, theta, lam=1e-6, num_rings=10, num_rays=None, b1=None, on_device=False):
+    """BeamGroups.jl:51-100 (cone of concentric fans).  on_device=True returns a DeviceSource with bit-identical rays."""
     if num_rays is None:
         num_rays = 100 * num_rings
     if num_rays < num_rings * 20:
@@ -273,24 +391,14 @@ def PointSource(pos, dir, theta, lam=1e-6, num_rings=10, num_rays=None, b1=None)
     if theta >= math.pi:
         raise ValueError("Point source opening half-angle must be <= pi")
     d, b1 = _basis(dir, b1)
-    b2 = la.normalize(la.cross(d, b1))
-    step = theta / (num_rings - 1)
-    dirs = [d]
-    num_rays -= 1
-    ndirs = [la.matvec(la.rotate3d(b2, step * i), d) for i in range(1, num_rings)]
-    circm = [la.norm(la.sub(nd, la.scale(la.dot(nd, d), d))) * 2 * math.pi for nd in ndirs]
-    ds = sum(circm) / num_rays
-    n_rays = [int(round(c / ds)) for c in circm]
-    n_rays[-1] += num_rays - sum(n_rays)
-    for nd, numEl in zip(ndirs, n_rays):
-        if numEl == 0:
-            continue
-        Rm = la.rotate3d(d, 2 * math.pi / numEl)
-        cdir = nd
-        for _ in range(numEl):
-            dirs.append(cdir)
-            cdir = la.matvec(Rm, cdir)
-    n = len(dirs)
-    b = RayBundle(np.tile(np.array(la.v3(pos)), (n, 1)), np.array(dirs), lam)
+    rings = source_rings("point", d, b1, theta, num_rings, num_rays)
+    if on_device:
+        from . import _lib as L
+        b = DeviceSource(L.SRC_POINT, num_rays, pos, _bundle_dir(d), lam, rings=rings)
+    else:
+        dirs = [d]
+        _expand_rings(rings, dirs.append)
+        n = len(dirs)
+        b = RayBundle(np.tile(np.array(la.v3(pos)), (n, 1)), np.array(dirs), lam)
     b.NA = math.sin(theta)
     return b

@@ -105,6 +105,7 @@ struct bmo_result {
     bmo_sys* sys = nullptr;   // system the result was traced through (may be freed before the result: never dereferenced after the trace)
     bmo_ctx* ctx = nullptr;
     std::vector<int32_t> part_object;   // part -> object of that system (segment export, structure check of bmo_retrace)
+    std::vector<int32_t> object_kind;   // bmo_obj_kind of every object of that system (bmo_spot_stats checks its detector)
     int32_t n_objects = 0;
     int mode = 0;           // 0 ray, 1 polarized ray, 2 gaussian beamlet
     int R = 1;              // rays per beam

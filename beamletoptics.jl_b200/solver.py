@@ -183,14 +183,15 @@ def cached_system(system, lambdas, device=0, norm_zero_rule=1):
     return dsys
 
 
-def trace_rays(dsys, pos, dir, lam_id, E0=None, pose_id=None, r_max=100, keep_segments=True, device_inputs=False):
+def trace_rays(dsys, pos, dir, lam_id, E0=None, pose_id=None, r_max=100, keep_segments=True, device_inputs=False, uniform_dir=False):
     """Thin wrapper of bmo_trace_rays.  With device_inputs=True pos/dir/lam_id/E0/pose_id are integer
-    device pointers (e.g. torch tensors' data_ptr()) and `n` must be given as pos=(ptr, n)."""
+    device pointers (e.g. torch tensors' data_ptr()) and `n` must be given as pos=(ptr, n); uniform_dir=True then
+    says that `dir` points at one direction for every ray (BMO_UNIFORM_DIR)."""
     flags = L.KEEP_SEGMENTS if keep_segments else 0
     h = C.c_void_p()
     if device_inputs:
         (ppos, n) = pos
-        flags |= L.INPUT_DEVICE
+        flags |= L.INPUT_DEVICE | (L.UNIFORM_DIR if uniform_dir else 0)
         L.check(L.lib().bmo_trace_rays(dsys.h, n, L.ptr(ppos), L.ptr(dir), L.ptr(lam_id), L.ptr(E0), L.ptr(pose_id), r_max, flags, C.byref(h)))
     else:
         pos = np.ascontiguousarray(pos, dtype=np.float64)
@@ -266,6 +267,8 @@ def _root_signature(beam):
         return (tuple(r.pos), tuple(r.dir), float(r.lam), tuple(complex(x) for x in r.E0) if r.polarized else None)
     if isinstance(beam, bm.BeamletBundle):
         return (hash(np.ascontiguousarray(beam.rays).tobytes()), hash(np.ascontiguousarray(beam.w0).tobytes()), hash(np.ascontiguousarray(beam.E0).tobytes()))
+    if isinstance(beam, bm.DeviceSource):
+        return (beam.signature(),)
     if isinstance(beam, bm.RayBundle):
         e = None if beam.E0 is None else hash(np.ascontiguousarray(beam.E0).tobytes())
         return (hash(np.ascontiguousarray(beam.pos).tobytes()), hash(np.ascontiguousarray(beam.dir).tobytes()), e)
@@ -382,11 +385,12 @@ def _collect_spots(system_flat, res):
                 o.data = np.concatenate([o.data, xz[sel]])
 
 
-def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rule=1, keep_segments=True):
-    """solve_system!(system, beam; r_max, retrace) for a Beam, GaussianBeamlet, RayBundle or
-    BeamletBundle (System.jl:444-468).  Returns the TraceResult (the reference returns nothing)."""
+def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rule=1, keep_segments=True, collect_spots=True):
+    """solve_system!(system, beam; r_max, retrace) for a Beam, GaussianBeamlet, RayBundle, DeviceSource or
+    BeamletBundle (System.jl:444-468).  Returns the TraceResult (the reference returns nothing).
+    collect_spots=False leaves Spotdetector.data alone: the hits stay on the device for spot_stats / TraceResult.spots."""
     if isinstance(beam, (list, tuple)):
-        return [solve_system_(system, b, r_max, retrace, device, norm_zero_rule, keep_segments) for b in beam]
+        return [solve_system_(system, b, r_max, retrace, device, norm_zero_rule, keep_segments, collect_spots) for b in beam]
     if isinstance(beam, bm.Beam):
         r0 = beam.rays[0]
         lams, lam_id = _lambda_ids([r0.lam])
@@ -401,7 +405,8 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
         beam._solution = res
         res._root_sig = _root_signature(beam)
         _rebuild_beam(beam, res, dsys.flat)
-        _collect_spots(dsys.flat, res)
+        if collect_spots:
+            _collect_spots(dsys.flat, res)
         _collect_psfs(dsys, res)
         return res
     if isinstance(beam, bm.GaussianBeamlet):
@@ -416,7 +421,8 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
         beam._solution = res
         res._root_sig = _root_signature(beam)
         _rebuild_gauss(beam, res, dsys.flat)
-        _collect_spots(dsys.flat, res)
+        if collect_spots:
+            _collect_spots(dsys.flat, res)
         _accumulate_pds(dsys, res)
         return res
     if isinstance(beam, bm.RayBundle):
@@ -431,7 +437,7 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
         prev = _previous_solution(beam, dsys, lams) if retrace else None
         if prev is not None:
             res = globals()["retrace"](dsys, prev, r_max, keep_segments)
-        elif not keep_segments and not splitters:      # one beam per ray: fused trace + Spotdetector read-back (pipelined copies)
+        elif not keep_segments and not splitters and collect_spots:   # one beam per ray: fused trace + Spotdetector read-back (pipelined copies)
             obj, xz, res = trace_rays_spots(dsys, beam.pos, bdir, blam, beam.E0, None, r_max)
             res._spots = (obj, xz)
         else:
@@ -439,7 +445,27 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
         res.lams = lams
         beam.result = beam._solution = res
         res._root_sig = _root_signature(beam)
-        _collect_spots(dsys.flat, res)
+        if collect_spots:
+            _collect_spots(dsys.flat, res)
+        if has_psf:
+            _collect_psfs(dsys, res)
+        return res
+    if isinstance(beam, bm.DeviceSource):
+        lams, _ = _lambda_ids([beam.lam])
+        dsys = cached_system(system, lams, device, norm_zero_rule)
+        has_psf = any(isinstance(o, co.PSFDetector) for o in dsys.flat.objects)
+        keep_segments = keep_segments or has_psf       # the PSF records are rebuilt from the segment table
+        prev = _previous_solution(beam, dsys, lams) if retrace else None
+        if prev is not None:
+            res = globals()["retrace"](dsys, prev, r_max, keep_segments)
+        else:      # the rays never leave the device: bmo_source -> bmo_trace_rays(BMO_INPUT_DEVICE)
+            n, ppos, pdir, uniform = beam.device_arrays(device)
+            res = trace_rays(dsys, (ppos, n), pdir, None, None, None, r_max, keep_segments, device_inputs=True, uniform_dir=uniform)
+        res.lams = lams
+        beam.result = beam._solution = res
+        res._root_sig = _root_signature(beam)
+        if collect_spots:
+            _collect_spots(dsys.flat, res)
         if has_psf:
             _collect_psfs(dsys, res)
         return res
@@ -454,10 +480,41 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
         res.lams = lams
         beam.result = beam._solution = res
         res._root_sig = _root_signature(beam)
-        _collect_spots(dsys.flat, res)
+        if collect_spots:
+            _collect_spots(dsys.flat, res)
         _accumulate_pds(dsys, res)
         return res
     raise TypeError(f"cannot trace {type(beam).__name__}")
+
+
+def spot_stats(result, detector, bins=None, window=None):
+    """Spot diagram of `detector` (a Spotdetector of the traced system, or its object index) reduced on the device
+    (bmo_spot_stats): dict of hits, centroid (x, z), rms, max_r (largest distance from the detector origin), lo / hi
+    (x, z) and outside (hits outside `window`).  With `bins` (n or (nx, nz)) also "counts", an (nz, nx) int64 histogram
+    over `window` = (x_lo, x_hi, z_lo, z_hi), by default the detector's face.  The statistics cover every spot entry of the
+    result on that detector (chief, waist and divergence rays of a beamlet result), whether or not they were collected."""
+    objs = result.dsys.flat.objects
+    if isinstance(detector, (int, np.integer)):
+        oi = int(detector)
+    else:
+        oi = next((i for i, o in enumerate(objs) if o is detector), -1)
+        if oi < 0:
+            raise L.BmoError("spot_stats: the detector is not part of the traced system")
+    counts, nx, nz = None, 0, 0
+    if bins is not None:
+        nx, nz = (int(bins), int(bins)) if np.ndim(bins) == 0 else (int(bins[0]), int(bins[1]))
+        if window is None and 0 <= oi < len(objs) and hasattr(objs[oi], "hw"):
+            hw = objs[oi].hw
+            window = (-hw, hw, -hw, hw)
+        counts = np.zeros((max(nz, 0), max(nx, 0)), np.int64)
+    win = None if window is None else np.ascontiguousarray(window, dtype=np.float64)
+    info = L.bmo_spot_info()
+    L.check(L.lib().bmo_spot_stats(result.h, oi, L.ptr(win), nx, nz, C.byref(info), L.ptr(counts), 0))
+    out = dict(hits=int(info.hits), centroid=(info.centroid[0], info.centroid[1]), rms=info.rms, max_r=info.max_r,
+               lo=(info.lo[0], info.lo[1]), hi=(info.hi[0], info.hi[1]), outside=int(info.outside))
+    if counts is not None:
+        out["counts"] = counts
+    return out
 
 
 # ---- PSFDetector (PSFDetector.jl) -----------------------------------------------------------------------

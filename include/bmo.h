@@ -177,7 +177,7 @@ typedef struct bmo_counters {
 } bmo_counters;
 
 int32_t bmo_init(int32_t device, bmo_ctx** ctx);
-int32_t bmo_shutdown(bmo_ctx* ctx);
+int32_t bmo_shutdown(bmo_ctx* ctx);   /* free the systems, results and sources made on ctx first: their free calls use the context */
 const char* bmo_last_error(void);
 int32_t bmo_set_stream(bmo_ctx* ctx, void* cuda_stream);  /* cudaStream_t; NULL = legacy default  */
 int32_t bmo_counters_get(bmo_ctx* ctx, bmo_counters* out);
@@ -297,6 +297,69 @@ int32_t bmo_result_spots(bmo_result* r, int32_t* det_object, double* xz);
 /* same, but leaves the data on the device: returns device pointers valid until bmo_result_free   */
 int32_t bmo_result_spots_device(bmo_result* r, const int32_t** det_object, const double** xz);
 int32_t bmo_result_free(bmo_result* r);
+
+/* ---- sources generated on the device (bmo_source.cu) -----------------------------------------------------
+ * replaces: building the rays of UniformDiscSource (BeamGroups.jl:222-245), CollimatedSource (:152-195) and PointSource
+ * (:51-100) on the host and copying them over.  The host computes every transcendental and every per-ring quantity (ring
+ * counts, rotate3d matrices, the basis) with the same code that builds its own bundles; the device expands the descriptor.
+ *   disc:        one thread per ray k: rho = sqrt((k + 0.5) / n), phi = k * phi0, r = radius * rho,
+ *                pos = pos + ((r cos phi) e1 + (r sin phi) e2); dir = `dir` for every ray.  CUDA's double sin / cos are not
+ *                correctly rounded: positions agree with the host to a few ulp, not to the bit.
+ *   collimated:  ray 0 = pos; ring ray j = pos + v_j with v_0 = ring.start (= r b1), v_{j+1} = ring.rot v_j;
+ *                dir = `dir` for every ray.
+ *   point:       pos for every ray; ray 0 has direction `dir`; ring ray j has v_j renormalised like RayBundle
+ *                (v * (1 / sqrt(vx vx + vy vy + vz vz))), v_0 = ring.start (= the ring's first direction).
+ * Ring sources run one thread per ring through the serial recurrence in linalg.matvec's operation order without FMA
+ * contraction, so they are bit-identical to the host constructors.                                               */
+enum bmo_source_kind { BMO_SRC_DISC = 0, BMO_SRC_COLLIMATED = 1, BMO_SRC_POINT = 2 };
+typedef struct bmo_source_ring {
+    int64_t first, count;   /* rays [first, first + count); rings are contiguous from ray 1; count 0 = skipped ring  */
+    double start[3];        /* collimated: first offset r * b1; point: first direction                                */
+    double rot[9];          /* rotate3d(dir, 2 pi / count), row-major                                                 */
+} bmo_source_ring;
+typedef struct bmo_source_desc {
+    int32_t kind;           /* bmo_source_kind                                                                        */
+    int32_t reserved;
+    int64_t n_rays;
+    int64_t n_rings;        /* ring sources: sum of the counts = n_rays - 1; discs: 0                                */
+    const bmo_source_ring* rings;   /* host array [n_rings]                                                          */
+    double pos[3];
+    double dir[3];          /* normalised the way RayBundle stores it                                                 */
+    double e1[3], e2[3];    /* disc basis (e2 = normalize(dir x e1))                                                 */
+    double radius, phi0;    /* disc: diameter / 2, 2 pi / (1 + sqrt 5)                                                 */
+} bmo_source_desc;
+typedef struct bmo_source bmo_source;
+/* Fills the device buffers of *src from the context's pool, enqueued on the context's stream.  BMO_EINVAL for an
+ * unknown kind, n_rays < 1, a non-finite value or rings that do not tile [1, n_rays).                             */
+int32_t bmo_source_create(bmo_ctx* ctx, const bmo_source_desc* desc, bmo_source** src);
+/* Device pointers for bmo_trace_rays(..., BMO_INPUT_DEVICE | (*uniform_dir ? BMO_UNIFORM_DIR : 0)): pos [n][3];
+ * dir [n][3], or one direction [3] when *uniform_dir is 1.  Valid until bmo_source_free.                         */
+int32_t bmo_source_device(bmo_source* src, int64_t* n, const double** pos, const double** dir, int32_t* uniform_dir);
+/* host copies (NULL ok): pos [n][3], dir [n][3] (a uniform direction is expanded to every ray)                   */
+int32_t bmo_source_rays(bmo_source* src, double* pos, double* dir);
+int32_t bmo_source_free(bmo_source* src);   /* before bmo_shutdown of the source's context */
+
+/* ---- spot-diagram reduction on the device --------------------------------------------------------------
+ * replaces: reading Spotdetector.data (Spotdetector.jl:50-61) back to compute what a spot diagram shows.  Works over the
+ * n_beams * R entries bmo_result_spots reports with det_object[k] == det_object (a beamlet result counts chief, waist and
+ * divergence).  rms = sqrt(sum((x - cx)^2 + (z - cz)^2) / hits) in a second pass; max_r = max sqrt(x x + z z) about the
+ * detector origin; with no hits every floating field is NaN.  The sums run over a fixed partition of the entry index
+ * whose partials are combined in index order, so two calls give the same bits; hits, outside, max_r, lo / hi and the
+ * histogram are exact.
+ * window (NULL ok, required with counts): x_lo, x_hi, z_lo, z_hi, finite with hi > lo; a hit outside the closed window
+ * counts in `outside`.  counts (NULL ok): [nz][nx], counts[j * nx + i] = hits with
+ * i = min(floor((x - x_lo) / (x_hi - x_lo) * nx), nx - 1), j likewise in z; overwritten.  Host pointer, or device
+ * pointer with BMO_INPUT_DEVICE.  (The struct cannot share the function's name in C, hence bmo_spot_info.)        */
+typedef struct bmo_spot_info {
+    int64_t hits;
+    int64_t outside;
+    double centroid[2];     /* mean x, mean z          */
+    double rms;
+    double max_r;
+    double lo[2], hi[2];    /* min / max of x and z    */
+} bmo_spot_info;
+int32_t bmo_spot_stats(bmo_result* r, int32_t det_object, const double* window, int32_t nx, int32_t nz, bmo_spot_info* out,
+                       int64_t* counts, uint32_t flags);
 
 enum bmo_status {
     BMO_ST_ACTIVE = 0,
