@@ -18,8 +18,9 @@ from .components import (AcylindricalSurface, CircularFlatSurface, ConcaveSpheri
 from .shapes import (AcylindricalSurfaceSDF, AsphericalSurfaceSDF, BoxSDF, CircularFlatMesh, ConcaveAsphericalSurfaceSDF, ConvexAsphericalSurfaceSDF, ConcaveCylinderSDF, ConcaveSphericalSurfaceSDF, ConvexCylinderSDF, ConvexSphericalSurfaceSDF, CubeMesh, CuboidMesh, CutSphereSDF,
                      CylinderSDF, Mesh, MeniscusLensSDF, PlanoSurfaceSDF, QuadraticFlatMesh, RectangularFlatMesh, RetroMesh,
                      RightAnglePrismSDF, RingSDF, SphereSDF, ThinLensSDF, UnionSDF, load_stl)
-from .solver import DeviceSystem, TraceResult, pd_accumulate, retrace, solve_system_, spot_stats, trace_beamlets, trace_rays, trace_rays_spots, upload_system
-from .sweep import flatten_poses, solve_pose_sweep, KinProgram, get_pose_tables, solve_pose_sweep_device
+from .solver import DeviceSystem, TraceResult, pd_accumulate, retrace, solve_system_, spot_stats, spot_stats_poses, trace_beamlets, trace_rays, trace_rays_spots, upload_system
+from .sweep import (flatten_poses, solve_pose_sweep, KinProgram, get_pose_tables, solve_pose_sweep_device, solve_spot_sweep,
+                    solve_spot_sweep_device, tile_ray_bundle)
 from . import parallel
 from .parallel import solve_system_sharded
 

@@ -108,6 +108,7 @@ EXPORTS = [
     "bmo_system_set_kinematics", "bmo_system_apply_poses", "bmo_system_get_pose",
     "bmo_debug_normals", "bmo_trim",
     "bmo_source_create", "bmo_source_device", "bmo_source_rays", "bmo_source_free", "bmo_spot_stats",
+    "bmo_source_create_poses", "bmo_source_pose_ids", "bmo_spot_stats_poses",
     "bmo_comm_unique_id", "bmo_comm_init", "bmo_comm_init_local", "bmo_comm_info", "bmo_pd_allreduce", "bmo_pd_allreduce_local", "bmo_comm_free",
 ]
 
@@ -161,6 +162,9 @@ def lib():
         L.bmo_source_rays.argtypes = [_vp, _vp, _vp]
         L.bmo_source_free.argtypes = [_vp]
         L.bmo_spot_stats.argtypes = [_vp, C.c_int32, _vp, C.c_int32, C.c_int32, C.POINTER(bmo_spot_info), _vp, C.c_uint32]
+        L.bmo_source_create_poses.argtypes = [_vp, C.POINTER(bmo_source_desc), C.c_int32, C.POINTER(_vp)]
+        L.bmo_source_pose_ids.argtypes = [_vp, _ip, C.POINTER(_vp)]
+        L.bmo_spot_stats_poses.argtypes = [_vp, C.c_int32, C.c_int32, _vp, C.c_int32, C.c_int32, C.POINTER(bmo_spot_info), _vp, C.c_uint32]
         L.bmo_comm_unique_id.argtypes = [_vp]
         L.bmo_comm_init.argtypes = [_vp, C.c_int32, C.c_int32, _vp, C.POINTER(_vp)]
         L.bmo_comm_init_local.argtypes = [C.c_int32, C.POINTER(_vp), C.POINTER(_vp)]

@@ -262,9 +262,10 @@ def _expand_rings(rings, emit):
 class DeviceSource:
     """A source whose rays are generated on the GPU (bmo_source_create) from a descriptor: the basis, the ring table and
     every transcendental are computed here by the code that builds the host bundles.  One bmo_source is created per
-    device on first use; `pos` / `dir` download the rays (device 0) for inspection.  solve_system_ traces it from the
-    device pointers, so no per-ray data crosses the bus.  The handles belong to the per-process contexts of _lib.context,
-    which live until the process ends, so freeing them from __del__ never outlives the context."""
+    (device, n_poses) on first use -- n_poses > 1 tiles the rays pose-major for a pose sweep (bmo_source_create_poses);
+    `pos` / `dir` download the untiled rays for inspection.  solve_system_ traces it from the device pointers, so no
+    per-ray data crosses the bus.  The handles belong to the per-process contexts of _lib.context, which live until the
+    process ends, so freeing them from __del__ never outlives the context."""
 
     def __init__(self, kind, n, pos, dir, lam, rings=(), e1=(0.0, 0.0, 0.0), e2=(0.0, 0.0, 0.0), radius=0.0, phi0=0.0):
         from . import _lib as L
@@ -292,32 +293,41 @@ class DeviceSource:
 
     def signature(self): return self._sig
 
-    def handle(self, device=0):
-        """The bmo_source of this descriptor on `device` (created on first use)."""
+    def handle(self, device=0, n_poses=1):
+        """The bmo_source of this descriptor on `device`, tiled `n_poses` times (created on first use)."""
         from . import _lib as L
-        if device not in self._handles:
+        key = (int(device), int(n_poses))
+        if key not in self._handles:
             h = C.c_void_p()
-            L.check(L.lib().bmo_source_create(L.context(device), C.byref(self.desc), C.byref(h)))
-            self._handles[device] = h
-        return self._handles[device]
+            L.check(L.lib().bmo_source_create_poses(L.context(device), C.byref(self.desc), key[1], C.byref(h)))
+            self._handles[key] = h
+        return self._handles[key]
 
-    def device_arrays(self, device=0):
-        """(n, pos, dir, uniform_dir): device pointers for bmo_trace_rays with BMO_INPUT_DEVICE."""
+    def device_arrays(self, device=0, n_poses=None):
+        """(n, pos, dir, uniform_dir): device pointers for bmo_trace_rays with BMO_INPUT_DEVICE.  With `n_poses` the rays
+        are tiled pose-major and the tuple ends with the pose-id pointer, (n * n_poses, pos, dir, uniform_dir, pose_id);
+        pose_id is None for one pose."""
         from . import _lib as L
+        h = self.handle(device, 1 if n_poses is None else n_poses)
         n, p, d, u = C.c_int64(), C.c_void_p(), C.c_void_p(), C.c_int32()
-        L.check(L.lib().bmo_source_device(self.handle(device), C.byref(n), C.byref(p), C.byref(d), C.byref(u)))
-        return int(n.value), p.value, d.value, bool(u.value)
+        L.check(L.lib().bmo_source_device(h, C.byref(n), C.byref(p), C.byref(d), C.byref(u)))
+        if n_poses is None:
+            return int(n.value), p.value, d.value, bool(u.value)
+        npo, pid = C.c_int32(), C.c_void_p()
+        L.check(L.lib().bmo_source_pose_ids(h, C.byref(npo), C.byref(pid)))
+        return int(n.value), p.value, d.value, bool(u.value), pid.value
 
-    def rays(self, device=0):
-        """Host copies (pos (n, 3), dir (n, 3)) of the rays generated on `device` (bmo_source_rays)."""
+    def rays(self, device=0, n_poses=1):
+        """Host copies (pos (n * n_poses, 3), dir (n * n_poses, 3)) of the rays generated on `device` (bmo_source_rays)."""
         from . import _lib as L
-        pos, dir = np.zeros((self.n, 3)), np.zeros((self.n, 3))
-        L.check(L.lib().bmo_source_rays(self.handle(device), L.ptr(pos), L.ptr(dir)))
+        m = self.n * int(n_poses)
+        pos, dir = np.zeros((m, 3)), np.zeros((m, 3))
+        L.check(L.lib().bmo_source_rays(self.handle(device, n_poses), L.ptr(pos), L.ptr(dir)))
         return pos, dir
 
     def _download(self):
         if self._host is None:
-            self._host = self.rays(next(iter(self._handles), 0))
+            self._host = self.rays(next(iter(self._handles), (0, 1))[0])
         return self._host
 
     @property

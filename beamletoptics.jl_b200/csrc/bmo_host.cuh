@@ -107,6 +107,7 @@ struct bmo_result {
     std::vector<int32_t> part_object;   // part -> object of that system (segment export, structure check of bmo_retrace)
     std::vector<int32_t> object_kind;   // bmo_obj_kind of every object of that system (bmo_spot_stats checks its detector)
     int32_t n_objects = 0;
+    int32_t n_poses = 1;    // poses of that system at trace time (bmo_spot_stats_poses checks its argument against it)
     int mode = 0;           // 0 ray, 1 polarized ray, 2 gaussian beamlet
     int R = 1;              // rays per beam
     int nsd = 12;           // doubles per segment record

@@ -2161,7 +2161,7 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
     bmo_result* res = new bmo_result();
     res->sys = sys; res->ctx = sys->ctx; res->part_object.resize(sys->parts.size()); for (size_t i = 0; i < sys->parts.size(); i++) res->part_object[i] = sys->parts[i].object;
     for (const bmo_object& ob : sys->objects) res->object_kind.push_back(ob.kind);
-    res->n_objects = (int32_t)sys->objects.size(); res->mode = mode; res->R = R; res->nsd = nf_seg(mode); res->n_roots = n; res->keep = flags & BMO_KEEP_SEGMENTS;
+    res->n_objects = (int32_t)sys->objects.size(); res->n_poses = sys->view.n_poses; res->mode = mode; res->R = R; res->nsd = nf_seg(mode); res->n_roots = n; res->keep = flags & BMO_KEEP_SEGMENTS;
     static const bool prof = getenv("BMO_HOST_PROFILE") != nullptr;
     const double tp0 = tnow_ms();
     BMO_CUDA(cudaEventRecord(ctx->ev0, st));

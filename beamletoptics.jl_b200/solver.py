@@ -487,31 +487,56 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
     raise TypeError(f"cannot trace {type(beam).__name__}")
 
 
-def spot_stats(result, detector, bins=None, window=None):
-    """Spot diagram of `detector` (a Spotdetector of the traced system, or its object index) reduced on the device
-    (bmo_spot_stats): dict of hits, centroid (x, z), rms, max_r (largest distance from the detector origin), lo / hi
-    (x, z) and outside (hits outside `window`).  With `bins` (n or (nx, nz)) also "counts", an (nz, nx) int64 histogram
-    over `window` = (x_lo, x_hi, z_lo, z_hi), by default the detector's face.  The statistics cover every spot entry of the
-    result on that detector (chief, waist and divergence rays of a beamlet result), whether or not they were collected."""
+def _spot_args(result, detector, bins, window, what):
+    """(object index, nx, nz, window array) of a spot_stats call; the window defaults to the detector's face."""
     objs = result.dsys.flat.objects
     if isinstance(detector, (int, np.integer)):
         oi = int(detector)
     else:
         oi = next((i for i, o in enumerate(objs) if o is detector), -1)
         if oi < 0:
-            raise L.BmoError("spot_stats: the detector is not part of the traced system")
-    counts, nx, nz = None, 0, 0
+            raise L.BmoError(f"{what}: the detector is not part of the traced system")
+    nx = nz = 0
     if bins is not None:
         nx, nz = (int(bins), int(bins)) if np.ndim(bins) == 0 else (int(bins[0]), int(bins[1]))
         if window is None and 0 <= oi < len(objs) and hasattr(objs[oi], "hw"):
             hw = objs[oi].hw
             window = (-hw, hw, -hw, hw)
-        counts = np.zeros((max(nz, 0), max(nx, 0)), np.int64)
     win = None if window is None else np.ascontiguousarray(window, dtype=np.float64)
+    return oi, nx, nz, win
+
+
+def spot_stats(result, detector, bins=None, window=None):
+    """Spot diagram of `detector` (a Spotdetector of the traced system, or its object index) reduced on the device
+    (bmo_spot_stats): dict of hits, centroid (x, z), rms, max_r (largest distance from the detector origin), lo / hi
+    (x, z) and outside (hits outside `window`).  With `bins` (n or (nx, nz)) also "counts", an (nz, nx) int64 histogram
+    over `window` = (x_lo, x_hi, z_lo, z_hi), by default the detector's face.  The statistics cover every spot entry of the
+    result on that detector (chief, waist and divergence rays of a beamlet result), whether or not they were collected."""
+    oi, nx, nz, win = _spot_args(result, detector, bins, window, "spot_stats")
+    counts = None if bins is None else np.zeros((max(nz, 0), max(nx, 0)), np.int64)
     info = L.bmo_spot_info()
     L.check(L.lib().bmo_spot_stats(result.h, oi, L.ptr(win), nx, nz, C.byref(info), L.ptr(counts), 0))
     out = dict(hits=int(info.hits), centroid=(info.centroid[0], info.centroid[1]), rms=info.rms, max_r=info.max_r,
                lo=(info.lo[0], info.lo[1]), hi=(info.hi[0], info.hi[1]), outside=int(info.outside))
+    if counts is not None:
+        out["counts"] = counts
+    return out
+
+
+def spot_stats_poses(result, detector, n_poses, bins=None, window=None):
+    """spot_stats for every pose of a pose sweep (bmo_spot_stats_poses): pose p covers the beams traced with pose id p
+    (children inherit their root's pose).  Returns a dict of arrays: hits (P,), outside (P,), centroid (P, 2), rms (P,),
+    max_r (P,), lo / hi (P, 2) and, with `bins`, counts (P, nz, nx) over `window` (by default the detector's face).  Pose p
+    has the bits spot_stats gives for a one-pose solve that lists the pose's hits in the same order, which a system
+    without beamsplitters always does."""
+    oi, nx, nz, win = _spot_args(result, detector, bins, window, "spot_stats_poses")
+    P = int(n_poses)
+    counts = None if bins is None else np.zeros((max(P, 0), max(nz, 0), max(nx, 0)), np.int64)
+    info = (L.bmo_spot_info * max(P, 1))()
+    L.check(L.lib().bmo_spot_stats_poses(result.h, oi, P, L.ptr(win), nx, nz, info, L.ptr(counts), 0))
+    a = np.frombuffer(info, dtype=np.dtype([("hits", np.int64), ("outside", np.int64), ("centroid", np.float64, 2), ("rms", np.float64),
+                                            ("max_r", np.float64), ("lo", np.float64, 2), ("hi", np.float64, 2)]))[:P]
+    out = {k: np.array(a[k]) for k in ("hits", "outside", "centroid", "rms", "max_r", "lo", "hi")}
     if counts is not None:
         out["counts"] = counts
     return out

@@ -1,10 +1,12 @@
 """Batched kinematic pose sweeps (BASELINE config 5): many `translate3d!/rotate3d!` poses of one
-system traced in a single launch, one Photodetector interferogram per pose.
+system traced in a single launch, one Photodetector interferogram or one spot diagram per pose.
 
 The reference solves one pose at a time (move -> empty!(pd) -> solve_system! -> optical_power(pd),
-test/runtests.jl:2092-2120).  Here every pose is flattened on the host with the unchanged kinematic
-API, the tables are stacked and uploaded once (bmo_system_set_poses), every beamlet is replicated per
-pose with a pose id, and the detector kernel writes fields[pose].
+test/runtests.jl:2092-2120; likewise empty!(sd) -> solve_system! -> sd.data for a Spotdetector).  Here
+every pose is flattened on the host with the unchanged kinematic API (or computed on the device from a
+KinProgram), the tables are stacked and uploaded once (bmo_system_set_poses), every beamlet or ray is
+replicated per pose with a pose id, and the detector kernel writes fields[pose] / the spot reduction
+writes the statistics of each pose.
 """
 import ctypes as C
 
@@ -13,7 +15,7 @@ import numpy as np
 from . import _lib as L
 from . import beams as bm
 from .flatten import FlatSystem
-from .solver import DeviceSystem, TraceResult, _lambda_ids
+from .solver import DeviceSystem, TraceResult, _lambda_ids, spot_stats_poses, trace_rays
 
 
 def flatten_poses(system, lambdas, n_poses, apply_pose, norm_zero_rule=1):
@@ -173,3 +175,68 @@ def solve_pose_sweep_device(system, beam, n_poses, program, pd, r_max=100, devic
         z = fields[:, 0::2] + 1j * fields[:, 1::2]
         out["fields"] = z.reshape(n_poses, n, n).transpose(0, 2, 1)
     return out
+
+
+# ---- spot diagrams over poses ------------------------------------------------------------------------------
+def tile_ray_bundle(beam, n_poses):
+    """A RayBundle tiled pose-major for a sweep: (pos (n P, 3), dir ((3,) uniform or (n P, 3)), lam (n P,), pose_id (n P,)),
+    ray i is ray i mod n and pose_id[i] = i // n -- the layout bmo_source_create_poses gives a DeviceSource."""
+    n = len(beam)
+    pos = np.ascontiguousarray(np.tile(beam.pos, (n_poses, 1)))
+    if getattr(beam, "uniform_dir", False) and n:
+        dir = np.ascontiguousarray(beam.dir[0])
+    else:
+        dir = np.ascontiguousarray(np.tile(beam.dir, (n_poses, 1)))
+    lam = np.ascontiguousarray(np.tile(np.broadcast_to(np.asarray(beam.lam, dtype=np.float64), (n,)), n_poses))
+    pose_id = np.ascontiguousarray(np.repeat(np.arange(n_poses, dtype=np.int32), n))
+    return pos, dir, lam, pose_id
+
+
+def _trace_spot_sweep(dsys, beam, lam_id, n_poses, r_max):
+    """Trace `beam` once per pose of `dsys` (segments not kept): a DeviceSource is tiled on the device, a RayBundle on
+    the host."""
+    if isinstance(beam, bm.DeviceSource):
+        n, ppos, pdir, uniform, pid = beam.device_arrays(dsys.device, n_poses)
+        return trace_rays(dsys, (ppos, n), pdir, None, None, pid, r_max, False, device_inputs=True, uniform_dir=uniform)
+    pos, dir, _, pose_id = tile_ray_bundle(beam, n_poses)
+    lam = None if len(dsys.flat.lambdas) == 1 else np.tile(lam_id, n_poses)
+    E0 = None if beam.E0 is None else np.tile(beam.E0, (n_poses, 1))
+    return trace_rays(dsys, pos, dir, lam, E0, pose_id, r_max, False)
+
+
+def _beam_lambdas(beam):
+    if isinstance(beam, bm.DeviceSource):
+        return _lambda_ids([beam.lam])
+    if not isinstance(beam, bm.RayBundle):
+        raise TypeError(f"a spot sweep traces a RayBundle or a DeviceSource, not {type(beam).__name__}")
+    return _lambda_ids(beam.lam)
+
+
+def solve_spot_sweep(system, beam, n_poses, apply_pose, detector, bins=None, window=None, r_max=100, device=0):
+    """Spot diagrams of `detector` (a Spotdetector) over `n_poses` poses of `system`: apply_pose(p) moves the host objects
+    into pose p (flatten_poses), the rays of `beam` (RayBundle or DeviceSource) are traced once per pose in one call and
+    reduced per pose on the device (spot_stats_poses).  Replaces the loop move -> empty!(sd) -> solve_system! -> sd.data.
+    Returns dict(stats=spot_stats_poses(...), result=TraceResult, dsys=DeviceSystem); the host objects are left in the
+    last pose."""
+    lams, lam_id = _beam_lambdas(beam)
+    f0, (prims, verts, bounds, det_pos, det_dir) = flatten_poses(system, lams, n_poses, apply_pose)
+    dsys = DeviceSystem(f0, device)
+    L.check(L.lib().bmo_system_set_poses(dsys.h, n_poses, L.ptr(prims), L.ptr(verts), L.ptr(bounds), L.ptr(det_pos), L.ptr(det_dir)))
+    dsys.n_poses = n_poses
+    res = _trace_spot_sweep(dsys, beam, lam_id, n_poses, r_max)
+    return dict(stats=spot_stats_poses(res, detector, n_poses, bins, window), result=res, dsys=dsys)
+
+
+def solve_spot_sweep_device(system, beam, n_poses, program, detector, bins=None, window=None, r_max=100, device=0):
+    """solve_spot_sweep with the poses produced on the device: `program(prog)` records the kinematic calls of the sweep on
+    a KinProgram (e.g. `prog.translate3d_(detector, offsets)`); the host objects are not moved.  A DeviceSource is tiled
+    on the device (bmo_source_create_poses), so no per-ray data crosses the bus."""
+    lams, lam_id = _beam_lambdas(beam)
+    f0 = FlatSystem(system, lams)
+    dsys = DeviceSystem(f0, device)
+    prog = KinProgram(f0, n_poses)
+    program(prog)
+    prog.apply(dsys)
+    dsys.n_poses = n_poses
+    res = _trace_spot_sweep(dsys, beam, lam_id, n_poses, r_max)
+    return dict(stats=spot_stats_poses(res, detector, n_poses, bins, window), result=res, dsys=dsys)

@@ -332,8 +332,18 @@ typedef struct bmo_source bmo_source;
 /* Fills the device buffers of *src from the context's pool, enqueued on the context's stream.  BMO_EINVAL for an
  * unknown kind, n_rays < 1, a non-finite value or rings that do not tile [1, n_rays).                             */
 int32_t bmo_source_create(bmo_ctx* ctx, const bmo_source_desc* desc, bmo_source** src);
+/* Pose-tiled source for a pose sweep: replaces building the same source once per step of the loop `translate3d!(obj, ...)
+ * -> empty!(sd) -> solve_system!(system, source) -> sd.data` (AbstractShape.jl:56-94, Spotdetector.jl:50-61,
+ * System.jl:444-468).  n_poses copies of the descriptor's rays, pose-major: ray i is ray i mod n_rays of the descriptor and
+ * pose_id[i] = i / n_rays, so every tile is bit-identical to bmo_source_create (discs keep rho = sqrt((k + 0.5) / n_rays);
+ * ring sources run their recurrence once and copy it).  bmo_source_create is the n_poses = 1 case.  BMO_EINVAL also for
+ * n_poses < 1 or n_rays * n_poses overflowing int64.                                                              */
+int32_t bmo_source_create_poses(bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, bmo_source** src);
+/* Device pose ids [n_rays * n_poses] for bmo_trace_rays(..., pose_id, BMO_INPUT_DEVICE); NULL for a one-pose source.
+ * Valid until bmo_source_free.                                                                                       */
+int32_t bmo_source_pose_ids(bmo_source* src, int32_t* n_poses, const int32_t** pose_id);
 /* Device pointers for bmo_trace_rays(..., BMO_INPUT_DEVICE | (*uniform_dir ? BMO_UNIFORM_DIR : 0)): pos [n][3];
- * dir [n][3], or one direction [3] when *uniform_dir is 1.  Valid until bmo_source_free.                         */
+ * dir [n][3], or one direction [3] when *uniform_dir is 1.  n counts the rays of every pose.  Valid until bmo_source_free. */
 int32_t bmo_source_device(bmo_source* src, int64_t* n, const double** pos, const double** dir, int32_t* uniform_dir);
 /* host copies (NULL ok): pos [n][3], dir [n][3] (a uniform direction is expanded to every ray)                   */
 int32_t bmo_source_rays(bmo_source* src, double* pos, double* dir);
@@ -360,6 +370,17 @@ typedef struct bmo_spot_info {
 } bmo_spot_info;
 int32_t bmo_spot_stats(bmo_result* r, int32_t det_object, const double* window, int32_t nx, int32_t nz, bmo_spot_info* out,
                        int64_t* counts, uint32_t flags);
+/* Per-pose spot statistics of a pose sweep: replaces reading sd.data after every step of the loop `translate3d!(obj, ...)
+ * -> empty!(sd) -> solve_system!(system, source) -> sd.data` (AbstractShape.jl:56-94, Spotdetector.jl:50-61,
+ * System.jl:444-468).  out[p] is bmo_spot_stats's definition over the entries of the beams whose pose is p (all R entries
+ * of a beamlet; children inherit their root's pose), taken in increasing entry index; counts (NULL ok): [n_poses][nz][nx]
+ * over the shared window, host pointer, or device pointer with BMO_INPUT_DEVICE.  The beams are ordered stably by pose and
+ * each pose's entries are cut into slices by bmo_spot_stats's formula on that pose's entry count, so out[p] has the bits
+ * bmo_spot_stats gives for a one-pose result that lists the pose's entries in the same order (always the case without
+ * beamsplitters: the roots follow the input order).  n_poses must be the pose count of the system at trace time
+ * (BMO_EINVAL otherwise), and bmo_spot_stats's argument checks apply.                                               */
+int32_t bmo_spot_stats_poses(bmo_result* r, int32_t det_object, int32_t n_poses, const double* window, int32_t nx, int32_t nz,
+                             bmo_spot_info* out, int64_t* counts, uint32_t flags);
 
 enum bmo_status {
     BMO_ST_ACTIVE = 0,
