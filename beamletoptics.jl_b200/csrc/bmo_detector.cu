@@ -17,7 +17,6 @@
 //       (tilted detectors, Beam.jl:186-199) take the reference-order path below.
 //   pd_field (BMO_PD_REFERENCE_ORDER)  every pair evaluated in the reference's operation order;
 //       kept as the cross-check of the fast kernel at full detector sizes.
-#include <cstdlib>
 #include "bmo_host.cuh"
 #include "bmo_interact.cuh"
 
@@ -319,8 +318,9 @@ BMO_D Cx pd_pair_fast(const PdFast& rc, V3 p1, bool& slow) {
     return mkc((rc.cre * re - rc.cim * im) * amp, (rc.cre * im + rc.cim * re) * amp);
 }
 
-template <int PDF_PX, int MINB>
-__global__ void __launch_bounds__(PDF_TX* PDF_TY, MINB) pd_field_fast(const PdParams P) {
+// One pixel per thread, 3 resident blocks per SM (80 registers): the fastest configuration measured (DESIGN §5).
+constexpr int PDF_PX = 1;
+__global__ void __launch_bounds__(PDF_TX* PDF_TY, 3) pd_field_fast(const PdParams P) {
     __shared__ PdFast s_rec[PDF_BATCH];
     const int tid = threadIdx.y * PDF_TX + threadIdx.x;
     const int i = blockIdx.x * PDF_TX + threadIdx.x;
@@ -541,17 +541,8 @@ static int32_t pd_run(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t po
             dim3 grid((n + PD_TILE - 1) / PD_TILE, (n + PD_TILE - 1) / PD_TILE, n_fields), block(PD_TILE, PD_TILE);
             pd_field<<<grid, block, 0, st>>>(pp);
         } else {
-            static const int variant = getenv("BMO_PD_VARIANT") ? atoi(getenv("BMO_PD_VARIANT")) : 13;   // tuning knob: 10*PX + MINB (13 = 80 registers, 3 blocks per SM: the fastest measured)
-            const int px = (variant == 22 || variant == 24) ? 2 : 1;
-            dim3 grid((n + PDF_TX - 1) / PDF_TX, (n + PDF_TY * px - 1) / (PDF_TY * px), n_fields), block(PDF_TX, PDF_TY);
-            switch (variant) {
-                case 13: pd_field_fast<1, 3><<<grid, block, 0, st>>>(pp); break;
-                case 15: pd_field_fast<1, 5><<<grid, block, 0, st>>>(pp); break;
-                case 16: pd_field_fast<1, 6><<<grid, block, 0, st>>>(pp); break;
-                case 22: pd_field_fast<2, 2><<<grid, block, 0, st>>>(pp); break;
-                case 24: pd_field_fast<2, 4><<<grid, block, 0, st>>>(pp); break;
-                default: pd_field_fast<1, 4><<<grid, block, 0, st>>>(pp); break;
-            }
+            dim3 grid((n + PDF_TX - 1) / PDF_TX, (n + PDF_TY * PDF_PX - 1) / (PDF_TY * PDF_PX), n_fields), block(PDF_TX, PDF_TY);
+            pd_field_fast<<<grid, block, 0, st>>>(pp);
         }
         BMO_CUDA(cudaEventRecord(ctx->evk1, st));
         ctx->launches++;

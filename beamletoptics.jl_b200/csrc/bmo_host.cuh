@@ -54,10 +54,9 @@ struct bmo_ctx {
     double trace_ms = 0, pd_ms = 0;
     int64_t pool_slack = 0;   // bytes by which bmo_retrace has grown the stream-ordered pool beyond its own needs (see there)
     int sm_count = 148;
-    // solve_rays_persistent (bmo_trace.cu: persistent_blocks): the variant and table size last sized, its resident blocks per SM
-    const void* persist_fn = nullptr;
+    // solve_rays_persistent (bmo_trace.cu: persistent_blocks): the table size last sized, its resident blocks per SM (-1: none yet)
     size_t persist_smem = 0;
-    int persist_blocks = 0;
+    int persist_blocks = -1;
 };
 
 struct bmo_sys {

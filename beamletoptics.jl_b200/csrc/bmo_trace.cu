@@ -12,18 +12,18 @@
 //                         slot, a dead one is flagged.  Systems with beamsplitters (NS = false): the children go
 //                         to a scratch area in queue order (warp ballots + prefix sums), scan_counts + spawn_children
 //                         number them deterministically and append the reflected ones to the queue.
-//   K1+K2 fused_wave0     plain rays through a splitter-free system, all waves of a chunk in one launch (used by
-//                         pipelined host-input calls, where the number of launches is what limits).
+//   K1+K2 fused_wave0     plain rays through a splitter-free system, all waves of a chunk in one launch: every wave of a
+//                         pipelined host-input call with plain rays, where the number of launches is what limits.
+//   K1r retrace_intersect_wave   K1 of a retrace call (stored path re-validated per beam).
+//   K3 compact_fused      queue compaction in one cooperative launch once the dead slots are the majority.
 // Plain rays through a splitter-free LEAN system whose segments are not kept need no waves at all: solve_rays_persistent
 // carries every ray from the caller's inputs to its last interaction in one launch.
-//   K1r retrace_intersect_wave   K1 of a retrace call (stored path re-validated per beam).
-//   K3 compact_fused      queue compaction in one cooperative launch once the dead slots are the majority
-//                         (compact_count + scan_counts + compact_scatter as the fallback).
 // With BMO_KEEP_SEGMENTS the segment records are written wave-major by K2 and gathered into
 // beam-major row records at the end (gather_segments, a warp-level transposition through shared memory).
 #include <chrono>
 #include <cstdlib>
 #include <cooperative_groups.h>
+#include <type_traits>
 #include "bmo_host.cuh"
 #include "bmo_interact.cuh"
 #include "bmo_lean.cuh"
@@ -132,9 +132,13 @@ BMO_D void stage_tables(const SysView& S, unsigned char* smem) {
 // STAGED: the small system tables (prims, parts, bounds) live in shared memory -- a compile-time fact,
 // so that the marching loop reads them with LDS instead of generic loads.
 // LEAN: every SDF part is a union of at most 4 plain primitives and every mesh is small (bmo_sys::all_lean): the union loop keeps
-// its member bounds in shared memory (LeanBounds, bmo_geom.cuh) and the BVH traversal is compiled out.
-template <int MINB, bool STAGED, bool RK, bool LEAN = false>
-__global__ void __launch_bounds__(IBLOCK, MINB) intersect_wave(const IntersectParams P) {
+// its member bounds in shared memory (LeanBounds, bmo_geom.cuh) and the BVH traversal is compiled out.  LEAN implies STAGED and
+// !RK (see k1_config).
+// Resident blocks per SM K1 is compiled for (DESIGN §5): 8 for the lean build (64 registers, the fastest of 6 / 7 / 8 on C2),
+// 7 for the general staged build (72 registers, the fastest of 4..8 on C2), 6 with the rare primitives, 4 without staged tables.
+constexpr int k1_min_blocks(bool staged, bool rk, bool lean) { return !staged ? 4 : lean ? 8 : rk ? 6 : 7; }
+template <bool STAGED, bool RK, bool LEAN = false>
+__global__ void __launch_bounds__(IBLOCK, k1_min_blocks(STAGED, RK, LEAN)) intersect_wave(const IntersectParams P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ float s_lb[LEAN ? LB_ROWS * LB_STRIDE : 1];
     __shared__ double s_ls[LEAN ? LS_SLOTS * LB_STRIDE : 1];
@@ -737,11 +741,8 @@ BMO_D void interact_body(const StepParams& P, const Hit& h_reg, const int wave_o
     }
 }
 
-#ifndef KMINB0
-#define KMINB0 6
-#endif
 template <int MODE, bool NS = false>
-__global__ void __launch_bounds__(Cfg<MODE>::BLOCK, MODE == 0 ? KMINB0 : 1) interact_wave(const StepParams P) {
+__global__ void __launch_bounds__(Cfg<MODE>::BLOCK, MODE == 0 ? 6 : 1) interact_wave(const StepParams P) {
     Hit none; none.part = -1; none.t = INFINITY; none.n = mk3(0, 0, 0);
     interact_body<MODE, false, NS>(P, none);
 }
@@ -749,8 +750,10 @@ __global__ void __launch_bounds__(Cfg<MODE>::BLOCK, MODE == 0 ? KMINB0 : 1) inte
 // ---- K1+K2 fused: plain rays through a system without beamsplitters (the sequential lens-stack path) --
 // One thread per ray does tracing_step! and interact3d back to back: the hit record never leaves the
 // registers and the ray state is read once.  Needs IBLOCK == Cfg<0>::BLOCK == Cfg<0>::UNITS.
-template <int MINB, bool STAGED, bool RK, bool LEAN = false>
-__global__ void __launch_bounds__(IBLOCK, MINB) fused_wave0(const StepParams P) {
+// Resident blocks per SM it is compiled for: 6 with staged tables (the lean build included), 4 without.
+constexpr int fused_min_blocks(bool staged) { return staged ? 6 : 4; }
+template <bool STAGED, bool RK, bool LEAN = false>
+__global__ void __launch_bounds__(IBLOCK, fused_min_blocks(STAGED)) fused_wave0(const StepParams P) {
     static_assert(IBLOCK == Cfg<0>::BLOCK && Cfg<0>::UNITS == IBLOCK, "fused_wave0 maps one thread to one ray like interact_wave<0>");
     __shared__ float s_lb[LEAN ? LB_ROWS * LB_STRIDE : 1];
     __shared__ double s_ls[LEAN ? LS_SLOTS * LB_STRIDE : 1];
@@ -832,9 +835,8 @@ struct SolveParams {
 // Per-thread scratch columns besides the march's (s_ls): the ray's refractive index (s_pn), wavelength id and segment index
 // (s_pi rows 0 / 1) are not needed by the march and would otherwise hold registers through it.  2 KB on top of the 22 KB of
 // intersect_wave's static scratch: with the LEAN gate's 24 KB of tables (staged_smem) a block stays within the 48 KB it gets
-// without opting in (checked at launch, persistent_blocks).
-template <int MINB>
-__global__ void __launch_bounds__(IBLOCK, MINB) solve_rays_persistent(const SolveParams P) {
+// without opting in (checked at launch, persistent_blocks).  6 resident blocks per SM: the fastest on C2 (DESIGN §5).
+__global__ void __launch_bounds__(IBLOCK, 6) solve_rays_persistent(const SolveParams P) {
     __shared__ float s_lb[LB_ROWS * LB_STRIDE];
     __shared__ double s_ls[LS_SLOTS * LB_STRIDE];
     __shared__ double s_pn[LB_STRIDE];
@@ -1058,45 +1060,10 @@ __global__ void __launch_bounds__(256) spawn_children(const SpawnParams P) {
 }
 
 // ---- K3: queue compaction (HBM-bound) ----------------------------------------------------------------
-// Dead slots are squeezed out when they make up more than half of the queue: per block, warp ballots
-// + prefix sums give every live unit its rank; scan_counts turns the block counts into offsets; the
-// scatter moves the live units to the front of the other queue buffer, order preserved.
+// Dead slots are squeezed out when they make up more than half of the queue: the live units move to the front of the other
+// queue buffer, order preserved.
 constexpr int CBLOCK = 256;
-__global__ void __launch_bounds__(CBLOCK) compact_count(const int32_t* qi, int64_t cap, int64_t n_slots, int R, int32_t* blk_cnt) {
-    __shared__ int s_w[CBLOCK / 32];
-    const int64_t u = (int64_t)blockIdx.x * CBLOCK + threadIdx.x;
-    const bool live = u < n_slots && qi[I_BEAM * cap + u * R] >= 0;
-    const unsigned bal = __ballot_sync(0xffffffffu, live);
-    if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = __popc(bal);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        int a = 0;
-        for (int k = 0; k < CBLOCK / 32; k++) a += s_w[k];
-        blk_cnt[blockIdx.x] = a;
-    }
-}
-__global__ void __launch_bounds__(CBLOCK) compact_scatter(Queue src, Queue dst, int64_t n_slots, int R, int nf, const long long* blk_off) {
-    __shared__ int s_w[CBLOCK / 32];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int64_t u = (int64_t)blockIdx.x * CBLOCK + threadIdx.x;
-    const int64_t ss = src.cap, ds = dst.cap;
-    const bool live = u < n_slots && src.i[I_BEAM * ss + u * R] >= 0;
-    const unsigned bal = __ballot_sync(0xffffffffu, live);
-    if (lane == 0) s_w[warp] = __popc(bal);
-    __syncthreads();
-    int woff = 0;
-    for (int k = 0; k < warp; k++) woff += s_w[k];
-    if (!live) return;
-    const int64_t du = blk_off[blockIdx.x] + woff + __popc(bal & lanemask_lt());
-    for (int r = 0; r < R; r++) {
-        const int64_t si = u * R + r, di = du * R + r;
-        for (int f = 0; f < nf; f++) dst.d[f * ds + di] = src.d[f * ss + si];
-#pragma unroll
-        for (int f = 0; f < NI_Q; f++) dst.i[f * ds + di] = src.i[f * ss + si];
-    }
-}
-
-// K3 in one launch (cooperative grid, one CTA slice per resident block, one contiguous sub-slice per warp): every warp counts
+// One cooperative launch (one CTA slice per resident block, one contiguous sub-slice per warp): every warp counts
 // the live units of its sub-slice, grid-wide barrier, own offset = sum of the lower blocks' counts (a few hundred values, L2
 // hits) + the lower warps of the block, then every warp scatters its sub-slice on its own, two 32-slot rows per step, all loads
 // of both rows issued before the first store -- no block barrier inside the copy loop, so the 8 warps of a block and the two
@@ -1837,12 +1804,23 @@ int32_t SubTrace::begin(const TraceInputs& in_h) {
 // Dynamic shared memory of the trace kernels (0 unless the tables are staged); lean: the LEAN builds apply (bmo_lean.cuh).
 static size_t staged_smem(const bmo_sys* sys, bool staged, bool& lean) {
     const SysView& V = sys->view;
-    static const bool lean_ok = !(getenv("BMO_LEAN") && atoi(getenv("BMO_LEAN")) == 0);   // tuning knob: BMO_LEAN=0 uses the general kernels everywhere
     const size_t tab_bytes = (size_t)V.n_prims * sizeof(bmo_prim) + (size_t)V.n_parts * (sizeof(bmo_part) + NBOUND * sizeof(double));
     // kernels compiled for lean unions + small meshes only; their tables live in shared memory next to 22 KB of per-thread
     // scratch (static), so the tables + part words have to fit in what is left of the 48 KB a block gets without opting in
-    lean = lean_ok && sys->all_lean && !sys->has_rare && staged && tab_bytes + (size_t)V.n_parts * 8 <= 24 * 1024;
+    lean = sys->all_lean && !sys->has_rare && staged && tab_bytes + (size_t)V.n_parts * 8 <= 24 * 1024;
     return staged ? tab_bytes + (lean ? (size_t)V.n_parts * 8 : 0) : 0;
+}
+
+// Calls f(STAGED, RK, LEAN) with the build of the trace kernels a call runs, as std::bool_constant arguments: staged tables,
+// the rare (cylindrical / aspheric) primitives compiled in, the LEAN build.  LEAN implies STAGED and !RK.
+template <class F> static void k1_config(bool staged, bool rk, bool lean, F&& f) {
+    using Y = std::true_type;
+    using N = std::false_type;
+    if (lean) f(Y{}, N{}, Y{});
+    else if (staged && rk) f(Y{}, Y{}, N{});
+    else if (staged) f(Y{}, N{}, N{});
+    else if (rk) f(N{}, Y{}, N{});
+    else f(N{}, N{}, N{});
 }
 
 // enqueue the next waves on this sub-batch's stream and the read-back of their totals
@@ -1890,88 +1868,37 @@ int32_t SubTrace::enqueue_chunk() {
         sp.S = sys->view; sp.cur = cur; sp.scr = scr; sp.hit = hit; sp.count = n_slots; sp.r_max = r_max; sp.keep = res->keep;
         sp.wave = wb; sp.B = beamtab(res); sp.blk_cnt = blk_cnt; sp.wave_totals = d_wtot + 2 * wave; sp.counters = ctx->d_counters;
         sp.rt = rt;
-        static const int minb_env = getenv("BMO_IMINB") ? atoi(getenv("BMO_IMINB")) : 0;
-        static const int minb = minb_env ? minb_env : 7;   // tuning knob: resident blocks per SM K1 is compiled for (C2: 4..8 measured, 7 = 72 registers is the fastest)
-        // tuning knob: 0 never fuse, 1 fuse in pipelined (launch-bound) calls [default], 2 always fuse.  Measured on C2:
-        // the fused kernel carries the interaction's registers through the march (0.282 vs 0.209 + 0.058 ms per
-        // wave), so it only pays where the number of launches is what limits the call.
-        static const int fuse_policy = getenv("BMO_FUSE") ? atoi(getenv("BMO_FUSE")) : 1;
-        const bool allow_fused = !rt.on && (fuse_policy == 2 || (fuse_policy == 1 && pipelined));
-        const bool rk = sys->has_rare;     // kernels compiled with the cylindrical / aspheric primitives
+        // Pipelined (launch-bound) calls run K1 and K2 fused, every wave of the chunk in one launch: the hit records stay in
+        // registers.  Measured on C2, the fused kernel carries the interaction's registers through the march (0.282 vs
+        // 0.209 + 0.058 ms per wave), so it only pays where the number of launches is what limits the call.  Pipelined calls
+        // have no beamsplitter, no retrace and no segment table.
+        const bool fused = pipelined && mode == 0;
+        const int nw = fused ? chunk - c : 1;   // waves of this launch
+        sp.n_waves = nw;
+        IntersectParams xp{};
+        xp.S = sys->view; xp.cur = cur; xp.hit = hit; xp.n_rays = n_slots * R; xp.r_max = r_max;
+        xp.counters = ctx->d_counters;
+        const unsigned grid = (unsigned)((n_slots * R + IBLOCK - 1) / IBLOCK);
         bool lean;
         const size_t smem = staged_smem(sys, staged, lean);
         BMO_CUDA(cudaEventRecord(ev[2 * c], st));
-        if (mode == 0 && !has_splitter && allow_fused) {
-            // sequential lens-stack path: intersect + interact in one kernel, hit records stay in registers; without a
-            // segment table to fill, all waves of this chunk run inside one launch (BMO_MULTIWAVE=0: one launch per wave)
-            static const bool multiwave = !(getenv("BMO_MULTIWAVE") && atoi(getenv("BMO_MULTIWAVE")) == 0);
-            const int nw = (multiwave && !res->keep) ? chunk - c : 1;
-            sp.n_waves = nw;
-            if (rk) {
-                if (!staged) fused_wave0<4, false, true><<<(unsigned)nblocks, IBLOCK, 0, st>>>(sp);
-                else fused_wave0<6, true, true><<<(unsigned)nblocks, IBLOCK, smem, st>>>(sp);
-            } else if (lean) {
-                static const int fminb = getenv("BMO_FMINB") ? atoi(getenv("BMO_FMINB")) : 6;   // tuning knob: resident blocks per SM of the fused lean kernel
-                if (fminb >= 8) fused_wave0<8, true, false, true><<<(unsigned)nblocks, IBLOCK, smem, st>>>(sp);
-                else if (fminb == 7) fused_wave0<7, true, false, true><<<(unsigned)nblocks, IBLOCK, smem, st>>>(sp);
-                else fused_wave0<6, true, false, true><<<(unsigned)nblocks, IBLOCK, smem, st>>>(sp);
-            } else {
-                if (!staged) fused_wave0<4, false, false><<<(unsigned)nblocks, IBLOCK, 0, st>>>(sp);
-                else if (minb <= 4) fused_wave0<4, true, false><<<(unsigned)nblocks, IBLOCK, smem, st>>>(sp);
-                else fused_wave0<6, true, false><<<(unsigned)nblocks, IBLOCK, smem, st>>>(sp);
-            }
-            BMO_LAUNCH(ctx, "fused_wave0");
-            BMO_CUDA(cudaEventRecord(ev[2 * c + 1], st));
+        k1_config(staged, sys->has_rare, lean, [&](auto S, auto K, auto L) {
+            if (fused) fused_wave0<S, K, L><<<(unsigned)nblocks, IBLOCK, smem, st>>>(sp);
+            // retrace call: K1r re-validates the stored path where there is one, ordinary tracing_step! elsewhere
+            else if (rt.on && mode == 0) retrace_intersect_wave<0, S, K, L><<<(unsigned)nblocks, Cfg<0>::BLOCK, smem, st>>>(sp);
+            else if (rt.on && mode == 1) retrace_intersect_wave<1, S, K, L><<<(unsigned)nblocks, Cfg<1>::BLOCK, smem, st>>>(sp);
+            else if (rt.on) retrace_intersect_wave<2, S, K, L><<<(unsigned)nblocks, Cfg<2>::BLOCK, smem, st>>>(sp);
+            else intersect_wave<S, K, L><<<grid, IBLOCK, smem, st>>>(xp);
+        });
+        BMO_LAUNCH(ctx, fused ? "fused_wave0" : rt.on ? "retrace_intersect_wave" : "intersect_wave");
+        BMO_CUDA(cudaEventRecord(ev[2 * c + 1], st));
+        if (fused) {
             for (int k = 1; k < nw; k++) {      // the waves folded into this launch: empty timing brackets, same bookkeeping
                 BMO_CUDA(cudaEventRecord(ev[2 * (c + k)], st));
                 BMO_CUDA(cudaEventRecord(ev[2 * (c + k) + 1], st));
             }
             wave += nw - 1; launched += nw - 1; c += nw - 1;
-        } else if (rt.on) {
-            // retrace call: K1r re-validates the stored path where there is one, ordinary tracing_step! elsewhere
-#define BMO_RETRACE_LAUNCH(M, RKV)                                                                                         \
-    do {                                                                                                                   \
-        if (lean) retrace_intersect_wave<M, true, false, true><<<(unsigned)nblocks, Cfg<M>::BLOCK, smem, st>>>(sp);        \
-        else if (staged) retrace_intersect_wave<M, true, RKV><<<(unsigned)nblocks, Cfg<M>::BLOCK, smem, st>>>(sp);         \
-        else retrace_intersect_wave<M, false, RKV><<<(unsigned)nblocks, Cfg<M>::BLOCK, 0, st>>>(sp);                       \
-    } while (0)
-            if (mode == 0) { if (rk) BMO_RETRACE_LAUNCH(0, true); else BMO_RETRACE_LAUNCH(0, false); }
-            else if (mode == 1) { if (rk) BMO_RETRACE_LAUNCH(1, true); else BMO_RETRACE_LAUNCH(1, false); }
-            else { if (rk) BMO_RETRACE_LAUNCH(2, true); else BMO_RETRACE_LAUNCH(2, false); }
-#undef BMO_RETRACE_LAUNCH
-            BMO_LAUNCH(ctx, "retrace_intersect_wave");
-            BMO_CUDA(cudaEventRecord(ev[2 * c + 1], st));
-            if (!has_splitter) {
-                if (mode == 0) interact_wave<0, true><<<(unsigned)nblocks, Cfg<0>::BLOCK, 0, st>>>(sp);
-                else if (mode == 1) interact_wave<1, true><<<(unsigned)nblocks, Cfg<1>::BLOCK, 0, st>>>(sp);
-                else interact_wave<2, true><<<(unsigned)nblocks, Cfg<2>::BLOCK, 0, st>>>(sp);
-            } else if (mode == 0) interact_wave<0><<<(unsigned)nblocks, Cfg<0>::BLOCK, 0, st>>>(sp);
-            else if (mode == 1) interact_wave<1><<<(unsigned)nblocks, Cfg<1>::BLOCK, 0, st>>>(sp);
-            else interact_wave<2><<<(unsigned)nblocks, Cfg<2>::BLOCK, 0, st>>>(sp);
-            BMO_LAUNCH(ctx, "interact_wave");
         } else {
-            IntersectParams xp{};
-            xp.S = sys->view; xp.cur = cur; xp.hit = hit; xp.n_rays = n_slots * R; xp.r_max = r_max;
-            xp.counters = ctx->d_counters;
-            const unsigned grid = (unsigned)((n_slots * R + IBLOCK - 1) / IBLOCK);
-            if (rk) {
-                if (!staged) intersect_wave<4, false, true><<<grid, IBLOCK, 0, st>>>(xp);
-                else intersect_wave<6, true, true><<<grid, IBLOCK, smem, st>>>(xp);
-            } else if (lean) {
-                // 8 blocks per SM (64 registers) is the fastest for the lean build (C2: 6 / 7 / 8 measured); BMO_IMINB=6 / 7 select the others
-                if (minb_env == 6) intersect_wave<6, true, false, true><<<grid, IBLOCK, smem, st>>>(xp);
-                else if (minb_env == 7) intersect_wave<7, true, false, true><<<grid, IBLOCK, smem, st>>>(xp);
-                else intersect_wave<8, true, false, true><<<grid, IBLOCK, smem, st>>>(xp);
-            } else {
-                if (!staged) intersect_wave<4, false, false><<<grid, IBLOCK, 0, st>>>(xp);
-                else if (minb <= 4) intersect_wave<4, true, false><<<grid, IBLOCK, smem, st>>>(xp);
-                else if (minb == 5) intersect_wave<5, true, false><<<grid, IBLOCK, smem, st>>>(xp);
-                else if (minb == 7) intersect_wave<7, true, false><<<grid, IBLOCK, smem, st>>>(xp);
-                else if (minb >= 8) intersect_wave<8, true, false><<<grid, IBLOCK, smem, st>>>(xp);
-                else intersect_wave<6, true, false><<<grid, IBLOCK, smem, st>>>(xp);
-            }
-            BMO_LAUNCH(ctx, "intersect_wave");
-            BMO_CUDA(cudaEventRecord(ev[2 * c + 1], st));
             if (!has_splitter) {
                 if (mode == 0) interact_wave<0, true><<<(unsigned)nblocks, Cfg<0>::BLOCK, 0, st>>>(sp);
                 else if (mode == 1) interact_wave<1, true><<<(unsigned)nblocks, Cfg<1>::BLOCK, 0, st>>>(sp);
@@ -2034,35 +1961,22 @@ int32_t SubTrace::finish_chunk() {
         const int64_t want = has_splitter ? 2 * alive * R : alive * R;
         if (next.cap < want) { free_queue(next, st); if ((rc = alloc_queue(next, want, nfq, NI_Q, st))) return rc; }
         BMO_CUDA(cudaEventRecord(evs0, st));
-        // one cooperative launch (BMO_COMPACT=0: the three-kernel version, also the fallback if the device refuses)
-        static const bool fused_ok = !(getenv("BMO_COMPACT") && atoi(getenv("BMO_COMPACT")) == 0);
-        static int coop_blocks = -1;   // blocks of compact_fused that are resident at once on this device
+        // one cooperative launch, as many blocks as are resident at once on this device
+        static int coop_blocks = -1;
         if (coop_blocks < 0) {
-            int per_sm = 0, sms = 0, coop = 0;
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, compact_fused, CBLOCK, 0);
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
-            cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device);
-            coop_blocks = coop ? per_sm * sms : 0;
+            int per_sm = 0, sms = 0;
+            BMO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, compact_fused, CBLOCK, 0));
+            BMO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
+            coop_blocks = std::max(1, per_sm * sms);
         }
-        bool done = false;
-        if (fused_ok && coop_blocks > 0) {
-            int64_t nb = std::min<int64_t>(coop_blocks, cblocks);
-            int64_t per = ((n_slots + nb - 1) / nb + CBLOCK - 1) / CBLOCK * CBLOCK;   // slots per block, whole rows
-            nb = (n_slots + per - 1) / per;
-            int R_ = R, nf_ = nfq;
-            int64_t ns_ = n_slots;
-            void* args[] = {&cur, &next, &ns_, &per, &R_, &nf_, &blk_cnt};
-            if (cudaLaunchCooperativeKernel((const void*)compact_fused, dim3((unsigned)nb), dim3(CBLOCK), args, 0, st) == cudaSuccess) done = true;
-            else cudaGetLastError();
-        }
-        if (!done) {
-            compact_count<<<(unsigned)cblocks, CBLOCK, 0, st>>>(cur.i, cur.cap, n_slots, R, blk_cnt);
-            BMO_LAUNCH(ctx, "compact_count");
-            scan_counts<<<1, 1024, 0, st>>>(blk_cnt, cblocks, 1, 1, blk_off, d_scan_tot);
-            BMO_LAUNCH(ctx, "scan_counts");
-            compact_scatter<<<(unsigned)cblocks, CBLOCK, 0, st>>>(cur, next, n_slots, R, nfq, blk_off);
-            BMO_LAUNCH(ctx, "compact_scatter");
-        } else BMO_LAUNCH(ctx, "compact_fused");
+        int64_t nb = std::min<int64_t>(coop_blocks, cblocks);
+        int64_t per = ((n_slots + nb - 1) / nb + CBLOCK - 1) / CBLOCK * CBLOCK;   // slots per block, whole rows
+        nb = (n_slots + per - 1) / per;
+        int R_ = R, nf_ = nfq;
+        int64_t ns_ = n_slots;
+        void* args[] = {&cur, &next, &ns_, &per, &R_, &nf_, &blk_cnt};
+        BMO_CUDA(cudaLaunchCooperativeKernel((const void*)compact_fused, dim3((unsigned)nb), dim3(CBLOCK), args, 0, st));
+        BMO_LAUNCH(ctx, "compact_fused");
         BMO_CUDA(cudaEventRecord(evs1, st));
         BMO_CUDA(cudaStreamSynchronize(st));
         float sms = 0;
@@ -2091,23 +2005,16 @@ void SubTrace::release() {
     ev.clear();
 }
 
-// The variant of solve_rays_persistent this process runs (tuning knob BMO_PMINB: resident blocks per SM it is compiled for, 4 - 8)
-static const void* persistent_kernel() {
-    static const int pminb = std::min(8, std::max(4, getenv("BMO_PMINB") ? atoi(getenv("BMO_PMINB")) : 6));
-    const void* fns[] = {(const void*)solve_rays_persistent<4>, (const void*)solve_rays_persistent<5>, (const void*)solve_rays_persistent<6>,
-                         (const void*)solve_rays_persistent<7>, (const void*)solve_rays_persistent<8>};
-    return fns[pminb - 4];
-}
-// Resident blocks per SM of persistent_kernel() with smem bytes of tables, 0 if a block would not fit the 48 KB of shared memory
-// it gets without opting in (static scratch + tables): such a call keeps the waves.  Cached per context.
+// Resident blocks per SM of solve_rays_persistent with smem bytes of tables, 0 if a block would not fit the 48 KB of shared
+// memory it gets without opting in (static scratch + tables): such a call keeps the waves.  Cached per context.
 static int32_t persistent_blocks(bmo_ctx* ctx, size_t smem, int* blocks) {
-    const void* fn = persistent_kernel();
-    if (ctx->persist_fn != fn || ctx->persist_smem != smem) {
+    if (ctx->persist_blocks < 0 || ctx->persist_smem != smem) {
         cudaFuncAttributes fa;
-        BMO_CUDA(cudaFuncGetAttributes(&fa, fn));
+        BMO_CUDA(cudaFuncGetAttributes(&fa, solve_rays_persistent));
         int b = 0;
-        if (fa.sharedSizeBytes + smem <= (size_t)48 * 1024) BMO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, fn, IBLOCK, smem));
-        ctx->persist_fn = fn; ctx->persist_smem = smem; ctx->persist_blocks = b;
+        if (fa.sharedSizeBytes + smem <= (size_t)48 * 1024)
+            BMO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, solve_rays_persistent, IBLOCK, smem));
+        ctx->persist_smem = smem; ctx->persist_blocks = b;
     }
     *blocks = ctx->persist_blocks;
     return BMO_OK;
@@ -2132,8 +2039,7 @@ static int32_t solve_persistent(bmo_sys* sys, const TraceInputs& in_h, int32_t r
     BMO_CUDA(cudaMemsetAsync(&ctx->d_counters->tiles, 0, 2 * sizeof(unsigned long long), st));   // tiles, most_nseg
     const int64_t grid = std::min<int64_t>((int64_t)blocks * ctx->sm_count, (n + IBLOCK - 1) / IBLOCK);
     BMO_CUDA(cudaEventRecord(ctx->evk0, st));
-    void* args[] = {&sp};
-    BMO_CUDA(cudaLaunchKernel(persistent_kernel(), dim3((unsigned)grid), dim3(IBLOCK), args, smem, st));
+    solve_rays_persistent<<<(unsigned)grid, IBLOCK, smem, st>>>(sp);
     BMO_LAUNCH(ctx, "solve_rays_persistent");
     BMO_CUDA(cudaEventRecord(ctx->evk1, st));
     BMO_CUDA(cudaMemcpyAsync(ctx->h_totals + 72, ctx->d_counters, sizeof(DevCounters), cudaMemcpyDeviceToHost, st));
@@ -2176,8 +2082,8 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
     const size_t table_bytes = (size_t)V.n_prims * sizeof(bmo_prim) + (size_t)V.n_parts * (sizeof(bmo_part) + NBOUND * sizeof(double));
     const bool staged = V.n_poses == 1 && table_bytes <= 40 * 1024;
 
-    // sub-batches (see SubTrace): only host inputs of splitter-free systems are pipelined
-    static const int max_sub = getenv("BMO_SUBBATCHES") ? std::min(8, std::max(1, atoi(getenv("BMO_SUBBATCHES")))) : 4;
+    // sub-batches (see SubTrace): only host inputs of splitter-free systems are pipelined, in up to 4 (6 and 8 measured slower)
+    constexpr int max_sub = 4;
     int n_sub = 1;
     if (!on_dev && !has_splitter && !res->keep) n_sub = (int)std::min<int64_t>(max_sub, std::max<int64_t>(1, n / (128 * 1024)));
     // Plain rays through a splitter-free LEAN system whose segments are not kept, in one stream: one launch solves them all

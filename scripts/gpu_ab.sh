@@ -1,4 +1,4 @@
-# A/B timing of library builds / tuning knobs on the C2 bench.  Usage: gpurun -- bash scripts/gpu_ab.sh TAG "ENV1=.. ENV2=..;ENV..." 
+# A/B timing on the C2 bench of library builds (BMO_LIB=path) and of the wave path (BMO_PERSIST=0).  Usage: bash scripts/gpu_ab.sh TAG "ENV1=.. ENV2=..;ENV..."
 TAG=${1:-ab}; SPECS=$2
 mkdir -p gpurun_out
 IFS=';' read -ra ARR <<< "$SPECS"
