@@ -18,6 +18,12 @@ UNIFORM_DIR = 8
 COMM_SYNC = 16
 COMM_ID_BYTES = 128
 SRC_DISC, SRC_COLLIMATED, SRC_POINT = 0, 1, 2     # bmo_source_kind
+SPOT_SLICE, SPOT_MAX_BLOCKS = 4096, 1024          # BMO_SPOT_PER
+
+
+def spot_per(m):
+    """BMO_SPOT_PER(m): entries per block of the spot reduction over m entries, 4096 * max(1, ceil(m / (4096 * 1024)))."""
+    return SPOT_SLICE * max(1, -(-int(m) // (SPOT_SLICE * SPOT_MAX_BLOCKS)))
 
 STATUS_NAMES = ["ACTIVE", "MISS", "ABSORBED", "RMAX", "SPLIT", "CLIPPED", "TORN", "ERROR"]
 
@@ -109,6 +115,7 @@ EXPORTS = [
     "bmo_debug_normals", "bmo_trim",
     "bmo_source_create", "bmo_source_device", "bmo_source_rays", "bmo_source_free", "bmo_spot_stats",
     "bmo_source_create_poses", "bmo_source_pose_ids", "bmo_spot_stats_poses",
+    "bmo_source_create_slice", "bmo_spot_stats_results", "bmo_spot_stats_sharded",
     "bmo_comm_unique_id", "bmo_comm_init", "bmo_comm_init_local", "bmo_comm_info", "bmo_pd_allreduce", "bmo_pd_allreduce_local", "bmo_comm_free",
 ]
 
@@ -172,6 +179,9 @@ def lib():
         L.bmo_pd_allreduce.argtypes = [_vp, _vp, C.c_int64, C.c_uint32]
         L.bmo_pd_allreduce_local.argtypes = [C.c_int32, C.POINTER(_vp), C.POINTER(_vp), C.c_int64, C.c_uint32]
         L.bmo_comm_free.argtypes = [_vp]
+        L.bmo_source_create_slice.argtypes = [_vp, C.POINTER(bmo_source_desc), C.c_int64, C.c_int64, C.POINTER(_vp)]
+        L.bmo_spot_stats_results.argtypes = [C.c_int32, C.POINTER(_vp), C.c_int32, _vp, C.c_int32, C.c_int32, C.POINTER(bmo_spot_info), _vp, C.c_uint32]
+        L.bmo_spot_stats_sharded.argtypes = [_vp, _vp, C.c_int32, _vp, C.c_int32, C.c_int32, C.POINTER(bmo_spot_info), _vp, C.c_uint32]
         _lib = L
     return _lib
 

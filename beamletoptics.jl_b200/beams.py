@@ -5,6 +5,7 @@ Single beams mirror the reference's objects (`Ray`, `Beam`, `GaussianBeamlet`); 
 `CollimatedSource` of a million rays is one bundle, not a million Python objects.
 Citations: /root/reference/src.
 """
+import copy
 import ctypes as C
 import math
 
@@ -262,10 +263,11 @@ def _expand_rings(rings, emit):
 class DeviceSource:
     """A source whose rays are generated on the GPU (bmo_source_create) from a descriptor: the basis, the ring table and
     every transcendental are computed here by the code that builds the host bundles.  One bmo_source is created per
-    (device, n_poses) on first use -- n_poses > 1 tiles the rays pose-major for a pose sweep (bmo_source_create_poses);
-    `pos` / `dir` download the untiled rays for inspection.  solve_system_ traces it from the device pointers, so no
-    per-ray data crosses the bus.  The handles belong to the per-process contexts of _lib.context, which live until the
-    process ends, so freeing them from __del__ never outlives the context."""
+    (device, n_poses, first, count) on first use -- n_poses > 1 tiles the rays pose-major for a pose sweep
+    (bmo_source_create_poses), a shard (`shard(first, count)`) holds the rays [first, first + count) of the source
+    (bmo_source_create_slice); `pos` / `dir` download the untiled rays for inspection.  solve_system_ traces it from the
+    device pointers, so no per-ray data crosses the bus.  The handles belong to the per-process contexts of _lib.context,
+    which live until the process ends, so freeing them from __del__ never outlives the context."""
 
     def __init__(self, kind, n, pos, dir, lam, rings=(), e1=(0.0, 0.0, 0.0), e2=(0.0, 0.0, 0.0), radius=0.0, phi0=0.0):
         from . import _lib as L
@@ -285,6 +287,7 @@ class DeviceSource:
         self._sig = bytes(desc) + bytes(memoryview(self._rings))[:len(rings) * C.sizeof(L.bmo_source_ring)] + np.float64(self.lam).tobytes()
         desc.rings = self._rings
         self.desc = desc
+        self.first = 0               # this source holds the rays [first, first + n) of the descriptor's desc.n_rays
         self._handles = {}
         self._host = None
         self.result = None
@@ -293,13 +296,32 @@ class DeviceSource:
 
     def signature(self): return self._sig
 
+    def shard(self, first, count):
+        """The rays [first, first + count) of this source as a DeviceSource of their own (bmo_source_create_slice): bit for
+        bit the same rays as those of the whole source, so that tracing the shards of a splitter-free system gives the
+        whole source's hits.  Offsets are relative to this source."""
+        first, count = int(first), int(count)
+        if first < 0 or count < 1 or first + count > self.n:
+            raise ValueError(f"shard [{first}, {first + count}) is not a non-empty part of the {self.n} rays")
+        s = copy.copy(self)
+        s.first, s.n = self.first + first, count
+        s._sig = self._sig + np.array([s.first, s.n], np.int64).tobytes()
+        s._handles, s._host, s.result = {}, None, None
+        s.__dict__.pop("_solution", None)
+        return s
+
     def handle(self, device=0, n_poses=1):
         """The bmo_source of this descriptor on `device`, tiled `n_poses` times (created on first use)."""
         from . import _lib as L
-        key = (int(device), int(n_poses))
+        key = (int(device), int(n_poses), self.first, self.n)
         if key not in self._handles:
             h = C.c_void_p()
-            L.check(L.lib().bmo_source_create_poses(L.context(device), C.byref(self.desc), key[1], C.byref(h)))
+            if (self.first, self.n) == (0, self.desc.n_rays):
+                L.check(L.lib().bmo_source_create_poses(L.context(device), C.byref(self.desc), key[1], C.byref(h)))
+            elif key[1] != 1:
+                raise ValueError("a shard of a source is traced with one pose")
+            else:
+                L.check(L.lib().bmo_source_create_slice(L.context(device), C.byref(self.desc), self.first, self.n, C.byref(h)))
             self._handles[key] = h
         return self._handles[key]
 
@@ -327,7 +349,7 @@ class DeviceSource:
 
     def _download(self):
         if self._host is None:
-            self._host = self.rays(next(iter(self._handles), (0, 1))[0])
+            self._host = self.rays(next(iter(self._handles), (0,))[0])
         return self._host
 
     @property

@@ -1,7 +1,11 @@
-// bmo_comm.cu -- the one exchange step of the path behind the C ABI: the Photodetector field of a beamlet bundle
-// that was sharded over several GPUs is the sum of the ranks' partial fields (the reference adds the beamlet
-// fields serially, `pd.field[i, j] += ...`, Photodetector.jl:103; its `for beam in beams(bg)` loop, System.jl:463-468,
-// is what gets sharded).  One complex128 all-reduce (2 n^2 doubles) over NVLink / NVSwitch through NCCL.
+// bmo_comm.cu -- the exchange steps of the path behind the C ABI.
+//   * The Photodetector field of a beamlet bundle that was sharded over several GPUs is the sum of the ranks' partial
+//     fields (the reference adds the beamlet fields serially, `pd.field[i, j] += ...`, Photodetector.jl:103; its
+//     `for beam in beams(bg)` loop, System.jl:463-468, is what gets sharded).  One complex128 all-reduce (2 n^2 doubles)
+//     over NVLink / NVSwitch through NCCL.
+//   * The spot diagram of a ray bundle sharded over several GPUs (bmo_spot_stats_sharded): every rank reduces its own
+//     Spotdetector entries to per-block partials (bmo_source.cu), the partials are all-gathered and combined in global block
+//     order on every rank, and the histograms are summed by one int64 all-reduce.  No spot leaves its GPU.
 //
 // NCCL is bound at run time (dlopen of libnccl.so.2) so that libbmo.so has no link-time dependency on it: a host
 // that never shards never needs the library, and inside a process that already carries one (PyTorch's bundled
@@ -27,10 +31,11 @@ typedef int (*fn_CommInitRank)(NcclComm*, int, NcclUniqueId, int);
 typedef int (*fn_CommInitAll)(NcclComm*, int, const int*);
 typedef int (*fn_CommDestroy)(NcclComm);
 typedef int (*fn_AllReduce)(const void*, void*, size_t, int /*dtype*/, int /*op*/, NcclComm, cudaStream_t);
+typedef int (*fn_AllGather)(const void*, void*, size_t, int /*dtype*/, NcclComm, cudaStream_t);
 typedef int (*fn_Group)(void);
 typedef const char* (*fn_ErrStr)(int);
 typedef int (*fn_GetVersion)(int*);
-constexpr int kNcclDouble = 8, kNcclSum = 0;
+constexpr int kNcclInt8 = 0, kNcclInt64 = 4, kNcclDouble = 8, kNcclSum = 0;
 
 struct Nccl {
     void* so = nullptr;
@@ -39,6 +44,7 @@ struct Nccl {
     fn_CommInitAll CommInitAll = nullptr;
     fn_CommDestroy CommDestroy = nullptr;
     fn_AllReduce AllReduce = nullptr;
+    fn_AllGather AllGather = nullptr;
     fn_Group GroupStart = nullptr, GroupEnd = nullptr;
     fn_ErrStr GetErrorString = nullptr;
     fn_GetVersion GetVersion = nullptr;
@@ -59,7 +65,7 @@ void load_nccl() {
     if (!g_nccl.so) return;
 #define SYM(field, name) g_nccl.field = (decltype(g_nccl.field))dlsym(g_nccl.so, name); if (!g_nccl.field) { g_nccl.why = std::string("symbol missing: ") + name; g_nccl.so = nullptr; return; }
     SYM(GetUniqueId, "ncclGetUniqueId") SYM(CommInitRank, "ncclCommInitRank") SYM(CommInitAll, "ncclCommInitAll")
-    SYM(CommDestroy, "ncclCommDestroy") SYM(AllReduce, "ncclAllReduce") SYM(GroupStart, "ncclGroupStart") SYM(GroupEnd, "ncclGroupEnd")
+    SYM(CommDestroy, "ncclCommDestroy") SYM(AllReduce, "ncclAllReduce") SYM(AllGather, "ncclAllGather") SYM(GroupStart, "ncclGroupStart") SYM(GroupEnd, "ncclGroupEnd")
     SYM(GetErrorString, "ncclGetErrorString") SYM(GetVersion, "ncclGetVersion")
 #undef SYM
 }
@@ -195,6 +201,85 @@ int32_t bmo_pd_allreduce_local(int32_t n, bmo_comm* const* comms, double* const*
         if (!on_dev || (flags & BMO_COMM_SYNC)) BMO_CUDA(cudaStreamSynchronize(comms[k]->ctx->stream));
     }
     return BMO_OK;
+}
+
+// the collective steps of bmo_spot_stats_sharded: NCCL on the context's stream; one rank needs no exchange
+struct NcclSpotExchange : SpotExchange {
+    bmo_comm* c;
+    explicit NcclSpotExchange(bmo_comm* comm) : c(comm) {}
+    int32_t gather(const void* mine, void* all, size_t bytes) override {
+        if (c->n_ranks == 1) { BMO_CUDA(cudaMemcpyAsync(all, mine, bytes, cudaMemcpyDeviceToDevice, c->ctx->stream)); return BMO_OK; }
+        BMO_NCCL(g_nccl.AllGather(mine, all, bytes, kNcclInt8, c->comm, c->ctx->stream));
+        return BMO_OK;
+    }
+    int32_t sum(int64_t* v, size_t n) override {
+        if (c->n_ranks > 1) BMO_NCCL(g_nccl.AllReduce(v, v, n, kNcclInt64, kNcclSum, c->comm, c->ctx->stream));
+        return BMO_OK;
+    }
+};
+
+int32_t bmo_spot_stats_sharded(bmo_comm* c, bmo_result* r, int32_t det_object, const double* window, int32_t nx, int32_t nz,
+                               bmo_spot_info* out, int64_t* counts, uint32_t flags) {
+    NvtxRange nvtx_("bmo_spot_stats_sharded");
+    const std::string fn = "bmo_spot_stats_sharded";
+    if (!c) return fail(BMO_EINVAL, fn + ": communicator NULL");
+    // Step 1: every rank's entry count, argument verdict and the arguments that must agree (detector, histogram shape,
+    // window), all-gathered, so that all ranks take the same branch below: a refusal on one rank is a refusal on every
+    // rank.  (Only arguments are agreed on: a CUDA or NCCL failure on one rank -- an allocation, a launch -- returns on
+    // that rank alone and leaves the others in the next collective, as with any NCCL collective.)
+    int32_t rc = BMO_OK;
+    if (!out) rc = fail(BMO_EINVAL, fn + ": NULL argument");
+    else if (r && r->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the result belongs to another context than the communicator");
+    if (!rc && r) rc = spot_check_result(fn, r, det_object);
+    if (!rc) rc = spot_check_args(fn, window, nx, nz, counts);
+    const std::string why = rc ? g_last_error : std::string();
+    const int W = c->n_ranks;
+    constexpr int K = 11;   // entries, verdict, then what must agree: det_object, histogram?, nx, nz, window?, window bits [4]
+    std::vector<int64_t> mine(K, 0), all((size_t)K * W);
+    mine[0] = r ? r->n_beams * r->R : 0; mine[1] = rc; mine[2] = det_object;
+    if (counts) { mine[3] = 1; mine[4] = nx; mine[5] = nz; }
+    if (window) { mine[6] = 1; std::memcpy(&mine[7], window, 4 * sizeof(double)); }
+    cudaStream_t st = c->ctx->stream;
+    BMO_CUDA(cudaSetDevice(c->ctx->device));
+    int64_t* d = nullptr;
+    BMO_CUDA(dev_alloc(&d, (size_t)K * (W + 1), st));
+    cudaError_t e = cudaMemcpyAsync(d, mine.data(), K * sizeof(int64_t), cudaMemcpyHostToDevice, st);
+    int nr = 0;
+    if (e == cudaSuccess) {
+        nr = W == 1 ? cudaMemcpyAsync(d + K, d, K * sizeof(int64_t), cudaMemcpyDeviceToDevice, st) != cudaSuccess
+                    : g_nccl.AllGather(d, d + K, K, kNcclInt64, c->comm, st);
+        if (!nr) e = cudaMemcpyAsync(all.data(), d + K, all.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
+        if (!nr && e == cudaSuccess) e = cudaStreamSynchronize(st);
+    }
+    dev_free(d, st);
+    if (e != cudaSuccess) return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e));
+    if (nr) return fail(BMO_ENCCL, fn + ": exchanging the arguments: " + (W == 1 ? std::string("copy failed") : std::string(g_nccl.GetErrorString(nr))));
+    for (int k = 0; k < W; k++) {
+        const int64_t* a = all.data() + (size_t)K * k;
+        if (a[1]) {      // the first refusal in rank order decides for every rank
+            if (k == c->rank) { g_last_error = why; return (int32_t)a[1]; }
+            return fail((int32_t)a[1], fn + ": rank " + std::to_string(k) + " refused its arguments");
+        }
+    }
+    std::vector<int64_t> entries((size_t)W);
+    int64_t N = 0;
+    for (int k = 0; k < W; k++) {
+        const int64_t* a = all.data() + (size_t)K * k;
+        if (!std::equal(a + 2, a + K, all.data() + 2))
+            return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " passes another detector, histogram shape or window than rank 0");
+        if (a[0] > INT64_MAX - N) return fail(BMO_EINVAL, fn + ": the ranks' entries overflow int64");
+        entries[k] = a[0];
+        N += a[0];
+    }
+    // Step 2: the global blocks must not cross a rank boundary
+    const int64_t per = spot_per(N);
+    for (int k = 0; k + 1 < W; k++)
+        if (entries[k] % per)
+            return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " holds " + std::to_string(entries[k]) + " entries, not a multiple of the " +
+                                        std::to_string(per) + " entries per block of " + std::to_string(N) + " (cut the shards with parallel.spot_shard_slice)");
+    // Steps 3-5: the two passes and the histogram (bmo_source.cu)
+    NcclSpotExchange x(c);
+    return spot_stats_shard(fn, c->ctx, r, det_object, window, nx, nz, entries, per, x, out, counts, flags);
 }
 
 int32_t bmo_comm_free(bmo_comm* c) {

@@ -274,4 +274,22 @@ template <class T> inline void dev_free(T*& p, cudaStream_t s) {
     p = nullptr;
 }
 
+// ---- spot statistics (bmo_source.cu), shared with bmo_spot_stats_sharded (bmo_comm.cu) ---------------------------
+// entries per block of a reduction over m spot entries: 4096 * max(1, ceil(m / (4096 * 1024))), the partition include/bmo.h fixes
+inline int64_t spot_per(int64_t m) { return BMO_SPOT_PER(m); }
+// bmo_spot_stats's argument checks: on the result (non-NULL, det_object a Spotdetector of its system), on the rest
+int32_t spot_check_result(const std::string& fn, const bmo_result* r, int32_t det_object);
+int32_t spot_check_args(const std::string& fn, const double* window, int32_t nx, int32_t nz, const void* counts);
+// the collective steps of bmo_spot_stats_sharded, on the context's stream
+struct SpotExchange {
+    virtual int32_t gather(const void* mine, void* all, size_t bytes) = 0;   // all[r * bytes ...] = rank r's `bytes` bytes
+    virtual int32_t sum(int64_t* v, size_t n) = 0;                            // v = the sum of every rank's v, in place
+    virtual ~SpotExchange() = default;
+};
+// this rank's part of bmo_spot_stats_sharded once the ranks agree on their arguments: entries[k] = entries of rank k, each a
+// multiple of `per` except the last rank's; r may be NULL on a rank without entries
+int32_t spot_stats_shard(const std::string& fn, bmo_ctx* ctx, bmo_result* r, int32_t det_object, const double* window, int32_t nx,
+                         int32_t nz, const std::vector<int64_t>& entries, int64_t per, SpotExchange& x, bmo_spot_info* out,
+                         int64_t* counts, uint32_t flags);
+
 }  // namespace bmo

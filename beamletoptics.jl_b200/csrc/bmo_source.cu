@@ -10,6 +10,8 @@
 // Pose-tiled sources (bmo_source_create_poses): n_poses copies of the rays, pose-major, with pose_id[i] = i / n_rays.  A
 // disc thread computes ray i mod n_rays with the untiled arithmetic (rho over n_rays), ring sources run the recurrence
 // once and source_tile replicates tile 0, so every tile is bit-identical to the untiled source.
+// Source slices (bmo_source_create_slice): rays [first, first + count) of the one-pose source.  A disc thread computes ray
+// first + i; a ring that overlaps the slice runs its recurrence from its own start and writes the rays inside the slice.
 // Spot statistics (bmo_spot_stats): two passes over a fixed partition of the spot entries (spot_sums: counts, sums,
 // extrema and the histogram; spot_spread: the squared distances to the centroid).  Each block reduces its slice in a
 // fixed order and the last block to finish combines the per-block partials in block order, so the result does not depend
@@ -18,6 +20,12 @@
 // by pose (cub radix sort on the pose id, skipped when the result is already pose-major), each pose's entry list is cut
 // with bmo_spot_stats's slice formula applied to that pose's entry count, and each pose has its own completion counters:
 // a pose reduces the same values in the same order as a one-pose result that lists its entries in the same order.
+// Several results (bmo_spot_stats_results): the same two kernels over the concatenation of the results' entries, cut by
+// the slice formula on the total; a table of (spot arrays, first concatenated entry) per result tells each thread where
+// an entry lives, so a block may straddle two results and still reduce what one result listing the same entries gives.
+// Several ranks (bmo_spot_stats_sharded, collective steps in bmo_comm.cu): each rank runs both passes over its own entries
+// without the last-block combine; the partials of all ranks are all-gathered and spot_combine runs the same combine loop
+// over them in global block order on every rank.
 // Compiled with -fmad=false; the arithmetic that must match the host bit for bit is spelled with __dmul_rn / __dadd_rn.
 #include <cmath>
 #include <cub/device/device_radix_sort.cuh>
@@ -26,8 +34,9 @@
 namespace bmo {
 
 struct SrcParams {
-    int64_t n, n_rings;             // rays of one tile, rings
-    int64_t total;                  // n * n_poses
+    int64_t n, n_rings;             // rays of the descriptor, rings
+    int64_t first, count;           // the rays [first, first + count) of the descriptor that one tile holds
+    int64_t total;                  // count * n_poses
     int32_t kind;
     double p[3], d[3], e1[3], e2[3], radius, phi0;
     const bmo_source_ring* rings;
@@ -47,19 +56,25 @@ __global__ void source_rings(SrcParams P) {
     if (t > P.n_rings) return;
     const bool point = P.kind == BMO_SRC_POINT;
     if (t == 0) {   // ray 0: the centre (collimated) or the axis (point); a collimated direction is stored once
-        for (int i = 0; i < 3; i++) { P.pos[i] = P.p[i]; P.dir[i] = P.d[i]; }
+        if (!point) for (int i = 0; i < 3; i++) P.dir[i] = P.d[i];
+        if (P.first == 0) for (int i = 0; i < 3; i++) { P.pos[i] = P.p[i]; P.dir[i] = P.d[i]; }
         return;
     }
+    // ray k of the descriptor is stored at k - first; the recurrence starts at the ring's first ray whatever the slice
     const bmo_source_ring g = P.rings[t - 1];
+    const int64_t stop = min(g.first + g.count, P.first + P.count);
+    if (stop <= P.first) return;
     double v[3] = {g.start[0], g.start[1], g.start[2]};
     const double* a = g.rot;
-    for (int64_t j = 0; j < g.count; j++) {
-        double* q = P.pos + 3 * (g.first + j);
-        if (point) {
-            q[0] = P.p[0]; q[1] = P.p[1]; q[2] = P.p[2];
-            renormalise(v, P.dir + 3 * (g.first + j));
-        } else {
-            for (int i = 0; i < 3; i++) q[i] = __dadd_rn(P.p[i], v[i]);
+    for (int64_t k = g.first; k < stop; k++) {
+        if (k >= P.first) {
+            double* q = P.pos + 3 * (k - P.first);
+            if (point) {
+                q[0] = P.p[0]; q[1] = P.p[1]; q[2] = P.p[2];
+                renormalise(v, P.dir + 3 * (k - P.first));
+            } else {
+                for (int i = 0; i < 3; i++) q[i] = __dadd_rn(P.p[i], v[i]);
+            }
         }
         double w[3];
         for (int i = 0; i < 3; i++)
@@ -68,13 +83,13 @@ __global__ void source_rings(SrcParams P) {
     }
 }
 
-// one thread per tiled ray t: ray k = t mod n of the descriptor (rho over the n rays of one tile)
+// one thread per stored ray t: ray k = first + t mod count of the descriptor (rho over its n rays)
 __global__ void source_disc(SrcParams P) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= P.total) return;
     if (t == 0) for (int i = 0; i < 3; i++) P.dir[i] = P.d[i];
-    const int64_t k = t % P.n;
-    if (P.pose_id) P.pose_id[t] = (int32_t)(t / P.n);
+    const int64_t k = P.first + t % P.count;
+    if (P.pose_id) P.pose_id[t] = (int32_t)(t / P.count);
     const double kd = (double)k;
     const double rho = __dsqrt_rn(__ddiv_rn(__dadd_rn(kd, 0.5), (double)P.n));
     const double phi = __dmul_rn(kd, P.phi0);
@@ -99,12 +114,16 @@ __global__ void source_tile(SrcParams P, int uniform) {
 
 // ---- spot statistics ------------------------------------------------------------------------------------------
 constexpr int SPOT_BLOCK = 256;
-constexpr int64_t SPOT_SLICE = 4096;     // entries per block (times a factor that keeps the grid at <= 1024 blocks)
 
 struct SpotPartial { unsigned long long hits, outside; double sx, sz, maxr, lo[2], hi[2], ssq; };
 
+// one result of a reduction over several: its spot arrays and the position of its entry 0 in the concatenated entries
+struct SpotRes { const int32_t* obj; const double* xz; int64_t first; };
+
 struct SpotParams {
-    const int32_t* obj; const double* xz;
+    const int32_t* obj; const double* xz;   // the one result (res == NULL)
+    const SpotRes* res;             // NULL, or [n_res + 1]: several results in list order; res[n_res].first = n
+    int32_t n_res;
     int64_t n, per;                 // one pose (pstart == NULL): entries, entries per block
     int32_t det, has_window, nx, nz;
     double win[4];
@@ -116,7 +135,8 @@ struct SpotParams {
     const int32_t* pblk;            // [n_poses + 1]: first block of each pose
     unsigned long long* counts;     // NULL: no histogram; else [n_poses][nz][nx]
     SpotPartial* part;              // [gridDim.x]
-    unsigned int* done;             // [n_poses][2] blocks of the pose finished with spot_sums / spot_spread
+    unsigned int* done;             // [n_poses][2] blocks of the pose finished with spot_sums / spot_spread; NULL: no
+                                    // combine (bmo_spot_stats_sharded combines the partials of every rank in spot_combine)
     bmo_spot_info* out;             // device, [n_poses]
 };
 
@@ -143,6 +163,31 @@ __device__ SpotSlice spot_slice(const SpotParams& P) {
 // entry index at position q of the ordered entry list (the R entries of a beam stay together, in entry order)
 __device__ __forceinline__ int64_t spot_entry(const SpotParams& P, int64_t q) {
     return P.order ? (int64_t)P.order[q / P.R] * P.R + q % P.R : q;
+}
+// several results: the one that holds position q of the concatenated entries (the last r with res[r].first <= q)
+__device__ int32_t spot_res_of(const SpotParams& P, int64_t q) {
+    int32_t lo = 0, hi = P.n_res;
+    while (hi - lo > 1) {
+        const int32_t mid = (lo + hi) / 2;
+        if (P.res[mid].first <= q) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+// the entry at position q: true with its (x, z) if it lies on the detector.  r is the thread's result cursor (several
+// results): a thread visits increasing q, so the cursor only moves forward.
+__device__ __forceinline__ bool spot_at(const SpotParams& P, int64_t q, int32_t& r, double& x, double& z) {
+    const int32_t* obj = P.obj;
+    const double* xz = P.xz;
+    int64_t k;
+    if (P.res) {
+        while (q >= P.res[r + 1].first) r++;
+        obj = P.res[r].obj; xz = P.res[r].xz; k = q - P.res[r].first;
+    } else {
+        k = spot_entry(P, q);
+    }
+    if (obj[k] != P.det) return false;
+    x = xz[2 * k]; z = xz[2 * k + 1];
+    return true;
 }
 
 // fixed-shape tree over the block's threads
@@ -173,6 +218,30 @@ __device__ bool last_block(unsigned int* done, int32_t nblk) {
     return last;
 }
 
+// the partials combined in block order: the loop the last block of spot_sums runs, and spot_combine over every rank's
+struct SpotAcc {
+    unsigned long long H = 0, O = 0;
+    double SX = 0, SZ = 0, M = -INFINITY, L0 = INFINITY, L1 = INFINITY, U0 = -INFINITY, U1 = -INFINITY;
+    template <class Part> __device__ void add(Part& p) {   // volatile in the last block, plain in spot_combine
+        H += p.hits; O += p.outside;
+        SX = __dadd_rn(SX, p.sx); SZ = __dadd_rn(SZ, p.sz);
+        M = fmax(M, p.maxr);
+        L0 = fmin(L0, p.lo[0]); L1 = fmin(L1, p.lo[1]); U0 = fmax(U0, p.hi[0]); U1 = fmax(U1, p.hi[1]);
+    }
+    __device__ bmo_spot_info info() const {
+        bmo_spot_info o;
+        o.hits = (int64_t)H; o.outside = (int64_t)O;
+        const double nan = __longlong_as_double(0x7ff8000000000000ll);
+        if (H == 0) {
+            o.centroid[0] = o.centroid[1] = o.rms = o.max_r = o.lo[0] = o.lo[1] = o.hi[0] = o.hi[1] = nan;
+        } else {
+            o.centroid[0] = __ddiv_rn(SX, (double)H); o.centroid[1] = __ddiv_rn(SZ, (double)H);
+            o.rms = nan; o.max_r = M; o.lo[0] = L0; o.lo[1] = L1; o.hi[0] = U0; o.hi[1] = U1;
+        }
+        return o;
+    }
+};
+
 __global__ void __launch_bounds__(SPOT_BLOCK) spot_sums(SpotParams P) {
     __shared__ double shd[SPOT_BLOCK];
     __shared__ unsigned long long shu[SPOT_BLOCK];
@@ -180,10 +249,10 @@ __global__ void __launch_bounds__(SPOT_BLOCK) spot_sums(SpotParams P) {
     unsigned long long* counts = P.counts ? P.counts + (size_t)sl.pose * P.nx * P.nz : nullptr;
     unsigned long long hits = 0, outside = 0;
     double sx = 0, sz = 0, maxr = -INFINITY, lox = INFINITY, loz = INFINITY, hix = -INFINITY, hiz = -INFINITY;
+    int32_t cur = P.res ? spot_res_of(P, sl.b0 + threadIdx.x) : 0;
     for (int64_t q = sl.b0 + threadIdx.x; q < sl.b1; q += SPOT_BLOCK) {
-        const int64_t k = spot_entry(P, q);
-        if (P.obj[k] != P.det) continue;
-        const double x = P.xz[2 * k], z = P.xz[2 * k + 1];
+        double x, z;
+        if (!spot_at(P, q, cur, x, z)) continue;
         hits++;
         sx = __dadd_rn(sx, x); sz = __dadd_rn(sz, z);
         maxr = fmax(maxr, __dsqrt_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(z, z))));
@@ -210,27 +279,12 @@ __global__ void __launch_bounds__(SPOT_BLOCK) spot_sums(SpotParams P) {
     r.hi[1] = block_reduce(hiz, shd, MaxD());
     r.ssq = 0;
     if (threadIdx.x == 0) P.part[blockIdx.x] = r;
-    if (!last_block(P.done + 2 * sl.pose, sl.nblk) || threadIdx.x != 0) return;
+    if (!P.done || !last_block(P.done + 2 * sl.pose, sl.nblk) || threadIdx.x != 0) return;
     // combine the pose's partials in block order
     const volatile SpotPartial* vp = P.part;
-    unsigned long long H = 0, O = 0;
-    double SX = 0, SZ = 0, M = -INFINITY, L0 = INFINITY, L1 = INFINITY, U0 = -INFINITY, U1 = -INFINITY;
-    for (int32_t b = sl.first; b < sl.first + sl.nblk; b++) {
-        H += vp[b].hits; O += vp[b].outside;
-        SX = __dadd_rn(SX, vp[b].sx); SZ = __dadd_rn(SZ, vp[b].sz);
-        M = fmax(M, vp[b].maxr);
-        L0 = fmin(L0, vp[b].lo[0]); L1 = fmin(L1, vp[b].lo[1]); U0 = fmax(U0, vp[b].hi[0]); U1 = fmax(U1, vp[b].hi[1]);
-    }
-    bmo_spot_info o;
-    o.hits = (int64_t)H; o.outside = (int64_t)O;
-    const double nan = __longlong_as_double(0x7ff8000000000000ll);
-    if (H == 0) {
-        o.centroid[0] = o.centroid[1] = o.rms = o.max_r = o.lo[0] = o.lo[1] = o.hi[0] = o.hi[1] = nan;
-    } else {
-        o.centroid[0] = __ddiv_rn(SX, (double)H); o.centroid[1] = __ddiv_rn(SZ, (double)H);
-        o.rms = nan; o.max_r = M; o.lo[0] = L0; o.lo[1] = L1; o.hi[0] = U0; o.hi[1] = U1;
-    }
-    P.out[sl.pose] = o;
+    SpotAcc a;
+    for (int32_t b = sl.first; b < sl.first + sl.nblk; b++) a.add(vp[b]);
+    P.out[sl.pose] = a.info();
 }
 
 __global__ void __launch_bounds__(SPOT_BLOCK) spot_spread(SpotParams P) {
@@ -240,18 +294,46 @@ __global__ void __launch_bounds__(SPOT_BLOCK) spot_spread(SpotParams P) {
     if (out->hits == 0) return;   // every block of the pose sees the same count: nothing to do, rms stays NaN
     const double cx = out->centroid[0], cz = out->centroid[1];
     double s = 0;
+    int32_t cur = P.res ? spot_res_of(P, sl.b0 + threadIdx.x) : 0;
     for (int64_t q = sl.b0 + threadIdx.x; q < sl.b1; q += SPOT_BLOCK) {
-        const int64_t k = spot_entry(P, q);
-        if (P.obj[k] != P.det) continue;
-        const double dx = __dsub_rn(P.xz[2 * k], cx), dz = __dsub_rn(P.xz[2 * k + 1], cz);
+        double x, z;
+        if (!spot_at(P, q, cur, x, z)) continue;
+        const double dx = __dsub_rn(x, cx), dz = __dsub_rn(z, cz);
         s = __dadd_rn(s, __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dz, dz)));
     }
     s = block_reduce(s, shd, AddD());
     if (threadIdx.x == 0) P.part[blockIdx.x].ssq = s;
-    if (!last_block(P.done + 2 * sl.pose + 1, sl.nblk) || threadIdx.x != 0) return;
+    if (!P.done || !last_block(P.done + 2 * sl.pose + 1, sl.nblk) || threadIdx.x != 0) return;
     const volatile SpotPartial* vp = P.part;
     double S = 0;
     for (int32_t b = sl.first; b < sl.first + sl.nblk; b++) S = __dadd_rn(S, vp[b].ssq);
+    out->rms = __dsqrt_rn(__ddiv_rn(S, (double)out->hits));
+}
+
+// bmo_spot_stats_sharded: the all-gathered partials of every rank, all[k * stride + b] for rank k's blocks b < ceil(entries[k] /
+// per), combined in global block order -- the combine loop of spot_sums (pass 0) or spot_spread (pass 1), on one thread
+// (a kernel of its own after the all-gather: plain loads, which the compiler may issue ahead of the serial sums)
+__global__ void spot_combine(const SpotPartial* __restrict__ all, int32_t n_ranks, int32_t stride, const int64_t* entries, int64_t per,
+                             int32_t pass, bmo_spot_info* out) {
+    if (pass == 0) {
+        SpotAcc a;
+        for (int32_t k = 0; k < n_ranks; k++) {
+            const SpotPartial* p = all + (int64_t)k * stride;
+            const int64_t nb = (entries[k] + per - 1) / per;
+#pragma unroll 8
+            for (int64_t b = 0; b < nb; b++) a.add(p[b]);
+        }
+        *out = a.info();
+        return;
+    }
+    if (out->hits == 0) return;
+    double S = 0;
+    for (int32_t k = 0; k < n_ranks; k++) {
+        const SpotPartial* p = all + (int64_t)k * stride;
+        const int64_t nb = (entries[k] + per - 1) / per;
+#pragma unroll 8
+        for (int64_t b = 0; b < nb; b++) S = __dadd_rn(S, p[b].ssq);
+    }
     out->rms = __dsqrt_rn(__ddiv_rn(S, (double)out->hits));
 }
 
@@ -348,20 +430,17 @@ int32_t bmo_source_free(bmo_source* s) {
     return BMO_OK;
 }
 
-int32_t bmo_source_create_poses(bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, bmo_source** out) {
-    NvtxRange nvtx_("bmo_source_create");
-    if (!ctx || !desc || !out) return fail(BMO_EINVAL, "bmo_source_create: NULL argument");
-    if (n_poses < 1) return fail(BMO_EINVAL, "bmo_source_create_poses: n_poses must be >= 1");
-    int32_t rc;
-    if ((rc = check_desc(desc))) return rc;
-    if (desc->n_rays > INT64_MAX / n_poses) return fail(BMO_EINVAL, "bmo_source_create_poses: n_rays * n_poses overflows int64");
+// n_poses copies of the rays [first, first + count) of the descriptor (n_poses > 1 only for the whole source)
+static int32_t source_create(const char* what, bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, int64_t first, int64_t count,
+                             bmo_source** out) {
+    const std::string fn(what);
     BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     bmo_source* s = new bmo_source();
-    s->ctx = ctx; s->n_rays = desc->n_rays; s->n_poses = n_poses; s->n = desc->n_rays * n_poses; s->uniform = desc->kind != BMO_SRC_POINT;
+    s->ctx = ctx; s->n_rays = desc->n_rays; s->n_poses = n_poses; s->n = count * n_poses; s->uniform = desc->kind != BMO_SRC_POINT;
     const int64_t n = s->n;
     SrcParams P{};
-    P.n = desc->n_rays; P.total = n; P.n_rings = desc->n_rings; P.kind = desc->kind;
+    P.n = desc->n_rays; P.first = first; P.count = count; P.total = n; P.n_rings = desc->n_rings; P.kind = desc->kind;
     for (int i = 0; i < 3; i++) { P.p[i] = desc->pos[i]; P.d[i] = desc->dir[i]; P.e1[i] = desc->e1[i]; P.e2[i] = desc->e2[i]; }
     P.radius = desc->radius; P.phi0 = desc->phi0;
     bmo_source_ring* d_rings = nullptr;
@@ -375,9 +454,10 @@ int32_t bmo_source_create_poses(bmo_ctx* ctx, const bmo_source_desc* desc, int32
     if (e != cudaSuccess) {
         dev_free(d_rings, st);
         bmo_source_free(s);
-        return fail(BMO_ECUDA, std::string("bmo_source_create: ") + cudaGetErrorString(e));
+        return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e));
     }
     P.rings = d_rings; P.pos = s->pos; P.dir = s->dir; P.pose_id = s->pose_id;
+    int32_t rc;
     if (desc->kind == BMO_SRC_DISC) {
         source_disc<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P);
         rc = launched(ctx, "source_disc");
@@ -396,8 +476,29 @@ int32_t bmo_source_create_poses(bmo_ctx* ctx, const bmo_source_desc* desc, int32
     return BMO_OK;
 }
 
+int32_t bmo_source_create_poses(bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, bmo_source** out) {
+    NvtxRange nvtx_("bmo_source_create");
+    if (!ctx || !desc || !out) return fail(BMO_EINVAL, "bmo_source_create: NULL argument");
+    if (n_poses < 1) return fail(BMO_EINVAL, "bmo_source_create_poses: n_poses must be >= 1");
+    int32_t rc;
+    if ((rc = check_desc(desc))) return rc;
+    if (desc->n_rays > INT64_MAX / n_poses) return fail(BMO_EINVAL, "bmo_source_create_poses: n_rays * n_poses overflows int64");
+    return source_create("bmo_source_create", ctx, desc, n_poses, 0, desc->n_rays, out);
+}
+
 int32_t bmo_source_create(bmo_ctx* ctx, const bmo_source_desc* desc, bmo_source** out) {
     return bmo_source_create_poses(ctx, desc, 1, out);
+}
+
+int32_t bmo_source_create_slice(bmo_ctx* ctx, const bmo_source_desc* desc, int64_t first, int64_t count, bmo_source** out) {
+    NvtxRange nvtx_("bmo_source_create_slice");
+    if (!ctx || !desc || !out) return fail(BMO_EINVAL, "bmo_source_create_slice: NULL argument");
+    int32_t rc;
+    if ((rc = check_desc(desc))) return rc;
+    if (first < 0 || count < 1 || first > desc->n_rays - count)
+        return fail(BMO_EINVAL, "bmo_source_create_slice: rays [" + std::to_string(first) + ", " + std::to_string(first) + " + " +
+                                    std::to_string(count) + ") are not a non-empty part of the source's " + std::to_string(desc->n_rays));
+    return source_create("bmo_source_create_slice", ctx, desc, 1, first, count, out);
 }
 
 int32_t bmo_source_pose_ids(bmo_source* s, int32_t* n_poses, const int32_t** pose_id) {
@@ -429,13 +530,14 @@ int32_t bmo_source_rays(bmo_source* s, double* pos, double* dir) {
     return BMO_OK;
 }
 
-// bmo_spot_stats (n_poses = 1: every entry, index order) and bmo_spot_stats_poses (n_poses = the result's pose count)
-static int32_t spot_stats(const char* what, bmo_result* r, int32_t det_object, int32_t n_poses, const double* window, int32_t nx,
-                          int32_t nz, bmo_spot_info* out, int64_t* counts, uint32_t flags) {
-    const std::string fn(what);
-    if (!r || !out) return fail(BMO_EINVAL, fn + ": NULL argument");
+int32_t bmo::spot_check_result(const std::string& fn, const bmo_result* r, int32_t det_object) {
+    if (!r) return fail(BMO_EINVAL, fn + ": NULL argument");
     if (det_object < 0 || det_object >= (int32_t)r->object_kind.size() || r->object_kind[det_object] != BMO_OBJ_SPOTDETECTOR)
         return fail(BMO_EINVAL, fn + ": object " + std::to_string(det_object) + " is not a Spotdetector of the result's system");
+    return BMO_OK;
+}
+
+int32_t bmo::spot_check_args(const std::string& fn, const double* window, int32_t nx, int32_t nz, const void* counts) {
     if (window) {
         for (int i = 0; i < 4; i++)
             if (!std::isfinite(window[i])) return fail(BMO_EINVAL, fn + ": window not finite");
@@ -445,11 +547,33 @@ static int32_t spot_stats(const char* what, bmo_result* r, int32_t det_object, i
         if (!window) return fail(BMO_EINVAL, fn + ": a histogram needs a window");
         if (nx < 1 || nz < 1) return fail(BMO_EINVAL, fn + ": nx and nz must be >= 1");
     }
+    return BMO_OK;
+}
+
+// bmo_spot_stats (one result, n_poses = 1: every entry, index order), bmo_spot_stats_poses (one result, n_poses = its pose
+// count) and bmo_spot_stats_results (several results, n_poses = 1: their entries concatenated in list order)
+static int32_t spot_stats(const char* what, int32_t n_res, bmo_result* const* rs, int32_t det_object, int32_t n_poses, const double* window,
+                          int32_t nx, int32_t nz, bmo_spot_info* out, int64_t* counts, uint32_t flags) {
+    const std::string fn(what);
+    if (!out) return fail(BMO_EINVAL, fn + ": NULL argument");
+    int32_t rc;
+    for (int32_t k = 0; k < n_res; k++) {
+        if ((rc = spot_check_result(fn, rs[k], det_object))) return rc;
+        if (rs[k]->ctx != rs[0]->ctx) return fail(BMO_EINVAL, fn + ": result " + std::to_string(k) + " belongs to another context than result 0");
+    }
+    if ((rc = spot_check_args(fn, window, nx, nz, counts))) return rc;
+    bmo_result* r = rs[0];
     bmo_ctx* ctx = r->ctx;
     BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const int64_t n = r->n_beams * r->R;
-    const auto slice = [](int64_t m) { return SPOT_SLICE * std::max<int64_t>(1, (m + SPOT_SLICE * 1024 - 1) / (SPOT_SLICE * 1024)); };
+    // several results: the table of their spot arrays and first concatenated entries, closed by the total
+    std::vector<SpotRes> rtab;
+    int64_t n = 0;
+    for (int32_t k = 0; k < n_res; k++) {
+        if (n_res > 1) rtab.push_back({rs[k]->spot_obj, rs[k]->spot_xz, n});
+        n += rs[k]->n_beams * rs[k]->R;
+    }
+    if (n_res > 1) rtab.push_back({nullptr, nullptr, n});
     const size_t np = (size_t)n_poses;
     const size_t bins = counts ? (size_t)nx * (size_t)nz : 0;
     const bool dev_counts = counts && (flags & BMO_INPUT_DEVICE);
@@ -463,9 +587,9 @@ static int32_t spot_stats(const char* what, bmo_result* r, int32_t det_object, i
     int64_t nblk = 0;
     int32_t* order = nullptr;
     cudaError_t e = cudaSuccess;
-    int32_t rc = BMO_OK;
+    rc = BMO_OK;
     if (n_poses == 1) {
-        P.per = slice(n);
+        P.per = spot_per(n);
         nblk = std::max<int64_t>(1, (n + P.per - 1) / P.per);
     } else {
         const int64_t nb = r->n_beams;
@@ -514,7 +638,7 @@ static int32_t spot_stats(const char* what, bmo_result* r, int32_t det_object, i
         int32_t* pblk = (int32_t*)(tab.data() + 2 * np + 1);
         for (size_t p = 0; p < np; p++) {
             const int64_t m = (int64_t)h[p] * r->R;
-            const int64_t per = slice(m);
+            const int64_t per = spot_per(m);
             tab[p + 1] = tab[p] + m;
             tab[np + 1 + p] = per;
             pblk[p] = (int32_t)nblk;
@@ -524,11 +648,12 @@ static int32_t spot_stats(const char* what, bmo_result* r, int32_t det_object, i
         if (nblk > INT32_MAX) { dev_free(order, st); return fail(BMO_EINVAL, fn + ": too many blocks"); }
     }
     // one scratch block: partials, two completion counters per pose, the statistics, the histogram of a host `counts`, the
-    // per-pose slice table
+    // per-pose slice table, the result table
     const size_t off_done = (size_t)nblk * sizeof(SpotPartial), done_bytes = (8 * np + 15) / 16 * 16;
     const size_t off_out = off_done + done_bytes, off_hist = off_out + np * sizeof(bmo_spot_info);
     const size_t off_tab = off_hist + (counts && !dev_counts ? np * bins * sizeof(int64_t) : 0);
-    const size_t bytes = off_tab + tab.size() * sizeof(int64_t);
+    const size_t off_res = off_tab + tab.size() * sizeof(int64_t);
+    const size_t bytes = off_res + rtab.size() * sizeof(SpotRes);
     char* scr = nullptr;
     e = dev_alloc(&scr, bytes, st);
     if (e != cudaSuccess) { dev_free(order, st); return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e)); }
@@ -538,6 +663,10 @@ static int32_t spot_stats(const char* what, bmo_result* r, int32_t det_object, i
     if (!tab.empty()) {
         P.pstart = (const int64_t*)(scr + off_tab); P.pper = P.pstart + np + 1; P.pblk = (const int32_t*)(P.pper + np);
         e = cudaMemcpyAsync(scr + off_tab, tab.data(), tab.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st);
+    }
+    if (!rtab.empty()) {
+        P.res = (const SpotRes*)(scr + off_res); P.n_res = n_res;
+        if (e == cudaSuccess) e = cudaMemcpyAsync(scr + off_res, rtab.data(), rtab.size() * sizeof(SpotRes), cudaMemcpyHostToDevice, st);
     }
     if (e == cudaSuccess) e = cudaMemsetAsync(P.done, 0, done_bytes, st);
     if (e == cudaSuccess && P.counts) e = cudaMemsetAsync(P.counts, 0, np * bins * sizeof(int64_t), st);
@@ -562,7 +691,7 @@ static int32_t spot_stats(const char* what, bmo_result* r, int32_t det_object, i
 int32_t bmo_spot_stats(bmo_result* r, int32_t det_object, const double* window, int32_t nx, int32_t nz, bmo_spot_info* out,
                        int64_t* counts, uint32_t flags) {
     NvtxRange nvtx_("bmo_spot_stats");
-    return spot_stats("bmo_spot_stats", r, det_object, 1, window, nx, nz, out, counts, flags);
+    return spot_stats("bmo_spot_stats", 1, &r, det_object, 1, window, nx, nz, out, counts, flags);
 }
 
 int32_t bmo_spot_stats_poses(bmo_result* r, int32_t det_object, int32_t n_poses, const double* window, int32_t nx, int32_t nz,
@@ -571,5 +700,59 @@ int32_t bmo_spot_stats_poses(bmo_result* r, int32_t det_object, int32_t n_poses,
     if (r && n_poses != r->n_poses)
         return fail(BMO_EINVAL, "bmo_spot_stats_poses: n_poses " + std::to_string(n_poses) + " differs from the " +
                                     std::to_string(r->n_poses) + " poses the result was traced with");
-    return spot_stats("bmo_spot_stats_poses", r, det_object, n_poses, window, nx, nz, out, counts, flags);
+    return spot_stats("bmo_spot_stats_poses", 1, &r, det_object, n_poses, window, nx, nz, out, counts, flags);
+}
+
+int32_t bmo_spot_stats_results(int32_t n_results, bmo_result* const* results, int32_t det_object, const double* window, int32_t nx,
+                               int32_t nz, bmo_spot_info* out, int64_t* counts, uint32_t flags) {
+    NvtxRange nvtx_("bmo_spot_stats_results");
+    if (n_results < 1 || !results) return fail(BMO_EINVAL, "bmo_spot_stats_results: needs n_results >= 1 results");
+    return spot_stats("bmo_spot_stats_results", n_results, results, det_object, 1, window, nx, nz, out, counts, flags);
+}
+
+int32_t bmo::spot_stats_shard(const std::string& fn, bmo_ctx* ctx, bmo_result* r, int32_t det_object, const double* window, int32_t nx,
+                              int32_t nz, const std::vector<int64_t>& entries, int64_t per, SpotExchange& x, bmo_spot_info* out,
+                              int64_t* counts, uint32_t flags) {
+    BMO_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int32_t W = (int32_t)entries.size();
+    int64_t stride = 1;             // blocks of the largest rank: every rank's partials are padded to it for the all-gather
+    for (int64_t m : entries) stride = std::max(stride, (m + per - 1) / per);
+    const int64_t n = r ? r->n_beams * r->R : 0, nblk = (n + per - 1) / per;
+    const size_t bins = counts ? (size_t)nx * (size_t)nz : 0;
+    const bool dev_counts = counts && (flags & BMO_INPUT_DEVICE);
+    // one scratch block: this rank's partials, every rank's, the entry counts, the statistics, the histogram of a host `counts`
+    const size_t part_bytes = (size_t)stride * sizeof(SpotPartial);
+    const size_t off_all = part_bytes, off_ent = off_all + (size_t)W * part_bytes, off_out = off_ent + (size_t)W * sizeof(int64_t);
+    const size_t off_hist = off_out + sizeof(bmo_spot_info), bytes = off_hist + (counts && !dev_counts ? bins * sizeof(int64_t) : 0);
+    char* scr = nullptr;
+    BMO_CUDA(dev_alloc(&scr, bytes, st));
+    SpotParams P{};
+    if (r) { P.obj = r->spot_obj; P.xz = r->spot_xz; P.R = r->R; }
+    P.n = n; P.per = per; P.det = det_object; P.n_poses = 1;
+    P.has_window = window != nullptr; P.nx = nx; P.nz = nz;
+    if (window) for (int i = 0; i < 4; i++) P.win[i] = window[i];
+    P.part = (SpotPartial*)scr; P.out = (bmo_spot_info*)(scr + off_out);
+    P.counts = counts ? (dev_counts ? (unsigned long long*)counts : (unsigned long long*)(scr + off_hist)) : nullptr;
+    const SpotPartial* all = (const SpotPartial*)(scr + off_all);
+    const int64_t* ent = (const int64_t*)(scr + off_ent);
+    int32_t rc = BMO_OK;
+    const auto cuda = [&](cudaError_t e) { if (!rc && e != cudaSuccess) rc = fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e)); };
+    cuda(cudaMemcpyAsync(scr + off_ent, entries.data(), (size_t)W * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    if (P.counts) cuda(cudaMemsetAsync(P.counts, 0, bins * sizeof(int64_t), st));
+    // pass 1: this rank's sums; every rank combines all partials in global block order
+    if (!rc && nblk) { spot_sums<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P); rc = launched(ctx, "spot_sums"); }
+    if (!rc) rc = x.gather(P.part, scr + off_all, part_bytes);
+    if (!rc) { spot_combine<<<1, 1, 0, st>>>(all, W, (int32_t)stride, ent, per, 0, P.out); rc = launched(ctx, "spot_combine"); }
+    // pass 2: the squared distances to the common centroid
+    if (!rc && nblk) { spot_spread<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P); rc = launched(ctx, "spot_spread"); }
+    if (!rc) rc = x.gather(P.part, scr + off_all, part_bytes);
+    if (!rc) { spot_combine<<<1, 1, 0, st>>>(all, W, (int32_t)stride, ent, per, 1, P.out); rc = launched(ctx, "spot_combine"); }
+    // the histogram: integer counts, summed exactly
+    if (!rc && P.counts) rc = x.sum((int64_t*)P.counts, bins);
+    if (!rc) cuda(cudaMemcpyAsync(out, P.out, sizeof(bmo_spot_info), cudaMemcpyDeviceToHost, st));
+    if (!rc && counts && !dev_counts) cuda(cudaMemcpyAsync(counts, P.counts, bins * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    cuda(cudaStreamSynchronize(st));
+    dev_free(scr, st);
+    return rc;
 }

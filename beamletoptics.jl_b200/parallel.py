@@ -3,12 +3,15 @@ plumbing (NCCL over NVLink on the GPU box, gloo in the CPU tests).
 
 Rays, beamlets and poses are independent, the system tables are small and replicated, so the path
 shards without a data-path collective: every rank traces its slice of the bundle on its own GPU and
-owns the corresponding slice of the outputs.  The single exchange step is the Photodetector: each
-rank accumulates *its* beamlets onto a full n x n complex128 partial field and the partial fields
-are summed with one all-reduce of 2 n^2 doubles (the reference adds the beamlet fields serially into
-`pd.field`, Photodetector.jl:103; addition order across ranks changes the sum at the 1e-16 level).
+owns the corresponding slice of the outputs.  The exchange steps are the Photodetector and the spot
+diagram.  Each rank accumulates *its* beamlets onto a full n x n complex128 partial field and the partial
+fields are summed with one all-reduce of 2 n^2 doubles (the reference adds the beamlet fields serially into
+`pd.field`, Photodetector.jl:103; addition order across ranks changes the sum at the 1e-16 level).  A spot
+diagram of a DeviceSource sharded with spot_shard_slice is reduced where the hits are (solve_spot_sharded:
+bmo_spot_stats_sharded all-gathers per-block partials, not hits) and has the bits of the unsharded solve.
 """
 import ctypes as C
+import math
 import os
 
 import numpy as np
@@ -59,6 +62,18 @@ class FieldComm:
         L.check(L.lib().bmo_pd_allreduce(self.h, L.ptr(field), int(n), 0))
         return field
 
+    def spot_stats(self, result, det_object, nx=0, nz=0, window=None):
+        """bmo_spot_stats_sharded, collective: every rank passes the TraceResult of its shard (None for a rank without rays)
+        and receives the spot statistics of all ranks' entries in rank order, as solver.spot_stats's dict ("counts": an
+        (nz, nx) int64 histogram over `window` when nx > 0).  BmoError on every rank if any rank's arguments are refused."""
+        from .solver import _spot_dict
+        counts = np.zeros((nz, nx), np.int64) if nx else None
+        win = None if window is None else np.ascontiguousarray(window, dtype=np.float64)
+        info = L.bmo_spot_info()
+        L.check(L.lib().bmo_spot_stats_sharded(self.h, None if result is None else result.h, int(det_object), L.ptr(win), int(nx), int(nz),
+                                               C.byref(info), L.ptr(counts), 0))
+        return _spot_dict(info, counts)
+
     def free(self):
         if self.h:
             L.lib().bmo_comm_free(self.h)
@@ -69,10 +84,15 @@ _default_comm = None
 
 
 def default_comm(group=None):
-    """The process-wide FieldComm (created on first use from the torch.distributed group; NCCL backends only)."""
+    """The process-wide FieldComm: created on first use from the torch.distributed group (NCCL backends only), or a
+    one-rank communicator on GPU LOCAL_RANK when this process is not part of a process group of several ranks."""
     global _default_comm
     if _default_comm is None:
-        _default_comm = FieldComm.from_torch(group=group)
+        import torch.distributed as dist
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+            _default_comm = FieldComm.from_torch(group=group)
+        else:
+            _default_comm = FieldComm(0, 1, FieldComm.unique_id(), world()[2])
     return _default_comm
 
 
@@ -87,6 +107,26 @@ def shard_slice(n, rank, world_size):
     base, rem = divmod(n, world_size)
     start = rank * base + min(rank, rem)
     return start, start + base + (1 if rank < rem else 0)
+
+
+def spot_shard_slice(n_rays, rank, world_size, R=1):
+    """(first, count): the contiguous rays of rank `rank` for bmo_spot_stats_sharded.  Every slice but the last holds a
+    multiple of BMO_SPOT_PER(n_rays * R) entries (R per ray), so no block of the spot reduction crosses a rank boundary, and
+    the slices are as even as that allows: they are cut in units of the fewest rays that fill whole blocks (per / gcd(per,
+    R) rays, at most `per`), the extra units go to the last ranks, and sizes differ by at most one unit.  A rank may get no
+    rays when there are fewer units than ranks."""
+    n_rays, rank, world_size = int(n_rays), int(rank), int(world_size)
+    if not (0 <= rank < world_size) or n_rays < 0:
+        raise ValueError(f"spot_shard_slice: rank {rank} of {world_size}, {n_rays} rays")
+    per = L.spot_per(n_rays * R)
+    unit = per // math.gcd(per, R)
+    base, rem = divmod(-(-n_rays // unit), world_size)
+
+    def start(k):   # first unit of rank k: ranks world_size - rem ... world_size - 1 take base + 1 units
+        return k * base + max(0, k - (world_size - rem))
+    first = min(n_rays, start(rank) * unit)
+    stop = n_rays if rank == world_size - 1 else min(n_rays, start(rank + 1) * unit)
+    return first, stop - first
 
 
 def shard_interleaved(n, rank, world_size):
@@ -157,6 +197,24 @@ def gather_rows(local, idx, n_total, group=None):
     for i, v in parts:
         out[i] = v
     return out
+
+
+def solve_spot_sharded(system, source, detector, bins=None, window=None, comm=None, r_max=100):
+    """The spot diagram of a DeviceSource traced across all ranks: this rank traces source.shard(*spot_shard_slice(...)) on
+    its GPU (the hits stay there) and bmo_spot_stats_sharded reduces every rank's hits.  Returns, on every rank, the dict
+    spot_stats gives for one unsharded solve of the whole source on one GPU -- bit for bit when the system has no
+    beamsplitters.  `comm`: a FieldComm (default: default_comm(), a one-rank communicator outside torchrun); the rank
+    traces on the communicator's GPU.  `bins` / `window` as in spot_stats."""
+    from .solver import _lambda_ids, _spot_args, cached_system, solve_system_
+    comm = default_comm() if comm is None else comm
+    first, count = spot_shard_slice(len(source), comm.rank, comm.world_size)
+    res = None
+    if count:
+        res = solve_system_(system, source.shard(first, count), r_max=r_max, retrace=False, device=comm.device, keep_segments=False,
+                            collect_spots=False)
+    dsys = res.dsys if res is not None else cached_system(system, _lambda_ids([source.lam])[0], comm.device)
+    oi, nx, nz, win = _spot_args(dsys.flat.objects, detector, bins, window, "solve_spot_sharded")
+    return comm.spot_stats(res, oi, nx, nz, win)
 
 
 def solve_system_sharded(system, bundle, r_max=100, interleaved=False, keep_segments=False, group=None, comm=None):

@@ -487,9 +487,9 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
     raise TypeError(f"cannot trace {type(beam).__name__}")
 
 
-def _spot_args(result, detector, bins, window, what):
-    """(object index, nx, nz, window array) of a spot_stats call; the window defaults to the detector's face."""
-    objs = result.dsys.flat.objects
+def _spot_args(objs, detector, bins, window, what):
+    """(object index, nx, nz, window array) of a spot_stats call on a system with objects `objs`; the window defaults to the
+    detector's face."""
     if isinstance(detector, (int, np.integer)):
         oi = int(detector)
     else:
@@ -506,21 +506,38 @@ def _spot_args(result, detector, bins, window, what):
     return oi, nx, nz, win
 
 
-def spot_stats(result, detector, bins=None, window=None):
-    """Spot diagram of `detector` (a Spotdetector of the traced system, or its object index) reduced on the device
-    (bmo_spot_stats): dict of hits, centroid (x, z), rms, max_r (largest distance from the detector origin), lo / hi
-    (x, z) and outside (hits outside `window`).  With `bins` (n or (nx, nz)) also "counts", an (nz, nx) int64 histogram
-    over `window` = (x_lo, x_hi, z_lo, z_hi), by default the detector's face.  The statistics cover every spot entry of the
-    result on that detector (chief, waist and divergence rays of a beamlet result), whether or not they were collected."""
-    oi, nx, nz, win = _spot_args(result, detector, bins, window, "spot_stats")
-    counts = None if bins is None else np.zeros((max(nz, 0), max(nx, 0)), np.int64)
-    info = L.bmo_spot_info()
-    L.check(L.lib().bmo_spot_stats(result.h, oi, L.ptr(win), nx, nz, C.byref(info), L.ptr(counts), 0))
+def _spot_dict(info, counts):
     out = dict(hits=int(info.hits), centroid=(info.centroid[0], info.centroid[1]), rms=info.rms, max_r=info.max_r,
                lo=(info.lo[0], info.lo[1]), hi=(info.hi[0], info.hi[1]), outside=int(info.outside))
     if counts is not None:
         out["counts"] = counts
     return out
+
+
+def spot_stats(result, detector, bins=None, window=None):
+    """Spot diagram of `detector` (a Spotdetector of the traced system, or its object index) reduced on the device
+    (bmo_spot_stats): dict of hits, centroid (x, z), rms, max_r (largest distance from the detector origin), lo / hi
+    (x, z) and outside (hits outside `window`).  With `bins` (n or (nx, nz)) also "counts", an (nz, nx) int64 histogram
+    over `window` = (x_lo, x_hi, z_lo, z_hi), by default the detector's face.  The statistics cover every spot entry of the
+    result on that detector (chief, waist and divergence rays of a beamlet result), whether or not they were collected.
+    `result` may be a list of results traced on one device (bmo_spot_stats_results): the spot diagram of all their entries,
+    in list order, as the reference's Spotdetector accumulates over several solve_system! calls until empty!; a bundle
+    traced in splitter-free pieces gives the bits of tracing it once."""
+    results = list(result) if isinstance(result, (list, tuple)) else [result]
+    if not results:
+        raise L.BmoError("spot_stats: no result")
+    oi, nx, nz, win = _spot_args(results[0].dsys.flat.objects, detector, bins, window, "spot_stats")
+    for r in results[1:]:
+        if _spot_args(r.dsys.flat.objects, detector, None, None, "spot_stats")[0] != oi:
+            raise L.BmoError("spot_stats: the detector has another object index in another result's system")
+    counts = None if bins is None else np.zeros((max(nz, 0), max(nx, 0)), np.int64)
+    info = L.bmo_spot_info()
+    if isinstance(result, (list, tuple)):
+        hs = (C.c_void_p * len(results))(*[r.h for r in results])
+        L.check(L.lib().bmo_spot_stats_results(len(results), hs, oi, L.ptr(win), nx, nz, C.byref(info), L.ptr(counts), 0))
+    else:
+        L.check(L.lib().bmo_spot_stats(result.h, oi, L.ptr(win), nx, nz, C.byref(info), L.ptr(counts), 0))
+    return _spot_dict(info, counts)
 
 
 def spot_stats_poses(result, detector, n_poses, bins=None, window=None):
@@ -529,7 +546,7 @@ def spot_stats_poses(result, detector, n_poses, bins=None, window=None):
     max_r (P,), lo / hi (P, 2) and, with `bins`, counts (P, nz, nx) over `window` (by default the detector's face).  Pose p
     has the bits spot_stats gives for a one-pose solve that lists the pose's hits in the same order, which a system
     without beamsplitters always does."""
-    oi, nx, nz, win = _spot_args(result, detector, bins, window, "spot_stats_poses")
+    oi, nx, nz, win = _spot_args(result.dsys.flat.objects, detector, bins, window, "spot_stats_poses")
     P = int(n_poses)
     counts = None if bins is None else np.zeros((max(P, 0), max(nz, 0), max(nx, 0)), np.int64)
     info = (L.bmo_spot_info * max(P, 1))()

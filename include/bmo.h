@@ -339,6 +339,13 @@ int32_t bmo_source_create(bmo_ctx* ctx, const bmo_source_desc* desc, bmo_source*
  * ring sources run their recurrence once and copy it).  bmo_source_create is the n_poses = 1 case.  BMO_EINVAL also for
  * n_poses < 1 or n_rays * n_poses overflowing int64.                                                              */
 int32_t bmo_source_create_poses(bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, bmo_source** src);
+/* Source slice, for sharding one source over several GPUs or tracing it in pieces: rays [first, first + count) of the one-pose
+ * source bmo_source_create would make, bit for bit (discs: to the same bits as those rays of the unsliced source, not closer
+ * to the host than it is).  A disc computes ray first + i with rho = sqrt((k + 0.5) / n_rays); each ring that overlaps the
+ * slice runs its recurrence from its own start and writes the rays inside the slice; ray 0 is written only when first == 0.
+ * bmo_source_device reports n = count, bmo_source_rays copies the slice, bmo_source_pose_ids gives NULL.  BMO_EINVAL for
+ * first < 0, count < 1, first + count > n_rays, and whatever bmo_source_create refuses.                              */
+int32_t bmo_source_create_slice(bmo_ctx* ctx, const bmo_source_desc* desc, int64_t first, int64_t count, bmo_source** src);
 /* Device pose ids [n_rays * n_poses] for bmo_trace_rays(..., pose_id, BMO_INPUT_DEVICE); NULL for a one-pose source.
  * Valid until bmo_source_free.                                                                                       */
 int32_t bmo_source_pose_ids(bmo_source* src, int32_t* n_poses, const int32_t** pose_id);
@@ -355,11 +362,15 @@ int32_t bmo_source_free(bmo_source* src);   /* before bmo_shutdown of the source
  * divergence).  rms = sqrt(sum((x - cx)^2 + (z - cz)^2) / hits) in a second pass; max_r = max sqrt(x x + z z) about the
  * detector origin; with no hits every floating field is NaN.  The sums run over a fixed partition of the entry index
  * whose partials are combined in index order, so two calls give the same bits; hits, outside, max_r, lo / hi and the
- * histogram are exact.
+ * histogram are exact.  The partition (part of this contract: bmo_spot_stats_results and bmo_spot_stats_sharded use it on
+ * the total of their entries, and the sharded call needs shards cut to it) gives each block BMO_SPOT_PER(m) consecutive
+ * entries of the m entries reduced, the last block the rest.
  * window (NULL ok, required with counts): x_lo, x_hi, z_lo, z_hi, finite with hi > lo; a hit outside the closed window
  * counts in `outside`.  counts (NULL ok): [nz][nx], counts[j * nx + i] = hits with
  * i = min(floor((x - x_lo) / (x_hi - x_lo) * nx), nx - 1), j likewise in z; overwritten.  Host pointer, or device
  * pointer with BMO_INPUT_DEVICE.  (The struct cannot share the function's name in C, hence bmo_spot_info.)        */
+/* entries per block of the partition of m spot entries: 4096 * max(1, ceil(m / (4096 * 1024))), so <= 1024 blocks          */
+#define BMO_SPOT_PER(m) (4096 * (((m) + 4096 * 1024 - 1) / (4096 * 1024) > 1 ? ((m) + 4096 * 1024 - 1) / (4096 * 1024) : 1))
 typedef struct bmo_spot_info {
     int64_t hits;
     int64_t outside;
@@ -381,6 +392,16 @@ int32_t bmo_spot_stats(bmo_result* r, int32_t det_object, const double* window, 
  * (BMO_EINVAL otherwise), and bmo_spot_stats's argument checks apply.                                               */
 int32_t bmo_spot_stats_poses(bmo_result* r, int32_t det_object, int32_t n_poses, const double* window, int32_t nx, int32_t nz,
                              bmo_spot_info* out, int64_t* counts, uint32_t flags);
+/* Spot statistics over several results on one device: replaces reading sd.data after several solve_system! calls into one
+ * Spotdetector without empty!(sd) in between (Spotdetector.jl:50-61): field points, one source per wavelength, or a bundle
+ * traced in pieces.  bmo_spot_stats's definition over the concatenation of the results' entries, the results in list order and
+ * each result's entries in entry order; the partition is BMO_SPOT_PER of the total entry count N = sum n_beams * R, and a
+ * block may straddle two results.  The output has the bits of bmo_spot_stats on one result that lists the same entries in the
+ * same order: without beamsplitters a bundle traced as k slices gives the bits of tracing it once, however it is cut.  The
+ * results must share one context and det_object must be a Spotdetector of every result's system; R = 1 and R = 3 results
+ * mix; poses are ignored.  BMO_EINVAL for n_results < 1, a NULL entry, and whatever bmo_spot_stats refuses.            */
+int32_t bmo_spot_stats_results(int32_t n_results, bmo_result* const* results, int32_t det_object, const double* window,
+                               int32_t nx, int32_t nz, bmo_spot_info* out, int64_t* counts, uint32_t flags);
 
 enum bmo_status {
     BMO_ST_ACTIVE = 0,
@@ -453,6 +474,22 @@ int32_t bmo_comm_info(bmo_comm* comm, int32_t* rank, int32_t* n_ranks, int32_t* 
  * stream; add BMO_COMM_SYNC to wait for it).                                                                    */
 int32_t bmo_pd_allreduce(bmo_comm* comm, double* field, int64_t n_complex, uint32_t flags);
 int32_t bmo_pd_allreduce_local(int32_t n, bmo_comm* const* comms, double* const* fields, int64_t n_complex, uint32_t flags);
+/* Spot statistics of a ray bundle sharded over ranks, collective: every rank of comm passes the result of its shard (NULL
+ * on a rank whose shard holds no rays); every rank receives the statistics (and histogram) of the concatenation of all
+ * ranks' entries in rank order, with the bits bmo_spot_stats_results gives for the shard results in rank order -- for
+ * aligned, splitter-free shards of one source the bits of one unsharded trace; with one rank, bmo_spot_stats's bits.
+ * Every rank except the last must hold a multiple of BMO_SPOT_PER(N) entries, N the total over all ranks, so that no
+ * block of the partition crosses a rank boundary.  det_object, nx, nz and the window must be the same on every rank.
+ * Steps, on the context's stream: (1) all-gather of each rank's entry count, argument verdict, det_object, histogram shape
+ * and window; a refusal on any rank (bmo_spot_stats's checks, another context, unaligned shards, a detector, histogram shape
+ * or window that differs from rank 0's) makes every rank return the same BMO_E* code; (2) each rank reduces its entries to
+ * per-block partials; (3) the partials are all-gathered and combined in global block order on every rank; (4) the same
+ * for the squared distances to the centroid; (5) one int64 all-reduce (sum) of the histogram.  Only the statistics and
+ * the histogram leave the device.  counts: host pointer, or device pointer with BMO_INPUT_DEVICE.  Only arguments are
+ * agreed on: a CUDA or NCCL failure on one rank (an allocation, a launch) returns BMO_ECUDA / BMO_ENCCL on that rank alone
+ * and leaves the other ranks waiting in the next collective, as any failed NCCL collective does.                     */
+int32_t bmo_spot_stats_sharded(bmo_comm* comm, bmo_result* r, int32_t det_object, const double* window, int32_t nx, int32_t nz,
+                               bmo_spot_info* out, int64_t* counts, uint32_t flags);
 int32_t bmo_comm_free(bmo_comm* comm);
 
 /* Give device memory back: the library keeps released blocks of 64 MiB and more in a per-device free list and smaller ones in
