@@ -6,6 +6,9 @@
 //   * The spot diagram of a ray bundle sharded over several GPUs (bmo_spot_stats_sharded): every rank reduces its own
 //     Spotdetector entries to per-block partials (bmo_source.cu), the partials are all-gathered and combined in global block
 //     order on every rank, and the histograms are summed by one int64 all-reduce.  No spot leaves its GPU.
+//   * The PSFDetector map of a ray bundle sharded over several GPUs (bmo_psf_allgather, bmo_psf_intensity_sharded): the hit
+//     records are all-gathered in rank order, every rank sums all records into its band of pixel columns, and the bands are
+//     all-gathered.  Each pixel is summed on one GPU over the records of one trace in order, so the map has one GPU's bits.
 //
 // NCCL is bound at run time (dlopen of libnccl.so.2) so that libbmo.so has no link-time dependency on it: a host
 // that never shards never needs the library, and inside a process that already carries one (PyTorch's bundled
@@ -218,31 +221,20 @@ struct NcclSpotExchange : SpotExchange {
     }
 };
 
-int32_t bmo_spot_stats_sharded(bmo_comm* c, bmo_result* r, int32_t det_object, const double* window, int32_t nx, int32_t nz,
-                               bmo_spot_info* out, int64_t* counts, uint32_t flags) {
-    NvtxRange nvtx_("bmo_spot_stats_sharded");
-    const std::string fn = "bmo_spot_stats_sharded";
-    if (!c) return fail(BMO_EINVAL, fn + ": communicator NULL");
-    // Step 1: every rank's entry count, argument verdict and the arguments that must agree (detector, histogram shape,
-    // window), all-gathered, so that all ranks take the same branch below: a refusal on one rank is a refusal on every
-    // rank.  (Only arguments are agreed on: a CUDA or NCCL failure on one rank -- an allocation, a launch -- returns on
-    // that rank alone and leaves the others in the next collective, as with any NCCL collective.)
-    int32_t rc = BMO_OK;
-    if (!out) rc = fail(BMO_EINVAL, fn + ": NULL argument");
-    else if (r && r->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the result belongs to another context than the communicator");
-    if (!rc && r) rc = spot_check_result(fn, r, det_object);
-    if (!rc) rc = spot_check_args(fn, window, nx, nz, counts);
-    const std::string why = rc ? g_last_error : std::string();
+// Step 1 of the collectives below: every rank's words, all-gathered into all[k * K + w] (word w of rank k, K = mine.size()).
+// Word 0 is the rank's argument verdict: BMO_OK, or the code its own checks returned (g_last_error then holds their message).  The
+// first refusal in rank order decides for every rank, so that all ranks take the same branch: that code is returned on every rank,
+// with the refusing rank's own message there.  (Only arguments are agreed on: a CUDA or NCCL failure on one rank -- an allocation,
+// a launch -- returns on that rank alone and leaves the others in the next collective, as with any NCCL collective.)
+static int32_t agree(bmo_comm* c, const std::string& fn, const std::vector<int64_t>& mine, std::vector<int64_t>& all) {
+    const std::string why = mine[0] ? g_last_error : std::string();
     const int W = c->n_ranks;
-    constexpr int K = 11;   // entries, verdict, then what must agree: det_object, histogram?, nx, nz, window?, window bits [4]
-    std::vector<int64_t> mine(K, 0), all((size_t)K * W);
-    mine[0] = r ? r->n_beams * r->R : 0; mine[1] = rc; mine[2] = det_object;
-    if (counts) { mine[3] = 1; mine[4] = nx; mine[5] = nz; }
-    if (window) { mine[6] = 1; std::memcpy(&mine[7], window, 4 * sizeof(double)); }
+    const size_t K = mine.size();
+    all.assign(K * W, 0);
     cudaStream_t st = c->ctx->stream;
     BMO_CUDA(cudaSetDevice(c->ctx->device));
     int64_t* d = nullptr;
-    BMO_CUDA(dev_alloc(&d, (size_t)K * (W + 1), st));
+    BMO_CUDA(dev_alloc(&d, K * (W + 1), st));
     cudaError_t e = cudaMemcpyAsync(d, mine.data(), K * sizeof(int64_t), cudaMemcpyHostToDevice, st);
     int nr = 0;
     if (e == cudaSuccess) {
@@ -255,21 +247,42 @@ int32_t bmo_spot_stats_sharded(bmo_comm* c, bmo_result* r, int32_t det_object, c
     if (e != cudaSuccess) return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e));
     if (nr) return fail(BMO_ENCCL, fn + ": exchanging the arguments: " + (W == 1 ? std::string("copy failed") : std::string(g_nccl.GetErrorString(nr))));
     for (int k = 0; k < W; k++) {
-        const int64_t* a = all.data() + (size_t)K * k;
-        if (a[1]) {      // the first refusal in rank order decides for every rank
-            if (k == c->rank) { g_last_error = why; return (int32_t)a[1]; }
-            return fail((int32_t)a[1], fn + ": rank " + std::to_string(k) + " refused its arguments");
+        const int32_t v = (int32_t)all[K * k];
+        if (v) {
+            if (k == c->rank) { g_last_error = why; return v; }
+            return fail(v, fn + ": rank " + std::to_string(k) + " refused its arguments");
         }
     }
+    return BMO_OK;
+}
+
+int32_t bmo_spot_stats_sharded(bmo_comm* c, bmo_result* r, int32_t det_object, const double* window, int32_t nx, int32_t nz,
+                               bmo_spot_info* out, int64_t* counts, uint32_t flags) {
+    NvtxRange nvtx_("bmo_spot_stats_sharded");
+    const std::string fn = "bmo_spot_stats_sharded";
+    if (!c) return fail(BMO_EINVAL, fn + ": communicator NULL");
+    // Step 1: every rank's argument verdict, entry count and the arguments that must agree (detector, histogram shape, window)
+    int32_t rc = BMO_OK;
+    if (!out) rc = fail(BMO_EINVAL, fn + ": NULL argument");
+    else if (r && r->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the result belongs to another context than the communicator");
+    if (!rc && r) rc = spot_check_result(fn, r, det_object);
+    if (!rc) rc = spot_check_args(fn, window, nx, nz, counts);
+    const int W = c->n_ranks;
+    constexpr int K = 11;   // verdict, entries, then what must agree: det_object, histogram?, nx, nz, window?, window bits [4]
+    std::vector<int64_t> mine(K, 0), all;
+    mine[0] = rc; mine[1] = r ? r->n_beams * r->R : 0; mine[2] = det_object;
+    if (counts) { mine[3] = 1; mine[4] = nx; mine[5] = nz; }
+    if (window) { mine[6] = 1; std::memcpy(&mine[7], window, 4 * sizeof(double)); }
+    if ((rc = agree(c, fn, mine, all))) return rc;
     std::vector<int64_t> entries((size_t)W);
     int64_t N = 0;
     for (int k = 0; k < W; k++) {
         const int64_t* a = all.data() + (size_t)K * k;
         if (!std::equal(a + 2, a + K, all.data() + 2))
             return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " passes another detector, histogram shape or window than rank 0");
-        if (a[0] > INT64_MAX - N) return fail(BMO_EINVAL, fn + ": the ranks' entries overflow int64");
-        entries[k] = a[0];
-        N += a[0];
+        if (a[1] > INT64_MAX - N) return fail(BMO_EINVAL, fn + ": the ranks' entries overflow int64");
+        entries[k] = a[1];
+        N += a[1];
     }
     // Step 2: the global blocks must not cross a rank boundary
     const int64_t per = spot_per(N);
@@ -280,6 +293,122 @@ int32_t bmo_spot_stats_sharded(bmo_comm* c, bmo_result* r, int32_t det_object, c
     // Steps 3-5: the two passes and the histogram (bmo_source.cu)
     NcclSpotExchange x(c);
     return spot_stats_shard(fn, c->ctx, r, det_object, window, nx, nz, entries, per, x, out, counts, flags);
+}
+
+int32_t bmo_psf_allgather(bmo_comm* c, bmo_psf* local, bmo_psf** all_out) {
+    NvtxRange nvtx_("bmo_psf_allgather");
+    const std::string fn = "bmo_psf_allgather";
+    if (!c) return fail(BMO_EINVAL, fn + ": communicator NULL");
+    // Step 1: every rank's verdict and record count; the total must fit int64
+    int32_t rc = BMO_OK;
+    if (!all_out) rc = fail(BMO_EINVAL, fn + ": NULL argument");
+    else if (local && local->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the records belong to another context than the communicator");
+    std::vector<int64_t> mine{rc, local ? local->n : 0}, all;
+    if ((rc = agree(c, fn, mine, all))) return rc;
+    const int W = c->n_ranks;
+    int64_t total = 0, most = 0;
+    std::vector<int64_t> first((size_t)W);
+    for (int k = 0; k < W; k++) {
+        const int64_t m = all[2 * k + 1];
+        if (m > INT64_MAX / (PSF_NREC + PSF_NFAST) / W - total) return fail(BMO_EINVAL, fn + ": the ranks' records overflow int64");
+        first[k] = total;
+        total += m;
+        most = std::max(most, m);
+    }
+    // Step 2: one all-gather of [most][PSF_NREC] records then [most][PSF_NFAST] fast words per rank, each rank's part copied into place
+    bmo_ctx* ctx = c->ctx;
+    cudaStream_t st = ctx->stream;
+    bmo_psf* p = new bmo_psf();
+    p->ctx = ctx;
+    auto done = [&](int32_t code) {
+        if (code) bmo_psf_free(p);
+        else *all_out = p;
+        return code;
+    };
+    if ((rc = psf_reserve(p, total, st))) return done(rc);
+    p->n = total;
+    if (total == 0) return done(BMO_OK);
+    const int64_t m = local ? local->n : 0;
+    constexpr size_t D = sizeof(double);
+    const size_t per = (size_t)most * (PSF_NREC + PSF_NFAST);   // doubles per rank
+    double* buf = nullptr;
+    rc = [&]() -> int32_t {
+        if (W == 1) {     // no exchange: a copy of this rank's records
+            BMO_CUDA(cudaMemcpyAsync(p->rec, local->rec, (size_t)m * PSF_NREC * D, cudaMemcpyDeviceToDevice, st));
+            BMO_CUDA(cudaMemcpyAsync(p->fast, local->fast, (size_t)m * PSF_NFAST * D, cudaMemcpyDeviceToDevice, st));
+            BMO_CUDA(cudaStreamSynchronize(st));
+            return BMO_OK;
+        }
+        BMO_CUDA(dev_alloc(&buf, per * (W + 1), st));
+        double* send = buf + per * W;
+        if (m) {
+            BMO_CUDA(cudaMemcpyAsync(send, local->rec, (size_t)m * PSF_NREC * D, cudaMemcpyDeviceToDevice, st));
+            BMO_CUDA(cudaMemcpyAsync(send + (size_t)most * PSF_NREC, local->fast, (size_t)m * PSF_NFAST * D, cudaMemcpyDeviceToDevice, st));
+        }
+        BMO_NCCL(g_nccl.AllGather(send, buf, per, kNcclDouble, c->comm, st));
+        for (int k = 0; k < W; k++) {
+            const int64_t mk = all[2 * k + 1];
+            if (!mk) continue;
+            const double* part = buf + per * k;
+            BMO_CUDA(cudaMemcpyAsync(p->rec + first[k] * PSF_NREC, part, (size_t)mk * PSF_NREC * D, cudaMemcpyDeviceToDevice, st));
+            BMO_CUDA(cudaMemcpyAsync(p->fast + first[k] * PSF_NFAST, part + (size_t)most * PSF_NREC, (size_t)mk * PSF_NFAST * D,
+                                     cudaMemcpyDeviceToDevice, st));
+        }
+        BMO_CUDA(cudaStreamSynchronize(st));
+        return BMO_OK;
+    }();
+    dev_free(buf, st);
+    return done(rc);
+}
+
+int32_t bmo_psf_intensity_sharded(bmo_comm* c, bmo_sys* sys, bmo_psf* all, int32_t psf_object, int32_t pose, int32_t n, const double* lims,
+                                  double x0_shift, double z0_shift, double* intensity, uint32_t flags) {
+    NvtxRange nvtx_("bmo_psf_intensity_sharded");
+    const std::string fn = "bmo_psf_intensity_sharded";
+    if (!c) return fail(BMO_EINVAL, fn + ": communicator NULL");
+    // Step 1: every rank's verdict and the arguments that must agree: n, pose, psf_object, the bits of lims and the shifts, and the
+    // record count (a rank that passes its own rather than the gathered records holds another count)
+    int32_t rc = psf_intensity_check(fn.c_str(), sys, all, psf_object, pose, n, lims, intensity);
+    if (!rc && sys->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the system belongs to another context than the communicator");
+    if (!rc && all->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the records belong to another context than the communicator");
+    constexpr int K = 11;   // verdict, n, pose, psf_object, lims bits [4], x0_shift bits, z0_shift bits, records
+    std::vector<int64_t> mine(K, 0), agreed;
+    mine[0] = rc; mine[1] = n; mine[2] = pose; mine[3] = psf_object;
+    if (lims) std::memcpy(&mine[4], lims, 4 * sizeof(double));
+    std::memcpy(&mine[8], &x0_shift, sizeof(double)); std::memcpy(&mine[9], &z0_shift, sizeof(double));
+    mine[10] = all ? all->n : 0;
+    if ((rc = agree(c, fn, mine, agreed))) return rc;
+    const int W = c->n_ranks;
+    for (int k = 1; k < W; k++)
+        if (!std::equal(agreed.begin() + (size_t)K * k + 1, agreed.begin() + (size_t)K * (k + 1), agreed.begin() + 1))
+            return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " passes another n, pose, detector, window, shift or record count than rank 0");
+    // Step 2: K6 on this rank's band of B = ceil(n / W) columns, then the bands all-gathered.  The map is column-major, so rank r's band
+    // of n * B doubles lands at n * (r * B): the first n * n doubles of the gathered bands are the map.
+    bmo_ctx* ctx = c->ctx;
+    BMO_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int64_t B = ((int64_t)n + W - 1) / W;
+    const int32_t j0 = (int32_t)std::min<int64_t>(n, c->rank * B), j1 = (int32_t)std::min<int64_t>(n, (c->rank + 1) * B);
+    const size_t nn = (size_t)n * n, band = (size_t)n * B;
+    const bool on_dev = flags & BMO_INPUT_DEVICE;
+    double* d_map = intensity;      // the caller's device buffer when the bands exactly fill it
+    if (!on_dev || band * W != nn) BMO_CUDA(dev_alloc(&d_map, band * W, st));
+    rc = [&]() -> int32_t {
+        int32_t r;
+        if ((r = psf_intensity_band(sys, all, psf_object, pose, n, lims, x0_shift, z0_shift, j0, j1, d_map + band * c->rank))) return r;
+        if (W > 1) BMO_NCCL(g_nccl.AllGather(d_map + band * c->rank, d_map, band, kNcclDouble, c->comm, st));
+        if (d_map != intensity)
+            BMO_CUDA(cudaMemcpyAsync(intensity, d_map, nn * sizeof(double), on_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
+        BMO_CUDA(cudaStreamSynchronize(st));
+        if (j1 > j0) {
+            float kms = 0;
+            BMO_CUDA(cudaEventElapsedTime(&kms, ctx->evk0, ctx->evk1));
+            ctx->psf_ms = kms;
+        }
+        return BMO_OK;
+    }();
+    if (d_map != intensity) dev_free(d_map, st);
+    return rc;
 }
 
 int32_t bmo_comm_free(bmo_comm* c) {

@@ -128,6 +128,14 @@ struct bmo_result {
     std::vector<WaveBuf> wavebufs;
 };
 
+// a PSFDetector's hit records on the device (bmo_psf.cu), in the order they were collected
+struct bmo_psf {
+    bmo_ctx* ctx = nullptr;
+    double* rec = nullptr;    // [cap][PSF_NREC]
+    double* fast = nullptr;   // [cap][PSF_NFAST]
+    int64_t n = 0, cap = 0;
+};
+
 namespace bmo {
 
 // ---- BVH (host build, median split on the longest centroid axis, <= 4 faces per leaf) ---------
@@ -291,5 +299,15 @@ struct SpotExchange {
 int32_t spot_stats_shard(const std::string& fn, bmo_ctx* ctx, bmo_result* r, int32_t det_object, const double* window, int32_t nx,
                          int32_t nz, const std::vector<int64_t>& entries, int64_t per, SpotExchange& x, bmo_spot_info* out,
                          int64_t* counts, uint32_t flags);
+
+// ---- PSFDetector records and K6 (bmo_psf.cu), shared with bmo_psf_allgather / bmo_psf_intensity_sharded (bmo_comm.cu) ----
+constexpr int PSF_NREC = 9;    // hit xyz, dir xyz, opl, proj, k
+constexpr int PSF_NFAST = 5;   // c0 = k (opl - hit . dir), k dir xyz, proj
+int32_t psf_reserve(bmo_psf* p, int64_t need, cudaStream_t st);   // capacity >= need records, the first p->n kept
+int32_t psf_intensity_check(const char* who, bmo_sys* sys, const bmo_psf* p, int32_t psf_object, int32_t pose, int32_t n,
+                            const double* lims, const double* intensity);
+// columns [j0, j1) of bmo_psf_intensity's map into d_out (device, [n][j1 - j0] column-major), enqueued on the context's stream
+int32_t psf_intensity_band(bmo_sys* sys, const bmo_psf* p, int32_t psf_object, int32_t pose, int32_t n, const double* lims,
+                           double x0_shift, double z0_shift, int32_t j0, int32_t j1, double* d_out);
 
 }  // namespace bmo

@@ -15,8 +15,6 @@
 namespace bmo {
 
 enum { S_PX = 0, S_PY, S_PZ, S_DX, S_DY, S_DZ, S_N, S_T, S_NX, S_NY, S_NZ };   // segment rows (bmo_trace.cu)
-constexpr int PSF_NREC = 9;    // hit xyz, dir xyz, opl, proj, k
-constexpr int PSF_NFAST = 5;   // c0 = k (opl - hit . dir), k dir xyz, proj
 
 struct PsfView {
     const double* seg_d; const int32_t* seg_part; int64_t rows; int nsd;   // segment table: row records [rows][nsd]
@@ -122,8 +120,8 @@ struct PsfParams {
     const double* fast; int64_t n_hits;
     const double* dp;            // detector pose: pos(3), dir(9 row-major)
     double x_lo, x_hi, z_lo, z_hi, x_shift, z_shift;
-    int32_t n, pad;
-    double* out;                 // [n][n] column-major [i + n*j]
+    int32_t n, j0, j1, pad;      // columns [j0, j1) of the n x n map
+    double* out;                 // [n][j1 - j0] column-major [i + n*(j - j0)]
 };
 BMO_D double lin_coord(int i, int n, double lo, double hi) {   // LinRange getindex (Base.lerpi)
     const double t = n == 1 ? 0.0 : (double)i / (double)(n - 1);
@@ -131,9 +129,9 @@ BMO_D double lin_coord(int i, int n, double lo, double hi) {   // LinRange getin
 }
 __global__ void __launch_bounds__(PSF_TX* PSF_TY, 4) psf_intensity_kernel(const PsfParams P) {
     __shared__ double s_h[PSF_BATCH * PSF_NFAST];
-    const int i = blockIdx.x * PSF_TX + threadIdx.x, j = blockIdx.y * PSF_TY + threadIdx.y;
+    const int i = blockIdx.x * PSF_TX + threadIdx.x, j = P.j0 + blockIdx.y * PSF_TY + threadIdx.y;
     const int tid = threadIdx.y * PSF_TX + threadIdx.x;
-    const bool inside = i < P.n && j < P.n;
+    const bool inside = i < P.n && j < P.j1;
     const double x = lin_coord(min(i, P.n - 1), P.n, P.x_lo, P.x_hi) + P.x_shift;
     const double z = lin_coord(min(j, P.n - 1), P.n, P.z_lo, P.z_hi) + P.z_shift;
     const double* dp = P.dp;
@@ -155,7 +153,7 @@ __global__ void __launch_bounds__(PSF_TX* PSF_TY, 4) psf_intensity_kernel(const 
             aim = fma(q[4], sn, aim);
         }
     }
-    if (inside) P.out[(int64_t)i + (int64_t)P.n * j] = are * are + aim * aim;
+    if (inside) P.out[(int64_t)i + (int64_t)P.n * (j - P.j0)] = are * are + aim * aim;
 }
 
 }  // namespace bmo
@@ -164,14 +162,7 @@ using namespace bmo;
 
 namespace bmo { __global__ void scan_flags(const int32_t* in, int64_t n, long long* out, long long* total); }
 
-struct bmo_psf {
-    bmo_ctx* ctx = nullptr;
-    double* rec = nullptr;    // [cap][PSF_NREC]
-    double* fast = nullptr;   // [cap][PSF_NFAST]
-    int64_t n = 0, cap = 0;
-};
-
-static int32_t psf_reserve(bmo_psf* p, int64_t need, cudaStream_t st) {
+int32_t bmo::psf_reserve(bmo_psf* p, int64_t need, cudaStream_t st) {
     if (need <= p->cap) return BMO_OK;
     const int64_t cap = std::max<int64_t>(need, 2 * p->cap);
     double *nr = nullptr, *nf = nullptr;
@@ -271,39 +262,72 @@ int32_t bmo_psf_lims(bmo_sys* sys, bmo_psf* p, int32_t psf_object, int32_t pose,
     return BMO_OK;
 }
 
-int32_t bmo_psf_intensity(bmo_sys* sys, bmo_psf* p, int32_t psf_object, int32_t pose, int32_t n, const double* lims, double x0_shift,
-                          double z0_shift, double* intensity, uint32_t flags) {
-    NvtxRange nvtx_("bmo_psf_intensity");
+// bmo_psf_intensity's argument checks (`who` names the caller in the message)
+int32_t bmo::psf_intensity_check(const char* who, bmo_sys* sys, const bmo_psf* p, int32_t psf_object, int32_t pose, int32_t n,
+                                 const double* lims, const double* intensity) {
     int32_t rc;
-    if ((rc = psf_check(sys, psf_object, "bmo_psf_intensity"))) return rc;
-    if (!p || !lims || !intensity) return fail(BMO_EINVAL, "bmo_psf_intensity: NULL argument");
-    if (n < 1) return fail(BMO_EINVAL, "bmo_psf_intensity: n must be >= 1");
-    if (pose < 0 || pose >= sys->view.n_poses) return fail(BMO_EINVAL, "bmo_psf_intensity: pose out of range");
+    if ((rc = psf_check(sys, psf_object, who))) return rc;
+    if (!p || !lims || !intensity) return fail(BMO_EINVAL, std::string(who) + ": NULL argument");
+    if (n < 1) return fail(BMO_EINVAL, std::string(who) + ": n must be >= 1");
+    if (pose < 0 || pose >= sys->view.n_poses) return fail(BMO_EINVAL, std::string(who) + ": pose out of range");
+    return BMO_OK;
+}
+
+// K6 on columns [j0, j1) of the map, enqueued on the context's stream between evk0 and evk1; no launch for an empty range
+int32_t bmo::psf_intensity_band(bmo_sys* sys, const bmo_psf* p, int32_t psf_object, int32_t pose, int32_t n, const double* lims,
+                                double x0_shift, double z0_shift, int32_t j0, int32_t j1, double* d_out) {
+    if (j1 == j0) return BMO_OK;
     bmo_ctx* ctx = sys->ctx;
-    BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const bool on_dev = flags & BMO_INPUT_DEVICE;
-    double* d_out = intensity;
-    if (!on_dev) BMO_CUDA(dev_alloc(&d_out, (size_t)n * n, st));
     PsfParams pp{};
     pp.fast = p->fast; pp.n_hits = p->n; pp.dp = sys->view.det_pose + 12 * ((int64_t)pose * sys->view.n_objects + psf_object);
     pp.x_lo = lims[0]; pp.x_hi = lims[1]; pp.z_lo = lims[2]; pp.z_hi = lims[3]; pp.x_shift = x0_shift; pp.z_shift = z0_shift;
-    pp.n = n; pp.out = d_out;
-    dim3 grid((n + PSF_TX - 1) / PSF_TX, (n + PSF_TY - 1) / PSF_TY), block(PSF_TX, PSF_TY);
+    pp.n = n; pp.j0 = j0; pp.j1 = j1; pp.out = d_out;
+    dim3 grid((n + PSF_TX - 1) / PSF_TX, (j1 - j0 + PSF_TY - 1) / PSF_TY), block(PSF_TX, PSF_TY);
     BMO_CUDA(cudaEventRecord(ctx->evk0, st));
     psf_intensity_kernel<<<grid, block, 0, st>>>(pp);
     BMO_CUDA(cudaEventRecord(ctx->evk1, st));
     ctx->launches++;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(BMO_ECUDA, std::string("psf_intensity: ") + cudaGetErrorString(e));
-    if (!on_dev) BMO_CUDA(cudaMemcpyAsync(intensity, d_out, (size_t)n * n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    ctx->psf_pairs += (int64_t)n * (j1 - j0) * p->n;
+    return BMO_OK;
+}
+
+// bmo_psf_intensity and bmo_psf_intensity_cols: columns [j0, j1) to a host or device buffer of n * (j1 - j0) doubles
+static int32_t psf_intensity_cols(const char* who, bmo_sys* sys, bmo_psf* p, int32_t psf_object, int32_t pose, int32_t n, const double* lims,
+                                  double x0_shift, double z0_shift, int32_t j0, int32_t j1, double* intensity, uint32_t flags) {
+    int32_t rc;
+    if ((rc = psf_intensity_check(who, sys, p, psf_object, pose, n, lims, intensity))) return rc;
+    if (!(0 <= j0 && j0 <= j1 && j1 <= n)) return fail(BMO_EINVAL, std::string(who) + ": column range outside 0 <= j0 <= j1 <= n");
+    if (j1 == j0) return BMO_OK;
+    bmo_ctx* ctx = sys->ctx;
+    BMO_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const bool on_dev = flags & BMO_INPUT_DEVICE;
+    const size_t n_out = (size_t)n * (size_t)(j1 - j0);
+    double* d_out = intensity;
+    if (!on_dev) BMO_CUDA(dev_alloc(&d_out, n_out, st));
+    if ((rc = psf_intensity_band(sys, p, psf_object, pose, n, lims, x0_shift, z0_shift, j0, j1, d_out))) return rc;
+    if (!on_dev) BMO_CUDA(cudaMemcpyAsync(intensity, d_out, n_out * sizeof(double), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
     float kms = 0;
     BMO_CUDA(cudaEventElapsedTime(&kms, ctx->evk0, ctx->evk1));
     ctx->psf_ms = kms;
-    ctx->psf_pairs += (int64_t)n * n * p->n;
     if (!on_dev) dev_free(d_out, st);
     return BMO_OK;
+}
+
+int32_t bmo_psf_intensity(bmo_sys* sys, bmo_psf* p, int32_t psf_object, int32_t pose, int32_t n, const double* lims, double x0_shift,
+                          double z0_shift, double* intensity, uint32_t flags) {
+    NvtxRange nvtx_("bmo_psf_intensity");
+    return psf_intensity_cols("bmo_psf_intensity", sys, p, psf_object, pose, n, lims, x0_shift, z0_shift, 0, n, intensity, flags);
+}
+
+int32_t bmo_psf_intensity_cols(bmo_sys* sys, bmo_psf* p, int32_t psf_object, int32_t pose, int32_t n, const double* lims, double x0_shift,
+                               double z0_shift, int32_t j0, int32_t j1, double* intensity, uint32_t flags) {
+    NvtxRange nvtx_("bmo_psf_intensity_cols");
+    return psf_intensity_cols("bmo_psf_intensity_cols", sys, p, psf_object, pose, n, lims, x0_shift, z0_shift, j0, j1, intensity, flags);
 }
 
 int32_t bmo_psf_count(bmo_psf* p, int64_t* n) {

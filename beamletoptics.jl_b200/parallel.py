@@ -8,7 +8,9 @@ diagram.  Each rank accumulates *its* beamlets onto a full n x n complex128 part
 fields are summed with one all-reduce of 2 n^2 doubles (the reference adds the beamlet fields serially into
 `pd.field`, Photodetector.jl:103; addition order across ranks changes the sum at the 1e-16 level).  A spot
 diagram of a DeviceSource sharded with spot_shard_slice is reduced where the hits are (solve_spot_sharded:
-bmo_spot_stats_sharded all-gathers per-block partials, not hits) and has the bits of the unsharded solve.
+bmo_spot_stats_sharded all-gathers per-block partials, not hits) and has the bits of the unsharded solve.  A PSFDetector map
+is sharded by pixel columns (solve_psf_sharded): the ranks all-gather their hit records in rank order, each sums all records
+into its band of columns, and the bands are all-gathered; for a splitter-free system the map has the bits of one solve.
 """
 import ctypes as C
 import math
@@ -73,6 +75,31 @@ class FieldComm:
         L.check(L.lib().bmo_spot_stats_sharded(self.h, None if result is None else result.h, int(det_object), L.ptr(win), int(nx), int(nz),
                                                C.byref(info), L.ptr(counts), 0))
         return _spot_dict(info, counts)
+
+    def psf_intensity(self, detector, n=100, crop_factor=1.0, center="centroid", x_min=math.inf, x_max=math.inf, z_min=math.inf,
+                      z_max=math.inf, x0_shift=0.0, z0_shift=0.0):
+        """PSFDetector.intensity over all ranks, collective: every rank passes its detector (after a solve, with or without hits
+        of its own) and receives (xs, zs, I) of the records of all ranks in rank order.  The records are all-gathered
+        (bmo_psf_allgather), the window is calc_local_lims of the gathered records with the x_min / z_min overrides of
+        PSFDetector.intensity, and bmo_psf_intensity_sharded computes this rank's band of pixel columns and all-gathers the
+        bands.  BmoError on every rank if any rank's arguments are refused."""
+        from .solver import psf_axes, psf_window
+        if detector._dsys is None:
+            raise L.BmoError("FieldComm.psf_intensity: the PSFDetector was not solved on this rank")
+        dsys, oi = detector._dsys, detector._index
+        lib = L.lib()
+        all_ = C.c_void_p()
+        L.check(lib.bmo_psf_allgather(self.h, C.c_void_p(detector._psf) if detector._psf else None, C.byref(all_)))
+        try:
+            lims = np.zeros(4)
+            L.check(lib.bmo_psf_lims(dsys.h, all_, oi, 0, float(crop_factor), 0 if center == "centroid" else 1, L.ptr(lims)))
+            lims = psf_window(lims, x_min, x_max, z_min, z_max)
+            I = np.zeros((n, n), order="F")
+            L.check(lib.bmo_psf_intensity_sharded(self.h, dsys.h, all_, oi, 0, int(n), L.ptr(lims), float(x0_shift), float(z0_shift),
+                                                  L.ptr(I), 0))
+        finally:
+            lib.bmo_psf_free(all_)
+        return psf_axes(n, lims, x0_shift, z0_shift) + (I,)
 
     def free(self):
         if self.h:
@@ -215,6 +242,38 @@ def solve_spot_sharded(system, source, detector, bins=None, window=None, comm=No
     dsys = res.dsys if res is not None else cached_system(system, _lambda_ids([source.lam])[0], comm.device)
     oi, nx, nz, win = _spot_args(dsys.flat.objects, detector, bins, window, "solve_spot_sharded")
     return comm.spot_stats(res, oi, nx, nz, win)
+
+
+def psf_shard_band(n, rank, world_size):
+    """Pixel columns [j0, j1) of rank `rank` in bmo_psf_intensity_sharded: bands of B = ceil(n / world_size) columns in rank
+    order, the last one cut at n; ranks past the last column get an empty band."""
+    B = -(-int(n) // int(world_size))
+    return min(n, rank * B), min(n, (rank + 1) * B)
+
+
+def solve_psf_sharded(system, source, detector, n=100, crop_factor=1.0, center="centroid", x_min=math.inf, x_max=math.inf,
+                      z_min=math.inf, z_max=math.inf, x0_shift=0.0, z0_shift=0.0, comm=None, r_max=100):
+    """The intensity map of `detector` (a PSFDetector of `system`) for a DeviceSource or RayBundle traced across all ranks: this
+    rank traces its shard_slice of the source (DeviceSource.shard / shard_bundle) on the communicator's GPU, its records are
+    appended to the detector as by solve_system_, and FieldComm.psf_intensity makes the map of all ranks' records.  Returns
+    (xs, zs, I) on every rank: for a system without beamsplitters the bits of solve_system_ of the whole source followed by
+    detector.intensity(...) on one GPU.  `comm`: a FieldComm (default: default_comm(), a one-rank communicator outside
+    torchrun).  A rank with an empty slice traces nothing and contributes no records."""
+    from .solver import _lambda_ids, cached_system, solve_system_
+    comm = default_comm() if comm is None else comm
+    first, stop = shard_slice(len(source), comm.rank, comm.world_size)
+    if isinstance(source, bm.DeviceSource):
+        part = source.shard(first, stop - first) if stop > first else None
+        lams = [source.lam]
+    else:
+        part = shard_bundle(source, comm.rank, comm.world_size)[0] if stop > first else None
+        lams = source.lam
+    if part is not None:
+        solve_system_(system, part, r_max=r_max, retrace=False, device=comm.device)
+    elif detector._dsys is None:          # no rays here: the detector's system and index for the collective
+        dsys = cached_system(system, _lambda_ids(lams)[0], comm.device)
+        detector._dsys, detector._index = dsys, next(i for i, o in enumerate(dsys.flat.objects) if o is detector)
+    return comm.psf_intensity(detector, n, crop_factor, center, x_min, x_max, z_min, z_max, x0_shift, z0_shift)
 
 
 def solve_system_sharded(system, bundle, r_max=100, interleaved=False, keep_segments=False, group=None, comm=None):

@@ -611,18 +611,29 @@ def psf_lims(psf, crop_factor=1.0, center="centroid"):
 def psf_intensity(psf, n=100, crop_factor=1.0, center="centroid", x_min=np.inf, x_max=np.inf, z_min=np.inf, z_max=np.inf,
                   x0_shift=0.0, z0_shift=0.0):
     dsys, oi = _psf_dsys(psf)
-    lims = list(psf_lims(psf, crop_factor, center))
-    if x_min != np.inf and x_max != np.inf:          # PSFDetector.jl:202-205
+    lims = psf_window(psf_lims(psf, crop_factor, center), x_min, x_max, z_min, z_max)
+    I = np.zeros((n, n), order="F")
+    L.check(L.lib().bmo_psf_intensity(dsys.h, C.c_void_p(psf._psf), oi, 0, int(n), L.ptr(lims), float(x0_shift), float(z0_shift), L.ptr(I), 0))
+    return psf_axes(n, lims, x0_shift, z0_shift) + (I,)
+
+
+def psf_window(lims, x_min=np.inf, x_max=np.inf, z_min=np.inf, z_max=np.inf):
+    """The (x_min, x_max, z_min, z_max) float64 array intensity(psf; ...) sums over: calc_local_lims's `lims`, with each axis
+    replaced where both of its bounds are given (PSFDetector.jl:202-205)."""
+    lims = [float(v) for v in lims]
+    if x_min != np.inf and x_max != np.inf:
         lims[0], lims[1] = float(x_min), float(x_max)
     if z_min != np.inf and z_max != np.inf:
         lims[2], lims[3] = float(z_min), float(z_max)
-    lims = np.array(lims, dtype=np.float64)
-    I = np.zeros((n, n), order="F")
-    L.check(L.lib().bmo_psf_intensity(dsys.h, C.c_void_p(psf._psf), oi, 0, int(n), L.ptr(lims), float(x0_shift), float(z0_shift), L.ptr(I), 0))
+    return np.array(lims, dtype=np.float64)
+
+
+def psf_axes(n, lims, x0_shift=0.0, z0_shift=0.0):
+    """(xs, zs) of an n x n intensity map over the window `lims`: LinRange(lo, hi, n) .+ shift (PSFDetector.jl:202-211)."""
     t = np.arange(n) / (n - 1) if n > 1 else np.zeros(1)
     xs = ((1 - t) * lims[0] + t * lims[1]) + x0_shift
     zs = ((1 - t) * lims[2] + t * lims[3]) + z0_shift
-    return xs, zs, I
+    return xs, zs
 
 
 def _accumulate_pds(dsys, res):

@@ -446,6 +446,12 @@ int32_t bmo_psf_lims(bmo_sys* sys, bmo_psf* psf, int32_t psf_object, int32_t pos
  * device pointer with BMO_INPUT_DEVICE.                                                                     */
 int32_t bmo_psf_intensity(bmo_sys* sys, bmo_psf* psf, int32_t psf_object, int32_t pose, int32_t n, const double* lims,
                           double x0_shift, double z0_shift, double* intensity, uint32_t flags);
+/* Columns [j0, j1) of bmo_psf_intensity's map: intensity[i + n*(j - j0)] for j in [j0, j1), n * (j1 - j0) doubles, with the bits
+ * bmo_psf_intensity gives those pixels (a pixel's sum depends only on (i, j), lims, the shifts and the records in order).  Host
+ * pointer, or device pointer with BMO_INPUT_DEVICE.  BMO_EINVAL unless 0 <= j0 <= j1 <= n (an empty range writes nothing); otherwise
+ * bmo_psf_intensity's checks.  The building block of a column-sharded map for a host that brings its own transport.           */
+int32_t bmo_psf_intensity_cols(bmo_sys* sys, bmo_psf* psf, int32_t psf_object, int32_t pose, int32_t n, const double* lims,
+                               double x0_shift, double z0_shift, int32_t j0, int32_t j1, double* intensity, uint32_t flags);
 int32_t bmo_psf_free(bmo_psf* psf);   /* empty!(psf) */
 
 /* pose sweep in one call: replaces the loop `translate3d!(mirror, ...); empty!(pd); solve_system!(system, beam);
@@ -490,6 +496,22 @@ int32_t bmo_pd_allreduce_local(int32_t n, bmo_comm* const* comms, double* const*
  * and leaves the other ranks waiting in the next collective, as any failed NCCL collective does.                     */
 int32_t bmo_spot_stats_sharded(bmo_comm* comm, bmo_result* r, int32_t det_object, const double* window, int32_t nx, int32_t nz,
                                bmo_spot_info* out, int64_t* counts, uint32_t flags);
+/* PSFDetector records of a ray bundle sharded over ranks, collective: every rank receives in *all a new handle, freed with
+ * bmo_psf_free, holding all ranks' records in rank order; `local` may be NULL on a rank without hits.  Steps, on the context's
+ * stream: (1) all-gather of each rank's record count and argument verdict (`local` on another context than comm, all NULL, a
+ * total that overflows int64); a refusal on any rank makes every rank return the same code; (2) one all-gather of both record
+ * arrays, padded to the largest count, each rank's part then copied into place.  With one rank, a device copy of `local`.  A
+ * CUDA or NCCL failure returns on the failing rank alone, as in bmo_spot_stats_sharded.                                  */
+int32_t bmo_psf_allgather(bmo_comm* comm, bmo_psf* local, bmo_psf** all);
+/* bmo_psf_intensity over ranks, collective: every rank passes the same gathered records (bmo_psf_allgather) and arguments and
+ * receives the whole n x n map (host pointer, or device pointer with BMO_INPUT_DEVICE).  Rank r sums every record into its band of
+ * pixel columns [r B, min(n, (r + 1) B)), B = ceil(n / n_ranks), and the bands are all-gathered: the map has bmo_psf_intensity's
+ * bits for the same records.  Step (1) all-gathers each rank's verdict (bmo_psf_intensity's checks; sys or psf on another
+ * context), n, pose, psf_object, the bits of lims and of the shifts, and the record count; a refusal or a mismatch with rank 0
+ * (a rank that passes its own, ungathered records holds another count) makes every rank return the same code.  With one rank
+ * there is no NCCL call.  Only arguments are agreed on, as in bmo_spot_stats_sharded.                                     */
+int32_t bmo_psf_intensity_sharded(bmo_comm* comm, bmo_sys* sys, bmo_psf* all, int32_t psf_object, int32_t pose, int32_t n,
+                                  const double* lims, double x0_shift, double z0_shift, double* intensity, uint32_t flags);
 int32_t bmo_comm_free(bmo_comm* comm);
 
 /* Give device memory back: the library keeps released blocks of 64 MiB and more in a per-device free list and smaller ones in
