@@ -3,6 +3,8 @@
 //
 //   interact3d(::AbstractSystem, ::PSFDetector, ::Beam{T, Ray{T}}, ::Ray) (:77-89) stores, per hit,
 //   position, direction, optical_path_length(beam), |dir . normal| and 2pi/lambda  -> psf_flag / psf_build
+//   (a GaussianBeamlet reaches it through the generic interact3d, Gaussian.jl:124-135: one record each for
+//   the chief, waist and divergence beam)
 //   calc_local_pos / calc_local_lims (:91-141)                                      -> psf_local / psf_reduce
 //   intensity(psf; n, ...) (:190-237): I[i, j] = | sum_h proj_h cis(k_h (opl_h + (p_ij - hit_h) . dir_h)) |^2
 //                                                                                  -> psf_intensity_kernel
@@ -20,16 +22,19 @@ struct PsfView {
     const double* seg_d; const int32_t* seg_part; int64_t rows; int nsd;   // segment table: row records [rows][nsd]
     const int32_t *nseg, *status, *lam, *parent;
     const long long* first_seg;
+    const double* popl;    // beamlets: OPL of the parent's chief beam (the tracer's running sum, also read by K4)
     int64_t n_beams;
+    int rays;              // rows per segment: 1, or 3 for beamlets (chief, waist, divergence interleaved)
 };
 
-// flags[b] = 1 if beam b ended on object `psf` (its last stored ray has an intersection with it)
+// flags[b] = 1 if beam b ended on object `psf` (its last stored ray -- a beamlet's chief ray -- has an intersection with it).
+// A torn or clipped beamlet never reached interact3d (System.jl:288-304): its status is not BMO_ST_ABSORBED.
 __global__ void psf_flag(PsfView R, SysView S, int psf_object, int32_t* flags) {
     const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= R.n_beams) return;
     int f = 0;
     if ((R.status[b] & 0xff) == BMO_ST_ABSORBED && R.nseg[b] > 0) {
-        const int part = R.seg_part[R.first_seg[b] + R.nseg[b] - 1];
+        const int part = R.seg_part[(R.first_seg[b] + R.nseg[b] - 1) * R.rays];
         if (part >= 0 && S.parts[part].object == psf_object) f = 1;
     }
     flags[b] = f;
@@ -51,24 +56,41 @@ __device__ double beam_opl(const PsfView& R, int b) {
     }
     return l0;
 }
+// optical_path_length of ray q of beamlet b (Beam.jl:137-149): only the chief beam has a parent (Gaussian.jl:107-111), whose
+// OPL the tracer kept in popl; then the beam's own rows in order.  No walk up the beamlet tree, so its depth is unbounded.
+__device__ double beamlet_opl(const PsfView& R, int64_t b, int q) {
+    double l0 = q == 0 ? R.popl[b] : 0.0;
+    const int64_t f = R.first_seg[b];
+    for (int s = 0; s < R.nseg[b]; s++) {
+        const int64_t row = (f + s) * 3 + q;
+        const double t = R.seg_d[(size_t)row * R.nsd + S_T];
+        if (isinf(t)) break;
+        l0 += t * R.seg_d[(size_t)row * R.nsd + S_N];
+    }
+    return l0;
+}
+// one thread per record: record q of flagged beam b goes to base + rays * offs[b] + q (a beamlet: chief, waist, divergence)
 __global__ void psf_build(PsfView R, SysView S, const int32_t* flags, const long long* offs, int64_t base, double* rec, double* fast) {
-    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= R.n_beams || !flags[b]) return;
-    const int64_t row = R.first_seg[b] + R.nseg[b] - 1;
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= R.n_beams * R.rays) return;
+    const int64_t b = i / R.rays;
+    const int q = (int)(i - b * R.rays);
+    if (!flags[b]) return;
+    const int64_t row = (R.first_seg[b] + R.nseg[b] - 1) * R.rays + q;
     const double* d = R.seg_d;
-    const int64_t rows = R.rows;
     const V3 pos = mk3(d[(size_t)(row) * R.nsd + S_PX], d[(size_t)(row) * R.nsd + S_PY], d[(size_t)(row) * R.nsd + S_PZ]);
     const V3 dir = mk3(d[(size_t)(row) * R.nsd + S_DX], d[(size_t)(row) * R.nsd + S_DY], d[(size_t)(row) * R.nsd + S_DZ]);
     const V3 nrm = mk3(d[(size_t)(row) * R.nsd + S_NX], d[(size_t)(row) * R.nsd + S_NY], d[(size_t)(row) * R.nsd + S_NZ]);
     const double t = d[(size_t)(row) * R.nsd + S_T];
     const V3 hit = pos + t * dir;
-    const double opl = beam_opl(R, (int)b);
+    const double opl = R.rays == 1 ? beam_opl(R, (int)b) : beamlet_opl(R, b, q);
     const double proj = fabs(dot(dir, nrm));
     const double k = kTwoPi / S.lambdas[R.lam[b]];
-    double* r = rec + (base + offs[b]) * PSF_NREC;
+    const int64_t o = base + R.rays * offs[b] + q;
+    double* r = rec + o * PSF_NREC;
     r[0] = hit.x; r[1] = hit.y; r[2] = hit.z; r[3] = dir.x; r[4] = dir.y; r[5] = dir.z; r[6] = opl; r[7] = proj; r[8] = k;
-    double* q = fast + (base + offs[b]) * PSF_NFAST;
-    q[0] = k * (opl - dot(hit, dir)); q[1] = k * dir.x; q[2] = k * dir.y; q[3] = k * dir.z; q[4] = proj;
+    double* qf = fast + o * PSF_NFAST;
+    qf[0] = k * (opl - dot(hit, dir)); qf[1] = k * dir.x; qf[2] = k * dir.y; qf[3] = k * dir.z; qf[4] = proj;
 }
 
 // local (x, z) of every hit (calc_local_pos, PSFDetector.jl:91-101)
@@ -188,7 +210,6 @@ int32_t bmo_psf_collect(bmo_sys* sys, bmo_result* r, int32_t psf_object, bmo_psf
     int32_t rc;
     if ((rc = psf_check(sys, psf_object, "bmo_psf_collect"))) return rc;
     if (!r || !psf) return fail(BMO_EINVAL, "bmo_psf_collect: NULL argument");
-    if (r->mode == 2) return fail(BMO_EINVAL, "bmo_psf_collect: GaussianBeamlet results are not supported (PSFDetector.jl:44-45: only Beam)");
     if (!r->keep || !r->seg_d) return fail(BMO_ESTATE, "bmo_psf_collect: the result has no segment table (trace with BMO_KEEP_SEGMENTS)");
     bmo_ctx* ctx = sys->ctx;
     BMO_CUDA(cudaSetDevice(ctx->device));
@@ -203,16 +224,16 @@ int32_t bmo_psf_collect(bmo_sys* sys, bmo_result* r, int32_t psf_object, bmo_psf
     BMO_CUDA(dev_alloc(&d_offs, (size_t)nb, st));
     PsfView v;
     v.seg_d = r->seg_d; v.seg_part = r->seg_part; v.rows = r->seg_rows; v.nsd = r->nsd; v.nseg = r->nseg; v.status = r->status; v.lam = r->lam;
-    v.parent = r->parent; v.first_seg = r->first_seg; v.n_beams = nb;
+    v.parent = r->parent; v.first_seg = r->first_seg; v.popl = r->popl; v.n_beams = nb; v.rays = r->mode == 2 ? 3 : 1;
     psf_flag<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(v, sys->view, psf_object, d_flags);
     scan_flags<<<1, 1024, 0, st>>>(d_flags, nb, d_offs, ctx->d_totals);
     ctx->launches += 2;
     BMO_CUDA(cudaMemcpyAsync(ctx->h_totals, ctx->d_totals, sizeof(long long), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
-    const int64_t m = ctx->h_totals[0];
+    const int64_t m = ctx->h_totals[0] * v.rays;    // records: one per ray of every flagged beam
     if (m > 0) {
         if ((rc = psf_reserve(p, p->n + m, st))) return rc;
-        psf_build<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(v, sys->view, d_flags, d_offs, p->n, p->rec, p->fast);
+        psf_build<<<(unsigned)((nb * v.rays + 255) / 256), 256, 0, st>>>(v, sys->view, d_flags, d_offs, p->n, p->rec, p->fast);
         ctx->launches++;
         p->n += m;
     }

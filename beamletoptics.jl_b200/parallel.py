@@ -253,8 +253,8 @@ def psf_shard_band(n, rank, world_size):
 
 def solve_psf_sharded(system, source, detector, n=100, crop_factor=1.0, center="centroid", x_min=math.inf, x_max=math.inf,
                       z_min=math.inf, z_max=math.inf, x0_shift=0.0, z0_shift=0.0, comm=None, r_max=100):
-    """The intensity map of `detector` (a PSFDetector of `system`) for a DeviceSource or RayBundle traced across all ranks: this
-    rank traces its shard_slice of the source (DeviceSource.shard / shard_bundle) on the communicator's GPU, its records are
+    """The intensity map of `detector` (a PSFDetector of `system`) for a DeviceSource, RayBundle or BeamletBundle traced across all
+    ranks: this rank traces its shard_slice of the source (DeviceSource.shard / shard_bundle) on the communicator's GPU, its records are
     appended to the detector as by solve_system_, and FieldComm.psf_intensity makes the map of all ranks' records.  Returns
     (xs, zs, I) on every rank: for a system without beamsplitters the bits of solve_system_ of the whole source followed by
     detector.intensity(...) on one GPU.  `comm`: a FieldComm (default: default_comm(), a one-rank communicator outside

@@ -423,6 +423,7 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
         _rebuild_gauss(beam, res, dsys.flat)
         if collect_spots:
             _collect_spots(dsys.flat, res)
+        _collect_psfs(dsys, res)
         _accumulate_pds(dsys, res)
         return res
     if isinstance(beam, bm.RayBundle):
@@ -482,6 +483,7 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
         res._root_sig = _root_signature(beam)
         if collect_spots:
             _collect_spots(dsys.flat, res)
+        _collect_psfs(dsys, res)
         _accumulate_pds(dsys, res)
         return res
     raise TypeError(f"cannot trace {type(beam).__name__}")
@@ -562,7 +564,7 @@ def spot_stats_poses(result, detector, n_poses, bins=None, window=None):
 # ---- PSFDetector (PSFDetector.jl) -----------------------------------------------------------------------
 def _collect_psfs(dsys, res):
     """interact3d(::PSFDetector, ::Beam, ::Ray) of every beam that ended on a PSF detector (push! order is
-    irrelevant for the sums that use the data)."""
+    irrelevant for the sums that use the data); a GaussianBeamlet pushes three records: chief, waist, divergence."""
     for oi, o in enumerate(dsys.flat.objects):
         if isinstance(o, co.PSFDetector):
             h = C.c_void_p(o._psf) if o._psf else C.c_void_p()

@@ -433,7 +433,12 @@ int32_t bmo_pd_power(bmo_sys* sys, int32_t pd_object, int32_t n_fields, const do
  * beam of `r` that ended on `psf_object`: hit position, direction, optical_path_length(beam) (through the
  * parents), |dir . normal| and 2 pi / lambda are appended to *psf (created when *psf == NULL; the reference's
  * detector also accumulates until empty!).  `r` must hold its segment table; PolarizedRay results add nothing
- * (no interact3d method, AbstractSystem.jl:30-33); GaussianBeamlet results are rejected.                      */
+ * (no interact3d method, AbstractSystem.jl:30-33).
+ * GaussianBeamlet results (Gaussian.jl:124-135): every beamlet absorbed with its chief ray on `psf_object` appends three
+ * records, chief, waist, divergence, each from its own ray's last hit (position, direction, |dir . normal|) with the
+ * beamlet's 2 pi / lambda.  OPL: the chief's is the OPL of the parent's chief beam (the children of a beamsplitter link only
+ * their chief beam to the parent, Gaussian.jl:107-111), at any depth of the beamlet tree, plus the chief's own t * n in
+ * order; the waist's and divergence's are their own t * n only.  A torn or clipped beamlet appends nothing.         */
 typedef struct bmo_psf bmo_psf;
 int32_t bmo_psf_collect(bmo_sys* sys, bmo_result* r, int32_t psf_object, bmo_psf** psf, int64_t* n_total);
 int32_t bmo_psf_count(bmo_psf* psf, int64_t* n);

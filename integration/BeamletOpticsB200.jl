@@ -294,7 +294,8 @@ end
 BeamletOptics.solve_system!(cs::CUDASystem, bg::BeamletOptics.AbstractBeamGroup; kw...) = BeamletOptics.solve_system!(cs, BeamletOptics.beams(bg); kw...)
 BeamletOptics.solve_system!(cs::CUDASystem, b::Beam; kw...) = BeamletOptics.solve_system!(cs, [b]; kw...)
 
-"""GaussianBeamlets: `bmo_trace_beamlets`, then `bmo_pd_accumulate` adds into every `Photodetector.field`."""
+"""GaussianBeamlets: `bmo_trace_beamlets`, then `bmo_pd_accumulate` adds into every `Photodetector.field` and
+`bmo_psf_collect` appends to every `PSFDetector`."""
 function BeamletOptics.solve_system!(cs::CUDASystem, gs::AbstractVector{<:GaussianBeamlet}; r_max = 100, retrace = true)
     λs = unique(Float64(g.λ) for g in gs)
     f = flatten(cs, λs); sys = upload(cs, f)
@@ -318,6 +319,7 @@ function BeamletOptics.solve_system!(cs::CUDASystem, gs::AbstractVector{<:Gaussi
             (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int32, Ptr{ComplexF64}, UInt32), sys, res[], oi - 1, 0, fld, UInt32(0)))
     end
     collect_spots!(f, res[])
+    collect_psfs!(f, sys, res[])                     # three records per beamlet: chief, waist, divergence
     rebuild_beamlets!(gs, f, res[])
     ccall((:bmo_result_free, libbmo), Int32, (Ptr{Cvoid},), res[])
     return nothing
