@@ -110,11 +110,11 @@ int32_t bmo_comm_init(bmo_ctx* ctx, int32_t n_ranks, int32_t rank, const uint8_t
     BMO_CUDA(cudaSetDevice(ctx->device));
     NcclUniqueId u;
     std::memcpy(u.internal, id, BMO_COMM_ID_BYTES);
-    bmo_comm* c = new bmo_comm();
+    std::unique_ptr<bmo_comm, FreeWith<bmo_comm_free>> c(new bmo_comm());
     c->ctx = ctx; c->rank = rank; c->n_ranks = n_ranks;
     int r = g_nccl.CommInitRank(&c->comm, n_ranks, u, rank);
-    if (r != 0) { delete c; return fail(BMO_ENCCL, std::string("ncclCommInitRank: ") + g_nccl.GetErrorString(r)); }
-    *out = c;
+    if (r != 0) return fail(BMO_ENCCL, std::string("ncclCommInitRank: ") + g_nccl.GetErrorString(r));
+    *out = c.release();
     return BMO_OK;
 }
 
@@ -233,19 +233,15 @@ static int32_t agree(bmo_comm* c, const std::string& fn, const std::vector<int64
     all.assign(K * W, 0);
     cudaStream_t st = c->ctx->stream;
     BMO_CUDA(cudaSetDevice(c->ctx->device));
-    int64_t* d = nullptr;
-    BMO_CUDA(dev_alloc(&d, K * (W + 1), st));
-    cudaError_t e = cudaMemcpyAsync(d, mine.data(), K * sizeof(int64_t), cudaMemcpyHostToDevice, st);
-    int nr = 0;
-    if (e == cudaSuccess) {
-        nr = W == 1 ? cudaMemcpyAsync(d + K, d, K * sizeof(int64_t), cudaMemcpyDeviceToDevice, st) != cudaSuccess
-                    : g_nccl.AllGather(d, d + K, K, kNcclInt64, c->comm, st);
-        if (!nr) e = cudaMemcpyAsync(all.data(), d + K, all.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
-        if (!nr && e == cudaSuccess) e = cudaStreamSynchronize(st);
-    }
-    dev_free(d, st);
-    if (e != cudaSuccess) return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e));
+    DevBuf<int64_t> buf;
+    BMO_CUDA(buf.alloc(K * (W + 1), st));
+    int64_t* d = buf.get();
+    BMO_CUDA(cudaMemcpyAsync(d, mine.data(), K * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    const int nr = W == 1 ? cudaMemcpyAsync(d + K, d, K * sizeof(int64_t), cudaMemcpyDeviceToDevice, st) != cudaSuccess
+                          : g_nccl.AllGather(d, d + K, K, kNcclInt64, c->comm, st);
     if (nr) return fail(BMO_ENCCL, fn + ": exchanging the arguments: " + (W == 1 ? std::string("copy failed") : std::string(g_nccl.GetErrorString(nr))));
+    BMO_CUDA(cudaMemcpyAsync(all.data(), d + K, all.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    BMO_CUDA(cudaStreamSynchronize(st));
     for (int k = 0; k < W; k++) {
         const int32_t v = (int32_t)all[K * k];
         if (v) {
@@ -318,47 +314,38 @@ int32_t bmo_psf_allgather(bmo_comm* c, bmo_psf* local, bmo_psf** all_out) {
     // Step 2: one all-gather of [most][PSF_NREC] records then [most][PSF_NFAST] fast words per rank, each rank's part copied into place
     bmo_ctx* ctx = c->ctx;
     cudaStream_t st = ctx->stream;
-    bmo_psf* p = new bmo_psf();
+    std::unique_ptr<bmo_psf, FreeWith<bmo_psf_free>> p(new bmo_psf());
     p->ctx = ctx;
-    auto done = [&](int32_t code) {
-        if (code) bmo_psf_free(p);
-        else *all_out = p;
-        return code;
-    };
-    if ((rc = psf_reserve(p, total, st))) return done(rc);
+    if ((rc = psf_reserve(p.get(), total, st))) return rc;
     p->n = total;
-    if (total == 0) return done(BMO_OK);
     const int64_t m = local ? local->n : 0;
     constexpr size_t D = sizeof(double);
     const size_t per = (size_t)most * (PSF_NREC + PSF_NFAST);   // doubles per rank
-    double* buf = nullptr;
-    rc = [&]() -> int32_t {
-        if (W == 1) {     // no exchange: a copy of this rank's records
-            BMO_CUDA(cudaMemcpyAsync(p->rec, local->rec, (size_t)m * PSF_NREC * D, cudaMemcpyDeviceToDevice, st));
-            BMO_CUDA(cudaMemcpyAsync(p->fast, local->fast, (size_t)m * PSF_NFAST * D, cudaMemcpyDeviceToDevice, st));
-            BMO_CUDA(cudaStreamSynchronize(st));
-            return BMO_OK;
-        }
-        BMO_CUDA(dev_alloc(&buf, per * (W + 1), st));
-        double* send = buf + per * W;
+    if (total > 0 && W == 1) {     // no exchange: a copy of this rank's records
+        BMO_CUDA(cudaMemcpyAsync(p->rec, local->rec, (size_t)m * PSF_NREC * D, cudaMemcpyDeviceToDevice, st));
+        BMO_CUDA(cudaMemcpyAsync(p->fast, local->fast, (size_t)m * PSF_NFAST * D, cudaMemcpyDeviceToDevice, st));
+        BMO_CUDA(cudaStreamSynchronize(st));
+    } else if (total > 0) {
+        DevBuf<double> buf;
+        BMO_CUDA(buf.alloc(per * (W + 1), st));
+        double* send = buf.get() + per * W;
         if (m) {
             BMO_CUDA(cudaMemcpyAsync(send, local->rec, (size_t)m * PSF_NREC * D, cudaMemcpyDeviceToDevice, st));
             BMO_CUDA(cudaMemcpyAsync(send + (size_t)most * PSF_NREC, local->fast, (size_t)m * PSF_NFAST * D, cudaMemcpyDeviceToDevice, st));
         }
-        BMO_NCCL(g_nccl.AllGather(send, buf, per, kNcclDouble, c->comm, st));
+        BMO_NCCL(g_nccl.AllGather(send, buf.get(), per, kNcclDouble, c->comm, st));
         for (int k = 0; k < W; k++) {
             const int64_t mk = all[2 * k + 1];
             if (!mk) continue;
-            const double* part = buf + per * k;
+            const double* part = buf.get() + per * k;
             BMO_CUDA(cudaMemcpyAsync(p->rec + first[k] * PSF_NREC, part, (size_t)mk * PSF_NREC * D, cudaMemcpyDeviceToDevice, st));
             BMO_CUDA(cudaMemcpyAsync(p->fast + first[k] * PSF_NFAST, part + (size_t)most * PSF_NREC, (size_t)mk * PSF_NFAST * D,
                                      cudaMemcpyDeviceToDevice, st));
         }
         BMO_CUDA(cudaStreamSynchronize(st));
-        return BMO_OK;
-    }();
-    dev_free(buf, st);
-    return done(rc);
+    }
+    *all_out = p.release();
+    return BMO_OK;
 }
 
 int32_t bmo_psf_intensity_sharded(bmo_comm* c, bmo_sys* sys, bmo_psf* all, int32_t psf_object, int32_t pose, int32_t n, const double* lims,
@@ -392,23 +379,22 @@ int32_t bmo_psf_intensity_sharded(bmo_comm* c, bmo_sys* sys, bmo_psf* all, int32
     const size_t nn = (size_t)n * n, band = (size_t)n * B;
     const bool on_dev = flags & BMO_INPUT_DEVICE;
     double* d_map = intensity;      // the caller's device buffer when the bands exactly fill it
-    if (!on_dev || band * W != nn) BMO_CUDA(dev_alloc(&d_map, band * W, st));
-    rc = [&]() -> int32_t {
-        int32_t r;
-        if ((r = psf_intensity_band(sys, all, psf_object, pose, n, lims, x0_shift, z0_shift, j0, j1, d_map + band * c->rank))) return r;
-        if (W > 1) BMO_NCCL(g_nccl.AllGather(d_map + band * c->rank, d_map, band, kNcclDouble, c->comm, st));
-        if (d_map != intensity)
-            BMO_CUDA(cudaMemcpyAsync(intensity, d_map, nn * sizeof(double), on_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
-        BMO_CUDA(cudaStreamSynchronize(st));
-        if (j1 > j0) {
-            float kms = 0;
-            BMO_CUDA(cudaEventElapsedTime(&kms, ctx->evk0, ctx->evk1));
-            ctx->psf_ms = kms;
-        }
-        return BMO_OK;
-    }();
-    if (d_map != intensity) dev_free(d_map, st);
-    return rc;
+    DevBuf<double> map_copy;
+    if (!on_dev || band * W != nn) {
+        BMO_CUDA(map_copy.alloc(band * W, st));
+        d_map = map_copy.get();
+    }
+    if ((rc = psf_intensity_band(sys, all, psf_object, pose, n, lims, x0_shift, z0_shift, j0, j1, d_map + band * c->rank))) return rc;
+    if (W > 1) BMO_NCCL(g_nccl.AllGather(d_map + band * c->rank, d_map, band, kNcclDouble, c->comm, st));
+    if (d_map != intensity)
+        BMO_CUDA(cudaMemcpyAsync(intensity, d_map, nn * sizeof(double), on_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
+    BMO_CUDA(cudaStreamSynchronize(st));
+    if (j1 > j0) {
+        float kms = 0;
+        BMO_CUDA(cudaEventElapsedTime(&kms, ctx->evk0, ctx->evk1));
+        ctx->psf_ms = kms;
+    }
+    return BMO_OK;
 }
 
 int32_t bmo_comm_free(bmo_comm* c) {

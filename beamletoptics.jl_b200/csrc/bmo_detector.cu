@@ -425,14 +425,12 @@ __global__ void __launch_bounds__(256) pd_power_reduce(const double* s_col, int 
 }
 // both steps on stream st; d_power: [n_fields] on the device
 static int32_t pd_power_launch(bmo_ctx* ctx, const double* d_fields, int n_fields, int n, double lo, double hi, double* d_power, cudaStream_t st) {
-    double* s_col = nullptr;
-    BMO_CUDA(dev_alloc(&s_col, (size_t)n_fields * n, st));
-    pd_power_columns<<<dim3((n + PWR_WARPS - 1) / PWR_WARPS, n_fields), 32 * PWR_WARPS, 0, st>>>(d_fields, n, lo, hi, s_col);
-    pd_power_reduce<<<n_fields, 256, 0, st>>>(s_col, n, lo, hi, d_power);
-    ctx->launches += 2;
-    cudaError_t e = cudaGetLastError();
-    dev_free(s_col, st);
-    if (e != cudaSuccess) return fail(BMO_ECUDA, std::string("pd_power: ") + cudaGetErrorString(e));
+    DevBuf<double> s_col;
+    BMO_CUDA(s_col.alloc((size_t)n_fields * n, st));
+    pd_power_columns<<<dim3((n + PWR_WARPS - 1) / PWR_WARPS, n_fields), 32 * PWR_WARPS, 0, st>>>(d_fields, n, lo, hi, s_col.get());
+    BMO_LAUNCH(ctx, "pd_power_columns");
+    pd_power_reduce<<<n_fields, 256, 0, st>>>(s_col.get(), n, lo, hi, d_power);
+    BMO_LAUNCH(ctx, "pd_power_reduce");
     return BMO_OK;
 }
 
@@ -487,32 +485,36 @@ static int32_t pd_run(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t po
     const bool on_dev = flags & BMO_INPUT_DEVICE;
     BMO_CUDA(cudaEventRecord(ctx->ev0, st));
     double* d_field = fields;
+    DevBuf<double> field_copy;   // of a host field
     if (!on_dev) {
-        BMO_CUDA(dev_alloc(&d_field, (size_t)n_fields * n * n * 2, st));
+        BMO_CUDA(field_copy.alloc((size_t)n_fields * n * n * 2, st));
+        d_field = field_copy.get();
         BMO_CUDA(cudaMemcpyAsync(d_field, fields, fbytes, cudaMemcpyHostToDevice, st));
     }
-    int32_t* d_flags = nullptr; long long* d_offs = nullptr; PdRec* d_recs = nullptr; long long* d_pose_off = nullptr;
-    PdFast* d_fast = nullptr;
+    DevBuf<int32_t> d_flags;
+    DevBuf<long long> d_offs, d_pose_off;
+    DevBuf<PdRec> d_recs;
+    DevBuf<PdFast> d_fast;
     const bool ref_order = flags & BMO_PD_REFERENCE_ORDER;
     const int64_t nb = r->n_beams;
-    BMO_CUDA(dev_alloc(&d_flags, (size_t)nb, st));
-    BMO_CUDA(dev_alloc(&d_offs, (size_t)nb, st));
+    BMO_CUDA(d_flags.alloc((size_t)nb, st));
+    BMO_CUDA(d_offs.alloc((size_t)nb, st));
     ResView rv = res_view(r);
-    pd_flag<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(rv, sys->view, pd_object, per_pose ? -1 : pose0, d_flags);
-    ctx->launches++;
-    scan_flags<<<1, 1024, 0, st>>>(d_flags, nb, d_offs, ctx->d_totals);
-    ctx->launches++;
+    pd_flag<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(rv, sys->view, pd_object, per_pose ? -1 : pose0, d_flags.get());
+    BMO_LAUNCH(ctx, "pd_flag");
+    scan_flags<<<1, 1024, 0, st>>>(d_flags.get(), nb, d_offs.get(), ctx->d_totals);
+    BMO_LAUNCH(ctx, "scan_flags");
     BMO_CUDA(cudaMemcpyAsync(ctx->h_totals, ctx->d_totals, sizeof(long long), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
     const int64_t m = ctx->h_totals[0];
     if (m > 0) {
-        BMO_CUDA(dev_alloc(&d_recs, (size_t)m, st));
-        pd_build<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(rv, sys->view, d_flags, d_offs, d_recs);
-        ctx->launches++;
+        BMO_CUDA(d_recs.alloc((size_t)m, st));
+        pd_build<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(rv, sys->view, d_flags.get(), d_offs.get(), d_recs.get());
+        BMO_LAUNCH(ctx, "pd_build");
         if (per_pose) {
             // group the records by pose (stable): tiny host round trip (m records)
             std::vector<PdRec> h((size_t)m);
-            BMO_CUDA(cudaMemcpyAsync(h.data(), d_recs, (size_t)m * sizeof(PdRec), cudaMemcpyDeviceToHost, st));
+            BMO_CUDA(cudaMemcpyAsync(h.data(), d_recs.get(), (size_t)m * sizeof(PdRec), cudaMemcpyDeviceToHost, st));
             BMO_CUDA(cudaStreamSynchronize(st));
             std::stable_sort(h.begin(), h.end(), [](const PdRec& a, const PdRec& b) { return a.pose < b.pose; });
             std::vector<long long> off((size_t)n_fields + 1, 0);
@@ -523,18 +525,19 @@ static int32_t pd_run(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t po
             }
             while (q < h.size() && (int)h[q].pose < pose0 + n_fields) q++;
             off[n_fields] = (long long)q;
-            BMO_CUDA(cudaMemcpyAsync(d_recs, h.data(), (size_t)m * sizeof(PdRec), cudaMemcpyHostToDevice, st));
-            BMO_CUDA(dev_alloc(&d_pose_off, off.size(), st));
-            BMO_CUDA(cudaMemcpyAsync(d_pose_off, off.data(), off.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+            BMO_CUDA(cudaMemcpyAsync(d_recs.get(), h.data(), (size_t)m * sizeof(PdRec), cudaMemcpyHostToDevice, st));
+            BMO_CUDA(d_pose_off.alloc(off.size(), st));
+            BMO_CUDA(cudaMemcpyAsync(d_pose_off.get(), off.data(), off.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
             BMO_CUDA(cudaStreamSynchronize(st));
         }
         if (!ref_order) {
-            BMO_CUDA(dev_alloc(&d_fast, (size_t)m, st));
-            pd_make_fast<<<(unsigned)((m + 127) / 128), 128, 0, st>>>(d_recs, d_fast, m);
-            ctx->launches++;
+            BMO_CUDA(d_fast.alloc((size_t)m, st));
+            pd_make_fast<<<(unsigned)((m + 127) / 128), 128, 0, st>>>(d_recs.get(), d_fast.get(), m);
+            BMO_LAUNCH(ctx, "pd_make_fast");
         }
         PdParams pp{};
-        pp.recs = d_recs; pp.fast = d_fast; pp.n_recs = m; pp.R = rv; pp.field = d_field; pp.det_pose = sys->view.det_pose; pp.pose_off = d_pose_off;
+        pp.recs = d_recs.get(); pp.fast = d_fast.get(); pp.n_recs = m; pp.R = rv; pp.field = d_field; pp.det_pose = sys->view.det_pose;
+        pp.pose_off = d_pose_off.get();
         pp.n = n; pp.pd_object = pd_object; pp.n_objects = sys->view.n_objects; pp.pose0 = pose0; pp.lo = ob.pd_lo; pp.hi = ob.pd_hi;
         BMO_CUDA(cudaEventRecord(ctx->evk0, st));
         if (ref_order) {
@@ -544,10 +547,8 @@ static int32_t pd_run(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t po
             dim3 grid((n + PDF_TX - 1) / PDF_TX, (n + PDF_TY * PDF_PX - 1) / (PDF_TY * PDF_PX), n_fields), block(PDF_TX, PDF_TY);
             pd_field_fast<<<grid, block, 0, st>>>(pp);
         }
+        BMO_LAUNCH(ctx, "pd_field");
         BMO_CUDA(cudaEventRecord(ctx->evk1, st));
-        ctx->launches++;
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return fail(BMO_ECUDA, std::string("pd_field: ") + cudaGetErrorString(e));
         ctx->px_beamlets += m * (int64_t)n * n;
     }
     if (!on_dev) {
@@ -559,8 +560,6 @@ static int32_t pd_run(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t po
     BMO_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
     ctx->pd_ms = ms;
     if (m > 0) { float kms = 0; BMO_CUDA(cudaEventElapsedTime(&kms, ctx->evk0, ctx->evk1)); ctx->k4_ms += kms; }
-    if (!on_dev) dev_free(d_field, st);
-    dev_free(d_flags, st); dev_free(d_offs, st); dev_free(d_recs, st); dev_free(d_pose_off, st); dev_free(d_fast, st);
     return BMO_OK;
 }
 
@@ -585,19 +584,18 @@ int32_t bmo_pd_sweep(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t n_p
     const bmo_object& ob = sys->objects[pd_object];
     const int n = ob.pd_n;
     const size_t cnt = (size_t)n_poses * n * n * 2;
-    double* d_field = nullptr; double* d_p = nullptr;
-    BMO_CUDA(dev_alloc(&d_field, cnt, st));
-    BMO_CUDA(cudaMemsetAsync(d_field, 0, cnt * sizeof(double), st));
-    int32_t rc = pd_run(sys, r, pd_object, 0, n_poses, d_field, (flags | BMO_INPUT_DEVICE), true);
-    if (rc) { dev_free(d_field, st); return rc; }
+    DevBuf<double> d_field, d_p;
+    BMO_CUDA(d_field.alloc(cnt, st));
+    BMO_CUDA(cudaMemsetAsync(d_field.get(), 0, cnt * sizeof(double), st));
+    int32_t rc = pd_run(sys, r, pd_object, 0, n_poses, d_field.get(), (flags | BMO_INPUT_DEVICE), true);
+    if (rc) return rc;
     if (power) {
-        BMO_CUDA(dev_alloc(&d_p, (size_t)n_poses, st));
-        if ((rc = pd_power_launch(ctx, d_field, n_poses, n, ob.pd_lo, ob.pd_hi, d_p, st))) { dev_free(d_field, st); dev_free(d_p, st); return rc; }
-        BMO_CUDA(cudaMemcpyAsync(power, d_p, (size_t)n_poses * sizeof(double), cudaMemcpyDeviceToHost, st));
+        BMO_CUDA(d_p.alloc((size_t)n_poses, st));
+        if ((rc = pd_power_launch(ctx, d_field.get(), n_poses, n, ob.pd_lo, ob.pd_hi, d_p.get(), st))) return rc;
+        BMO_CUDA(cudaMemcpyAsync(power, d_p.get(), (size_t)n_poses * sizeof(double), cudaMemcpyDeviceToHost, st));
     }
-    if (fields) BMO_CUDA(cudaMemcpyAsync(fields, d_field, cnt * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (fields) BMO_CUDA(cudaMemcpyAsync(fields, d_field.get(), cnt * sizeof(double), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
-    dev_free(d_field, st); dev_free(d_p, st);
     return BMO_OK;
 }
 int32_t bmo_pd_power(bmo_sys* sys, int32_t pd_object, int32_t n_fields, const double* fields, double* power, uint32_t flags) {
@@ -611,18 +609,19 @@ int32_t bmo_pd_power(bmo_sys* sys, int32_t pd_object, int32_t n_fields, const do
     const int n = ob.pd_n;
     const bool on_dev = flags & BMO_INPUT_DEVICE;
     const double* d_f = fields;
-    double* d_tmp = nullptr; double* d_p = nullptr;
+    double* d_p = power;
+    DevBuf<double> f_copy, p_copy;   // of host fields and power
     if (!on_dev) {
-        BMO_CUDA(dev_alloc(&d_tmp, (size_t)n_fields * n * n * 2, st));
-        BMO_CUDA(cudaMemcpyAsync(d_tmp, fields, (size_t)n_fields * n * n * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
-        d_f = d_tmp;
-        BMO_CUDA(dev_alloc(&d_p, (size_t)n_fields, st));
-    } else d_p = power;
+        BMO_CUDA(f_copy.alloc((size_t)n_fields * n * n * 2, st));
+        BMO_CUDA(cudaMemcpyAsync(f_copy.get(), fields, (size_t)n_fields * n * n * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
+        d_f = f_copy.get();
+        BMO_CUDA(p_copy.alloc((size_t)n_fields, st));
+        d_p = p_copy.get();
+    }
     { int32_t rc = pd_power_launch(ctx, d_f, n_fields, n, ob.pd_lo, ob.pd_hi, d_p, st); if (rc) return rc; }
     if (!on_dev) {
         BMO_CUDA(cudaMemcpyAsync(power, d_p, (size_t)n_fields * sizeof(double), cudaMemcpyDeviceToHost, st));
         BMO_CUDA(cudaStreamSynchronize(st));
-        dev_free(d_tmp, st); dev_free(d_p, st);
     }
     return BMO_OK;
 }

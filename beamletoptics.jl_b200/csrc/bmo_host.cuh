@@ -1,10 +1,17 @@
 // bmo_host.cuh -- host-side state of libbmo.so: context, uploaded system, result tables, error
-// handling and the BVH builder.  Shared by bmo_trace.cu and bmo_detector.cu.
+// handling, device-memory owners and the BVH builder.  Shared by every .cu file of the library.
+//
+// Ownership: a C-ABI call holds each temporary device allocation in a DevBuf, so that any early return frees it.  The
+// long-lived objects (bmo_ctx, bmo_sys, bmo_result, bmo_psf, bmo_source, bmo_comm) are freed by their own free function
+// only; while a call builds one it holds it in a std::unique_ptr with that function as deleter (FreeWith) and hands it out
+// on success.  A call that replaces live tables of an object builds the new ones in owners first and swaps them in only
+// when everything has succeeded.
 #pragma once
 #include <algorithm>
 #include <cstdio>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <utility>
@@ -59,6 +66,24 @@ struct bmo_ctx {
     int persist_blocks = -1;
 };
 
+namespace bmo {
+// Every kernel launch is followed by this check: it counts the launch in ctx->launches and reports a launch error from the
+// call that made it, not from some later call.
+inline int32_t launch_check(bmo_ctx* ctx, const char* what) {
+    ctx->launches++;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(BMO_ECUDA, std::string(what) + ": " + cudaGetErrorString(e));
+    return BMO_OK;
+}
+// Owner of a cudaMalloc'ed table of an uploaded system (bmo_sys): freed with the system, or when a new table replaces it.
+struct CudaFree { void operator()(void* p) const { cudaFree(p); } };
+template <class T> using DevTable = std::unique_ptr<T, CudaFree>;
+// Owner of a long-lived C-ABI object while it is being built: freed by the object's own free function (bmo_system_free, ...)
+// unless the call succeeds and releases it to the caller.
+template <auto Free> struct FreeWith { template <class T> void operator()(T* p) const { Free(p); } };
+}  // namespace bmo
+#define BMO_LAUNCH(ctx, what) do { int32_t rc_ = bmo::launch_check(ctx, what); if (rc_) return rc_; } while (0)
+
 struct bmo_sys {
     bmo_ctx* ctx = nullptr;
     bmo::SysView view{};         // device pointers
@@ -71,17 +96,17 @@ struct bmo_sys {
     int64_t n_vertices = 0, n_faces = 0;
     bool has_rare = false;       // some primitive is a cylindrical / aspheric surface: the trace kernels compiled with them are used
     bool all_lean = false;       // every SDF part is a union of <= 4 plain primitives and no mesh has a BVH: the LEAN trace kernels are used
-    // owned device buffers
-    bmo_prim* d_prims = nullptr; bmo_part* d_parts = nullptr; bmo_object* d_objects = nullptr;
-    bmo::MeshView* d_meshes = nullptr; double* d_vertices = nullptr; int32_t* d_faces = nullptr;
-    bmo::BvhNode* d_nodes = nullptr; int32_t* d_bvh_faces = nullptr; double* d_ntable = nullptr;
-    double* d_bounds = nullptr; double* d_detpose = nullptr; double* d_lambdas = nullptr; double* d_jones = nullptr; double* d_ext = nullptr;
+    // owned device tables (`view` holds the same addresses)
+    bmo::DevTable<bmo_prim> d_prims; bmo::DevTable<bmo_part> d_parts; bmo::DevTable<bmo_object> d_objects;
+    bmo::DevTable<bmo::MeshView> d_meshes; bmo::DevTable<double> d_vertices; bmo::DevTable<int32_t> d_faces;
+    bmo::DevTable<bmo::BvhNode> d_nodes; bmo::DevTable<int32_t> d_bvh_faces; bmo::DevTable<double> d_ntable;
+    bmo::DevTable<double> d_bounds, d_detpose, d_lambdas, d_jones, d_ext;
     // pose-0 copies to restore after a sweep
     std::vector<double> h_vertices, h_bounds, h_detpose;
     // K5 (bmo_pose.cu): kinematic tree + the uploaded tables every pose starts from
     std::vector<bmo_kin_node> kin_nodes;
-    bmo_kin_node* d_kin_nodes = nullptr; double* d_prim_bounds = nullptr;
-    bmo_prim* d_prims0 = nullptr; double* d_vertices0 = nullptr; double* d_detpose0 = nullptr;
+    bmo::DevTable<bmo_kin_node> d_kin_nodes; bmo::DevTable<double> d_prim_bounds;
+    bmo::DevTable<bmo_prim> d_prims0; bmo::DevTable<double> d_vertices0, d_detpose0;
     // high-water marks of earlier branching traces, keyed by (mode, root beams): queue units, beams and scratch
     // units the call ended with.  The next call of the same shape allocates them up front (no growth copies,
     // identical request sizes for the pool).
@@ -272,14 +297,49 @@ struct BigBlocks {
         return true;
     }
 };
+// *p = NULL when the allocation fails
 template <class T> inline cudaError_t dev_alloc(T** p, size_t n, cudaStream_t s) {
     const size_t bytes = size_class(std::max<size_t>(n, 1) * sizeof(T));
-    if (bytes >= BigBlocks::kMin) return BigBlocks::of_device().get((void**)p, bytes, s);
-    return cudaMallocAsync((void**)p, bytes, s);
+    void* q = nullptr;
+    const cudaError_t e = bytes >= BigBlocks::kMin ? BigBlocks::of_device().get(&q, bytes, s) : cudaMallocAsync(&q, bytes, s);
+    *p = e == cudaSuccess ? (T*)q : nullptr;
+    return e;
 }
 template <class T> inline void dev_free(T*& p, cudaStream_t s) {
     if (p && !BigBlocks::of_device().put((void*)p, s)) cudaFreeAsync((void*)p, s);
     p = nullptr;
+}
+
+// Owner of one dev_alloc block: freed (stream-ordered, on the stream it was allocated on) when the owner goes out of scope, so
+// that every early return of a C-ABI call releases its temporaries.
+template <class T> class DevBuf {
+public:
+    DevBuf() = default;
+    DevBuf(DevBuf&& o) noexcept : p_(o.p_), st_(o.st_) { o.p_ = nullptr; }
+    DevBuf& operator=(DevBuf&& o) noexcept {
+        if (this != &o) { reset(); p_ = o.p_; st_ = o.st_; o.p_ = nullptr; }
+        return *this;
+    }
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() { reset(); }
+    cudaError_t alloc(size_t n, cudaStream_t st) { reset(); st_ = st; return dev_alloc(&p_, n, st); }
+    T* get() const { return p_; }
+    void reset() { dev_free(p_, st_); }
+    T* release() { T* p = p_; p_ = nullptr; return p; }   // hand the block to a long-lived object
+private:
+    T* p_ = nullptr;
+    cudaStream_t st_ = nullptr;
+};
+
+// A cudaMalloc'ed table of n elements (at least one), filled from the host when h is given: *out only on success
+template <class T> inline int32_t upload(DevTable<T>& out, const T* h, size_t n) {
+    T* p = nullptr;
+    BMO_CUDA(cudaMalloc((void**)&p, std::max<size_t>(n, 1) * sizeof(T)));
+    DevTable<T> t(p);
+    if (h && n) BMO_CUDA(cudaMemcpy(p, h, n * sizeof(T), cudaMemcpyHostToDevice));
+    out = std::move(t);
+    return BMO_OK;
 }
 
 // ---- spot statistics (bmo_source.cu), shared with bmo_spot_stats_sharded (bmo_comm.cu) ---------------------------

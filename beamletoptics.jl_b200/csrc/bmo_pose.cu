@@ -251,13 +251,6 @@ __global__ void __launch_bounds__(PBLOCK) apply_poses_kernel(const PoseParams P)
 
 }  // namespace bmo
 
-template <class T> static int32_t up(T** dptr, const T* h, size_t n) {
-    if (*dptr) { cudaFree(*dptr); *dptr = nullptr; }
-    BMO_CUDA(cudaMalloc((void**)dptr, std::max<size_t>(n, 1) * sizeof(T)));
-    if (n) BMO_CUDA(cudaMemcpy(*dptr, h, n * sizeof(T), cudaMemcpyHostToDevice));
-    return BMO_OK;
-}
-
 int32_t bmo_system_set_kinematics(bmo_sys* s, int32_t n_nodes, const bmo_kin_node* nodes, const double* prim_bounds) {
     if (!s || n_nodes < 1 || !nodes || (!prim_bounds && !s->prims.empty())) return fail(BMO_EINVAL, "bmo_system_set_kinematics: bad arguments");
     const int n_prims = (int)s->prims.size(), n_meshes = (int)s->meshes.size(), n_objects = (int)s->objects.size();
@@ -288,13 +281,17 @@ int32_t bmo_system_set_kinematics(bmo_sys* s, int32_t n_nodes, const bmo_kin_nod
     }
     BMO_CUDA(cudaSetDevice(s->ctx->device));
     BMO_CUDA(cudaStreamSynchronize(s->ctx->stream));
-    s->kin_nodes.assign(nodes, nodes + n_nodes);
+    // the new tables replace the live ones only once all of them are on the device
+    DevTable<bmo_kin_node> d_kin_nodes; DevTable<double> d_prim_bounds; DevTable<bmo_prim> d_prims0; DevTable<double> d_vertices0, d_detpose0;
     int32_t rc;
-    if ((rc = up(&s->d_kin_nodes, nodes, (size_t)n_nodes))) return rc;
-    if ((rc = up(&s->d_prim_bounds, prim_bounds, (size_t)10 * n_prims))) return rc;
-    if ((rc = up(&s->d_prims0, s->prims.data(), s->prims.size()))) return rc;
-    if ((rc = up(&s->d_vertices0, s->h_vertices.data(), s->h_vertices.size()))) return rc;
-    if ((rc = up(&s->d_detpose0, s->h_detpose.data(), s->h_detpose.size()))) return rc;
+    if ((rc = upload(d_kin_nodes, nodes, (size_t)n_nodes))) return rc;
+    if ((rc = upload(d_prim_bounds, prim_bounds, (size_t)10 * n_prims))) return rc;
+    if ((rc = upload(d_prims0, s->prims.data(), s->prims.size()))) return rc;
+    if ((rc = upload(d_vertices0, s->h_vertices.data(), s->h_vertices.size()))) return rc;
+    if ((rc = upload(d_detpose0, s->h_detpose.data(), s->h_detpose.size()))) return rc;
+    s->kin_nodes.assign(nodes, nodes + n_nodes);
+    s->d_kin_nodes = std::move(d_kin_nodes); s->d_prim_bounds = std::move(d_prim_bounds); s->d_prims0 = std::move(d_prims0);
+    s->d_vertices0 = std::move(d_vertices0); s->d_detpose0 = std::move(d_detpose0);
     return BMO_OK;
 }
 
@@ -318,44 +315,40 @@ int32_t bmo_system_apply_poses(bmo_sys* s, int32_t n_poses, int32_t n_ops, const
             for (int j = op.node; j < op.node + nd.size; j++)
                 if (s->kin_nodes[j].kind == BMO_KIN_MESH && s->meshes[s->kin_nodes[j].index].n_nodes > 0) mesh_with_bvh_moves = true;
     }
+    const size_t smem = (size_t)n_nodes * 12 * sizeof(double);
+    if (smem > 200 * 1024) return fail(BMO_EINVAL, "bmo_system_apply_poses: kinematic tree too large for one block's shared memory");
     bmo_ctx* ctx = s->ctx;
     BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     BMO_CUDA(cudaStreamSynchronize(st));
     const size_t np = (size_t)n_poses, n_prims = s->prims.size(), n_parts = s->parts.size(), n_objects = s->objects.size();
-    auto renew = [&](auto** dptr, size_t n) -> int32_t {
-        if (*dptr) { cudaFree(*dptr); *dptr = nullptr; }
-        BMO_CUDA(cudaMalloc((void**)dptr, std::max<size_t>(n, 1) * sizeof(**dptr)));
-        return BMO_OK;
-    };
+    // the kernel writes new tables; they replace the live ones only once it has run
+    DevTable<bmo_prim> d_prims; DevTable<double> d_vertices, d_bounds, d_detpose;
     int32_t rc;
-    if ((rc = renew(&s->d_prims, np * n_prims))) return rc;
-    if ((rc = renew(&s->d_vertices, np * 3 * (size_t)s->n_vertices))) return rc;
-    if ((rc = renew(&s->d_bounds, np * NBOUND * n_parts))) return rc;
-    if ((rc = renew(&s->d_detpose, np * 12 * n_objects))) return rc;
-    bmo_kin_op* d_ops = nullptr; double* d_par = nullptr;
-    BMO_CUDA(cudaMalloc((void**)&d_ops, std::max<size_t>(n_ops, 1) * sizeof(bmo_kin_op)));
-    BMO_CUDA(cudaMalloc((void**)&d_par, std::max<size_t>(np * n_params * 9, 1) * sizeof(double)));
-    if (n_ops) BMO_CUDA(cudaMemcpyAsync(d_ops, ops, (size_t)n_ops * sizeof(bmo_kin_op), cudaMemcpyHostToDevice, st));
-    if (n_params) BMO_CUDA(cudaMemcpyAsync(d_par, params, np * n_params * 9 * sizeof(double), cudaMemcpyHostToDevice, st));
+    if ((rc = upload(d_prims, (const bmo_prim*)nullptr, np * n_prims))) return rc;
+    if ((rc = upload(d_vertices, (const double*)nullptr, np * 3 * (size_t)s->n_vertices))) return rc;
+    if ((rc = upload(d_bounds, (const double*)nullptr, np * NBOUND * n_parts))) return rc;
+    if ((rc = upload(d_detpose, (const double*)nullptr, np * 12 * n_objects))) return rc;
+    DevBuf<bmo_kin_op> d_ops;
+    DevBuf<double> d_par;
+    BMO_CUDA(d_ops.alloc((size_t)n_ops, st));
+    BMO_CUDA(d_par.alloc(np * n_params * 9, st));
+    if (n_ops) BMO_CUDA(cudaMemcpyAsync(d_ops.get(), ops, (size_t)n_ops * sizeof(bmo_kin_op), cudaMemcpyHostToDevice, st));
+    if (n_params) BMO_CUDA(cudaMemcpyAsync(d_par.get(), params, np * n_params * 9 * sizeof(double), cudaMemcpyHostToDevice, st));
     PoseParams P{};
-    P.nodes = s->d_kin_nodes; P.n_nodes = n_nodes; P.ops = d_ops; P.n_ops = n_ops; P.params = d_par; P.n_params = n_params;
-    P.prims0 = s->d_prims0; P.n_prims = (int32_t)n_prims; P.parts = s->d_parts; P.n_parts = (int32_t)n_parts;
-    P.meshes = s->d_meshes; P.n_meshes = (int32_t)s->meshes.size(); P.vertices0 = s->d_vertices0; P.n_vertices = s->n_vertices;
-    P.detpose0 = s->d_detpose0; P.n_objects = (int32_t)n_objects; P.prim_bounds = s->d_prim_bounds;
-    P.prims = s->d_prims; P.vertices = s->d_vertices; P.bounds = s->d_bounds; P.detpose = s->d_detpose;
+    P.nodes = s->d_kin_nodes.get(); P.n_nodes = n_nodes; P.ops = d_ops.get(); P.n_ops = n_ops; P.params = d_par.get(); P.n_params = n_params;
+    P.prims0 = s->d_prims0.get(); P.n_prims = (int32_t)n_prims; P.parts = s->d_parts.get(); P.n_parts = (int32_t)n_parts;
+    P.meshes = s->d_meshes.get(); P.n_meshes = (int32_t)s->meshes.size(); P.vertices0 = s->d_vertices0.get(); P.n_vertices = s->n_vertices;
+    P.detpose0 = s->d_detpose0.get(); P.n_objects = (int32_t)n_objects; P.prim_bounds = s->d_prim_bounds.get();
+    P.prims = d_prims.get(); P.vertices = d_vertices.get(); P.bounds = d_bounds.get(); P.detpose = d_detpose.get();
     P.bound_rel = 1e-9; P.bound_abs = 1e-6;   // flatten.py BOUND_REL / BOUND_ABS
-    const size_t smem = (size_t)n_nodes * 12 * sizeof(double);
-    if (smem > 200 * 1024) { cudaFree(d_ops); cudaFree(d_par); return fail(BMO_EINVAL, "bmo_system_apply_poses: kinematic tree too large for one block's shared memory"); }
     if (smem > 48 * 1024) BMO_CUDA(cudaFuncSetAttribute(apply_poses_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     apply_poses_kernel<<<(unsigned)n_poses, PBLOCK, smem, st>>>(P);
-    ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    cudaFree(d_ops); cudaFree(d_par);
-    if (e != cudaSuccess) return fail(BMO_ECUDA, std::string("apply_poses_kernel: ") + cudaGetErrorString(e));
+    BMO_LAUNCH(ctx, "apply_poses_kernel");
+    BMO_CUDA(cudaStreamSynchronize(st));
+    s->d_prims = std::move(d_prims); s->d_vertices = std::move(d_vertices); s->d_bounds = std::move(d_bounds); s->d_detpose = std::move(d_detpose);
     SysView& v = s->view;
-    v.prims = s->d_prims; v.vertices = s->d_vertices; v.bounds = s->d_bounds; v.det_pose = s->d_detpose;
+    v.prims = s->d_prims.get(); v.vertices = s->d_vertices.get(); v.bounds = s->d_bounds.get(); v.det_pose = s->d_detpose.get();
     v.n_poses = n_poses;
     v.bvh_ok = mesh_with_bvh_moves ? 0 : 1;
     return BMO_OK;
@@ -366,9 +359,9 @@ int32_t bmo_system_get_pose(bmo_sys* s, int32_t pose, bmo_prim* prims, double* v
     BMO_CUDA(cudaSetDevice(s->ctx->device));
     BMO_CUDA(cudaStreamSynchronize(s->ctx->stream));
     const size_t n_prims = s->prims.size(), n_parts = s->parts.size(), n_objects = s->objects.size(), p = (size_t)pose;
-    if (prims && n_prims) BMO_CUDA(cudaMemcpy(prims, s->d_prims + p * n_prims, n_prims * sizeof(bmo_prim), cudaMemcpyDeviceToHost));
-    if (vertices && s->n_vertices) BMO_CUDA(cudaMemcpy(vertices, s->d_vertices + p * 3 * s->n_vertices, (size_t)3 * s->n_vertices * sizeof(double), cudaMemcpyDeviceToHost));
-    if (bounds) BMO_CUDA(cudaMemcpy(bounds, s->d_bounds + p * NBOUND * n_parts, NBOUND * n_parts * sizeof(double), cudaMemcpyDeviceToHost));
-    if (det_pose) BMO_CUDA(cudaMemcpy(det_pose, s->d_detpose + p * 12 * n_objects, 12 * n_objects * sizeof(double), cudaMemcpyDeviceToHost));
+    if (prims && n_prims) BMO_CUDA(cudaMemcpy(prims, s->d_prims.get() + p * n_prims, n_prims * sizeof(bmo_prim), cudaMemcpyDeviceToHost));
+    if (vertices && s->n_vertices) BMO_CUDA(cudaMemcpy(vertices, s->d_vertices.get() + p * 3 * s->n_vertices, (size_t)3 * s->n_vertices * sizeof(double), cudaMemcpyDeviceToHost));
+    if (bounds) BMO_CUDA(cudaMemcpy(bounds, s->d_bounds.get() + p * NBOUND * n_parts, NBOUND * n_parts * sizeof(double), cudaMemcpyDeviceToHost));
+    if (det_pose) BMO_CUDA(cudaMemcpy(det_pose, s->d_detpose.get() + p * 12 * n_objects, 12 * n_objects * sizeof(double), cudaMemcpyDeviceToHost));
     return BMO_OK;
 }

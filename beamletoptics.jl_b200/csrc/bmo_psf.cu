@@ -187,15 +187,15 @@ namespace bmo { __global__ void scan_flags(const int32_t* in, int64_t n, long lo
 int32_t bmo::psf_reserve(bmo_psf* p, int64_t need, cudaStream_t st) {
     if (need <= p->cap) return BMO_OK;
     const int64_t cap = std::max<int64_t>(need, 2 * p->cap);
-    double *nr = nullptr, *nf = nullptr;
-    BMO_CUDA(dev_alloc(&nr, (size_t)cap * PSF_NREC, st));
-    BMO_CUDA(dev_alloc(&nf, (size_t)cap * PSF_NFAST, st));
+    DevBuf<double> nr, nf;
+    BMO_CUDA(nr.alloc((size_t)cap * PSF_NREC, st));
+    BMO_CUDA(nf.alloc((size_t)cap * PSF_NFAST, st));
     if (p->n > 0) {
-        BMO_CUDA(cudaMemcpyAsync(nr, p->rec, (size_t)p->n * PSF_NREC * sizeof(double), cudaMemcpyDeviceToDevice, st));
-        BMO_CUDA(cudaMemcpyAsync(nf, p->fast, (size_t)p->n * PSF_NFAST * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        BMO_CUDA(cudaMemcpyAsync(nr.get(), p->rec, (size_t)p->n * PSF_NREC * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        BMO_CUDA(cudaMemcpyAsync(nf.get(), p->fast, (size_t)p->n * PSF_NFAST * sizeof(double), cudaMemcpyDeviceToDevice, st));
     }
     dev_free(p->rec, st); dev_free(p->fast, st);
-    p->rec = nr; p->fast = nf; p->cap = cap;
+    p->rec = nr.release(); p->fast = nf.release(); p->cap = cap;
     return BMO_OK;
 }
 
@@ -214,33 +214,35 @@ int32_t bmo_psf_collect(bmo_sys* sys, bmo_result* r, int32_t psf_object, bmo_psf
     bmo_ctx* ctx = sys->ctx;
     BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    if (!*psf) { *psf = new bmo_psf(); (*psf)->ctx = ctx; }
-    bmo_psf* p = *psf;
+    std::unique_ptr<bmo_psf, FreeWith<bmo_psf_free>> fresh;   // a new record set: the caller's once the call succeeds
+    if (!*psf) { fresh.reset(new bmo_psf()); fresh->ctx = ctx; }
+    bmo_psf* p = *psf ? *psf : fresh.get();
     if (p->ctx != ctx) return fail(BMO_EINVAL, "bmo_psf_collect: detector data lives on another context");
-    if (r->mode == 1) { if (n_total) *n_total = p->n; return BMO_OK; }   // PolarizedRay: no interact3d method -> no data (AbstractSystem.jl:30-33)
-    const int64_t nb = r->n_beams;
-    int32_t* d_flags = nullptr; long long* d_offs = nullptr;
-    BMO_CUDA(dev_alloc(&d_flags, (size_t)nb, st));
-    BMO_CUDA(dev_alloc(&d_offs, (size_t)nb, st));
-    PsfView v;
-    v.seg_d = r->seg_d; v.seg_part = r->seg_part; v.rows = r->seg_rows; v.nsd = r->nsd; v.nseg = r->nseg; v.status = r->status; v.lam = r->lam;
-    v.parent = r->parent; v.first_seg = r->first_seg; v.popl = r->popl; v.n_beams = nb; v.rays = r->mode == 2 ? 3 : 1;
-    psf_flag<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(v, sys->view, psf_object, d_flags);
-    scan_flags<<<1, 1024, 0, st>>>(d_flags, nb, d_offs, ctx->d_totals);
-    ctx->launches += 2;
-    BMO_CUDA(cudaMemcpyAsync(ctx->h_totals, ctx->d_totals, sizeof(long long), cudaMemcpyDeviceToHost, st));
-    BMO_CUDA(cudaStreamSynchronize(st));
-    const int64_t m = ctx->h_totals[0] * v.rays;    // records: one per ray of every flagged beam
-    if (m > 0) {
-        if ((rc = psf_reserve(p, p->n + m, st))) return rc;
-        psf_build<<<(unsigned)((nb * v.rays + 255) / 256), 256, 0, st>>>(v, sys->view, d_flags, d_offs, p->n, p->rec, p->fast);
-        ctx->launches++;
-        p->n += m;
+    if (r->mode != 1) {   // PolarizedRay: no interact3d method -> no data (AbstractSystem.jl:30-33)
+        const int64_t nb = r->n_beams;
+        DevBuf<int32_t> d_flags;
+        DevBuf<long long> d_offs;
+        BMO_CUDA(d_flags.alloc((size_t)nb, st));
+        BMO_CUDA(d_offs.alloc((size_t)nb, st));
+        PsfView v;
+        v.seg_d = r->seg_d; v.seg_part = r->seg_part; v.rows = r->seg_rows; v.nsd = r->nsd; v.nseg = r->nseg; v.status = r->status; v.lam = r->lam;
+        v.parent = r->parent; v.first_seg = r->first_seg; v.popl = r->popl; v.n_beams = nb; v.rays = r->mode == 2 ? 3 : 1;
+        psf_flag<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(v, sys->view, psf_object, d_flags.get());
+        BMO_LAUNCH(ctx, "psf_flag");
+        scan_flags<<<1, 1024, 0, st>>>(d_flags.get(), nb, d_offs.get(), ctx->d_totals);
+        BMO_LAUNCH(ctx, "scan_flags");
+        BMO_CUDA(cudaMemcpyAsync(ctx->h_totals, ctx->d_totals, sizeof(long long), cudaMemcpyDeviceToHost, st));
+        BMO_CUDA(cudaStreamSynchronize(st));
+        const int64_t m = ctx->h_totals[0] * v.rays;    // records: one per ray of every flagged beam
+        if (m > 0) {
+            if ((rc = psf_reserve(p, p->n + m, st))) return rc;
+            psf_build<<<(unsigned)((nb * v.rays + 255) / 256), 256, 0, st>>>(v, sys->view, d_flags.get(), d_offs.get(), p->n, p->rec, p->fast);
+            BMO_LAUNCH(ctx, "psf_build");
+            p->n += m;
+        }
+        BMO_CUDA(cudaStreamSynchronize(st));
     }
-    dev_free(d_flags, st); dev_free(d_offs, st);
-    BMO_CUDA(cudaStreamSynchronize(st));
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(BMO_ECUDA, std::string("bmo_psf_collect: ") + cudaGetErrorString(e));
+    if (fresh) *psf = fresh.release();
     if (n_total) *n_total = p->n;
     return BMO_OK;
 }
@@ -262,22 +264,23 @@ int32_t bmo_psf_lims(bmo_sys* sys, bmo_psf* p, int32_t psf_object, int32_t pose,
     bmo_ctx* ctx = sys->ctx;
     BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    double *xs = nullptr, *zs = nullptr, *d_out = nullptr;
-    BMO_CUDA(dev_alloc(&xs, (size_t)p->n, st)); BMO_CUDA(dev_alloc(&zs, (size_t)p->n, st)); BMO_CUDA(dev_alloc(&d_out, 8, st));
+    DevBuf<double> xs, zs, d_out;
+    BMO_CUDA(xs.alloc((size_t)p->n, st)); BMO_CUDA(zs.alloc((size_t)p->n, st)); BMO_CUDA(d_out.alloc(8, st));
     const double* dp = sys->view.det_pose + 12 * ((int64_t)pose * sys->view.n_objects + psf_object);
-    psf_local<<<(unsigned)((p->n + 255) / 256), 256, 0, st>>>(p->rec, p->n, dp, xs, zs);
-    psf_reduce<<<1, 512, 0, st>>>(p->rec, xs, zs, p->n, 0, 0.0, 0.0, d_out);
+    psf_local<<<(unsigned)((p->n + 255) / 256), 256, 0, st>>>(p->rec, p->n, dp, xs.get(), zs.get());
+    BMO_LAUNCH(ctx, "psf_local");
+    psf_reduce<<<1, 512, 0, st>>>(p->rec, xs.get(), zs.get(), p->n, 0, 0.0, 0.0, d_out.get());
+    BMO_LAUNCH(ctx, "psf_reduce");
     double h[7];
-    BMO_CUDA(cudaMemcpyAsync(h, d_out, sizeof(h), cudaMemcpyDeviceToHost, st));
+    BMO_CUDA(cudaMemcpyAsync(h, d_out.get(), sizeof(h), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
     double x0, z0;
     if (center == 0) { x0 = h[1] / h[0]; z0 = h[2] / h[0]; }          // :122-125 projection-weighted centroid
     else { x0 = (h[3] + h[4]) / 2; z0 = (h[5] + h[6]) / 2; }           // :127-128 bounding-box midpoint
-    psf_reduce<<<1, 512, 0, st>>>(p->rec, xs, zs, p->n, 1, x0, z0, d_out);
-    BMO_CUDA(cudaMemcpyAsync(h, d_out, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    psf_reduce<<<1, 512, 0, st>>>(p->rec, xs.get(), zs.get(), p->n, 1, x0, z0, d_out.get());
+    BMO_LAUNCH(ctx, "psf_reduce");
+    BMO_CUDA(cudaMemcpyAsync(h, d_out.get(), 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
-    ctx->launches += 3;
-    dev_free(xs, st); dev_free(zs, st); dev_free(d_out, st);
     const double hwx = h[0] * crop_factor, hwz = h[1] * crop_factor;
     lims[0] = x0 - hwx; lims[1] = x0 + hwx; lims[2] = z0 - hwz; lims[3] = z0 + hwz;
     return BMO_OK;
@@ -307,10 +310,8 @@ int32_t bmo::psf_intensity_band(bmo_sys* sys, const bmo_psf* p, int32_t psf_obje
     dim3 grid((n + PSF_TX - 1) / PSF_TX, (j1 - j0 + PSF_TY - 1) / PSF_TY), block(PSF_TX, PSF_TY);
     BMO_CUDA(cudaEventRecord(ctx->evk0, st));
     psf_intensity_kernel<<<grid, block, 0, st>>>(pp);
+    BMO_LAUNCH(ctx, "psf_intensity");
     BMO_CUDA(cudaEventRecord(ctx->evk1, st));
-    ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(BMO_ECUDA, std::string("psf_intensity: ") + cudaGetErrorString(e));
     ctx->psf_pairs += (int64_t)n * (j1 - j0) * p->n;
     return BMO_OK;
 }
@@ -328,14 +329,17 @@ static int32_t psf_intensity_cols(const char* who, bmo_sys* sys, bmo_psf* p, int
     const bool on_dev = flags & BMO_INPUT_DEVICE;
     const size_t n_out = (size_t)n * (size_t)(j1 - j0);
     double* d_out = intensity;
-    if (!on_dev) BMO_CUDA(dev_alloc(&d_out, n_out, st));
+    DevBuf<double> out_copy;   // of a host map
+    if (!on_dev) {
+        BMO_CUDA(out_copy.alloc(n_out, st));
+        d_out = out_copy.get();
+    }
     if ((rc = psf_intensity_band(sys, p, psf_object, pose, n, lims, x0_shift, z0_shift, j0, j1, d_out))) return rc;
     if (!on_dev) BMO_CUDA(cudaMemcpyAsync(intensity, d_out, n_out * sizeof(double), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
     float kms = 0;
     BMO_CUDA(cudaEventElapsedTime(&kms, ctx->evk0, ctx->evk1));
     ctx->psf_ms = kms;
-    if (!on_dev) dev_free(d_out, st);
     return BMO_OK;
 }
 

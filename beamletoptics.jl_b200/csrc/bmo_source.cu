@@ -386,13 +386,6 @@ struct bmo_source {
     int32_t* pose_id = nullptr; // [n], NULL for one pose
 };
 
-static int32_t launched(bmo_ctx* ctx, const char* what) {
-    ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(BMO_ECUDA, std::string(what) + ": " + cudaGetErrorString(e));
-    return BMO_OK;
-}
-
 static bool finite3(const double* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); }
 
 static int32_t check_desc(const bmo_source_desc* d) {
@@ -431,48 +424,38 @@ int32_t bmo_source_free(bmo_source* s) {
 }
 
 // n_poses copies of the rays [first, first + count) of the descriptor (n_poses > 1 only for the whole source)
-static int32_t source_create(const char* what, bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, int64_t first, int64_t count,
-                             bmo_source** out) {
-    const std::string fn(what);
+static int32_t source_create(bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, int64_t first, int64_t count, bmo_source** out) {
     BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    bmo_source* s = new bmo_source();
+    std::unique_ptr<bmo_source, FreeWith<bmo_source_free>> s(new bmo_source());
     s->ctx = ctx; s->n_rays = desc->n_rays; s->n_poses = n_poses; s->n = count * n_poses; s->uniform = desc->kind != BMO_SRC_POINT;
     const int64_t n = s->n;
     SrcParams P{};
     P.n = desc->n_rays; P.first = first; P.count = count; P.total = n; P.n_rings = desc->n_rings; P.kind = desc->kind;
     for (int i = 0; i < 3; i++) { P.p[i] = desc->pos[i]; P.d[i] = desc->dir[i]; P.e1[i] = desc->e1[i]; P.e2[i] = desc->e2[i]; }
     P.radius = desc->radius; P.phi0 = desc->phi0;
-    bmo_source_ring* d_rings = nullptr;
-    cudaError_t e = dev_alloc(&s->pos, (size_t)n * 3, st);
-    if (e == cudaSuccess) e = dev_alloc(&s->dir, s->uniform ? (size_t)3 : (size_t)n * 3, st);
-    if (e == cudaSuccess && n_poses > 1) e = dev_alloc(&s->pose_id, (size_t)n, st);
-    if (e == cudaSuccess && desc->kind != BMO_SRC_DISC && desc->n_rings > 0) {
-        e = dev_alloc(&d_rings, (size_t)desc->n_rings, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d_rings, desc->rings, (size_t)desc->n_rings * sizeof(bmo_source_ring), cudaMemcpyHostToDevice, st);
+    BMO_CUDA(dev_alloc(&s->pos, (size_t)n * 3, st));
+    BMO_CUDA(dev_alloc(&s->dir, s->uniform ? (size_t)3 : (size_t)n * 3, st));
+    if (n_poses > 1) BMO_CUDA(dev_alloc(&s->pose_id, (size_t)n, st));
+    DevBuf<bmo_source_ring> d_rings;
+    if (desc->kind != BMO_SRC_DISC && desc->n_rings > 0) {
+        BMO_CUDA(d_rings.alloc((size_t)desc->n_rings, st));
+        BMO_CUDA(cudaMemcpyAsync(d_rings.get(), desc->rings, (size_t)desc->n_rings * sizeof(bmo_source_ring), cudaMemcpyHostToDevice, st));
     }
-    if (e != cudaSuccess) {
-        dev_free(d_rings, st);
-        bmo_source_free(s);
-        return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e));
-    }
-    P.rings = d_rings; P.pos = s->pos; P.dir = s->dir; P.pose_id = s->pose_id;
-    int32_t rc;
+    P.rings = d_rings.get(); P.pos = s->pos; P.dir = s->dir; P.pose_id = s->pose_id;
     if (desc->kind == BMO_SRC_DISC) {
         source_disc<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P);
-        rc = launched(ctx, "source_disc");
+        BMO_LAUNCH(ctx, "source_disc");
     } else {
         // the serial recurrence runs once (tile 0); further poses are copies of it
         source_rings<<<(unsigned)((desc->n_rings + 1 + 63) / 64), 64, 0, st>>>(P);
-        rc = launched(ctx, "source_rings");
-        if (!rc && n_poses > 1) {
+        BMO_LAUNCH(ctx, "source_rings");
+        if (n_poses > 1) {
             source_tile<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P, s->uniform ? 1 : 0);
-            rc = launched(ctx, "source_tile");
+            BMO_LAUNCH(ctx, "source_tile");
         }
     }
-    dev_free(d_rings, st);
-    if (rc) { bmo_source_free(s); return rc; }
-    *out = s;
+    *out = s.release();
     return BMO_OK;
 }
 
@@ -483,7 +466,7 @@ int32_t bmo_source_create_poses(bmo_ctx* ctx, const bmo_source_desc* desc, int32
     int32_t rc;
     if ((rc = check_desc(desc))) return rc;
     if (desc->n_rays > INT64_MAX / n_poses) return fail(BMO_EINVAL, "bmo_source_create_poses: n_rays * n_poses overflows int64");
-    return source_create("bmo_source_create", ctx, desc, n_poses, 0, desc->n_rays, out);
+    return source_create(ctx, desc, n_poses, 0, desc->n_rays, out);
 }
 
 int32_t bmo_source_create(bmo_ctx* ctx, const bmo_source_desc* desc, bmo_source** out) {
@@ -498,7 +481,7 @@ int32_t bmo_source_create_slice(bmo_ctx* ctx, const bmo_source_desc* desc, int64
     if (first < 0 || count < 1 || first > desc->n_rays - count)
         return fail(BMO_EINVAL, "bmo_source_create_slice: rays [" + std::to_string(first) + ", " + std::to_string(first) + " + " +
                                     std::to_string(count) + ") are not a non-empty part of the source's " + std::to_string(desc->n_rays));
-    return source_create("bmo_source_create_slice", ctx, desc, 1, first, count, out);
+    return source_create(ctx, desc, 1, first, count, out);
 }
 
 int32_t bmo_source_pose_ids(bmo_source* s, int32_t* n_poses, const int32_t** pose_id) {
@@ -585,54 +568,42 @@ static int32_t spot_stats(const char* what, int32_t n_res, bmo_result* const* rs
     // needs the per-pose counts to size the grid: one read-back of n_poses + 1 words.
     std::vector<int64_t> tab;   // pstart [n_poses + 1], pper [n_poses], then pblk [n_poses + 1] as int32 pairs
     int64_t nblk = 0;
-    int32_t* order = nullptr;
-    cudaError_t e = cudaSuccess;
-    rc = BMO_OK;
+    DevBuf<int32_t> order;
     if (n_poses == 1) {
         P.per = spot_per(n);
         nblk = std::max<int64_t>(1, (n + P.per - 1) / P.per);
     } else {
         const int64_t nb = r->n_beams;
         if (nb > INT32_MAX) return fail(BMO_EINVAL, fn + ": more beams than a 32-bit beam id can number");
-        unsigned long long* cnt = nullptr;   // [n_poses] counts, then the flags word
-        BMO_CUDA(dev_alloc(&cnt, np + 1, st));
+        DevBuf<unsigned long long> cnt;   // [n_poses] counts, then the flags word
+        BMO_CUDA(cnt.alloc(np + 1, st));
         std::vector<unsigned long long> h(np + 1);
-        e = cudaMemsetAsync(cnt, 0, (np + 1) * sizeof(unsigned long long), st);
-        if (e == cudaSuccess && nb > 0) {
+        BMO_CUDA(cudaMemsetAsync(cnt.get(), 0, (np + 1) * sizeof(unsigned long long), st));
+        if (nb > 0) {
             const int64_t runs = (nb + POSE_RUN - 1) / POSE_RUN;
-            spot_pose_count<<<(unsigned)((runs + 255) / 256), 256, 0, st>>>(r->pose, nb, n_poses, cnt, (unsigned int*)(cnt + np));
-            rc = launched(ctx, "spot_pose_count");
+            spot_pose_count<<<(unsigned)((runs + 255) / 256), 256, 0, st>>>(r->pose, nb, n_poses, cnt.get(), (unsigned int*)(cnt.get() + np));
+            BMO_LAUNCH(ctx, "spot_pose_count");
         }
-        if (!rc && e == cudaSuccess) e = cudaMemcpyAsync(h.data(), cnt, (np + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
-        if (!rc && e == cudaSuccess) e = cudaStreamSynchronize(st);
-        dev_free(cnt, st);
-        if (rc) return rc;
-        if (e != cudaSuccess) return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e));
+        BMO_CUDA(cudaMemcpyAsync(h.data(), cnt.get(), (np + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        BMO_CUDA(cudaStreamSynchronize(st));
+        cnt.reset();
         if (h[np] & 2u) return fail(BMO_EINVAL, fn + ": a beam of the result carries a pose id outside [0, n_poses)");
         if (h[np] & 1u) {   // not pose-major (beamsplitter children, or pose ids in any order): stable radix sort on the pose id
-            int32_t *keys = nullptr, *iota = nullptr;
-            void* tmp = nullptr;
+            DevBuf<int32_t> keys, iota;
+            DevBuf<char> tmp;
             size_t tmp_bytes = 0;
             const int end_bit = 32 - __builtin_clz((unsigned)(n_poses - 1));
-            e = cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, (const int32_t*)r->pose, keys, (const int32_t*)iota, order, (int)nb, 0, end_bit, st);
-            if (e == cudaSuccess) e = dev_alloc(&order, (size_t)nb, st);
-            if (e == cudaSuccess) e = dev_alloc(&keys, (size_t)nb, st);
-            if (e == cudaSuccess) e = dev_alloc(&iota, (size_t)nb, st);
-            if (e == cudaSuccess) e = dev_alloc((char**)&tmp, tmp_bytes, st);
-            if (e == cudaSuccess) {
-                iota32<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(iota, nb);
-                rc = launched(ctx, "iota32");
-            }
-            if (!rc && e == cudaSuccess) {
-                e = cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, (const int32_t*)r->pose, keys, (const int32_t*)iota, order, (int)nb, 0, end_bit, st);
-                if (e == cudaSuccess) rc = launched(ctx, "radix sort by pose");
-            }
-            dev_free(keys, st); dev_free(iota, st); dev_free(tmp, st);
-            if (rc || e != cudaSuccess) {
-                dev_free(order, st);
-                if (rc) return rc;
-                return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e));
-            }
+            BMO_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, (const int32_t*)r->pose, keys.get(), (const int32_t*)iota.get(), order.get(),
+                                                     (int)nb, 0, end_bit, st));
+            BMO_CUDA(order.alloc((size_t)nb, st));
+            BMO_CUDA(keys.alloc((size_t)nb, st));
+            BMO_CUDA(iota.alloc((size_t)nb, st));
+            BMO_CUDA(tmp.alloc(tmp_bytes, st));
+            iota32<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(iota.get(), nb);
+            BMO_LAUNCH(ctx, "iota32");
+            BMO_CUDA(cub::DeviceRadixSort::SortPairs(tmp.get(), tmp_bytes, (const int32_t*)r->pose, keys.get(), (const int32_t*)iota.get(), order.get(),
+                                                     (int)nb, 0, end_bit, st));
+            BMO_LAUNCH(ctx, "radix sort by pose");
         }
         tab.assign(2 * np + 1 + (np + 2) / 2, 0);
         int32_t* pblk = (int32_t*)(tab.data() + 2 * np + 1);
@@ -645,7 +616,7 @@ static int32_t spot_stats(const char* what, int32_t n_res, bmo_result* const* rs
             nblk += std::max<int64_t>(1, (m + per - 1) / per);
         }
         pblk[np] = (int32_t)nblk;
-        if (nblk > INT32_MAX) { dev_free(order, st); return fail(BMO_EINVAL, fn + ": too many blocks"); }
+        if (nblk > INT32_MAX) return fail(BMO_EINVAL, fn + ": too many blocks");
     }
     // one scratch block: partials, two completion counters per pose, the statistics, the histogram of a host `counts`, the
     // per-pose slice table, the result table
@@ -654,37 +625,29 @@ static int32_t spot_stats(const char* what, int32_t n_res, bmo_result* const* rs
     const size_t off_tab = off_hist + (counts && !dev_counts ? np * bins * sizeof(int64_t) : 0);
     const size_t off_res = off_tab + tab.size() * sizeof(int64_t);
     const size_t bytes = off_res + rtab.size() * sizeof(SpotRes);
-    char* scr = nullptr;
-    e = dev_alloc(&scr, bytes, st);
-    if (e != cudaSuccess) { dev_free(order, st); return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e)); }
+    DevBuf<char> buf;
+    BMO_CUDA(buf.alloc(bytes, st));
+    char* scr = buf.get();
     P.part = (SpotPartial*)scr; P.done = (unsigned int*)(scr + off_done); P.out = (bmo_spot_info*)(scr + off_out);
     P.counts = counts ? (dev_counts ? (unsigned long long*)counts : (unsigned long long*)(scr + off_hist)) : nullptr;
-    P.order = order;
+    P.order = order.get();
     if (!tab.empty()) {
         P.pstart = (const int64_t*)(scr + off_tab); P.pper = P.pstart + np + 1; P.pblk = (const int32_t*)(P.pper + np);
-        e = cudaMemcpyAsync(scr + off_tab, tab.data(), tab.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st);
+        BMO_CUDA(cudaMemcpyAsync(scr + off_tab, tab.data(), tab.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
     }
     if (!rtab.empty()) {
         P.res = (const SpotRes*)(scr + off_res); P.n_res = n_res;
-        if (e == cudaSuccess) e = cudaMemcpyAsync(scr + off_res, rtab.data(), rtab.size() * sizeof(SpotRes), cudaMemcpyHostToDevice, st);
+        BMO_CUDA(cudaMemcpyAsync(scr + off_res, rtab.data(), rtab.size() * sizeof(SpotRes), cudaMemcpyHostToDevice, st));
     }
-    if (e == cudaSuccess) e = cudaMemsetAsync(P.done, 0, done_bytes, st);
-    if (e == cudaSuccess && P.counts) e = cudaMemsetAsync(P.counts, 0, np * bins * sizeof(int64_t), st);
-    if (e == cudaSuccess) {
-        spot_sums<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P);
-        rc = launched(ctx, "spot_sums");
-        if (!rc) {
-            spot_spread<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P);
-            rc = launched(ctx, "spot_spread");
-        }
-        if (!rc) e = cudaMemcpyAsync(out, P.out, np * sizeof(bmo_spot_info), cudaMemcpyDeviceToHost, st);
-        if (!rc && e == cudaSuccess && counts && !dev_counts) e = cudaMemcpyAsync(counts, P.counts, np * bins * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
-        if (!rc && e == cudaSuccess) e = cudaStreamSynchronize(st);
-    }
-    dev_free(scr, st);
-    dev_free(order, st);
-    if (rc) return rc;
-    if (e != cudaSuccess) return fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e));
+    BMO_CUDA(cudaMemsetAsync(P.done, 0, done_bytes, st));
+    if (P.counts) BMO_CUDA(cudaMemsetAsync(P.counts, 0, np * bins * sizeof(int64_t), st));
+    spot_sums<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P);
+    BMO_LAUNCH(ctx, "spot_sums");
+    spot_spread<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P);
+    BMO_LAUNCH(ctx, "spot_spread");
+    BMO_CUDA(cudaMemcpyAsync(out, P.out, np * sizeof(bmo_spot_info), cudaMemcpyDeviceToHost, st));
+    if (counts && !dev_counts) BMO_CUDA(cudaMemcpyAsync(counts, P.counts, np * bins * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    BMO_CUDA(cudaStreamSynchronize(st));
     return BMO_OK;
 }
 
@@ -725,8 +688,9 @@ int32_t bmo::spot_stats_shard(const std::string& fn, bmo_ctx* ctx, bmo_result* r
     const size_t part_bytes = (size_t)stride * sizeof(SpotPartial);
     const size_t off_all = part_bytes, off_ent = off_all + (size_t)W * part_bytes, off_out = off_ent + (size_t)W * sizeof(int64_t);
     const size_t off_hist = off_out + sizeof(bmo_spot_info), bytes = off_hist + (counts && !dev_counts ? bins * sizeof(int64_t) : 0);
-    char* scr = nullptr;
-    BMO_CUDA(dev_alloc(&scr, bytes, st));
+    DevBuf<char> buf;
+    BMO_CUDA(buf.alloc(bytes, st));
+    char* scr = buf.get();
     SpotParams P{};
     if (r) { P.obj = r->spot_obj; P.xz = r->spot_xz; P.R = r->R; }
     P.n = n; P.per = per; P.det = det_object; P.n_poses = 1;
@@ -736,23 +700,23 @@ int32_t bmo::spot_stats_shard(const std::string& fn, bmo_ctx* ctx, bmo_result* r
     P.counts = counts ? (dev_counts ? (unsigned long long*)counts : (unsigned long long*)(scr + off_hist)) : nullptr;
     const SpotPartial* all = (const SpotPartial*)(scr + off_all);
     const int64_t* ent = (const int64_t*)(scr + off_ent);
-    int32_t rc = BMO_OK;
-    const auto cuda = [&](cudaError_t e) { if (!rc && e != cudaSuccess) rc = fail(BMO_ECUDA, fn + ": " + cudaGetErrorString(e)); };
-    cuda(cudaMemcpyAsync(scr + off_ent, entries.data(), (size_t)W * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    if (P.counts) cuda(cudaMemsetAsync(P.counts, 0, bins * sizeof(int64_t), st));
+    int32_t rc;
+    BMO_CUDA(cudaMemcpyAsync(scr + off_ent, entries.data(), (size_t)W * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    if (P.counts) BMO_CUDA(cudaMemsetAsync(P.counts, 0, bins * sizeof(int64_t), st));
     // pass 1: this rank's sums; every rank combines all partials in global block order
-    if (!rc && nblk) { spot_sums<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P); rc = launched(ctx, "spot_sums"); }
-    if (!rc) rc = x.gather(P.part, scr + off_all, part_bytes);
-    if (!rc) { spot_combine<<<1, 1, 0, st>>>(all, W, (int32_t)stride, ent, per, 0, P.out); rc = launched(ctx, "spot_combine"); }
+    if (nblk) { spot_sums<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P); BMO_LAUNCH(ctx, "spot_sums"); }
+    if ((rc = x.gather(P.part, scr + off_all, part_bytes))) return rc;
+    spot_combine<<<1, 1, 0, st>>>(all, W, (int32_t)stride, ent, per, 0, P.out);
+    BMO_LAUNCH(ctx, "spot_combine");
     // pass 2: the squared distances to the common centroid
-    if (!rc && nblk) { spot_spread<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P); rc = launched(ctx, "spot_spread"); }
-    if (!rc) rc = x.gather(P.part, scr + off_all, part_bytes);
-    if (!rc) { spot_combine<<<1, 1, 0, st>>>(all, W, (int32_t)stride, ent, per, 1, P.out); rc = launched(ctx, "spot_combine"); }
+    if (nblk) { spot_spread<<<(unsigned)nblk, SPOT_BLOCK, 0, st>>>(P); BMO_LAUNCH(ctx, "spot_spread"); }
+    if ((rc = x.gather(P.part, scr + off_all, part_bytes))) return rc;
+    spot_combine<<<1, 1, 0, st>>>(all, W, (int32_t)stride, ent, per, 1, P.out);
+    BMO_LAUNCH(ctx, "spot_combine");
     // the histogram: integer counts, summed exactly
-    if (!rc && P.counts) rc = x.sum((int64_t*)P.counts, bins);
-    if (!rc) cuda(cudaMemcpyAsync(out, P.out, sizeof(bmo_spot_info), cudaMemcpyDeviceToHost, st));
-    if (!rc && counts && !dev_counts) cuda(cudaMemcpyAsync(counts, P.counts, bins * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    cuda(cudaStreamSynchronize(st));
-    dev_free(scr, st);
-    return rc;
+    if (P.counts && (rc = x.sum((int64_t*)P.counts, bins))) return rc;
+    BMO_CUDA(cudaMemcpyAsync(out, P.out, sizeof(bmo_spot_info), cudaMemcpyDeviceToHost, st));
+    if (counts && !dev_counts) BMO_CUDA(cudaMemcpyAsync(counts, P.counts, bins * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    BMO_CUDA(cudaStreamSynchronize(st));
+    return BMO_OK;
 }

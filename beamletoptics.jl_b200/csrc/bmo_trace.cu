@@ -1285,14 +1285,6 @@ using namespace bmo;
 // =================================================================================================
 // host side
 // =================================================================================================
-static int32_t launch_check(bmo_ctx* ctx, const char* what) {
-    ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(BMO_ECUDA, std::string(what) + ": " + cudaGetErrorString(e));
-    return BMO_OK;
-}
-#define BMO_LAUNCH(ctx, what) do { int32_t rc_ = launch_check(ctx, what); if (rc_) return rc_; } while (0)
-
 // (exported functions get C linkage from their declarations in include/bmo.h)
 
 const char* bmo_last_error(void) { return g_last_error.c_str(); }
@@ -1308,7 +1300,7 @@ int32_t bmo_init(int32_t device, bmo_ctx** out) {
     cudaDeviceProp prop;
     BMO_CUDA(cudaGetDeviceProperties(&prop, device));
     if (prop.major < 10) return fail(BMO_ECUDA, std::string("bmo_init: ") + prop.name + " is not an sm_100-class device");
-    bmo_ctx* c = new bmo_ctx();
+    std::unique_ptr<bmo_ctx, FreeWith<bmo_shutdown>> c(new bmo_ctx());
     c->device = device;
     c->sm_count = prop.multiProcessorCount;
     BMO_CUDA(cudaEventCreate(&c->ev0));
@@ -1323,7 +1315,7 @@ int32_t bmo_init(int32_t device, bmo_ctx** out) {
     BMO_CUDA(cudaDeviceGetDefaultMemPool(&pool, device));
     uint64_t thr = UINT64_MAX;  // keep freed blocks cached: the wave loop reuses them every call
     BMO_CUDA(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr));
-    *out = c;
+    *out = c.release();
     return BMO_OK;
 }
 int32_t bmo_shutdown(bmo_ctx* c) {
@@ -1332,7 +1324,11 @@ int32_t bmo_shutdown(bmo_ctx* c) {
     cudaStreamSynchronize(c->stream);
     BigBlocks::of_device().drop_parked();
     cudaFree(c->d_counters); cudaFree(c->d_totals); cudaFreeHost(c->h_totals);
-    cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1);
+    std::vector<cudaEvent_t> evs = c->ev_pool;
+    evs.insert(evs.end(), {c->ev0, c->ev1, c->evk0, c->evk1, c->evs0, c->evs1});
+    for (cudaEvent_t e : evs)
+        if (e) cudaEventDestroy(e);   // (a context that bmo_init gave up on may lack some)
+    for (cudaStream_t s : c->aux_streams) cudaStreamDestroy(s);
     delete c;
     return BMO_OK;
 }
@@ -1413,6 +1409,11 @@ static int32_t validate_tables(const bmo_tables* t) {
         for (int64_t f = 3 * me.first_face; f < 3 * (me.first_face + me.n_faces); f++)
             if (t->faces[f] < 0 || t->faces[f] >= me.n_vertices) return fail(BMO_EINVAL, "face vertex index out of range");
     }
+    for (int p = 0; p < t->n_prims; p++) {
+        const bmo_prim& pr = t->prims[p];
+        if (pr.type >= BMO_PRIM_CONVEX_ASPH && (!t->ext || pr.ext_first < 0 || pr.ext_count < 7 || (int64_t)pr.ext_first + pr.ext_count > t->n_ext))
+            return fail(BMO_EINVAL, "aspheric primitive without a parameter block in tables.ext");
+    }
     return BMO_OK;
 }
 
@@ -1456,19 +1457,13 @@ static void patch_asph(bmo_prim* p, size_t n, const double* d_ext) {
         }
 }
 
-template <class T> static int32_t upload(T** dptr, const T* h, size_t n) {
-    BMO_CUDA(cudaMalloc((void**)dptr, std::max<size_t>(n, 1) * sizeof(T)));
-    if (n) BMO_CUDA(cudaMemcpy(*dptr, h, n * sizeof(T), cudaMemcpyHostToDevice));
-    return BMO_OK;
-}
-
 int32_t bmo_system_upload(bmo_ctx* ctx, const bmo_tables* t, bmo_sys** out) {
     NvtxRange nvtx_("bmo_system_upload");
     if (!ctx || !out) return fail(BMO_EINVAL, "bmo_system_upload: NULL argument");
     int32_t rc = validate_tables(t);
     if (rc) return rc;
     BMO_CUDA(cudaSetDevice(ctx->device));
-    bmo_sys* s = new bmo_sys();
+    std::unique_ptr<bmo_sys, FreeWith<bmo_system_free>> s(new bmo_sys());
     s->ctx = ctx;
     s->prims.assign(t->prims, t->prims + t->n_prims);
     for (auto& pr : s->prims) pr.reserved = prim_flags(pr);
@@ -1505,47 +1500,40 @@ int32_t bmo_system_upload(bmo_ctx* ctx, const bmo_tables* t, bmo_sys** out) {
     for (int p = 0; p < t->n_parts; p++)
         for (int k = 0; k < NBOUND; k++) s->h_bounds[NBOUND * p + k] = t->parts[p].bound[k];
     std::vector<double> ntab(t->n_table, t->n_table + (size_t)std::max(t->n_rows, 0) * t->n_lambda);
-    if (t->n_ext > 0 && (rc = upload(&s->d_ext, t->ext, (size_t)t->n_ext))) return rc;
-    for (const bmo_prim& pr : s->prims)
-        if ((pr.type >= BMO_PRIM_CONVEX_ASPH && pr.type <= BMO_PRIM_CONCAVE_ACYL) &&
-            (!t->ext || pr.ext_first < 0 || pr.ext_count < 7 || (int64_t)pr.ext_first + pr.ext_count > t->n_ext))
-            return fail(BMO_EINVAL, "aspheric primitive without a parameter block in tables.ext");
-    patch_asph(s->prims.data(), s->prims.size(), s->d_ext);
+    if (t->n_ext > 0 && (rc = upload(s->d_ext, t->ext, (size_t)t->n_ext))) return rc;
+    patch_asph(s->prims.data(), s->prims.size(), s->d_ext.get());
     flag_rare_parts(s->prims.data(), s->prims.size(), 1, s->parts);
     for (const bmo_prim& pr : s->prims) s->has_rare |= pr.type >= BMO_PRIM_CONVEX_CYL;
     s->all_lean = system_is_lean(s->prims, s->parts, s->meshes);
-    if ((rc = upload(&s->d_prims, s->prims.data(), s->prims.size()))) return rc;
-    if ((rc = upload(&s->d_parts, s->parts.data(), s->parts.size()))) return rc;
-    if ((rc = upload(&s->d_objects, s->objects.data(), s->objects.size()))) return rc;
-    if ((rc = upload(&s->d_meshes, s->meshes.data(), s->meshes.size()))) return rc;
-    if ((rc = upload(&s->d_vertices, s->h_vertices.data(), s->h_vertices.size()))) return rc;
-    if ((rc = upload(&s->d_faces, t->faces, (size_t)3 * t->n_faces))) return rc;
-    if ((rc = upload(&s->d_nodes, nodes.data(), nodes.size()))) return rc;
-    if ((rc = upload(&s->d_bvh_faces, order.data(), (size_t)t->n_faces))) return rc;
-    if ((rc = upload(&s->d_ntable, ntab.data(), ntab.size()))) return rc;
-    if ((rc = upload(&s->d_bounds, s->h_bounds.data(), s->h_bounds.size()))) return rc;
-    if ((rc = upload(&s->d_detpose, s->h_detpose.data(), s->h_detpose.size()))) return rc;
-    if ((rc = upload(&s->d_lambdas, s->lambdas.data(), s->lambdas.size()))) return rc;
-    if (t->n_jones > 0 && (rc = upload(&s->d_jones, t->jones, (size_t)10 * t->n_jones))) return rc;
+    if ((rc = upload(s->d_prims, s->prims.data(), s->prims.size()))) return rc;
+    if ((rc = upload(s->d_parts, s->parts.data(), s->parts.size()))) return rc;
+    if ((rc = upload(s->d_objects, s->objects.data(), s->objects.size()))) return rc;
+    if ((rc = upload(s->d_meshes, s->meshes.data(), s->meshes.size()))) return rc;
+    if ((rc = upload(s->d_vertices, s->h_vertices.data(), s->h_vertices.size()))) return rc;
+    if ((rc = upload(s->d_faces, t->faces, (size_t)3 * t->n_faces))) return rc;
+    if ((rc = upload(s->d_nodes, nodes.data(), nodes.size()))) return rc;
+    if ((rc = upload(s->d_bvh_faces, order.data(), (size_t)t->n_faces))) return rc;
+    if ((rc = upload(s->d_ntable, ntab.data(), ntab.size()))) return rc;
+    if ((rc = upload(s->d_bounds, s->h_bounds.data(), s->h_bounds.size()))) return rc;
+    if ((rc = upload(s->d_detpose, s->h_detpose.data(), s->h_detpose.size()))) return rc;
+    if ((rc = upload(s->d_lambdas, s->lambdas.data(), s->lambdas.size()))) return rc;
+    if (t->n_jones > 0 && (rc = upload(s->d_jones, t->jones, (size_t)10 * t->n_jones))) return rc;
     SysView& v = s->view;
-    v.prims = s->d_prims; v.parts = s->d_parts; v.objects = s->d_objects; v.meshes = s->d_meshes;
-    v.vertices = s->d_vertices; v.faces = s->d_faces; v.nodes = s->d_nodes; v.bvh_faces = s->d_bvh_faces;
-    v.n_table = s->d_ntable; v.bounds = s->d_bounds; v.det_pose = s->d_detpose; v.lambdas = s->d_lambdas; v.jones = s->d_jones; v.ext = s->d_ext;
+    v.prims = s->d_prims.get(); v.parts = s->d_parts.get(); v.objects = s->d_objects.get(); v.meshes = s->d_meshes.get();
+    v.vertices = s->d_vertices.get(); v.faces = s->d_faces.get(); v.nodes = s->d_nodes.get(); v.bvh_faces = s->d_bvh_faces.get();
+    v.n_table = s->d_ntable.get(); v.bounds = s->d_bounds.get(); v.det_pose = s->d_detpose.get(); v.lambdas = s->d_lambdas.get();
+    v.jones = s->d_jones.get(); v.ext = s->d_ext.get();
     v.n_prims = t->n_prims; v.n_parts = t->n_parts; v.n_objects = t->n_objects; v.n_meshes = t->n_meshes;
     v.n_lambda = t->n_lambda; v.n_poses = 1; v.bvh_ok = 1; v.zr = t->norm_zero_rule; v.n_vertices = t->n_vertices;
     v.n_system = t->n_system;
-    *out = s;
+    *out = s.release();
     return BMO_OK;
 }
 int32_t bmo_system_free(bmo_sys* s) {
     if (!s) return BMO_OK;
     cudaSetDevice(s->ctx->device);
     cudaStreamSynchronize(s->ctx->stream);
-    cudaFree(s->d_prims); cudaFree(s->d_parts); cudaFree(s->d_objects); cudaFree(s->d_meshes); cudaFree(s->d_vertices);
-    cudaFree(s->d_faces); cudaFree(s->d_nodes); cudaFree(s->d_bvh_faces); cudaFree(s->d_ntable); cudaFree(s->d_bounds);
-    cudaFree(s->d_detpose); cudaFree(s->d_lambdas); cudaFree(s->d_jones); cudaFree(s->d_ext);
-    cudaFree(s->d_kin_nodes); cudaFree(s->d_prim_bounds); cudaFree(s->d_prims0); cudaFree(s->d_vertices0); cudaFree(s->d_detpose0);
-    delete s;
+    delete s;   // the device tables go with it
     return BMO_OK;
 }
 int32_t bmo_system_set_poses(bmo_sys* s, int32_t n_poses, const bmo_prim* prims, const double* vertices, const double* bounds,
@@ -1553,41 +1541,42 @@ int32_t bmo_system_set_poses(bmo_sys* s, int32_t n_poses, const bmo_prim* prims,
     if (!s || n_poses < 1) return fail(BMO_EINVAL, "bmo_system_set_poses: bad arguments");
     BMO_CUDA(cudaSetDevice(s->ctx->device));
     BMO_CUDA(cudaStreamSynchronize(s->ctx->stream));
-    SysView& v = s->view;
     const size_t np = (size_t)n_poses;
-    auto reup = [&](auto** dptr, const auto* h, size_t n) -> int32_t {
-        cudaFree(*dptr); *dptr = nullptr;
-        return upload(dptr, h, n);
-    };
+    // the new tables replace the live ones only once all of them are on the device
+    DevTable<bmo_prim> d_prims; DevTable<double> d_vertices, d_bounds, d_detpose;
     int32_t rc;
     if (n_poses == 1 && !prims) {  // restore the uploaded tables
-        if ((rc = reup(&s->d_prims, s->prims.data(), s->prims.size()))) return rc;
-        if ((rc = reup(&s->d_vertices, s->h_vertices.data(), s->h_vertices.size()))) return rc;
-        if ((rc = reup(&s->d_bounds, s->h_bounds.data(), s->h_bounds.size()))) return rc;
-        if ((rc = reup(&s->d_detpose, s->h_detpose.data(), s->h_detpose.size()))) return rc;
+        if ((rc = upload(d_prims, s->prims.data(), s->prims.size()))) return rc;
+        if ((rc = upload(d_vertices, s->h_vertices.data(), s->h_vertices.size()))) return rc;
+        if ((rc = upload(d_bounds, s->h_bounds.data(), s->h_bounds.size()))) return rc;
+        if ((rc = upload(d_detpose, s->h_detpose.data(), s->h_detpose.size()))) return rc;
     } else {
         if (!prims || !bounds || (!vertices && s->n_vertices > 0) || !det_pos || !det_dir) return fail(BMO_EINVAL, "bmo_system_set_poses: NULL table");
         std::vector<bmo_prim> pp(prims, prims + np * s->prims.size());
         for (auto& pr : pp) pr.reserved = prim_flags(pr);
-        patch_asph(pp.data(), pp.size(), s->d_ext);
+        patch_asph(pp.data(), pp.size(), s->d_ext.get());
         flag_rare_parts(pp.data(), s->prims.size(), np, s->parts);
-        if ((rc = reup(&s->d_prims, pp.data(), pp.size()))) return rc;
-        if ((rc = reup(&s->d_vertices, vertices, np * 3 * (size_t)s->n_vertices))) return rc;
-        if ((rc = reup(&s->d_bounds, bounds, np * NBOUND * s->parts.size()))) return rc;
+        if ((rc = upload(d_prims, pp.data(), pp.size()))) return rc;
+        if ((rc = upload(d_vertices, vertices, np * 3 * (size_t)s->n_vertices))) return rc;
+        if ((rc = upload(d_bounds, bounds, np * NBOUND * s->parts.size()))) return rc;
         std::vector<double> dp(np * 12 * s->objects.size());
         for (size_t i = 0; i < np * s->objects.size(); i++) {
             for (int k = 0; k < 3; k++) dp[12 * i + k] = det_pos[3 * i + k];
             for (int k = 0; k < 9; k++) dp[12 * i + 3 + k] = det_dir[9 * i + k];
         }
-        if ((rc = reup(&s->d_detpose, dp.data(), dp.size()))) return rc;
+        if ((rc = upload(d_detpose, dp.data(), dp.size()))) return rc;
     }
-    v.prims = s->d_prims; v.vertices = s->d_vertices; v.bounds = s->d_bounds; v.det_pose = s->d_detpose;
+    s->d_prims = std::move(d_prims); s->d_vertices = std::move(d_vertices); s->d_bounds = std::move(d_bounds); s->d_detpose = std::move(d_detpose);
+    SysView& v = s->view;
+    v.prims = s->d_prims.get(); v.vertices = s->d_vertices.get(); v.bounds = s->d_bounds.get(); v.det_pose = s->d_detpose.get();
     v.n_poses = n_poses;
     v.bvh_ok = (n_poses == 1 && !prims) ? 1 : 0;   // moved vertices: the BVH boxes are stale, meshes fall back to the face loop
     return BMO_OK;
 }
 
 // ---- trace driver -----------------------------------------------------------------------------------
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+static void free_wavebuf(WaveBuf& w, cudaStream_t st) { dev_free(w.d, st); dev_free(w.part, st); dev_free(w.beam, st); dev_free(w.seg, st); }
 static int32_t alloc_queue(Queue& q, int64_t cap, int nf, int ni, cudaStream_t st) {
     q.cap = cap;
     BMO_CUDA(dev_alloc(&q.d, (size_t)nf * cap, st));
@@ -1596,17 +1585,18 @@ static int32_t alloc_queue(Queue& q, int64_t cap, int nf, int ni, cudaStream_t s
 }
 // enlarge a queue (SoA planes of stride cap) keeping its contents
 static int32_t grow_queue(Queue& q, int64_t new_cap, int nf, int ni, cudaStream_t st) {
-    Queue nq;
-    int32_t rc = alloc_queue(nq, new_cap, nf, ni, st);
-    if (rc) return rc;
+    DevBuf<double> d;
+    DevBuf<int32_t> i;
+    BMO_CUDA(d.alloc((size_t)nf * new_cap, st));
+    BMO_CUDA(i.alloc((size_t)ni * new_cap, st));
     if (q.cap) {
-        BMO_CUDA(cudaMemcpy2DAsync(nq.d, (size_t)new_cap * sizeof(double), q.d, (size_t)q.cap * sizeof(double), (size_t)q.cap * sizeof(double), nf,
+        BMO_CUDA(cudaMemcpy2DAsync(d.get(), (size_t)new_cap * sizeof(double), q.d, (size_t)q.cap * sizeof(double), (size_t)q.cap * sizeof(double), nf,
                                    cudaMemcpyDeviceToDevice, st));
-        BMO_CUDA(cudaMemcpy2DAsync(nq.i, (size_t)new_cap * sizeof(int32_t), q.i, (size_t)q.cap * sizeof(int32_t), (size_t)q.cap * sizeof(int32_t), ni,
+        BMO_CUDA(cudaMemcpy2DAsync(i.get(), (size_t)new_cap * sizeof(int32_t), q.i, (size_t)q.cap * sizeof(int32_t), (size_t)q.cap * sizeof(int32_t), ni,
                                    cudaMemcpyDeviceToDevice, st));
     }
     dev_free(q.d, st); dev_free(q.i, st);
-    q = nq;
+    q.d = d.release(); q.i = i.release(); q.cap = new_cap;
     return BMO_OK;
 }
 static void free_queue(Queue& q, cudaStream_t st) { dev_free(q.d, st); dev_free(q.i, st); q.cap = 0; }
@@ -1618,11 +1608,11 @@ static BeamTab beamtab(bmo_result* r) {
     return b;
 }
 template <class T> static int32_t grow(T*& p, int64_t old_n, int64_t new_n, cudaStream_t st) {
-    T* np_ = nullptr;
-    BMO_CUDA(dev_alloc(&np_, (size_t)new_n, st));
-    if (p && old_n) BMO_CUDA(cudaMemcpyAsync(np_, p, (size_t)old_n * sizeof(T), cudaMemcpyDeviceToDevice, st));
+    DevBuf<T> np_;
+    BMO_CUDA(np_.alloc((size_t)new_n, st));
+    if (p && old_n) BMO_CUDA(cudaMemcpyAsync(np_.get(), p, (size_t)old_n * sizeof(T), cudaMemcpyDeviceToDevice, st));
     dev_free(p, st);
-    p = np_;
+    p = np_.release();
     return BMO_OK;
 }
 // Per-beam tables of a trace that cannot add beams (no beamsplitter in the system): one allocation instead of 8-12.
@@ -1680,16 +1670,16 @@ static int32_t ensure_first_seg(bmo_result* res) {
         BMO_LAUNCH(ctx, "scan_counts(nseg)");
     } else {
         const int64_t nblk = (nb + 1023) / 1024;
-        int32_t* bsum = nullptr; long long* boff = nullptr;
-        BMO_CUDA(dev_alloc(&bsum, (size_t)nblk, st));
-        BMO_CUDA(dev_alloc(&boff, (size_t)nblk, st));
-        scan_local<<<(unsigned)nblk, 1024, 0, st>>>(res->nseg, nb, res->first_seg, bsum);
+        DevBuf<int32_t> bsum;
+        DevBuf<long long> boff;
+        BMO_CUDA(bsum.alloc((size_t)nblk, st));
+        BMO_CUDA(boff.alloc((size_t)nblk, st));
+        scan_local<<<(unsigned)nblk, 1024, 0, st>>>(res->nseg, nb, res->first_seg, bsum.get());
         BMO_LAUNCH(ctx, "scan_local");
-        scan_counts<<<1, 1024, 0, st>>>(bsum, nblk, 1, 1, boff, ctx->d_totals);
+        scan_counts<<<1, 1024, 0, st>>>(bsum.get(), nblk, 1, 1, boff.get(), ctx->d_totals);
         BMO_LAUNCH(ctx, "scan_counts(blocks)");
-        scan_add<<<(unsigned)nblk, 1024, 0, st>>>(res->first_seg, nb, boff);
+        scan_add<<<(unsigned)nblk, 1024, 0, st>>>(res->first_seg, nb, boff.get());
         BMO_LAUNCH(ctx, "scan_add");
-        dev_free(bsum, st); dev_free(boff, st);
     }
     BMO_CUDA(cudaMemcpyAsync(ctx->h_totals, ctx->d_totals, sizeof(long long), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaMemcpyAsync(res->first_seg + nb, ctx->d_totals, sizeof(long long), cudaMemcpyDeviceToDevice, st));
@@ -1705,14 +1695,15 @@ struct TraceInputs {
     bool dir_uniform = false;   // BMO_UNIFORM_DIR
 };
 
-template <class T> static int32_t stage_in(const T* h, size_t n, bool on_device, cudaStream_t st, const T** out, std::vector<void*>& tmp) {
+// *out = the device copy of a host input (owned by tmp), or the input itself when it is on the device already
+template <class T> static int32_t stage_in(const T* h, size_t n, bool on_device, cudaStream_t st, const T** out, std::vector<DevBuf<char>>& tmp) {
     if (!h) { *out = nullptr; return BMO_OK; }
     if (on_device) { *out = h; return BMO_OK; }
-    T* d = nullptr;
-    BMO_CUDA(dev_alloc(&d, n, st));
-    BMO_CUDA(cudaMemcpyAsync(d, h, n * sizeof(T), cudaMemcpyHostToDevice, st));
-    tmp.push_back((void*)d);
-    *out = d;
+    DevBuf<char> d;
+    BMO_CUDA(d.alloc(n * sizeof(T), st));
+    BMO_CUDA(cudaMemcpyAsync(d.get(), h, n * sizeof(T), cudaMemcpyHostToDevice, st));
+    *out = (const T*)d.get();
+    tmp.push_back(std::move(d));
     return BMO_OK;
 }
 
@@ -1730,7 +1721,7 @@ struct SubTrace {
     bool has_splitter = false, staged = false, on_dev = false, pipelined = false;
     int64_t beam0 = 0, n = 0;              // global id of the first root beam, number of root beams
     TraceInputs in{};                      // device pointers of this sub-batch's inputs
-    std::vector<void*> tmp;                // staged input copies
+    std::vector<DevBuf<char>> tmp;         // staged input copies
     Queue cur, next, scr;
     HitBuf hit;
     int32_t* blk_cnt = nullptr; long long* blk_off = nullptr; int64_t blk_cap = 0;
@@ -1751,10 +1742,13 @@ struct SubTrace {
     // start counting afresh (System.jl:141-150): a tree of g generations needs up to g * r_max waves.  The host gives up
     // after 64 generations' worth (the reference would recurse as deep as the tree is).
     int64_t max_waves() const { return has_splitter ? (int64_t)64 * (r_max + 1) : (int64_t)r_max + 1; }
+    SubTrace() = default;
+    SubTrace(const SubTrace&) = delete;
+    SubTrace& operator=(const SubTrace&) = delete;
+    ~SubTrace();
     int32_t begin(const TraceInputs& in_h);
     int32_t enqueue_chunk();
     int32_t finish_chunk();
-    void release();
 };
 
 static double tnow_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
@@ -1849,13 +1843,15 @@ int32_t SubTrace::enqueue_chunk() {
             blk_cap = nblocks;
         }
         WaveBuf wb{};
-        if (res->keep) {
-            wb.count = n_slots * R;
-            BMO_CUDA(dev_alloc(&wb.d, (size_t)nsd * wb.count, st));
-            BMO_CUDA(dev_alloc(&wb.part, (size_t)wb.count, st));
-            BMO_CUDA(dev_alloc(&wb.beam, (size_t)wb.count, st));
-            BMO_CUDA(dev_alloc(&wb.seg, (size_t)wb.count, st));
-            res->wavebufs.push_back(wb);
+        if (res->keep) {     // owned by the result from the first allocation on
+            res->wavebufs.push_back(WaveBuf{});
+            WaveBuf& w = res->wavebufs.back();
+            w.count = n_slots * R;
+            BMO_CUDA(dev_alloc(&w.d, (size_t)nsd * w.count, st));
+            BMO_CUDA(dev_alloc(&w.part, (size_t)w.count, st));
+            BMO_CUDA(dev_alloc(&w.beam, (size_t)w.count, st));
+            BMO_CUDA(dev_alloc(&w.seg, (size_t)w.count, st));
+            wb = w;
         }
         if (hit.cap < n_slots * R) {
             dev_free(hit.d, st); dev_free(hit.part, st); dev_free(hit.flag, st);
@@ -1995,14 +1991,14 @@ int32_t SubTrace::finish_chunk() {
     return BMO_OK;
 }
 
-void SubTrace::release() {
+// The host waits for an auxiliary stream before its buffers go: after a failed call it may still write to the result, which
+// is freed on the caller's stream.
+SubTrace::~SubTrace() {
+    if (ctx && st != ctx->stream) cudaStreamSynchronize(st);
     free_queue(cur, st); free_queue(next, st); free_queue(scr, st);
     dev_free(hit.d, st); dev_free(hit.part, st); dev_free(hit.flag, st);
     dev_free(blk_cnt, st); dev_free(blk_off, st);
     dev_free(d_wtot, st); dev_free(d_scan_tot, st);
-    for (void* p : tmp) dev_free(p, st);
-    tmp.clear();
-    ev.clear();
 }
 
 // Resident blocks per SM of solve_rays_persistent with smem bytes of tables, 0 if a block would not fit the 48 KB of shared
@@ -2029,7 +2025,7 @@ static int32_t solve_persistent(bmo_sys* sys, const TraceInputs& in_h, int32_t r
     cudaStream_t st = ctx->stream;
     const int64_t n = in_h.n;
     int32_t rc;
-    std::vector<void*> tmp;
+    std::vector<DevBuf<char>> tmp;
     SolveParams sp{};
     sp.S = sys->view; sp.n = n; sp.r_max = r_max; sp.dir_uniform = in_h.dir_uniform; sp.B = beamtab(res); sp.counters = ctx->d_counters;
     if ((rc = stage_in(in_h.pos, (size_t)n * 3, on_dev, st, &sp.pos, tmp))) return rc;
@@ -2047,7 +2043,6 @@ static int32_t solve_persistent(bmo_sys* sys, const TraceInputs& in_h, int32_t r
         if (spot_obj_out) BMO_CUDA(cudaMemcpyAsync(spot_obj_out, res->spot_obj, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         BMO_CUDA(cudaMemcpyAsync(spot_xz_out, res->spot_xz, (size_t)2 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
     }
-    for (void* p : tmp) dev_free(p, st);
     return BMO_OK;
 }
 
@@ -2064,7 +2059,7 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
     const int R = mode == 2 ? 3 : 1;
     const int64_t n = in_h.n;
 
-    bmo_result* res = new bmo_result();
+    std::unique_ptr<bmo_result, FreeWith<bmo_result_free>> res(new bmo_result());
     res->sys = sys; res->ctx = sys->ctx; res->part_object.resize(sys->parts.size()); for (size_t i = 0; i < sys->parts.size(); i++) res->part_object[i] = sys->parts[i].object;
     for (const bmo_object& ob : sys->objects) res->object_kind.push_back(ob.kind);
     res->n_objects = (int32_t)sys->objects.size(); res->n_poses = sys->view.n_poses; res->mode = mode; res->R = R; res->nsd = nf_seg(mode); res->n_roots = n; res->keep = flags & BMO_KEEP_SEGMENTS;
@@ -2077,7 +2072,7 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
     bool has_splitter = false;
     for (const bmo_object& ob : sys->objects)
         has_splitter |= ob.kind == BMO_OBJ_THIN_BS || ob.kind == BMO_OBJ_PLATE_BS || ob.kind == BMO_OBJ_CUBE_BS;
-    if ((rc = has_splitter ? ensure_beams(res, n, st) : alloc_beams_slab(res, n, st))) return rc;
+    if ((rc = has_splitter ? ensure_beams(res.get(), n, st) : alloc_beams_slab(res.get(), n, st))) return rc;
     const SysView& V = sys->view;
     const size_t table_bytes = (size_t)V.n_prims * sizeof(bmo_prim) + (size_t)V.n_parts * (sizeof(bmo_part) + NBOUND * sizeof(double));
     const bool staged = V.n_poses == 1 && table_bytes <= 40 * 1024;
@@ -2092,18 +2087,13 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
     bool lean;
     const size_t smem = staged_smem(sys, staged, lean);
     int pblocks = 0;
-    if (persist_ok && mode == 0 && !has_splitter && !prev_rt && !res->keep && lean && n_sub == 1 && (rc = persistent_blocks(ctx, smem, &pblocks))) {
-        bmo_result_free(res);
+    if (persist_ok && mode == 0 && !has_splitter && !prev_rt && !res->keep && lean && n_sub == 1 && (rc = persistent_blocks(ctx, smem, &pblocks)))
         return rc;
-    }
     const bool persistent = pblocks > 0;
     int wave = 0;
     double tp1 = tp0, tp2 = tp0, tp_wave_sync = 0;   // host timeline (BMO_HOST_PROFILE)
     if (persistent) {
-        if ((rc = solve_persistent(sys, in_h, r_max, on_dev, smem, pblocks, res, spot_obj_out, spot_xz_out))) {
-            bmo_result_free(res);
-            return rc;
-        }
+        if ((rc = solve_persistent(sys, in_h, r_max, on_dev, smem, pblocks, res.get(), spot_obj_out, spot_xz_out))) return rc;
         res->n_beams = n;
         tp1 = tp2 = tnow_ms();
     } else {
@@ -2112,22 +2102,25 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
             BMO_CUDA(cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
             ctx->aux_streams.push_back(s2);
         }
-        cudaEvent_t ev_fork = nullptr;
+        std::unique_ptr<CUevent_st, EventDestroy> ev_fork;
         if (n_sub > 1) {   // the auxiliary streams start after everything already queued on the caller's stream (result tables included)
-            BMO_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
-            BMO_CUDA(cudaEventRecord(ev_fork, st));
+            cudaEvent_t e;
+            BMO_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            ev_fork.reset(e);
+            BMO_CUDA(cudaEventRecord(ev_fork.get(), st));
         }
+        // released at the end of this block, before the segment gather allocates the segment table
         std::vector<SubTrace> subs((size_t)n_sub);
         for (int k = 0; k < n_sub; k++) {
             SubTrace& s = subs[k];
-            s.sys = sys; s.ctx = ctx; s.res = res; s.st = k == 0 ? st : ctx->aux_streams[k - 1]; s.slot = k;
+            s.sys = sys; s.ctx = ctx; s.res = res.get(); s.st = k == 0 ? st : ctx->aux_streams[k - 1]; s.slot = k;
             s.mode = mode; s.R = R; s.nfq = nf_queue(mode); s.nfs = nf_scratch(mode); s.nsd = res->nsd;
             s.units = mode == 2 ? Cfg<2>::UNITS : Cfg<0>::UNITS;
             s.r_max = r_max; s.has_splitter = has_splitter; s.staged = staged; s.on_dev = on_dev; s.pipelined = n_sub > 1;
             s.beam0 = n * k / n_sub; s.n = n * (k + 1) / n_sub - s.beam0;
             s.spot_obj_out = spot_obj_out; s.spot_xz_out = spot_xz_out;
             if (prev_rt) s.rt = *prev_rt;
-            if (k > 0) BMO_CUDA(cudaStreamWaitEvent(s.st, ev_fork, 0));
+            if (k > 0) BMO_CUDA(cudaStreamWaitEvent(s.st, ev_fork.get(), 0));
             if (!has_splitter && n_sub == 1 && !prev_rt) {
                 auto it = sys->hints.find({mode, n});
                 if (it != sys->hints.end()) s.first_chunk = it->second.first_chunk;
@@ -2140,7 +2133,7 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
                     const bmo_sys::TraceHint& hh = it->second;
                     if (hh.slots * R > s.cur.cap && (rc = grow_queue(s.cur, hh.slots * R, s.nfq, NI_Q, s.st))) return rc;
                     if (hh.scr > s.scr.cap) { free_queue(s.scr, s.st); if ((rc = alloc_queue(s.scr, hh.scr, s.nfs, NI_S, s.st))) return rc; }
-                    if ((rc = ensure_beams(res, hh.beams, s.st))) return rc;
+                    if ((rc = ensure_beams(res.get(), hh.beams, s.st))) return rc;
                 }
             }
             if ((rc = s.enqueue_chunk())) return rc;     // the first sub-batch is already copying / tracing while the others are set up
@@ -2174,21 +2167,19 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
             bmo_sys::TraceHint& hh = sys->hints[{mode, n}];
             hh.slots = std::max(hh.slots, subs[0].cur.cap / R); hh.scr = std::max(hh.scr, subs[0].scr.cap); hh.beams = std::max(hh.beams, res->cap_beams);
         }
-        // join: the caller's stream continues after every sub-batch (copies of the Spotdetector hits included)
+        // join: the caller's stream continues after every sub-batch (copies of the Spotdetector hits included); the host
+        // waits for each auxiliary stream as its sub-batch is released
         for (int k = 1; k < n_sub; k++) {
-            BMO_CUDA(cudaEventRecord(ev_fork, subs[k].st));
-            BMO_CUDA(cudaStreamWaitEvent(st, ev_fork, 0));
-            BMO_CUDA(cudaStreamSynchronize(subs[k].st));
+            BMO_CUDA(cudaEventRecord(ev_fork.get(), subs[k].st));
+            BMO_CUDA(cudaStreamWaitEvent(st, ev_fork.get(), 0));
         }
-        for (auto& s : subs) s.release();
-        if (ev_fork) cudaEventDestroy(ev_fork);
     }
     const int nsd = res->nsd;
     // segment table: first_seg = exclusive scan of nseg, then gather wave-major -> beam-major
     // (spot-only traces compute first_seg lazily, see ensure_first_seg)
     if (res->keep) {
         const double tf0 = tnow_ms();
-        if ((rc = ensure_first_seg(res))) return rc;
+        if ((rc = ensure_first_seg(res.get()))) return rc;
         if (prof) { cudaStreamSynchronize(st); fprintf(stderr, "[bmo]   finalize: first_seg scan %.3f ms\n", tnow_ms() - tf0); }
         res->seg_rows = res->n_segments * R;
         BMO_CUDA(dev_alloc(&res->seg_d, (size_t)nsd * res->seg_rows, st));
@@ -2198,7 +2189,7 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
             if (nsd == 17) gather_segments<17><<<(unsigned)((wb.count + 255) / 256), 256, 0, st>>>(wb, R, res->first_seg, res->seg_d, res->seg_part);
             else gather_segments<11><<<(unsigned)((wb.count + 255) / 256), 256, 0, st>>>(wb, R, res->first_seg, res->seg_d, res->seg_part);
             BMO_LAUNCH(ctx, "gather_segments");
-            dev_free(wb.d, st); dev_free(wb.part, st); dev_free(wb.beam, st); dev_free(wb.seg, st);
+            free_wavebuf(wb, st);   // as soon as it is gathered: peak memory
         }
         res->wavebufs.clear();
         if (prof) { cudaStreamSynchronize(st); fprintf(stderr, "[bmo]   finalize: + gather %.3f ms\n", tnow_ms() - tf0); }
@@ -2225,15 +2216,12 @@ static int32_t trace_common(bmo_sys* sys, int mode, const TraceInputs& in_h, int
         ctx->interactions_seen = (int64_t)h.interactions;
         const int64_t bad = (int64_t)h.bad_ids - ctx->bad_ids_seen;
         ctx->bad_ids_seen = (int64_t)h.bad_ids;
-        if (bad > 0) {
-            bmo_result_free(res);
+        if (bad > 0)
             return fail(BMO_EINVAL, "trace: " + std::to_string(bad) + " beam(s) carry a lambda_id outside [0, n_lambda) or a pose_id outside [0, n_poses)");
-        }
     }
     if (prof) fprintf(stderr, "[bmo] trace n=%lld waves=%d sub-batches=%d: setup %.3f ms, wave loop %.3f ms (of which waiting %.3f), finalize %.3f ms\n",
                       (long long)n, wave, n_sub, tp1 - tp0, tp2 - tp1, tp_wave_sync, tnow_ms() - tp2);
-    if (out) *out = res;
-    else bmo_result_free(res);
+    if (out) *out = res.release();
     return BMO_OK;
 }
 
@@ -2295,32 +2283,32 @@ int32_t bmo_retrace(bmo_sys* sys, bmo_result* prev, int32_t r_max, uint32_t flag
     PrevRoots pr{};
     pr.seg_d = prev->seg_d; pr.first_seg = prev->first_seg; pr.rows = prev->seg_rows; pr.nsd = prev->nsd; pr.lam = prev->lam; pr.pose = prev->pose;
     pr.w0 = prev->w0; pr.e0 = prev->e0; pr.n = n; pr.mode = mode;
+    DevBuf<double> grays, ow0, oe0, pos, dir, E0;
+    DevBuf<int32_t> olam, opose, child;
     if (mode == 2) {
-        BMO_CUDA(dev_alloc(&pr.grays, (size_t)n * 18, st)); BMO_CUDA(dev_alloc(&pr.ow0, (size_t)n, st)); BMO_CUDA(dev_alloc(&pr.oe0, (size_t)n * 2, st));
+        BMO_CUDA(grays.alloc((size_t)n * 18, st)); BMO_CUDA(ow0.alloc((size_t)n, st)); BMO_CUDA(oe0.alloc((size_t)n * 2, st));
     } else {
-        BMO_CUDA(dev_alloc(&pr.pos, (size_t)n * 3, st)); BMO_CUDA(dev_alloc(&pr.dir, (size_t)n * 3, st));
-        if (mode == 1) BMO_CUDA(dev_alloc(&pr.E0, (size_t)n * 6, st));
+        BMO_CUDA(pos.alloc((size_t)n * 3, st)); BMO_CUDA(dir.alloc((size_t)n * 3, st));
+        if (mode == 1) BMO_CUDA(E0.alloc((size_t)n * 6, st));
     }
-    BMO_CUDA(dev_alloc(&pr.olam, (size_t)n, st)); BMO_CUDA(dev_alloc(&pr.opose, (size_t)n, st));
+    BMO_CUDA(olam.alloc((size_t)n, st)); BMO_CUDA(opose.alloc((size_t)n, st));
+    pr.grays = grays.get(); pr.ow0 = ow0.get(); pr.oe0 = oe0.get(); pr.pos = pos.get(); pr.dir = dir.get(); pr.E0 = E0.get();
+    pr.olam = olam.get(); pr.opose = opose.get();
     gather_prev_roots<<<(unsigned)((n * R + 255) / 256), 256, 0, st>>>(pr);
     BMO_LAUNCH(ctx, "gather_prev_roots");
-    int32_t* child = nullptr;
-    BMO_CUDA(dev_alloc(&child, (size_t)2 * prev->n_beams, st));
-    BMO_CUDA(cudaMemsetAsync(child, 0xff, (size_t)2 * prev->n_beams * sizeof(int32_t), st));
+    BMO_CUDA(child.alloc((size_t)2 * prev->n_beams, st));
+    BMO_CUDA(cudaMemsetAsync(child.get(), 0xff, (size_t)2 * prev->n_beams * sizeof(int32_t), st));
     if (prev->n_beams > n) {
-        build_child_table<<<(unsigned)((prev->n_beams - n + 255) / 256), 256, 0, st>>>(prev->parent, prev->slot, n, prev->n_beams, child);
+        build_child_table<<<(unsigned)((prev->n_beams - n + 255) / 256), 256, 0, st>>>(prev->parent, prev->slot, n, prev->n_beams, child.get());
         BMO_LAUNCH(ctx, "build_child_table");
     }
     RetraceView rt;
-    rt.nseg = prev->nseg; rt.first_seg = prev->first_seg; rt.seg_part = prev->seg_part; rt.child = child; rt.w0 = prev->w0; rt.on = 1;
+    rt.nseg = prev->nseg; rt.first_seg = prev->first_seg; rt.seg_part = prev->seg_part; rt.child = child.get(); rt.w0 = prev->w0; rt.on = 1;
     TraceInputs in{};
     in.n = n; in.pos = pr.pos; in.dir = pr.dir; in.E0 = pr.E0; in.grays = pr.grays; in.w0 = pr.ow0; in.ge0 = pr.oe0; in.lam = pr.olam; in.pose = pr.opose;
     uint32_t f = (flags | BMO_INPUT_DEVICE);
     if (mode == 2) f |= BMO_KEEP_SEGMENTS;
-    rc = trace_common(sys, mode, in, r_max, f, out, nullptr, nullptr, &rt);
-    dev_free(pr.grays, st); dev_free(pr.ow0, st); dev_free(pr.oe0, st); dev_free(pr.pos, st); dev_free(pr.dir, st); dev_free(pr.E0, st);
-    dev_free(pr.olam, st); dev_free(pr.opose, st); dev_free(child, st);
-    return rc;
+    return trace_common(sys, mode, in, r_max, f, out, nullptr, nullptr, &rt);
 }
 int32_t bmo_trace_beamlets(bmo_sys* sys, int64_t n, const double* rays, const int32_t* lambda_id, const double* w0, const double* E0,
                            const int32_t* pose_id, int32_t r_max, uint32_t flags, bmo_result** out) {
@@ -2422,7 +2410,7 @@ int32_t bmo_result_free(bmo_result* r) {
     }
     dev_free(r->first_seg, st);
     dev_free(r->seg_d, st); dev_free(r->seg_part, st);
-    for (auto& wb : r->wavebufs) { dev_free(wb.d, st); dev_free(wb.part, st); dev_free(wb.beam, st); dev_free(wb.seg, st); }
+    for (auto& wb : r->wavebufs) free_wavebuf(wb, st);
     delete r;
     return BMO_OK;
 }
@@ -2441,19 +2429,19 @@ int32_t bmo_measure_fp64_peak(bmo_ctx* ctx, double* tflops) {
     if (!ctx || !tflops) return fail(BMO_EINVAL, "NULL");
     BMO_CUDA(cudaSetDevice(ctx->device));
     const int blocks = ctx->sm_count * 8, threads = 256, iters = 1 << 16;
-    double* d = nullptr;
-    BMO_CUDA(cudaMalloc((void**)&d, (size_t)blocks * threads * sizeof(double)));
+    DevBuf<double> d;
+    BMO_CUDA(d.alloc((size_t)blocks * threads, ctx->stream));
     float best = 1e30f;
     for (int rep = 0; rep < 5; rep++) {
         BMO_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
-        dfma_probe<<<blocks, threads, 0, ctx->stream>>>(d, iters);
+        dfma_probe<<<blocks, threads, 0, ctx->stream>>>(d.get(), iters);
+        BMO_LAUNCH(ctx, "dfma_probe");
         BMO_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
         BMO_CUDA(cudaStreamSynchronize(ctx->stream));
         float ms;
         BMO_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
         if (rep > 0 && ms < best) best = ms;
     }
-    cudaFree(d);
     *tflops = 2.0 * 8 * iters * (double)blocks * threads / (best * 1e-3) / 1e12;
     return BMO_OK;
 }
@@ -2480,17 +2468,17 @@ int32_t bmo_debug_normals(bmo_sys* sys, int64_t n, const double* points, const i
     bmo_ctx* ctx = sys->ctx;
     BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    double *d_pts = nullptr, *d_a = nullptr, *d_b = nullptr; int32_t* d_idx = nullptr;
-    BMO_CUDA(dev_alloc(&d_pts, (size_t)3 * n, st)); BMO_CUDA(dev_alloc(&d_a, (size_t)3 * n, st)); BMO_CUDA(dev_alloc(&d_b, (size_t)3 * n, st));
-    BMO_CUDA(dev_alloc(&d_idx, (size_t)n, st));
-    BMO_CUDA(cudaMemcpyAsync(d_pts, points, (size_t)3 * n * sizeof(double), cudaMemcpyHostToDevice, st));
-    BMO_CUDA(cudaMemcpyAsync(d_idx, prim_idx, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    debug_normals_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(sys->view, n, d_pts, d_idx, d_a, d_b);
+    DevBuf<double> d_pts, d_a, d_b;
+    DevBuf<int32_t> d_idx;
+    BMO_CUDA(d_pts.alloc((size_t)3 * n, st)); BMO_CUDA(d_a.alloc((size_t)3 * n, st)); BMO_CUDA(d_b.alloc((size_t)3 * n, st));
+    BMO_CUDA(d_idx.alloc((size_t)n, st));
+    BMO_CUDA(cudaMemcpyAsync(d_pts.get(), points, (size_t)3 * n * sizeof(double), cudaMemcpyHostToDevice, st));
+    BMO_CUDA(cudaMemcpyAsync(d_idx.get(), prim_idx, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    debug_normals_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(sys->view, n, d_pts.get(), d_idx.get(), d_a.get(), d_b.get());
     BMO_LAUNCH(ctx, "debug_normals_kernel");
-    BMO_CUDA(cudaMemcpyAsync(out_fast, d_a, (size_t)3 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
-    BMO_CUDA(cudaMemcpyAsync(out_generic, d_b, (size_t)3 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    BMO_CUDA(cudaMemcpyAsync(out_fast, d_a.get(), (size_t)3 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    BMO_CUDA(cudaMemcpyAsync(out_generic, d_b.get(), (size_t)3 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
-    dev_free(d_pts, st); dev_free(d_a, st); dev_free(d_b, st); dev_free(d_idx, st);
     return BMO_OK;
 }
 
