@@ -39,14 +39,16 @@ __global__ void psf_flag(PsfView R, SysView S, int psf_object, int32_t* flags) {
     }
     flags[b] = f;
 }
-// optical_path_length(beam) (Beam.jl:137-149): the parent's OPL first, then the beam's own rays in order
+// optical_path_length(beam) (Beam.jl:137-149): the parent's OPL first, then the beam's own rays in order.  The ancestor of
+// each generation is found by walking up from b again (O(depth^2) parent reads, paid only by deep records), so a beam tree of
+// any depth sums root first without a fixed-size chain.
 __device__ double beam_opl(const PsfView& R, int b) {
-    int chain[64];
     int depth = 0;
-    for (int c = b; c >= 0 && depth < 64; c = R.parent[c]) chain[depth++] = c;
+    for (int c = R.parent[b]; c >= 0; c = R.parent[c]) depth++;
     double l0 = 0.0;
-    for (int d = depth - 1; d >= 0; d--) {
-        const int c = chain[d];
+    for (int d = depth; d >= 0; d--) {
+        int c = b;
+        for (int u = 0; u < d; u++) c = R.parent[c];
         const int64_t f = R.first_seg[c];
         for (int s = 0; s < R.nseg[c]; s++) {
             const double t = R.seg_d[(size_t)(f + s) * R.nsd + S_T];
