@@ -7,7 +7,7 @@ is spelled `f_` here.  There is no CPU fallback.
 """
 from . import linalg
 from ._lib import BmoError, counters, counters_reset, measure_fp64_peak
-from .beams import (Beam, BeamletBundle, CollimatedSource, DeviceSource, GaussianBeamlet, Intersection, PointSource, PolarizedRay, Ray,
+from .beams import (Beam, BeamletBundle, CollimatedSource, DeviceBeamletSource, DeviceSource, GaussianBeamlet, Intersection, PointSource, PolarizedRay, Ray,
                     RayBundle, UniformDiscSource)
 from .components import (AcylindricalSurface, CircularFlatSurface, ConcaveSphericalMirror, CubeBeamsplitter, EvenAsphericalSurface, LensFromSurfaces, SphericalSurface, CylindricalLens, CylindricalSurface, RectangularFlatSurface, DiscreteRefractiveIndex, DoubletLens, IntersectableObject, Lens,
                          MeshDummy, Mirror, NonInteractableObject, ObjectGroup, PSFDetector, Photodetector, PolarizationFilter, Prism, RectangularCompensatorPlate,

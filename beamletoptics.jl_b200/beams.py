@@ -269,9 +269,10 @@ class DeviceSource:
     device pointers, so no per-ray data crosses the bus.  The handles belong to the per-process contexts of _lib.context,
     which live until the process ends, so freeing them from __del__ never outlives the context."""
 
-    def __init__(self, kind, n, pos, dir, lam, rings=(), e1=(0.0, 0.0, 0.0), e2=(0.0, 0.0, 0.0), radius=0.0, phi0=0.0):
+    def __init__(self, kind, n, pos, dir, lam, rings=(), e1=(0.0, 0.0, 0.0), e2=(0.0, 0.0, 0.0), radius=0.0, phi0=0.0, direction=None):
         from . import _lib as L
         self.kind, self.n, self.lam = kind, int(n), float(lam)
+        self.direction = la.v3(dir if direction is None else direction)   # as the constructor was given it (beamlets' from_params)
         self.uniform_dir = kind != L.SRC_POINT
         self.E0 = None
         self._rings = (L.bmo_source_ring * max(1, len(rings)))()
@@ -315,15 +316,28 @@ class DeviceSource:
         from . import _lib as L
         key = (int(device), int(n_poses), self.first, self.n)
         if key not in self._handles:
-            h = C.c_void_p()
-            if (self.first, self.n) == (0, self.desc.n_rays):
-                L.check(L.lib().bmo_source_create_poses(L.context(device), C.byref(self.desc), key[1], C.byref(h)))
-            elif key[1] != 1:
+            whole = (self.first, self.n) == (0, self.desc.n_rays)
+            if not whole and key[1] != 1:
                 raise ValueError("a shard of a source is traced with one pose")
-            else:
-                L.check(L.lib().bmo_source_create_slice(L.context(device), C.byref(self.desc), self.first, self.n, C.byref(h)))
+            h = C.c_void_p()
+            L.check(self._create(L.context(device), key[1], whole, h))
             self._handles[key] = h
         return self._handles[key]
+
+    def _create(self, ctx, n_poses, whole, h):
+        from . import _lib as L
+        if whole:
+            return L.lib().bmo_source_create_poses(ctx, C.byref(self.desc), n_poses, C.byref(h))
+        return L.lib().bmo_source_create_slice(ctx, C.byref(self.desc), self.first, self.n, C.byref(h))
+
+    def beamlets(self, w0, M2=1.0, P0=1e-3, z0=0.0, support=(1.0, 0.0, 0.0)):
+        """GaussianBeamlets on the rays of this source, generated on the GPU (bmo_source_create_beamlets): beamlet i has the
+        bits of BeamletBundle.from_params(P, self.direction, self.lam, w0, M2, P0, z0, support) at the position P of ray i as
+        `rays()` gives it.  A point source is refused (its rays have no common direction)."""
+        from . import _lib as L
+        if self.kind == L.SRC_POINT:
+            raise ValueError("a point source has no beamlet source: its rays differ in direction")
+        return DeviceBeamletSource(self, beamlet_desc(self.direction, self.lam, w0, M2, P0, z0, support))
 
     def device_arrays(self, device=0, n_poses=None):
         """(n, pos, dir, uniform_dir): device pointers for bmo_trace_rays with BMO_INPUT_DEVICE.  With `n_poses` the rays
@@ -371,6 +385,74 @@ class DeviceSource:
             pass
 
 
+def beamlet_desc(direction, lam, w0, M2=1.0, P0=1e-3, z0=0.0, support=(1.0, 0.0, 0.0)):
+    """The bmo_beamlet_desc of GaussianBeamlets with these parameters: the constants BeamletBundle.from_params forms, by its
+    code.  ValueError for w0 <= 0 and for non-finite input or constants."""
+    from . import _lib as L
+    vals = [lam, w0, M2, P0, z0] + list(la.v3(direction)) + list(la.v3(support))
+    if not all(math.isfinite(float(v)) for v in vals):
+        raise ValueError("beamlet parameters must be finite")
+    if not float(w0) > 0:
+        raise ValueError(f"w0 must be > 0, not {w0}")
+    if la.norm(la.v3(direction)) == 0 or la.norm(la.v3(support)) == 0:
+        raise ValueError("direction and support must not be zero vectors")
+    w0a, lama, P0a = np.float64(w0), np.float64(lam), np.float64(P0)
+    d = la.normalize(la.v3(direction))
+    s1 = la.normalize(la.v3(support))
+    tant = math.tan(M2 * lama / (math.pi * w0a))
+    I0 = 2 * P0a / (math.pi * (w0a * w0a))
+    b = L.bmo_beamlet_desc()
+    b.dv[:] = [float(x) for x in la.normalize(d)]
+    b.dd[:] = [float(x) for x in la.normalize(la.normalize(la.add(d, la.scale(tant, s1))))]
+    b.s[:] = [float(x) for x in s1]
+    b.w0, b.div_offset = float(w0a), float(-z0 * tant)
+    b.E0[:] = [float(np.sqrt(2 * I0 * Z_VACUUM)), 0.0]
+    if not all(math.isfinite(x) for x in list(b.dv) + list(b.dd) + list(b.s) + [b.div_offset, b.E0[0]]):
+        raise ValueError("beamlet constants are not finite")
+    return b
+
+
+class DeviceBeamletSource(DeviceSource):
+    """GaussianBeamlets generated on the GPU on the rays of a DeviceSource (DeviceSource.beamlets): the source's descriptor
+    plus one bmo_beamlet_desc, expanded by bmo_source_create_beamlets per (device, n_poses, first, count) like the ray source's
+    handles.  `shard(first, count)` gives the beamlets [first, first + count); solve_system_, the pose sweeps and the sharded
+    solves trace it from the device pointers, so no per-beamlet data crosses the bus."""
+
+    def __init__(self, source, bdesc):
+        self.__dict__.update(source.__dict__)
+        self.bdesc = bdesc
+        self.w0, self.E0 = float(bdesc.w0), complex(bdesc.E0[0], bdesc.E0[1])
+        self._sig = source._sig + bytes(bdesc)
+        self._handles, self._host, self.result = {}, None, None
+        self.__dict__.pop("_solution", None)
+
+    def _create(self, ctx, n_poses, whole, h):
+        from . import _lib as L
+        return L.lib().bmo_source_create_beamlets(ctx, C.byref(self.desc), C.byref(self.bdesc), n_poses, self.first, self.n, C.byref(h))
+
+    def device_beamlets(self, device=0, n_poses=None):
+        """(n, rays, w0, E0): device pointers for bmo_trace_beamlets with BMO_INPUT_DEVICE.  With `n_poses` the beamlets are
+        tiled pose-major and the tuple ends with the pose-id pointer (None for one pose)."""
+        from . import _lib as L
+        h = self.handle(device, 1 if n_poses is None else n_poses)
+        n, r, w, e = C.c_int64(), C.c_void_p(), C.c_void_p(), C.c_void_p()
+        L.check(L.lib().bmo_source_beamlets_device(h, C.byref(n), C.byref(r), C.byref(w), C.byref(e)))
+        if n_poses is None:
+            return int(n.value), r.value, w.value, e.value
+        npo, pid = C.c_int32(), C.c_void_p()
+        L.check(L.lib().bmo_source_pose_ids(h, C.byref(npo), C.byref(pid)))
+        return int(n.value), r.value, w.value, e.value, pid.value
+
+    def beamlets(self, device=0, n_poses=1):
+        """Host copies (rays (n * n_poses, 3, 6), w0 (n * n_poses,), E0 (n * n_poses,) complex) of the beamlets generated on
+        `device` (bmo_source_beamlets)."""
+        from . import _lib as L
+        m = self.n * int(n_poses)
+        rays, w0, e = np.zeros((m, 3, 6)), np.zeros(m), np.zeros((m, 2))
+        L.check(L.lib().bmo_source_beamlets(self.handle(device, n_poses), L.ptr(rays), L.ptr(w0), L.ptr(e)))
+        return rays, w0, e.view(np.complex128).reshape(m)
+
+
 def UniformDiscSource(pos, dir, diameter, lam=1e-6, num_rays=1000, e1=None, on_device=False):
     """BeamGroups.jl:222-245 (Fibonacci disc); `e1` fixes the reference's random in-plane basis.  on_device=True returns a
     DeviceSource whose positions are computed on the GPU (within a few ulp of these: CUDA's sin / cos)."""
@@ -380,7 +462,7 @@ def UniformDiscSource(pos, dir, diameter, lam=1e-6, num_rays=1000, e1=None, on_d
     phi0 = 2 * math.pi / (1 + math.sqrt(5))
     if on_device:
         from . import _lib as L
-        b = DeviceSource(L.SRC_DISC, num_rays, pos, _bundle_dir(d), lam, e1=e1, e2=e2, radius=R, phi0=phi0)
+        b = DeviceSource(L.SRC_DISC, num_rays, pos, _bundle_dir(d), lam, e1=e1, e2=e2, radius=R, phi0=phi0, direction=dir)
         b.diameter = float(diameter)
         return b
     k = np.arange(num_rays, dtype=np.float64)
@@ -405,7 +487,7 @@ def CollimatedSource(pos, dir, diameter, lam=1e-6, num_rings=10, num_rays=None, 
     rings = source_rings("collimated", d, b1, diameter, num_rings, num_rays)
     if on_device:
         from . import _lib as L
-        b = DeviceSource(L.SRC_COLLIMATED, num_rays, p0, _bundle_dir(d), lam, rings=rings)
+        b = DeviceSource(L.SRC_COLLIMATED, num_rays, p0, _bundle_dir(d), lam, rings=rings, direction=dir)
     else:
         pts = [p0]
         _expand_rings(rings, lambda v: pts.append(la.add(p0, v)))

@@ -12,6 +12,9 @@
 // once and source_tile replicates tile 0, so every tile is bit-identical to the untiled source.
 // Source slices (bmo_source_create_slice): rays [first, first + count) of the one-pose source.  A disc thread computes ray
 // first + i; a ring that overlaps the slice runs its recurrence from its own start and writes the rays inside the slice.
+// Beamlet sources (bmo_source_create_beamlets): the kernels above write the chief positions of one tile (or slice) into a
+// temporary, and source_beamlets writes every tile's [18] rays, w0, E0 and pose id from them and the host's constants, one
+// thread per beamlet, with from_params' additions and products.
 // Spot statistics (bmo_spot_stats): two passes over a fixed partition of the spot entries (spot_sums: counts, sums,
 // extrema and the histogram; spot_spread: the squared distances to the centroid).  Each block reduces its slice in a
 // fixed order and the last block to finish combines the per-block partials in block order, so the result does not depend
@@ -110,6 +113,35 @@ __global__ void source_tile(SrcParams P, int uniform) {
     for (int i = 0; i < 3; i++) P.pos[3 * t + i] = P.pos[3 * k + i];
     if (!uniform)
         for (int i = 0; i < 3; i++) P.dir[3 * t + i] = P.dir[3 * k + i];
+}
+
+struct BeamletParams {
+    const double* pos;              // [count][3]: the chief positions of one tile
+    int64_t count, total;           // beamlets of a tile, of all tiles
+    double dv[3], dd[3], s[3], w0, div_offset, e0[2];
+    double *rays, *w0_out, *e0_out; // [total][18], [total], [total][2]
+    int32_t* pose_id;               // [total], NULL for one pose
+};
+
+// one thread per stored beamlet t: tile t / count, beamlet t mod count of the tile; from_params' rows and operation order
+__global__ void source_beamlets(BeamletParams B) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= B.total) return;
+    const int64_t k = t % B.count;
+    const double p[3] = {B.pos[3 * k], B.pos[3 * k + 1], B.pos[3 * k + 2]};
+    double* r = B.rays + 18 * t;
+    for (int i = 0; i < 3; i++) {
+        r[i] = p[i];
+        r[3 + i] = B.dv[i];
+        r[6 + i] = __dadd_rn(p[i], __dmul_rn(B.s[i], B.w0));
+        r[9 + i] = B.dv[i];
+        r[12 + i] = __dadd_rn(p[i], __dmul_rn(B.s[i], B.div_offset));
+        r[15 + i] = B.dd[i];
+    }
+    B.w0_out[t] = B.w0;
+    B.e0_out[2 * t] = B.e0[0];
+    B.e0_out[2 * t + 1] = B.e0[1];
+    if (B.pose_id) B.pose_id[t] = (int32_t)(t / B.count);
 }
 
 // ---- spot statistics ------------------------------------------------------------------------------------------
@@ -384,6 +416,10 @@ struct bmo_source {
     double* pos = nullptr;      // [n][3]
     double* dir = nullptr;      // [n][3], or [3] when uniform
     int32_t* pose_id = nullptr; // [n], NULL for one pose
+    bool beamlets = false;      // bmo_source_create_beamlets: rays / w0 / e0 instead of pos / dir
+    double* rays = nullptr;     // [n][18]
+    double* w0 = nullptr;       // [n]
+    double* e0 = nullptr;       // [n][2]
 };
 
 static bool finite3(const double* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); }
@@ -419,30 +455,29 @@ int32_t bmo_source_free(bmo_source* s) {
     dev_free(s->pos, s->ctx->stream);
     dev_free(s->dir, s->ctx->stream);
     dev_free(s->pose_id, s->ctx->stream);
+    dev_free(s->rays, s->ctx->stream);
+    dev_free(s->w0, s->ctx->stream);
+    dev_free(s->e0, s->ctx->stream);
     delete s;
     return BMO_OK;
 }
 
-// n_poses copies of the rays [first, first + count) of the descriptor (n_poses > 1 only for the whole source)
-static int32_t source_create(bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, int64_t first, int64_t count, bmo_source** out) {
-    BMO_CUDA(cudaSetDevice(ctx->device));
+// n_poses copies of the rays [first, first + count) of the descriptor into pos [count * n_poses][3], dir ([3] for a uniform
+// direction) and pose_id (NULL for one pose); n_poses > 1 only for the whole source
+static int32_t expand_rays(bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, int64_t first, int64_t count, double* pos,
+                           double* dir, int32_t* pose_id) {
     cudaStream_t st = ctx->stream;
-    std::unique_ptr<bmo_source, FreeWith<bmo_source_free>> s(new bmo_source());
-    s->ctx = ctx; s->n_rays = desc->n_rays; s->n_poses = n_poses; s->n = count * n_poses; s->uniform = desc->kind != BMO_SRC_POINT;
-    const int64_t n = s->n;
+    const int64_t n = count * n_poses;
     SrcParams P{};
     P.n = desc->n_rays; P.first = first; P.count = count; P.total = n; P.n_rings = desc->n_rings; P.kind = desc->kind;
     for (int i = 0; i < 3; i++) { P.p[i] = desc->pos[i]; P.d[i] = desc->dir[i]; P.e1[i] = desc->e1[i]; P.e2[i] = desc->e2[i]; }
     P.radius = desc->radius; P.phi0 = desc->phi0;
-    BMO_CUDA(dev_alloc(&s->pos, (size_t)n * 3, st));
-    BMO_CUDA(dev_alloc(&s->dir, s->uniform ? (size_t)3 : (size_t)n * 3, st));
-    if (n_poses > 1) BMO_CUDA(dev_alloc(&s->pose_id, (size_t)n, st));
     DevBuf<bmo_source_ring> d_rings;
     if (desc->kind != BMO_SRC_DISC && desc->n_rings > 0) {
         BMO_CUDA(d_rings.alloc((size_t)desc->n_rings, st));
         BMO_CUDA(cudaMemcpyAsync(d_rings.get(), desc->rings, (size_t)desc->n_rings * sizeof(bmo_source_ring), cudaMemcpyHostToDevice, st));
     }
-    P.rings = d_rings.get(); P.pos = s->pos; P.dir = s->dir; P.pose_id = s->pose_id;
+    P.rings = d_rings.get(); P.pos = pos; P.dir = dir; P.pose_id = pose_id;
     if (desc->kind == BMO_SRC_DISC) {
         source_disc<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P);
         BMO_LAUNCH(ctx, "source_disc");
@@ -451,10 +486,24 @@ static int32_t source_create(bmo_ctx* ctx, const bmo_source_desc* desc, int32_t 
         source_rings<<<(unsigned)((desc->n_rings + 1 + 63) / 64), 64, 0, st>>>(P);
         BMO_LAUNCH(ctx, "source_rings");
         if (n_poses > 1) {
-            source_tile<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P, s->uniform ? 1 : 0);
+            source_tile<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P, desc->kind != BMO_SRC_POINT ? 1 : 0);
             BMO_LAUNCH(ctx, "source_tile");
         }
     }
+    return BMO_OK;
+}
+
+static int32_t source_create(bmo_ctx* ctx, const bmo_source_desc* desc, int32_t n_poses, int64_t first, int64_t count, bmo_source** out) {
+    BMO_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    std::unique_ptr<bmo_source, FreeWith<bmo_source_free>> s(new bmo_source());
+    s->ctx = ctx; s->n_rays = desc->n_rays; s->n_poses = n_poses; s->n = count * n_poses; s->uniform = desc->kind != BMO_SRC_POINT;
+    const int64_t n = s->n;
+    BMO_CUDA(dev_alloc(&s->pos, (size_t)n * 3, st));
+    BMO_CUDA(dev_alloc(&s->dir, s->uniform ? (size_t)3 : (size_t)n * 3, st));
+    if (n_poses > 1) BMO_CUDA(dev_alloc(&s->pose_id, (size_t)n, st));
+    int32_t rc;
+    if ((rc = expand_rays(ctx, desc, n_poses, first, count, s->pos, s->dir, s->pose_id))) return rc;
     *out = s.release();
     return BMO_OK;
 }
@@ -484,6 +533,78 @@ int32_t bmo_source_create_slice(bmo_ctx* ctx, const bmo_source_desc* desc, int64
     return source_create(ctx, desc, 1, first, count, out);
 }
 
+static bool finite_n(const double* v, int n) {
+    for (int i = 0; i < n; i++)
+        if (!std::isfinite(v[i])) return false;
+    return true;
+}
+
+int32_t bmo_source_create_beamlets(bmo_ctx* ctx, const bmo_source_desc* desc, const bmo_beamlet_desc* bd, int32_t n_poses, int64_t first,
+                                   int64_t count, bmo_source** out) {
+    NvtxRange nvtx_("bmo_source_create_beamlets");
+    const std::string fn = "bmo_source_create_beamlets";
+    if (!ctx || !desc || !bd || !out) return fail(BMO_EINVAL, fn + ": NULL argument");
+    int32_t rc;
+    if ((rc = check_desc(desc))) return rc;
+    if (desc->kind == BMO_SRC_POINT) return fail(BMO_EINVAL, fn + ": a point source's rays have no common direction for its beamlets");
+    if (!finite_n(bd->dv, 3) || !finite_n(bd->dd, 3) || !finite_n(bd->s, 3) || !std::isfinite(bd->w0) || !std::isfinite(bd->div_offset) ||
+        !finite_n(bd->E0, 2))
+        return fail(BMO_EINVAL, fn + ": beamlet constants not finite");
+    if (!(bd->w0 > 0)) return fail(BMO_EINVAL, fn + ": w0 must be > 0");
+    if (n_poses < 1) return fail(BMO_EINVAL, fn + ": n_poses must be >= 1");
+    if (first < 0 || count < 1 || first > desc->n_rays - count)
+        return fail(BMO_EINVAL, fn + ": beamlets [" + std::to_string(first) + ", " + std::to_string(first) + " + " + std::to_string(count) +
+                                    ") are not a non-empty part of the source's " + std::to_string(desc->n_rays));
+    if (n_poses > 1 && (first != 0 || count != desc->n_rays)) return fail(BMO_EINVAL, fn + ": a slice of a source is made with one pose");
+    if (count > INT64_MAX / n_poses) return fail(BMO_EINVAL, fn + ": count * n_poses overflows int64");
+    BMO_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    std::unique_ptr<bmo_source, FreeWith<bmo_source_free>> s(new bmo_source());
+    s->ctx = ctx; s->n_rays = desc->n_rays; s->n_poses = n_poses; s->n = count * n_poses; s->beamlets = true;
+    const int64_t n = s->n;
+    // the chief positions of one tile, by the ray source's own kernels
+    DevBuf<double> pos, dir;
+    BMO_CUDA(pos.alloc((size_t)count * 3, st));
+    BMO_CUDA(dir.alloc(3, st));
+    if ((rc = expand_rays(ctx, desc, 1, first, count, pos.get(), dir.get(), nullptr))) return rc;
+    BMO_CUDA(dev_alloc(&s->rays, (size_t)n * 18, st));
+    BMO_CUDA(dev_alloc(&s->w0, (size_t)n, st));
+    BMO_CUDA(dev_alloc(&s->e0, (size_t)n * 2, st));
+    if (n_poses > 1) BMO_CUDA(dev_alloc(&s->pose_id, (size_t)n, st));
+    BeamletParams B{};
+    B.pos = pos.get(); B.count = count; B.total = n;
+    for (int i = 0; i < 3; i++) { B.dv[i] = bd->dv[i]; B.dd[i] = bd->dd[i]; B.s[i] = bd->s[i]; }
+    B.w0 = bd->w0; B.div_offset = bd->div_offset; B.e0[0] = bd->E0[0]; B.e0[1] = bd->E0[1];
+    B.rays = s->rays; B.w0_out = s->w0; B.e0_out = s->e0; B.pose_id = s->pose_id;
+    source_beamlets<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(B);
+    BMO_LAUNCH(ctx, "source_beamlets");
+    *out = s.release();
+    return BMO_OK;
+}
+
+int32_t bmo_source_beamlets_device(bmo_source* s, int64_t* n, const double** rays, const double** w0, const double** E0) {
+    if (!s) return fail(BMO_EINVAL, "bmo_source_beamlets_device: source NULL");
+    if (!s->beamlets) return fail(BMO_EINVAL, "bmo_source_beamlets_device: a ray source holds no beamlets (bmo_source_device)");
+    if (n) *n = s->n;
+    if (rays) *rays = s->rays;
+    if (w0) *w0 = s->w0;
+    if (E0) *E0 = s->e0;
+    return BMO_OK;
+}
+
+int32_t bmo_source_beamlets(bmo_source* s, double* rays, double* w0, double* E0) {
+    if (!s) return fail(BMO_EINVAL, "bmo_source_beamlets: source NULL");
+    if (!s->beamlets) return fail(BMO_EINVAL, "bmo_source_beamlets: a ray source holds no beamlets (bmo_source_rays)");
+    BMO_CUDA(cudaSetDevice(s->ctx->device));
+    cudaStream_t st = s->ctx->stream;
+    const size_t n = (size_t)s->n;
+    if (rays) BMO_CUDA(cudaMemcpyAsync(rays, s->rays, n * 18 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (w0) BMO_CUDA(cudaMemcpyAsync(w0, s->w0, n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (E0) BMO_CUDA(cudaMemcpyAsync(E0, s->e0, n * 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    BMO_CUDA(cudaStreamSynchronize(st));
+    return BMO_OK;
+}
+
 int32_t bmo_source_pose_ids(bmo_source* s, int32_t* n_poses, const int32_t** pose_id) {
     if (!s) return fail(BMO_EINVAL, "bmo_source_pose_ids: source NULL");
     if (n_poses) *n_poses = s->n_poses;
@@ -493,6 +614,7 @@ int32_t bmo_source_pose_ids(bmo_source* s, int32_t* n_poses, const int32_t** pos
 
 int32_t bmo_source_device(bmo_source* s, int64_t* n, const double** pos, const double** dir, int32_t* uniform_dir) {
     if (!s) return fail(BMO_EINVAL, "bmo_source_device: source NULL");
+    if (s->beamlets) return fail(BMO_EINVAL, "bmo_source_device: a beamlet source holds no rays (bmo_source_beamlets_device)");
     if (n) *n = s->n;
     if (pos) *pos = s->pos;
     if (dir) *dir = s->dir;
@@ -502,6 +624,7 @@ int32_t bmo_source_device(bmo_source* s, int64_t* n, const double** pos, const d
 
 int32_t bmo_source_rays(bmo_source* s, double* pos, double* dir) {
     if (!s) return fail(BMO_EINVAL, "bmo_source_rays: source NULL");
+    if (s->beamlets) return fail(BMO_EINVAL, "bmo_source_rays: a beamlet source holds no rays (bmo_source_beamlets)");
     BMO_CUDA(cudaSetDevice(s->ctx->device));
     cudaStream_t st = s->ctx->stream;
     const size_t n = (size_t)s->n;

@@ -253,8 +253,9 @@ def psf_shard_band(n, rank, world_size):
 
 def solve_psf_sharded(system, source, detector, n=100, crop_factor=1.0, center="centroid", x_min=math.inf, x_max=math.inf,
                       z_min=math.inf, z_max=math.inf, x0_shift=0.0, z0_shift=0.0, comm=None, r_max=100):
-    """The intensity map of `detector` (a PSFDetector of `system`) for a DeviceSource, RayBundle or BeamletBundle traced across all
-    ranks: this rank traces its shard_slice of the source (DeviceSource.shard / shard_bundle) on the communicator's GPU, its records are
+    """The intensity map of `detector` (a PSFDetector of `system`) for a DeviceSource, DeviceBeamletSource, RayBundle or BeamletBundle
+    traced across all ranks: this rank traces its shard_slice of the source (DeviceSource.shard, which builds only those rays or
+    beamlets on the device / shard_bundle) on the communicator's GPU, its records are
     appended to the detector as by solve_system_, and FieldComm.psf_intensity makes the map of all ranks' records.  Returns
     (xs, zs, I) on every rank: for a system without beamsplitters the bits of solve_system_ of the whole source followed by
     detector.intensity(...) on one GPU.  `comm`: a FieldComm (default: default_comm(), a one-rank communicator outside
@@ -279,16 +280,24 @@ def solve_psf_sharded(system, source, detector, n=100, crop_factor=1.0, center="
 def solve_system_sharded(system, bundle, r_max=100, interleaved=False, keep_segments=False, group=None, comm=None):
     """solve_system! of a bundle across all ranks: this rank traces its shard on GPU LOCAL_RANK; every
     Photodetector of `system` ends up with the field of the *whole* bundle on every rank (all-reduce);
-    Spotdetector data stay rank-local (disjoint slices).  Returns (TraceResult of the shard, indices)."""
+    Spotdetector data stay rank-local (disjoint slices).  A DeviceSource or DeviceBeamletSource is cut into contiguous
+    shard_slice parts, each rank building only its own on the device (interleaved=True is refused: a device shard is
+    contiguous).  Returns (TraceResult of the shard, indices)."""
     from . import components as co
     from .solver import solve_system_
     rank, ws, local = world()
-    part, idx = shard_bundle(bundle, rank, ws, interleaved)
+    if isinstance(bundle, bm.DeviceSource):
+        if interleaved:
+            raise ValueError("a device source is sharded in contiguous slices, not interleaved")
+        start, stop = shard_slice(len(bundle), rank, ws)
+        part, idx = (bundle.shard(start, stop - start) if stop > start else None), np.arange(start, stop)
+    else:
+        part, idx = shard_bundle(bundle, rank, ws, interleaved)
     pds = [o for o in system.leaves() if isinstance(o, co.Photodetector)]
     before = [pd.field.copy() for pd in pds]
     for pd in pds:                       # accumulate this rank's beamlets onto a zeroed partial field
         pd.field[...] = 0
-    res = solve_system_(system, part, r_max=r_max, device=local, keep_segments=keep_segments) if len(part) else None
+    res = solve_system_(system, part, r_max=r_max, device=local, keep_segments=keep_segments) if part is not None and len(part) else None
     for pd, old in zip(pds, before):
         allreduce_field(pd.field, group, comm)
         pd.field += old                  # the reference's `+=` onto whatever the detector already held

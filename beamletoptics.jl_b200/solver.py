@@ -232,14 +232,21 @@ def trace_rays_spots(dsys, pos, dir, lam_id, E0=None, pose_id=None, r_max=100, w
     return obj, xz, TraceResult(dsys, h)
 
 
-def trace_beamlets(dsys, rays, lam_id, w0, E0, pose_id=None, r_max=100):
+def trace_beamlets(dsys, rays, lam_id, w0, E0, pose_id=None, r_max=100, device_inputs=False):
+    """Thin wrapper of bmo_trace_beamlets.  With device_inputs=True rays/lam_id/w0/E0/pose_id are integer device pointers
+    (lam_id and pose_id may be None) and `n` must be given as rays=(ptr, n), as in trace_rays."""
+    h = C.c_void_p()
+    if device_inputs:
+        (prays, n) = rays
+        L.check(L.lib().bmo_trace_beamlets(dsys.h, n, L.ptr(prays), L.ptr(lam_id), L.ptr(w0), L.ptr(E0), L.ptr(pose_id), r_max, L.INPUT_DEVICE,
+                                           C.byref(h)))
+        return TraceResult(dsys, h)
     rays = np.ascontiguousarray(rays, dtype=np.float64).reshape(-1, 18)
     lam_id = np.ascontiguousarray(lam_id, dtype=np.int32)
     w0 = np.ascontiguousarray(w0, dtype=np.float64)
     ec = np.ascontiguousarray(E0, dtype=np.complex128)
     e = np.ascontiguousarray(np.stack([ec.real, ec.imag], axis=-1))
     pid = None if pose_id is None else np.ascontiguousarray(pose_id, dtype=np.int32)
-    h = C.c_void_p()
     L.check(L.lib().bmo_trace_beamlets(dsys.h, rays.shape[0], L.ptr(rays), L.ptr(lam_id), L.ptr(w0), L.ptr(e), L.ptr(pid), r_max, 0, C.byref(h)))
     return TraceResult(dsys, h)
 
@@ -386,8 +393,8 @@ def _collect_spots(system_flat, res):
 
 
 def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rule=1, keep_segments=True, collect_spots=True):
-    """solve_system!(system, beam; r_max, retrace) for a Beam, GaussianBeamlet, RayBundle, DeviceSource or
-    BeamletBundle (System.jl:444-468).  Returns the TraceResult (the reference returns nothing).
+    """solve_system!(system, beam; r_max, retrace) for a Beam, GaussianBeamlet, RayBundle, DeviceSource, BeamletBundle or
+    DeviceBeamletSource (System.jl:444-468).  Returns the TraceResult (the reference returns nothing).
     collect_spots=False leaves Spotdetector.data alone: the hits stay on the device for spot_stats / TraceResult.spots."""
     if isinstance(beam, (list, tuple)):
         return [solve_system_(system, b, r_max, retrace, device, norm_zero_rule, keep_segments, collect_spots) for b in beam]
@@ -450,6 +457,23 @@ def solve_system_(system, beam, r_max=100, retrace=True, device=0, norm_zero_rul
             _collect_spots(dsys.flat, res)
         if has_psf:
             _collect_psfs(dsys, res)
+        return res
+    if isinstance(beam, bm.DeviceBeamletSource):
+        lams, _ = _lambda_ids([beam.lam])
+        dsys = cached_system(system, lams, device, norm_zero_rule)
+        prev = _previous_solution(beam, dsys, lams) if retrace else None
+        if prev is not None:
+            res = globals()["retrace"](dsys, prev, r_max)
+        else:      # the beamlets never leave the device: bmo_source -> bmo_trace_beamlets(BMO_INPUT_DEVICE)
+            n, rays, w0, E0 = beam.device_beamlets(device)
+            res = trace_beamlets(dsys, (rays, n), None, w0, E0, None, r_max, device_inputs=True)
+        res.lams = lams
+        beam.result = beam._solution = res
+        res._root_sig = _root_signature(beam)
+        if collect_spots:
+            _collect_spots(dsys.flat, res)
+        _collect_psfs(dsys, res)
+        _accumulate_pds(dsys, res)
         return res
     if isinstance(beam, bm.DeviceSource):
         lams, _ = _lambda_ids([beam.lam])

@@ -15,7 +15,7 @@ import numpy as np
 from . import _lib as L
 from . import beams as bm
 from .flatten import FlatSystem
-from .solver import DeviceSystem, TraceResult, _lambda_ids, spot_stats_poses, trace_rays
+from .solver import DeviceSystem, _lambda_ids, spot_stats_poses, trace_beamlets, trace_rays
 
 
 def flatten_poses(system, lambdas, n_poses, apply_pose, norm_zero_rule=1):
@@ -38,24 +38,13 @@ def flatten_poses(system, lambdas, n_poses, apply_pose, norm_zero_rule=1):
 
 
 def solve_pose_sweep(system, beam, n_poses, apply_pose, pd, r_max=100, device=0, want_fields=True):
-    """Trace `beam` (GaussianBeamlet or BeamletBundle) through `n_poses` poses of `system`.
+    """Trace `beam` (GaussianBeamlet, BeamletBundle or DeviceBeamletSource) through `n_poses` poses of `system`.
     Returns dict(fields=(n_poses, n, n) complex, power=(n_poses,), result=TraceResult)."""
-    if isinstance(beam, bm.GaussianBeamlet):
-        beam = bm.BeamletBundle(np.array([beam.rays18()]), [beam.lam], [beam.w0], [beam.E0])
-    lams, lam_id = _lambda_ids(beam.lam)
+    lams, lam_id, beam = _beamlet_lambdas(beam)
     f0, (prims, verts, bounds, det_pos, det_dir) = flatten_poses(system, lams, n_poses, apply_pose)
     dsys = DeviceSystem(f0, device)
     L.check(L.lib().bmo_system_set_poses(dsys.h, n_poses, L.ptr(prims), L.ptr(verts), L.ptr(bounds), L.ptr(det_pos), L.ptr(det_dir)))
-    nb = len(beam)
-    rays = np.ascontiguousarray(np.tile(beam.rays.reshape(nb, 18), (n_poses, 1)))
-    lam_ids = np.ascontiguousarray(np.tile(lam_id, n_poses))
-    w0 = np.ascontiguousarray(np.tile(beam.w0, n_poses))
-    E0 = np.tile(beam.E0, n_poses)
-    e = np.ascontiguousarray(np.stack([E0.real, E0.imag], axis=-1))
-    pose_id = np.ascontiguousarray(np.repeat(np.arange(n_poses, dtype=np.int32), nb))
-    h = C.c_void_p()
-    L.check(L.lib().bmo_trace_beamlets(dsys.h, rays.shape[0], L.ptr(rays), L.ptr(lam_ids), L.ptr(w0), L.ptr(e), L.ptr(pose_id), r_max, 0, C.byref(h)))
-    res = TraceResult(dsys, h)
+    res = _trace_beamlet_sweep(dsys, beam, lam_id, n_poses, r_max)
     pd_index = f0.object_index(pd)
     n = pd.n
     # one call: per-pose fields accumulated and integrated on the device; the fields only come back when asked for
@@ -147,24 +136,13 @@ def get_pose_tables(dsys, pose):
 def solve_pose_sweep_device(system, beam, n_poses, program, pd, r_max=100, device=0, want_fields=True):
     """solve_pose_sweep with the poses produced on the device: `program(prog)` records the kinematic calls of the
     sweep on a KinProgram (e.g. `prog.translate3d_(mirror, offsets)`); the host objects are not moved."""
-    if isinstance(beam, bm.GaussianBeamlet):
-        beam = bm.BeamletBundle(np.array([beam.rays18()]), [beam.lam], [beam.w0], [beam.E0])
-    lams, lam_id = _lambda_ids(beam.lam)
+    lams, lam_id, beam = _beamlet_lambdas(beam)
     f0 = FlatSystem(system, lams)
     dsys = DeviceSystem(f0, device)
     prog = KinProgram(f0, n_poses)
     program(prog)
     prog.apply(dsys)
-    nb = len(beam)
-    rays = np.ascontiguousarray(np.tile(beam.rays.reshape(nb, 18), (n_poses, 1)))
-    lam_ids = np.ascontiguousarray(np.tile(lam_id, n_poses))
-    w0 = np.ascontiguousarray(np.tile(beam.w0, n_poses))
-    E0 = np.tile(beam.E0, n_poses)
-    e = np.ascontiguousarray(np.stack([E0.real, E0.imag], axis=-1))
-    pose_id = np.ascontiguousarray(np.repeat(np.arange(n_poses, dtype=np.int32), nb))
-    h = C.c_void_p()
-    L.check(L.lib().bmo_trace_beamlets(dsys.h, rays.shape[0], L.ptr(rays), L.ptr(lam_ids), L.ptr(w0), L.ptr(e), L.ptr(pose_id), r_max, 0, C.byref(h)))
-    res = TraceResult(dsys, h)
+    res = _trace_beamlet_sweep(dsys, beam, lam_id, n_poses, r_max)
     pd_index = f0.object_index(pd)
     n = pd.n
     fields = np.zeros((n_poses, n * n * 2)) if want_fields else None
@@ -202,6 +180,27 @@ def _trace_spot_sweep(dsys, beam, lam_id, n_poses, r_max):
     lam = None if len(dsys.flat.lambdas) == 1 else np.tile(lam_id, n_poses)
     E0 = None if beam.E0 is None else np.tile(beam.E0, (n_poses, 1))
     return trace_rays(dsys, pos, dir, lam, E0, pose_id, r_max, False)
+
+
+def _beamlet_lambdas(beam):
+    """(lambdas, lambda ids, beam) of a pose sweep's beamlets; a GaussianBeamlet becomes a one-beamlet BeamletBundle."""
+    if isinstance(beam, bm.DeviceBeamletSource):
+        return _lambda_ids([beam.lam]) + (beam,)
+    if isinstance(beam, bm.GaussianBeamlet):
+        beam = bm.BeamletBundle(np.array([beam.rays18()]), [beam.lam], [beam.w0], [beam.E0])
+    return _lambda_ids(beam.lam) + (beam,)
+
+
+def _trace_beamlet_sweep(dsys, beam, lam_id, n_poses, r_max):
+    """Trace the beamlets of `beam` once per pose of `dsys`: a DeviceBeamletSource is tiled on the device, a BeamletBundle on
+    the host, both pose-major with pose_id[i] = i // len(beam)."""
+    if isinstance(beam, bm.DeviceBeamletSource):
+        n, rays, w0, E0, pid = beam.device_beamlets(dsys.device, n_poses)
+        return trace_beamlets(dsys, (rays, n), None, w0, E0, pid, r_max, device_inputs=True)
+    nb = len(beam)
+    rays = np.tile(beam.rays.reshape(nb, 18), (n_poses, 1))
+    pose_id = np.repeat(np.arange(n_poses, dtype=np.int32), nb)
+    return trace_beamlets(dsys, rays, np.tile(lam_id, n_poses), np.tile(beam.w0, n_poses), np.tile(beam.E0, n_poses), pose_id, r_max)
 
 
 def _beam_lambdas(beam):

@@ -346,15 +346,53 @@ int32_t bmo_source_create_poses(bmo_ctx* ctx, const bmo_source_desc* desc, int32
  * bmo_source_device reports n = count, bmo_source_rays copies the slice, bmo_source_pose_ids gives NULL.  BMO_EINVAL for
  * first < 0, count < 1, first + count > n_rays, and whatever bmo_source_create refuses.                              */
 int32_t bmo_source_create_slice(bmo_ctx* ctx, const bmo_source_desc* desc, int64_t first, int64_t count, bmo_source** src);
-/* Device pose ids [n_rays * n_poses] for bmo_trace_rays(..., pose_id, BMO_INPUT_DEVICE); NULL for a one-pose source.
- * Valid until bmo_source_free.                                                                                       */
+/* Device pose ids [n_rays * n_poses] for bmo_trace_rays(..., pose_id, BMO_INPUT_DEVICE) or, of a beamlet source,
+ * bmo_trace_beamlets; NULL for a one-pose source.  Valid until bmo_source_free.                                      */
 int32_t bmo_source_pose_ids(bmo_source* src, int32_t* n_poses, const int32_t** pose_id);
 /* Device pointers for bmo_trace_rays(..., BMO_INPUT_DEVICE | (*uniform_dir ? BMO_UNIFORM_DIR : 0)): pos [n][3];
- * dir [n][3], or one direction [3] when *uniform_dir is 1.  n counts the rays of every pose.  Valid until bmo_source_free. */
+ * dir [n][3], or one direction [3] when *uniform_dir is 1.  n counts the rays of every pose.  Valid until bmo_source_free.
+ * BMO_EINVAL on a beamlet source (bmo_source_create_beamlets).                                                          */
 int32_t bmo_source_device(bmo_source* src, int64_t* n, const double** pos, const double** dir, int32_t* uniform_dir);
-/* host copies (NULL ok): pos [n][3], dir [n][3] (a uniform direction is expanded to every ray)                   */
+/* host copies (NULL ok): pos [n][3], dir [n][3] (a uniform direction is expanded to every ray); BMO_EINVAL on a
+ * beamlet source                                                                                                 */
 int32_t bmo_source_rays(bmo_source* src, double* pos, double* dir);
 int32_t bmo_source_free(bmo_source* src);   /* before bmo_shutdown of the source's context */
+
+/* ---- Gaussian beamlet sources generated on the device ----------------------------------------------------------------
+ * replaces: BeamletBundle.from_params / GaussianBeamlet (Gaussian.jl:215-256) over the rays of a disc or collimated source, built
+ * on the host and copied over (144 B of rays, w0, E0 and a wavelength id per beamlet, once per pose for a pose sweep).  Every
+ * beamlet shares one set of parameters; the host computes every scalar and vector below with the code of from_params, and the
+ * device only adds and multiplies, in from_params' order, without FMA contraction.  Beamlet i at source position P (the
+ * position bmo_source_rays gives ray i of the same source descriptor):
+ *   chief       pos P,                 dir dv
+ *   waist       pos P + s * w0,        dir dv
+ *   divergence  pos P + s * div_offset, dir dd
+ *   w0[i] = w0, E0[i] = E0.
+ * With d = normalize(direction), s = normalize(support), tan_t = tan(M2 lambda / (pi w0)), I0 = 2 P0 / (pi w0^2):
+ * dv = normalize(d), dd = normalize(normalize(d + tan_t s)), div_offset = -z0 tan_t, E0 = sqrt(2 I0 Z0) + 0i.       */
+typedef struct bmo_beamlet_desc {
+    double dv[3];           /* chief and waist direction                                                             */
+    double dd[3];           /* divergence direction                                                                  */
+    double s[3];            /* normalised support vector                                                             */
+    double w0;              /* waist radius, > 0                                                                     */
+    double div_offset;      /* -z0 tan_t: offset of the divergence ray along s                                      */
+    double E0[2];           /* field amplitude (re, im)                                                              */
+} bmo_beamlet_desc;
+/* Beamlets [first, first + count) of the one-pose source, tiled n_poses times pose-major (beamlet i is beamlet first + i mod
+ * count, pose_id[i] = i / count; n_poses > 1 only for the whole source, first = 0 and count = n_rays).  The positions are those
+ * bmo_source_create_slice / _poses give the same descriptor, so each tile and slice has the bits of the matching rows of the
+ * whole one-pose source.  BMO_EINVAL for whatever bmo_source_create refuses, a point source (its directions differ per ray),
+ * non-finite constants, w0 <= 0, n_poses < 1, n_poses > 1 on a slice, a slice outside the source and count * n_poses
+ * overflowing int64.  bmo_source_device and bmo_source_rays refuse a beamlet source with BMO_EINVAL; bmo_source_pose_ids
+ * gives its pose ids (NULL for one pose).                                                                                */
+int32_t bmo_source_create_beamlets(bmo_ctx* ctx, const bmo_source_desc* desc, const bmo_beamlet_desc* beamlet, int32_t n_poses,
+                                   int64_t first, int64_t count, bmo_source** src);
+/* Device pointers for bmo_trace_beamlets(..., BMO_INPUT_DEVICE) (lambda_id NULL: the source's one wavelength is lambdas[0]):
+ * rays [n][3][6], w0 [n], E0 [n][2]; n counts the beamlets of every pose.  Valid until bmo_source_free.  BMO_EINVAL on a ray
+ * source.                                                                                                                 */
+int32_t bmo_source_beamlets_device(bmo_source* src, int64_t* n, const double** rays, const double** w0, const double** E0);
+/* host copies (NULL ok): rays [n][3][6], w0 [n], E0 [n][2].  BMO_EINVAL on a ray source.                                  */
+int32_t bmo_source_beamlets(bmo_source* src, double* rays, double* w0, double* E0);
 
 /* ---- spot-diagram reduction on the device --------------------------------------------------------------
  * replaces: reading Spotdetector.data (Spotdetector.jl:50-61) back to compute what a spot diagram shows.  Works over the
