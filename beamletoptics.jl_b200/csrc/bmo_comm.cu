@@ -9,6 +9,8 @@
 //   * The PSFDetector map of a ray bundle sharded over several GPUs (bmo_psf_allgather, bmo_psf_intensity_sharded): the hit
 //     records are all-gathered in rank order, every rank sums all records into its band of pixel columns, and the bands are
 //     all-gathered.  Each pixel is summed on one GPU over the records of one trace in order, so the map has one GPU's bits.
+//   * The Photodetector pose sweep sharded over GPUs by pose range (bmo_pd_sweep_sharded): every rank sweeps its contiguous
+//     poses with bmo_pd_sweep's code, the fields stay where they are, and the powers are all-gathered into pose order.
 //
 // NCCL is bound at run time (dlopen of libnccl.so.2) so that libbmo.so has no link-time dependency on it: a host
 // that never shards never needs the library, and inside a process that already carries one (PyTorch's bundled
@@ -394,6 +396,74 @@ int32_t bmo_psf_intensity_sharded(bmo_comm* c, bmo_sys* sys, bmo_psf* all, int32
         BMO_CUDA(cudaEventElapsedTime(&kms, ctx->evk0, ctx->evk1));
         ctx->psf_ms = kms;
     }
+    return BMO_OK;
+}
+
+int32_t bmo_pd_sweep_sharded(bmo_comm* c, bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t n_poses, int32_t first, int32_t count,
+                             double* fields, double* power, uint32_t flags) {
+    NvtxRange nvtx_("bmo_pd_sweep_sharded");
+    const std::string fn = "bmo_pd_sweep_sharded";
+    if (!c) return fail(BMO_EINVAL, fn + ": communicator NULL");
+    // Step 1: every rank's verdict (bmo_pd_sweep's checks on this rank's poses) and the arguments that must agree
+    int32_t rc = BMO_OK;
+    if (!sys || !power) rc = fail(BMO_EINVAL, fn + ": NULL argument");
+    else if (sys->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the system belongs to another context than the communicator");
+    else if (n_poses < 1 || first < 0 || count < 0 || count > n_poses - first)
+        rc = fail(BMO_EINVAL, fn + ": poses [first, first + count) outside [0, n_poses)");
+    else if (count > sys->view.n_poses) rc = fail(BMO_EINVAL, fn + ": the system holds fewer poses than count");
+    else if (pd_object < 0 || pd_object >= (int)sys->objects.size() || sys->objects[pd_object].kind != BMO_OBJ_PHOTODETECTOR)
+        rc = fail(BMO_EINVAL, fn + ": object is not a Photodetector");
+    else if (count > 0 && !r) rc = fail(BMO_EINVAL, fn + ": NULL result on a rank with poses");
+    else if (count > 0 && r->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the result belongs to another context than the communicator");
+    else if (count > 0 && r->mode != 2) rc = fail(BMO_EINVAL, fn + ": result does not hold Gaussian beamlets (Photodetector.jl:57-60)");
+    const int n = rc ? 0 : sys->objects[pd_object].pd_n;
+    constexpr int K = 6;   // verdict, then pd_object, n, n_poses (as rank 0's), first, count (tiling [0, n_poses) in rank order)
+    std::vector<int64_t> mine{rc, pd_object, n, n_poses, first, count}, all;
+    if ((rc = agree(c, fn, mine, all))) return rc;
+    const int W = c->n_ranks;
+    int64_t next = 0, most = 0;
+    for (int k = 0; k < W; k++) {
+        const int64_t* a = all.data() + (size_t)K * k;
+        if (!std::equal(a + 1, a + 4, all.data() + 1))
+            return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " passes another detector, detector size or pose count than rank 0");
+        if (a[4] != next)
+            return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " sweeps from pose " + std::to_string(a[4]) + ", not " + std::to_string(next) +
+                                        " (the ranks' poses must tile [0, n_poses) in rank order)");
+        next += a[5];
+        most = std::max(most, a[5]);
+    }
+    if (next != n_poses)
+        return fail(BMO_EINVAL, fn + ": the ranks sweep " + std::to_string(next) + " of " + std::to_string(n_poses) + " poses");
+    // Step 2: this rank's fields and powers, on the device
+    bmo_ctx* ctx = c->ctx;
+    BMO_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const bool on_dev = flags & BMO_INPUT_DEVICE;
+    const cudaMemcpyKind out_kind = on_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    const size_t fcount = (size_t)count * n * n * 2;
+    DevBuf<double> f_buf, p_buf;
+    BMO_CUDA(p_buf.alloc((size_t)most * (W > 1 ? W + 1 : 1), st));   // [W][most] gathered, then this rank's powers
+    double* my_power = p_buf.get() + (W > 1 ? (size_t)most * W : 0);
+    if (count > 0) {
+        double* d_field = fields;     // the caller's device buffer
+        if (!on_dev || !fields) {
+            BMO_CUDA(f_buf.alloc(fcount, st));
+            d_field = f_buf.get();
+        }
+        if ((rc = pd_sweep_device(sys, r, pd_object, count, d_field, my_power, flags))) return rc;
+        if (fields && !on_dev) BMO_CUDA(cudaMemcpyAsync(fields, d_field, fcount * sizeof(double), cudaMemcpyDeviceToHost, st));
+    }
+    // Step 3: the powers of all ranks, padded to the largest count, and each rank's part copied into pose order
+    if (W == 1) {
+        BMO_CUDA(cudaMemcpyAsync(power, my_power, (size_t)count * sizeof(double), out_kind, st));
+    } else {
+        BMO_NCCL(g_nccl.AllGather(my_power, p_buf.get(), (size_t)most, kNcclDouble, c->comm, st));
+        for (int k = 0; k < W; k++) {
+            const int64_t fk = all[(size_t)K * k + 4], ck = all[(size_t)K * k + 5];
+            if (ck) BMO_CUDA(cudaMemcpyAsync(power + fk, p_buf.get() + (size_t)most * k, (size_t)ck * sizeof(double), out_kind, st));
+        }
+    }
+    BMO_CUDA(cudaStreamSynchronize(st));
     return BMO_OK;
 }
 

@@ -17,6 +17,8 @@
 //       (tilted detectors, Beam.jl:186-199) take the reference-order path below.
 //   pd_field (BMO_PD_REFERENCE_ORDER)  every pair evaluated in the reference's operation order;
 //       kept as the cross-check of the fast kernel at full detector sizes.
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include "bmo_host.cuh"
 #include "bmo_interact.cuh"
 
@@ -66,12 +68,13 @@ struct ResView {
     int64_t n_beams;
 };
 
-// flags[b] = 1 if beam b ended on detector `pd` after a full interaction (all three rays on the PD shape)
-__global__ void pd_flag(ResView R, SysView S, int pd_object, int pose_filter, int32_t* flags) {
+// flags[b] = 1 if beam b of a pose in [pose_lo, pose_hi) ended on detector `pd` after a full interaction (all three rays on
+// the PD shape)
+__global__ void pd_flag(ResView R, SysView S, int pd_object, int pose_lo, int pose_hi, int32_t* flags) {
     const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= R.n_beams) return;
     int f = 0;
-    if ((R.status[b] & 0xff) == BMO_ST_ABSORBED && R.nseg[b] > 0 && (pose_filter < 0 || R.pose[b] == pose_filter)) {
+    if ((R.status[b] & 0xff) == BMO_ST_ABSORBED && R.nseg[b] > 0 && R.pose[b] >= pose_lo && R.pose[b] < pose_hi) {
         const int64_t row = (R.first_seg[b] + R.nseg[b] - 1) * 3;
         const int part = R.seg_part[row];
         if (part >= 0 && S.parts[part].object == pd_object) f = 1;
@@ -119,6 +122,41 @@ __global__ void pd_build(ResView R, SysView S, const int32_t* flags, const long 
     rc.first_row = (double)f; rc.nseg = (double)n; rc.pose = (double)R.pose[b]; rc.pad = 0;
     recs[offs[b]] = rc;
 }
+// Grouping the records of a sweep by pose, on the device (pd_run):
+//   pd_pose_count  cnt[p - pose0] = records of pose p (the beams flagged by pd_flag), and *unsorted = 1 when some beam's pose id
+//                  is smaller than its predecessor's.  Records are numbered in beam order, so without such a beam they are
+//                  already grouped; the test looks at every beam, flagged or not, which can only ask for a sort that was not needed.
+//   pd_pose_keys   (pose - pose0, record index) of every record: the pairs a stable radix sort orders by pose
+//   pd_gather      out[i] = in[order[i]]
+__global__ void pd_pose_count(const int32_t* pose, const int32_t* flags, int64_t nb, int32_t pose0, unsigned long long* cnt,
+                              long long* unsorted) {
+    const int64_t b0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * POSE_RUN, b1 = min(nb, b0 + POSE_RUN);
+    int32_t cur = -1;
+    unsigned long long c = 0;
+    bool down = false;
+    for (int64_t b = b0; b < b1; b++) {
+        const int32_t p = pose[b];
+        down |= b > 0 && pose[b - 1] > p;
+        if (!flags[b]) continue;
+        if (p != cur && c) { atomicAdd(cnt + (cur - pose0), c); c = 0; }
+        cur = p; c++;
+    }
+    add_pose_count(cnt, cur - pose0, c, c > 0);
+    if (down) *unsorted = 1;
+}
+__global__ void pd_pose_keys(const int32_t* pose, const int32_t* flags, const long long* offs, int64_t nb, int32_t pose0, int32_t* keys,
+                             int32_t* idx) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= nb || !flags[b]) return;
+    const long long q = offs[b];
+    keys[q] = pose[b] - pose0;
+    idx[q] = (int32_t)q;
+}
+__global__ void pd_gather(const PdRec* in, const int32_t* order, PdRec* out, int64_t m) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < m) out[i] = in[order[i]];
+}
+
 // PdRec -> PdFast (after the records have been grouped by pose)
 __global__ void pd_make_fast(const PdRec* recs, PdFast* fast, int64_t m) {
     const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -500,35 +538,62 @@ static int32_t pd_run(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t po
     BMO_CUDA(d_flags.alloc((size_t)nb, st));
     BMO_CUDA(d_offs.alloc((size_t)nb, st));
     ResView rv = res_view(r);
-    pd_flag<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(rv, sys->view, pd_object, per_pose ? -1 : pose0, d_flags.get());
+    // only the records of poses [pose0, pose0 + n_fields) are built
+    pd_flag<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(rv, sys->view, pd_object, pose0, pose0 + n_fields, d_flags.get());
     BMO_LAUNCH(ctx, "pd_flag");
     scan_flags<<<1, 1024, 0, st>>>(d_flags.get(), nb, d_offs.get(), ctx->d_totals);
     BMO_LAUNCH(ctx, "scan_flags");
-    BMO_CUDA(cudaMemcpyAsync(ctx->h_totals, ctx->d_totals, sizeof(long long), cudaMemcpyDeviceToHost, st));
+    // per pose: the record count of every pose (cnt, closed by a zero so that its exclusive scan ends with m) and, next to m,
+    // whether the records need sorting -- read back with m
+    DevBuf<unsigned long long> cnt;
+    if (per_pose) {
+        BMO_CUDA(cnt.alloc((size_t)n_fields + 1, st));
+        BMO_CUDA(cudaMemsetAsync(cnt.get(), 0, ((size_t)n_fields + 1) * sizeof(unsigned long long), st));
+        BMO_CUDA(cudaMemsetAsync(ctx->d_totals + 1, 0, sizeof(long long), st));
+        const int64_t runs = (nb + POSE_RUN - 1) / POSE_RUN;
+        pd_pose_count<<<(unsigned)((runs + 255) / 256), 256, 0, st>>>(r->pose, d_flags.get(), nb, pose0, cnt.get(), ctx->d_totals + 1);
+        BMO_LAUNCH(ctx, "pd_pose_count");
+    }
+    BMO_CUDA(cudaMemcpyAsync(ctx->h_totals, ctx->d_totals, (per_pose ? 2 : 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
     const int64_t m = ctx->h_totals[0];
+    const bool unsorted = per_pose && ctx->h_totals[1] != 0;
     if (m > 0) {
         BMO_CUDA(d_recs.alloc((size_t)m, st));
         pd_build<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(rv, sys->view, d_flags.get(), d_offs.get(), d_recs.get());
         BMO_LAUNCH(ctx, "pd_build");
         if (per_pose) {
-            // group the records by pose (stable): tiny host round trip (m records)
-            std::vector<PdRec> h((size_t)m);
-            BMO_CUDA(cudaMemcpyAsync(h.data(), d_recs.get(), (size_t)m * sizeof(PdRec), cudaMemcpyDeviceToHost, st));
-            BMO_CUDA(cudaStreamSynchronize(st));
-            std::stable_sort(h.begin(), h.end(), [](const PdRec& a, const PdRec& b) { return a.pose < b.pose; });
-            std::vector<long long> off((size_t)n_fields + 1, 0);
-            size_t q = 0;
-            for (int p = 0; p < n_fields; p++) {
-                while (q < h.size() && (int)h[q].pose < pose0 + p) q++;
-                off[p] = (long long)q;
+            // group the records by pose, stably (the order std::stable_sort by pose gives), on the device; one pose needs no sort
+            if (unsorted && n_fields > 1) {
+                if (m > INT32_MAX) return fail(BMO_EINVAL, "bmo_pd_accumulate_poses: more records than a 32-bit index can number");
+                DevBuf<int32_t> keys, idx, keys_out, order;
+                DevBuf<PdRec> sorted;
+                DevBuf<char> tmp;
+                size_t tmp_bytes = 0;
+                const int end_bit = 32 - __builtin_clz((unsigned)(n_fields - 1));
+                BMO_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys.get(), keys_out.get(), idx.get(), order.get(), (int)m, 0, end_bit, st));
+                BMO_CUDA(keys.alloc((size_t)m, st));
+                BMO_CUDA(idx.alloc((size_t)m, st));
+                BMO_CUDA(keys_out.alloc((size_t)m, st));
+                BMO_CUDA(order.alloc((size_t)m, st));
+                BMO_CUDA(tmp.alloc(tmp_bytes, st));
+                pd_pose_keys<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(r->pose, d_flags.get(), d_offs.get(), nb, pose0, keys.get(), idx.get());
+                BMO_LAUNCH(ctx, "pd_pose_keys");
+                BMO_CUDA(cub::DeviceRadixSort::SortPairs(tmp.get(), tmp_bytes, keys.get(), keys_out.get(), idx.get(), order.get(), (int)m, 0, end_bit, st));
+                BMO_LAUNCH(ctx, "radix sort by pose");
+                BMO_CUDA(sorted.alloc((size_t)m, st));
+                pd_gather<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(d_recs.get(), order.get(), sorted.get(), m);
+                BMO_LAUNCH(ctx, "pd_gather");
+                d_recs = std::move(sorted);
             }
-            while (q < h.size() && (int)h[q].pose < pose0 + n_fields) q++;
-            off[n_fields] = (long long)q;
-            BMO_CUDA(cudaMemcpyAsync(d_recs.get(), h.data(), (size_t)m * sizeof(PdRec), cudaMemcpyHostToDevice, st));
-            BMO_CUDA(d_pose_off.alloc(off.size(), st));
-            BMO_CUDA(cudaMemcpyAsync(d_pose_off.get(), off.data(), off.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
-            BMO_CUDA(cudaStreamSynchronize(st));
+            size_t scan_bytes = 0;
+            BMO_CUDA(d_pose_off.alloc((size_t)n_fields + 1, st));
+            long long* cnt_in = reinterpret_cast<long long*>(cnt.get());
+            BMO_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, cnt_in, d_pose_off.get(), n_fields + 1, st));
+            DevBuf<char> scan_tmp;
+            BMO_CUDA(scan_tmp.alloc(scan_bytes, st));
+            BMO_CUDA(cub::DeviceScan::ExclusiveSum(scan_tmp.get(), scan_bytes, cnt_in, d_pose_off.get(), n_fields + 1, st));
+            BMO_LAUNCH(ctx, "pose offsets");
         }
         if (!ref_order) {
             BMO_CUDA(d_fast.alloc((size_t)m, st));
@@ -581,22 +646,26 @@ int32_t bmo_pd_sweep(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t n_p
     bmo_ctx* ctx = sys->ctx;
     BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const bmo_object& ob = sys->objects[pd_object];
-    const int n = ob.pd_n;
+    const int n = sys->objects[pd_object].pd_n;
     const size_t cnt = (size_t)n_poses * n * n * 2;
     DevBuf<double> d_field, d_p;
     BMO_CUDA(d_field.alloc(cnt, st));
-    BMO_CUDA(cudaMemsetAsync(d_field.get(), 0, cnt * sizeof(double), st));
-    int32_t rc = pd_run(sys, r, pd_object, 0, n_poses, d_field.get(), (flags | BMO_INPUT_DEVICE), true);
+    if (power) BMO_CUDA(d_p.alloc((size_t)n_poses, st));
+    const int32_t rc = pd_sweep_device(sys, r, pd_object, n_poses, d_field.get(), d_p.get(), flags);
     if (rc) return rc;
-    if (power) {
-        BMO_CUDA(d_p.alloc((size_t)n_poses, st));
-        if ((rc = pd_power_launch(ctx, d_field.get(), n_poses, n, ob.pd_lo, ob.pd_hi, d_p.get(), st))) return rc;
-        BMO_CUDA(cudaMemcpyAsync(power, d_p.get(), (size_t)n_poses * sizeof(double), cudaMemcpyDeviceToHost, st));
-    }
+    if (power) BMO_CUDA(cudaMemcpyAsync(power, d_p.get(), (size_t)n_poses * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (fields) BMO_CUDA(cudaMemcpyAsync(fields, d_field.get(), cnt * sizeof(double), cudaMemcpyDeviceToHost, st));
     BMO_CUDA(cudaStreamSynchronize(st));
     return BMO_OK;
+}
+int32_t bmo::pd_sweep_device(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t n_poses, double* d_field, double* d_power, uint32_t flags) {
+    bmo_ctx* ctx = sys->ctx;
+    const bmo_object& ob = sys->objects[pd_object];
+    const int n = ob.pd_n;
+    BMO_CUDA(cudaMemsetAsync(d_field, 0, (size_t)n_poses * n * n * 2 * sizeof(double), ctx->stream));
+    int32_t rc = pd_run(sys, r, pd_object, 0, n_poses, d_field, (flags | BMO_INPUT_DEVICE), true);
+    if (!rc && d_power) rc = pd_power_launch(ctx, d_field, n_poses, n, ob.pd_lo, ob.pd_hi, d_power, ctx->stream);
+    return rc;
 }
 int32_t bmo_pd_power(bmo_sys* sys, int32_t pd_object, int32_t n_fields, const double* fields, double* power, uint32_t flags) {
     if (!sys || !fields || !power) return fail(BMO_EINVAL, "bmo_pd_power: NULL argument");

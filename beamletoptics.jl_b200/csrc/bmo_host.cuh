@@ -342,6 +342,25 @@ template <class T> inline int32_t upload(DevTable<T>& out, const T* h, size_t n)
     return BMO_OK;
 }
 
+// ---- per-pose counts of a result's beams (spot_pose_count in bmo_source.cu, pd_pose_count in bmo_detector.cu) ----------------
+// Each thread counts a run of POSE_RUN consecutive beams and adds a count when the pose changes, and the lanes of a warp that
+// flush the same pose add once: a pose-major result takes about one atomic per warp, not per beam.
+constexpr int64_t POSE_RUN = 64;
+__device__ __forceinline__ void add_pose_count(unsigned long long* cnt, int32_t p, unsigned long long c, bool act) {
+    const unsigned live = __ballot_sync(0xffffffffu, act);
+    if (!act) return;
+    const unsigned same = __match_any_sync(live, p);
+    unsigned long long sum = 0;
+    for (unsigned m = same; m; m &= m - 1) sum += __shfl_sync(same, c, __ffs(m) - 1);
+    if ((int)(threadIdx.x & 31) == __ffs(same) - 1) atomicAdd(cnt + p, sum);
+}
+
+// ---- Photodetector pose sweep (bmo_detector.cu), shared with bmo_pd_sweep_sharded (bmo_comm.cu) ----------------------------
+// bmo_pd_sweep's work without its copies, enqueued on the context's stream: d_field ([n_poses][n*n*2], device) is zeroed and
+// receives the fields of poses [0, n_poses), d_power ([n_poses], device, NULL: not wanted) their optical powers.  The caller
+// has checked the arguments.
+int32_t pd_sweep_device(bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t n_poses, double* d_field, double* d_power, uint32_t flags);
+
 // ---- spot statistics (bmo_source.cu), shared with bmo_spot_stats_sharded (bmo_comm.cu) ---------------------------
 // entries per block of a reduction over m spot entries: 4096 * max(1, ceil(m / (4096 * 1024))), the partition include/bmo.h fixes
 inline int64_t spot_per(int64_t m) { return BMO_SPOT_PER(m); }

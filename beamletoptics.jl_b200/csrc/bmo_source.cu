@@ -370,17 +370,7 @@ __global__ void spot_combine(const SpotPartial* __restrict__ all, int32_t n_rank
 }
 
 // per-pose beam counts of a result; bit 0 of *flags: the poses are not in non-decreasing beam order, bit 1: a pose id
-// outside [0, n_poses).  Each thread counts a run of POSE_RUN consecutive beams and adds a count when the pose changes, and
-// the lanes of a warp that flush the same pose add once: a pose-major result takes about one atomic per warp, not per beam.
-constexpr int64_t POSE_RUN = 64;
-__device__ __forceinline__ void add_pose_count(unsigned long long* cnt, int32_t p, unsigned long long c, bool act) {
-    const unsigned live = __ballot_sync(0xffffffffu, act);
-    if (!act) return;
-    const unsigned same = __match_any_sync(live, p);
-    unsigned long long sum = 0;
-    for (unsigned m = same; m; m &= m - 1) sum += __shfl_sync(same, c, __ffs(m) - 1);
-    if ((int)(threadIdx.x & 31) == __ffs(same) - 1) atomicAdd(cnt + p, sum);
-}
+// outside [0, n_poses).  Counted in runs of POSE_RUN beams (add_pose_count, bmo_host.cuh).
 __global__ void spot_pose_count(const int32_t* pose, int64_t nb, int32_t n_poses, unsigned long long* cnt, unsigned int* flags) {
     const int64_t b0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * POSE_RUN, b1 = min(nb, b0 + POSE_RUN);
     int32_t cur = -1;

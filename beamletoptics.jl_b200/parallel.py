@@ -10,7 +10,9 @@ fields are summed with one all-reduce of 2 n^2 doubles (the reference adds the b
 diagram of a DeviceSource sharded with spot_shard_slice is reduced where the hits are (solve_spot_sharded:
 bmo_spot_stats_sharded all-gathers per-block partials, not hits) and has the bits of the unsharded solve.  A PSFDetector map
 is sharded by pixel columns (solve_psf_sharded): the ranks all-gather their hit records in rank order, each sums all records
-into its band of columns, and the bands are all-gathered; for a splitter-free system the map has the bits of one solve.
+into its band of columns, and the bands are all-gathered; for a splitter-free system the map has the bits of one solve.  A
+Photodetector pose sweep is sharded by pose range (solve_pose_sweep_sharded): each rank traces its poses into fields of its own,
+which never leave it, and only the powers are all-gathered; every pose has the bits of the one-GPU sweep.
 """
 import ctypes as C
 import math
@@ -100,6 +102,25 @@ class FieldComm:
         finally:
             lib.bmo_psf_free(all_)
         return psf_axes(n, lims, x0_shift, z0_shift) + (I,)
+
+    def pd_sweep(self, dsys, result, pd_index, n_poses, first, count, want_fields=True):
+        """bmo_pd_sweep_sharded, collective: this rank's `dsys` holds poses [first, first + count) of an n_poses-pose sweep as its
+        poses 0 .. count - 1 and `result` is their trace (None on a rank without poses).  Returns (power (n_poses,) of every
+        rank's poses in pose order, this rank's fields (count, n, n) complex or None).  BmoError on every rank if any rank's
+        arguments are refused."""
+        from . import components as co
+        objs = dsys.flat.objects
+        n = objs[pd_index].n if 0 <= pd_index < len(objs) and isinstance(objs[pd_index], co.Photodetector) else 0   # else refused
+        fields = np.zeros((count, n * n * 2)) if want_fields and count > 0 and n > 0 else None
+        power = np.zeros(max(int(n_poses), 0))
+        L.check(L.lib().bmo_pd_sweep_sharded(self.h, dsys.h, None if result is None else result.h, int(pd_index), int(n_poses), int(first),
+                                             int(count), L.ptr(fields), L.ptr(power), 0))
+        if not want_fields:
+            return power, None
+        if fields is None:
+            return power, np.zeros((0, n, n), np.complex128)
+        z = fields[:, 0::2] + 1j * fields[:, 1::2]
+        return power, z.reshape(count, n, n).transpose(0, 2, 1)   # stored column-major [i + n*j] -> [pose, i, j]
 
     def free(self):
         if self.h:
@@ -275,6 +296,42 @@ def solve_psf_sharded(system, source, detector, n=100, crop_factor=1.0, center="
         dsys = cached_system(system, _lambda_ids(lams)[0], comm.device)
         detector._dsys, detector._index = dsys, next(i for i, o in enumerate(dsys.flat.objects) if o is detector)
     return comm.psf_intensity(detector, n, crop_factor, center, x_min, x_max, z_min, z_max, x0_shift, z0_shift)
+
+
+def solve_pose_sweep_sharded(system, beam, n_poses, pd, program=None, apply_pose=None, comm=None, want_fields=True, r_max=100):
+    """A Photodetector pose sweep (solve_pose_sweep_device / solve_pose_sweep) across all ranks: this rank sweeps its shard_slice
+    [first, first + count) of the n_poses poses on the communicator's GPU and bmo_pd_sweep_sharded gathers the powers.  Exactly one
+    of `program` (records the kinematic calls of the whole sweep on a KinProgram; the rank applies its rows) and `apply_pose`
+    (apply_pose(p) moves the host objects into pose p; called for the rank's p only) is given.  `beam`: GaussianBeamlet,
+    BeamletBundle or DeviceBeamletSource, tiled `count` times.  Returns, on every rank, dict(power=(n_poses,), fields=(count, n, n)
+    complex of this rank's poses or None, first=first, result=TraceResult or None, dsys=DeviceSystem): pose p's power and field
+    have the bits of the one-GPU sweep (DESIGN §14).  `comm`: a FieldComm (default: default_comm())."""
+    from . import sweep as sw
+    from .flatten import FlatSystem
+    from .solver import DeviceSystem
+    if (program is None) == (apply_pose is None):
+        raise ValueError("solve_pose_sweep_sharded: give exactly one of program and apply_pose")
+    n_poses = int(n_poses)
+    if n_poses < 1:
+        raise ValueError(f"solve_pose_sweep_sharded: n_poses = {n_poses}, at least one pose is needed")
+    comm = default_comm() if comm is None else comm
+    first, stop = shard_slice(n_poses, comm.rank, comm.world_size)
+    count = stop - first
+    lams, lam_id, beam = sw._beamlet_lambdas(beam)
+    if apply_pose is not None and count:
+        f0, (prims, verts, bounds, det_pos, det_dir) = sw.flatten_poses(system, lams, count, lambda k: apply_pose(first + k))
+        dsys = DeviceSystem(f0, comm.device)
+        L.check(L.lib().bmo_system_set_poses(dsys.h, count, L.ptr(prims), L.ptr(verts), L.ptr(bounds), L.ptr(det_pos), L.ptr(det_dir)))
+    else:
+        f0 = FlatSystem(system, lams)
+        dsys = DeviceSystem(f0, comm.device)
+        if count:
+            prog = sw.KinProgram(f0, n_poses)
+            program(prog)
+            prog.apply(dsys, first, count)
+    res = sw._trace_beamlet_sweep(dsys, beam, lam_id, count, r_max) if count else None
+    power, fields = comm.pd_sweep(dsys, res, f0.object_index(pd), n_poses, first, count, want_fields)
+    return dict(power=power, fields=fields, first=first, result=res, dsys=dsys)
 
 
 def solve_system_sharded(system, bundle, r_max=100, interleaved=False, keep_segments=False, group=None, comm=None):

@@ -111,15 +111,27 @@ class KinProgram:
         else:
             self.ops.append((self.ROT_LEAF, a, 0, k))
 
-    def apply(self, dsys):
-        """Install the kinematic tree (once per DeviceSystem) and run the program: dsys then holds n_poses poses."""
+    def param_table(self, first=0, count=None):
+        """Rows [first, first + count) of the parameter table ([pose][param][9]; count=None: to the last pose)."""
+        first = int(first)
+        count = self.n_poses - first if count is None else int(count)
+        if first < 0 or count < 1 or first + count > self.n_poses:
+            raise ValueError(f"KinProgram: poses [{first}, {first + count}) outside [0, {self.n_poses})")
+        if not self.params:
+            return np.zeros((count, 0, 9))
+        return np.ascontiguousarray(np.stack([p[first:first + count] for p in self.params], axis=1))
+
+    def apply(self, dsys, first=0, count=None):
+        """Install the kinematic tree (once per DeviceSystem) and run the program for poses [first, first + count) (count=None:
+        to the last pose): dsys then holds them as its poses 0 .. count - 1, each with the bits of the same pose of the whole
+        program (the device computes every pose from its own row of the parameter table)."""
+        params = self.param_table(first, count)
         lib = L.lib()
         if getattr(dsys, "_kin_installed", None) is not self.flat:
             L.check(lib.bmo_system_set_kinematics(dsys.h, len(self.nodes), C.byref(self.nodes), L.ptr(self.prim_bounds)))
             dsys._kin_installed = self.flat
         ops = (L.bmo_kin_op * max(len(self.ops), 1))(*[L.bmo_kin_op(*o) for o in self.ops])
-        params = np.ascontiguousarray(np.stack(self.params, axis=1)) if self.params else np.zeros((self.n_poses, 0, 9))
-        L.check(lib.bmo_system_apply_poses(dsys.h, self.n_poses, len(self.ops), C.byref(ops), len(self.params), L.ptr(params)))
+        L.check(lib.bmo_system_apply_poses(dsys.h, params.shape[0], len(self.ops), C.byref(ops), len(self.params), L.ptr(params)))
 
 
 def get_pose_tables(dsys, pose):

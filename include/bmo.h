@@ -555,6 +555,19 @@ int32_t bmo_psf_allgather(bmo_comm* comm, bmo_psf* local, bmo_psf** all);
  * there is no NCCL call.  Only arguments are agreed on, as in bmo_spot_stats_sharded.                                     */
 int32_t bmo_psf_intensity_sharded(bmo_comm* comm, bmo_sys* sys, bmo_psf* all, int32_t psf_object, int32_t pose, int32_t n,
                                   const double* lims, double x0_shift, double z0_shift, double* intensity, uint32_t flags);
+/* bmo_pd_sweep over ranks by pose range, collective: rank k sweeps poses [first_k, first_k + count_k) of an n_poses-pose sweep.
+ * Its `sys` holds those count_k poses as its poses 0 .. count_k - 1 and `r` is their trace (pose ids 0 .. count_k - 1); a rank
+ * with count == 0 passes r = NULL and still takes part.  fields: this rank's [count][n*n*2] (NULL ok), never exchanged; power:
+ * [n_poses] on every rank.  Both host pointers, or device pointers with BMO_INPUT_DEVICE.  Steps, on the context's stream:
+ * (1) all-gather of each rank's verdict (bmo_pd_sweep's checks on its poses; sys or r on another context than comm), pd_object,
+ * the detector's n, n_poses, first and count; a refusal, another pd_object, n or n_poses than rank 0's, or ranges that do not
+ * tile [0, n_poses) in rank order make every rank return the same code; (2) the rank's fields and powers with bmo_pd_sweep's
+ * code; (3) one all-gather of the powers, padded to the largest count, each rank's part then copied into pose order.  A pose's
+ * field and power have the bits bmo_pd_sweep gives it in one sweep of all poses when the rank's trace holds the same records
+ * for it in the same order (DESIGN §14).  With one rank there is no NCCL call.  Only arguments are agreed on, as in
+ * bmo_spot_stats_sharded.                                                                                                     */
+int32_t bmo_pd_sweep_sharded(bmo_comm* comm, bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t n_poses, int32_t first, int32_t count,
+                             double* fields, double* power, uint32_t flags);
 int32_t bmo_comm_free(bmo_comm* comm);
 
 /* Give device memory back: the library keeps released blocks of 64 MiB and more in a per-device free list and smaller ones in
