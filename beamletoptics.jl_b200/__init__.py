@@ -22,7 +22,7 @@ from .solver import DeviceSystem, TraceResult, pd_accumulate, retrace, solve_sys
 from .sweep import (flatten_poses, solve_pose_sweep, KinProgram, get_pose_tables, solve_pose_sweep_device, solve_spot_sweep,
                     solve_spot_sweep_device, tile_ray_bundle)
 from . import parallel
-from .parallel import solve_pose_sweep_sharded, solve_spot_sharded, solve_system_sharded
+from .parallel import solve_pose_sweep_sharded, solve_spot_sharded, solve_spot_sweep_sharded, solve_system_sharded
 
 
 # function-style kinematic API of the reference: translate3d!(obj, v) -> translate3d_(obj, v)

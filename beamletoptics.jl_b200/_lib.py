@@ -122,6 +122,7 @@ EXPORTS = [
     "bmo_source_create_poses", "bmo_source_pose_ids", "bmo_spot_stats_poses",
     "bmo_source_create_slice", "bmo_spot_stats_results", "bmo_spot_stats_sharded",
     "bmo_psf_intensity_cols", "bmo_psf_allgather", "bmo_psf_intensity_sharded", "bmo_pd_sweep_sharded",
+    "bmo_spot_stats_poses_sharded",
     "bmo_source_create_beamlets", "bmo_source_beamlets_device", "bmo_source_beamlets",
     "bmo_comm_unique_id", "bmo_comm_init", "bmo_comm_init_local", "bmo_comm_info", "bmo_pd_allreduce", "bmo_pd_allreduce_local", "bmo_comm_free",
 ]
@@ -194,6 +195,8 @@ def lib():
         L.bmo_psf_allgather.argtypes = [_vp, _vp, C.POINTER(_vp)]
         L.bmo_psf_intensity_sharded.argtypes = [_vp, _vp, _vp, C.c_int32, C.c_int32, C.c_int32, _vp, C.c_double, C.c_double, _vp, C.c_uint32]
         L.bmo_pd_sweep_sharded.argtypes = [_vp, _vp, _vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _vp, _vp, C.c_uint32]
+        L.bmo_spot_stats_poses_sharded.argtypes = [_vp, _vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _vp, C.c_int32, C.c_int32,
+                                                   C.POINTER(bmo_spot_info), _vp, C.c_uint32]
         L.bmo_source_create_beamlets.argtypes = [_vp, C.POINTER(bmo_source_desc), C.POINTER(bmo_beamlet_desc), C.c_int32, C.c_int64, C.c_int64,
                                                  C.POINTER(_vp)]
         L.bmo_source_beamlets_device.argtypes = [_vp, C.POINTER(C.c_int64), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp)]

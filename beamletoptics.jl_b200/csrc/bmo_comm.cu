@@ -11,6 +11,9 @@
 //     all-gathered.  Each pixel is summed on one GPU over the records of one trace in order, so the map has one GPU's bits.
 //   * The Photodetector pose sweep sharded over GPUs by pose range (bmo_pd_sweep_sharded): every rank sweeps its contiguous
 //     poses with bmo_pd_sweep's code, the fields stay where they are, and the powers are all-gathered into pose order.
+//   * The spot-diagram pose sweep sharded over GPUs by pose range (bmo_spot_stats_poses_sharded): every rank reduces its
+//     contiguous poses with bmo_spot_stats_poses' code, and the statistics and histograms are all-gathered into pose order.
+//     Each pose is reduced from its own entries alone, so no sum crosses a rank.
 //
 // NCCL is bound at run time (dlopen of libnccl.so.2) so that libbmo.so has no link-time dependency on it: a host
 // that never shards never needs the library, and inside a process that already carries one (PyTorch's bundled
@@ -399,6 +402,55 @@ int32_t bmo_psf_intensity_sharded(bmo_comm* c, bmo_sys* sys, bmo_psf* all, int32
     return BMO_OK;
 }
 
+// The pose ranges of a sweep sharded by pose range (bmo_pd_sweep_sharded, bmo_spot_stats_poses_sharded).  Step 1 agrees on K words
+// per rank: the verdict, the words that must equal rank 0's, then the rank's first pose and pose count.  Every rank's items of one
+// pose -- a power, a bmo_spot_info, a histogram -- have the same size, so step 3 is one all-gather of each rank's items, padded to
+// the largest count, and one copy of each rank's part into pose order.
+struct PoseShards {
+    bmo_comm* c;
+    int W;
+    std::vector<int64_t> first, count;
+    int64_t most = 0;        // the largest count
+    explicit PoseShards(bmo_comm* comm) : c(comm), W(comm->n_ranks), first((size_t)W), count((size_t)W) {}
+
+    // Step 1, once `all` is agreed: another `what` than rank 0's, or ranges that do not tile [0, n_poses) in rank order, is refused
+    int32_t check(const std::string& fn, const std::vector<int64_t>& all, int64_t n_poses, const char* what) {
+        const size_t K = all.size() / W;
+        int64_t next = 0;
+        for (int k = 0; k < W; k++) {
+            const int64_t* a = all.data() + K * k;
+            if (!std::equal(a + 1, a + K - 2, all.data() + 1))
+                return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " passes another " + what + " than rank 0");
+            first[k] = a[K - 2];
+            count[k] = a[K - 1];
+            if (first[k] != next)
+                return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " sweeps from pose " + std::to_string(first[k]) + ", not " +
+                                            std::to_string(next) + " (the ranks' poses must tile [0, n_poses) in rank order)");
+            next += count[k];
+            most = std::max(most, count[k]);
+        }
+        if (next != n_poses)
+            return fail(BMO_EINVAL, fn + ": the ranks sweep " + std::to_string(next) + " of " + std::to_string(n_poses) + " poses");
+        return BMO_OK;
+    }
+    // The device buffer of step 3 holds items() items: [W][most] gathered, then this rank's own `most` from item mine() (one rank:
+    // only its own, from item 0).
+    size_t items() const { return (size_t)most * (W > 1 ? W + 1 : 1); }
+    size_t mine() const { return W > 1 ? (size_t)most * W : 0; }
+    // Step 3 on the context's stream, not synchronised: buf's own items (`item` bytes each) of every rank into dst, pose p at item p
+    // (dst: host pointer, or device pointer with kind cudaMemcpyDeviceToDevice).  With one rank a copy, no NCCL call.
+    int32_t gather(void* buf, size_t item, void* dst, cudaMemcpyKind kind) {
+        cudaStream_t st = c->ctx->stream;
+        char* b = (char*)buf;
+        const size_t part = (size_t)most * item;
+        if (W > 1) BMO_NCCL(g_nccl.AllGather(b + mine() * item, b, part, kNcclInt8, c->comm, st));
+        for (int k = 0; k < W; k++)
+            if (count[k])
+                BMO_CUDA(cudaMemcpyAsync((char*)dst + (size_t)first[k] * item, b + (W > 1 ? part * k : 0), (size_t)count[k] * item, kind, st));
+        return BMO_OK;
+    }
+};
+
 int32_t bmo_pd_sweep_sharded(bmo_comm* c, bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t n_poses, int32_t first, int32_t count,
                              double* fields, double* power, uint32_t flags) {
     NvtxRange nvtx_("bmo_pd_sweep_sharded");
@@ -417,52 +469,81 @@ int32_t bmo_pd_sweep_sharded(bmo_comm* c, bmo_sys* sys, bmo_result* r, int32_t p
     else if (count > 0 && r->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the result belongs to another context than the communicator");
     else if (count > 0 && r->mode != 2) rc = fail(BMO_EINVAL, fn + ": result does not hold Gaussian beamlets (Photodetector.jl:57-60)");
     const int n = rc ? 0 : sys->objects[pd_object].pd_n;
-    constexpr int K = 6;   // verdict, then pd_object, n, n_poses (as rank 0's), first, count (tiling [0, n_poses) in rank order)
+    // verdict, then pd_object, n, n_poses (as rank 0's), first, count (tiling [0, n_poses) in rank order)
     std::vector<int64_t> mine{rc, pd_object, n, n_poses, first, count}, all;
     if ((rc = agree(c, fn, mine, all))) return rc;
-    const int W = c->n_ranks;
-    int64_t next = 0, most = 0;
-    for (int k = 0; k < W; k++) {
-        const int64_t* a = all.data() + (size_t)K * k;
-        if (!std::equal(a + 1, a + 4, all.data() + 1))
-            return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " passes another detector, detector size or pose count than rank 0");
-        if (a[4] != next)
-            return fail(BMO_EINVAL, fn + ": rank " + std::to_string(k) + " sweeps from pose " + std::to_string(a[4]) + ", not " + std::to_string(next) +
-                                        " (the ranks' poses must tile [0, n_poses) in rank order)");
-        next += a[5];
-        most = std::max(most, a[5]);
-    }
-    if (next != n_poses)
-        return fail(BMO_EINVAL, fn + ": the ranks sweep " + std::to_string(next) + " of " + std::to_string(n_poses) + " poses");
+    PoseShards ps(c);
+    if ((rc = ps.check(fn, all, n_poses, "detector, detector size or pose count"))) return rc;
     // Step 2: this rank's fields and powers, on the device
     bmo_ctx* ctx = c->ctx;
     BMO_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const bool on_dev = flags & BMO_INPUT_DEVICE;
-    const cudaMemcpyKind out_kind = on_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
     const size_t fcount = (size_t)count * n * n * 2;
     DevBuf<double> f_buf, p_buf;
-    BMO_CUDA(p_buf.alloc((size_t)most * (W > 1 ? W + 1 : 1), st));   // [W][most] gathered, then this rank's powers
-    double* my_power = p_buf.get() + (W > 1 ? (size_t)most * W : 0);
+    BMO_CUDA(p_buf.alloc(ps.items(), st));
     if (count > 0) {
         double* d_field = fields;     // the caller's device buffer
         if (!on_dev || !fields) {
             BMO_CUDA(f_buf.alloc(fcount, st));
             d_field = f_buf.get();
         }
-        if ((rc = pd_sweep_device(sys, r, pd_object, count, d_field, my_power, flags))) return rc;
+        if ((rc = pd_sweep_device(sys, r, pd_object, count, d_field, p_buf.get() + ps.mine(), flags))) return rc;
         if (fields && !on_dev) BMO_CUDA(cudaMemcpyAsync(fields, d_field, fcount * sizeof(double), cudaMemcpyDeviceToHost, st));
     }
-    // Step 3: the powers of all ranks, padded to the largest count, and each rank's part copied into pose order
-    if (W == 1) {
-        BMO_CUDA(cudaMemcpyAsync(power, my_power, (size_t)count * sizeof(double), out_kind, st));
-    } else {
-        BMO_NCCL(g_nccl.AllGather(my_power, p_buf.get(), (size_t)most, kNcclDouble, c->comm, st));
-        for (int k = 0; k < W; k++) {
-            const int64_t fk = all[(size_t)K * k + 4], ck = all[(size_t)K * k + 5];
-            if (ck) BMO_CUDA(cudaMemcpyAsync(power + fk, p_buf.get() + (size_t)most * k, (size_t)ck * sizeof(double), out_kind, st));
-        }
+    // Step 3: the powers of all ranks in pose order
+    if ((rc = ps.gather(p_buf.get(), sizeof(double), power, on_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost))) return rc;
+    BMO_CUDA(cudaStreamSynchronize(st));
+    return BMO_OK;
+}
+
+int32_t bmo_spot_stats_poses_sharded(bmo_comm* c, bmo_result* r, int32_t det_object, int32_t n_poses, int32_t first, int32_t count,
+                                     const double* window, int32_t nx, int32_t nz, bmo_spot_info* out, int64_t* counts, uint32_t flags) {
+    NvtxRange nvtx_("bmo_spot_stats_poses_sharded");
+    const std::string fn = "bmo_spot_stats_poses_sharded";
+    if (!c) return fail(BMO_EINVAL, fn + ": communicator NULL");
+    // Step 1: every rank's verdict (bmo_spot_stats_poses' checks on this rank's poses) and the arguments that must agree
+    int32_t rc = BMO_OK;
+    if (!out) rc = fail(BMO_EINVAL, fn + ": NULL argument");
+    else if (n_poses < 1 || first < 0 || count < 0 || count > n_poses - first)
+        rc = fail(BMO_EINVAL, fn + ": poses [first, first + count) outside [0, n_poses)");
+    else if (count > 0 && !r) rc = fail(BMO_EINVAL, fn + ": NULL result on a rank with poses");
+    else if (count > 0 && r->ctx != c->ctx) rc = fail(BMO_EINVAL, fn + ": the result belongs to another context than the communicator");
+    else if (count > 0 && r->n_poses != count)
+        rc = fail(BMO_EINVAL, fn + ": count " + std::to_string(count) + " differs from the " + std::to_string(r->n_poses) +
+                                  " poses the result was traced with");
+    else if (count > 0) rc = spot_check_result(fn, r, det_object);
+    if (!rc) rc = spot_check_args(fn, window, nx, nz, counts);
+    // verdict, then det_object, n_poses, histogram?, nx, nz, window?, window bits [4] (as rank 0's), first, count (tiling [0, n_poses))
+    std::vector<int64_t> mine(13, 0), all;
+    mine[0] = rc; mine[1] = det_object; mine[2] = n_poses;
+    if (counts) { mine[3] = 1; mine[4] = nx; mine[5] = nz; }
+    if (window) { mine[6] = 1; std::memcpy(&mine[7], window, 4 * sizeof(double)); }
+    mine[11] = first; mine[12] = count;
+    if ((rc = agree(c, fn, mine, all))) return rc;
+    PoseShards ps(c);
+    if ((rc = ps.check(fn, all, n_poses, "detector, pose count, histogram shape or window"))) return rc;
+    // Step 2: this rank's statistics with bmo_spot_stats_poses' code, its histograms into the device buffer of step 3
+    bmo_ctx* ctx = c->ctx;
+    BMO_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const size_t bins = counts ? (size_t)nx * (size_t)nz : 0;
+    DevBuf<bmo_spot_info> i_buf;
+    DevBuf<int64_t> h_buf;
+    BMO_CUDA(i_buf.alloc(ps.items(), st));
+    if (counts) BMO_CUDA(h_buf.alloc(ps.items() * bins, st));
+    std::vector<bmo_spot_info> info((size_t)count);
+    if (count > 0) {
+        if ((rc = spot_stats(fn.c_str(), 1, &r, det_object, count, window, nx, nz, info.data(), counts ? h_buf.get() + ps.mine() * bins : nullptr,
+                             BMO_INPUT_DEVICE)))
+            return rc;
+        BMO_CUDA(cudaMemcpyAsync(i_buf.get() + ps.mine(), info.data(), (size_t)count * sizeof(bmo_spot_info), cudaMemcpyHostToDevice, st));
     }
+    // Step 3: the statistics and histograms of all ranks in pose order
+    if ((rc = ps.gather(i_buf.get(), sizeof(bmo_spot_info), out, cudaMemcpyDeviceToHost))) return rc;
+    if (counts && (rc = ps.gather(h_buf.get(), bins * sizeof(int64_t), counts,
+                                  (flags & BMO_INPUT_DEVICE) ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost)))
+        return rc;
     BMO_CUDA(cudaStreamSynchronize(st));
     return BMO_OK;
 }

@@ -367,6 +367,10 @@ inline int64_t spot_per(int64_t m) { return BMO_SPOT_PER(m); }
 // bmo_spot_stats's argument checks: on the result (non-NULL, det_object a Spotdetector of its system), on the rest
 int32_t spot_check_result(const std::string& fn, const bmo_result* r, int32_t det_object);
 int32_t spot_check_args(const std::string& fn, const double* window, int32_t nx, int32_t nz, const void* counts);
+// bmo_spot_stats, bmo_spot_stats_poses and bmo_spot_stats_results (n_res results, n_poses poses) under the name `what`: out is a
+// host pointer, counts a host pointer or, with BMO_INPUT_DEVICE, a device pointer; the stream is synchronised on return
+int32_t spot_stats(const char* what, int32_t n_res, bmo_result* const* rs, int32_t det_object, int32_t n_poses, const double* window,
+                   int32_t nx, int32_t nz, bmo_spot_info* out, int64_t* counts, uint32_t flags);
 // the collective steps of bmo_spot_stats_sharded, on the context's stream
 struct SpotExchange {
     virtual int32_t gather(const void* mine, void* all, size_t bytes) = 0;   // all[r * bytes ...] = rank r's `bytes` bytes

@@ -648,8 +648,8 @@ int32_t bmo::spot_check_args(const std::string& fn, const double* window, int32_
 
 // bmo_spot_stats (one result, n_poses = 1: every entry, index order), bmo_spot_stats_poses (one result, n_poses = its pose
 // count) and bmo_spot_stats_results (several results, n_poses = 1: their entries concatenated in list order)
-static int32_t spot_stats(const char* what, int32_t n_res, bmo_result* const* rs, int32_t det_object, int32_t n_poses, const double* window,
-                          int32_t nx, int32_t nz, bmo_spot_info* out, int64_t* counts, uint32_t flags) {
+int32_t bmo::spot_stats(const char* what, int32_t n_res, bmo_result* const* rs, int32_t det_object, int32_t n_poses, const double* window,
+                        int32_t nx, int32_t nz, bmo_spot_info* out, int64_t* counts, uint32_t flags) {
     const std::string fn(what);
     if (!out) return fail(BMO_EINVAL, fn + ": NULL argument");
     int32_t rc;

@@ -12,7 +12,9 @@ bmo_spot_stats_sharded all-gathers per-block partials, not hits) and has the bit
 is sharded by pixel columns (solve_psf_sharded): the ranks all-gather their hit records in rank order, each sums all records
 into its band of columns, and the bands are all-gathered; for a splitter-free system the map has the bits of one solve.  A
 Photodetector pose sweep is sharded by pose range (solve_pose_sweep_sharded): each rank traces its poses into fields of its own,
-which never leave it, and only the powers are all-gathered; every pose has the bits of the one-GPU sweep.
+which never leave it, and only the powers are all-gathered; every pose has the bits of the one-GPU sweep.  A spot-diagram pose
+sweep is sharded the same way (solve_spot_sweep_sharded): each rank reduces its own poses, whose hits never leave it, and the
+per-pose statistics and histograms are all-gathered; every pose has the bits of the one-GPU sweep.
 """
 import ctypes as C
 import math
@@ -121,6 +123,20 @@ class FieldComm:
             return power, np.zeros((0, n, n), np.complex128)
         z = fields[:, 0::2] + 1j * fields[:, 1::2]
         return power, z.reshape(count, n, n).transpose(0, 2, 1)   # stored column-major [i + n*j] -> [pose, i, j]
+
+    def spot_sweep(self, result, det_object, n_poses, first, count, nx=0, nz=0, window=None):
+        """bmo_spot_stats_poses_sharded, collective: `result` is this rank's trace of poses [first, first + count) of an n_poses-pose
+        sweep, traced as its poses 0 .. count - 1 (None on a rank without poses).  Returns, on every rank, solver.spot_stats_poses's
+        dict of all n_poses poses in pose order ("counts": (n_poses, nz, nx) int64 histograms over `window` when nx > 0).  BmoError
+        on every rank if any rank's arguments are refused."""
+        from .solver import _spot_pose_dict
+        P = int(n_poses)
+        counts = np.zeros((max(P, 0), max(int(nz), 0), max(int(nx), 0)), np.int64) if nx else None
+        win = None if window is None else np.ascontiguousarray(window, dtype=np.float64)
+        info = (L.bmo_spot_info * max(P, 1))()
+        L.check(L.lib().bmo_spot_stats_poses_sharded(self.h, None if result is None else result.h, int(det_object), P, int(first), int(count),
+                                                     L.ptr(win), int(nx), int(nz), info, L.ptr(counts), 0))
+        return _spot_pose_dict(info, P, counts)
 
     def free(self):
         if self.h:
@@ -307,31 +323,69 @@ def solve_pose_sweep_sharded(system, beam, n_poses, pd, program=None, apply_pose
     complex of this rank's poses or None, first=first, result=TraceResult or None, dsys=DeviceSystem): pose p's power and field
     have the bits of the one-GPU sweep (DESIGN §14).  `comm`: a FieldComm (default: default_comm())."""
     from . import sweep as sw
-    from .flatten import FlatSystem
-    from .solver import DeviceSystem
-    if (program is None) == (apply_pose is None):
-        raise ValueError("solve_pose_sweep_sharded: give exactly one of program and apply_pose")
-    n_poses = int(n_poses)
-    if n_poses < 1:
-        raise ValueError(f"solve_pose_sweep_sharded: n_poses = {n_poses}, at least one pose is needed")
+    n_poses = _check_sweep_args("solve_pose_sweep_sharded", n_poses, program, apply_pose)
     comm = default_comm() if comm is None else comm
     first, stop = shard_slice(n_poses, comm.rank, comm.world_size)
     count = stop - first
     lams, lam_id, beam = sw._beamlet_lambdas(beam)
+    f0, dsys = _pose_range_system(system, lams, n_poses, first, count, program, apply_pose, comm.device)
+    res = sw._trace_beamlet_sweep(dsys, beam, lam_id, count, r_max) if count else None
+    power, fields = comm.pd_sweep(dsys, res, f0.object_index(pd), n_poses, first, count, want_fields)
+    return dict(power=power, fields=fields, first=first, result=res, dsys=dsys)
+
+
+def solve_spot_sweep_sharded(system, beam, n_poses, detector, program=None, apply_pose=None, bins=None, window=None, comm=None, r_max=100):
+    """A spot-diagram pose sweep (solve_spot_sweep_device / solve_spot_sweep) across all ranks: this rank sweeps its shard_slice
+    [first, first + count) of the n_poses poses on the communicator's GPU and bmo_spot_stats_poses_sharded gathers the statistics.
+    Exactly one of `program` (records the kinematic calls of the whole sweep on a KinProgram; the rank applies its rows) and
+    `apply_pose` (apply_pose(p) moves the host objects into pose p; called for the rank's p only) is given.  `beam`: RayBundle or
+    DeviceSource, traced once per local pose.  `bins` / `window` as in spot_stats_poses.  Returns, on every rank,
+    dict(stats=spot_stats_poses's dict of all n_poses poses, first=first, result=TraceResult or None, dsys=DeviceSystem): pose p has
+    the bits of the one-GPU sweep (DESIGN §15).  `comm`: a FieldComm (default: default_comm())."""
+    from . import sweep as sw
+    from .solver import _spot_args
+    n_poses = _check_sweep_args("solve_spot_sweep_sharded", n_poses, program, apply_pose)
+    comm = default_comm() if comm is None else comm
+    first, stop = shard_slice(n_poses, comm.rank, comm.world_size)
+    count = stop - first
+    lams, lam_id = sw._beam_lambdas(beam)
+    f0, dsys = _pose_range_system(system, lams, n_poses, first, count, program, apply_pose, comm.device)
+    oi, nx, nz, win = _spot_args(f0.objects, detector, bins, window, "solve_spot_sweep_sharded")
+    res = sw._trace_spot_sweep(dsys, beam, lam_id, count, r_max) if count else None
+    stats = comm.spot_sweep(res, oi, n_poses, first, count, nx, nz, win)
+    return dict(stats=stats, first=first, result=res, dsys=dsys)
+
+
+def _check_sweep_args(what, n_poses, program, apply_pose):
+    """n_poses as an int, once exactly one of program and apply_pose is given and there is at least one pose."""
+    if (program is None) == (apply_pose is None):
+        raise ValueError(f"{what}: give exactly one of program and apply_pose")
+    n_poses = int(n_poses)
+    if n_poses < 1:
+        raise ValueError(f"{what}: n_poses = {n_poses}, at least one pose is needed")
+    return n_poses
+
+
+def _pose_range_system(system, lams, n_poses, first, count, program, apply_pose, device):
+    """(FlatSystem, DeviceSystem on `device`) of a sweep's poses [first, first + count), held as the system's poses 0 .. count - 1,
+    each with the bits of the same pose of the whole sweep: `program` records the kinematic calls of all n_poses poses on a
+    KinProgram and its rows [first, first + count) are applied on the device, or apply_pose(p) moves the host objects into pose p
+    for those p only.  With count == 0 the system is uploaded as it is."""
+    from . import sweep as sw
+    from .flatten import FlatSystem
+    from .solver import DeviceSystem
     if apply_pose is not None and count:
         f0, (prims, verts, bounds, det_pos, det_dir) = sw.flatten_poses(system, lams, count, lambda k: apply_pose(first + k))
-        dsys = DeviceSystem(f0, comm.device)
+        dsys = DeviceSystem(f0, device)
         L.check(L.lib().bmo_system_set_poses(dsys.h, count, L.ptr(prims), L.ptr(verts), L.ptr(bounds), L.ptr(det_pos), L.ptr(det_dir)))
     else:
         f0 = FlatSystem(system, lams)
-        dsys = DeviceSystem(f0, comm.device)
+        dsys = DeviceSystem(f0, device)
         if count:
             prog = sw.KinProgram(f0, n_poses)
             program(prog)
             prog.apply(dsys, first, count)
-    res = sw._trace_beamlet_sweep(dsys, beam, lam_id, count, r_max) if count else None
-    power, fields = comm.pd_sweep(dsys, res, f0.object_index(pd), n_poses, first, count, want_fields)
-    return dict(power=power, fields=fields, first=first, result=res, dsys=dsys)
+    return f0, dsys
 
 
 def solve_system_sharded(system, bundle, r_max=100, interleaved=False, keep_segments=False, group=None, comm=None):

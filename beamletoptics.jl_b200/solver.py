@@ -577,6 +577,11 @@ def spot_stats_poses(result, detector, n_poses, bins=None, window=None):
     counts = None if bins is None else np.zeros((max(P, 0), max(nz, 0), max(nx, 0)), np.int64)
     info = (L.bmo_spot_info * max(P, 1))()
     L.check(L.lib().bmo_spot_stats_poses(result.h, oi, P, L.ptr(win), nx, nz, info, L.ptr(counts), 0))
+    return _spot_pose_dict(info, P, counts)
+
+
+def _spot_pose_dict(info, P, counts):
+    """spot_stats_poses's dict of the first P entries of a bmo_spot_info array (and the (P, nz, nx) counts or None)."""
     a = np.frombuffer(info, dtype=np.dtype([("hits", np.int64), ("outside", np.int64), ("centroid", np.float64, 2), ("rms", np.float64),
                                             ("max_r", np.float64), ("lo", np.float64, 2), ("hi", np.float64, 2)]))[:P]
     out = {k: np.array(a[k]) for k in ("hits", "outside", "centroid", "rms", "max_r", "lo", "hi")}

@@ -568,6 +568,21 @@ int32_t bmo_psf_intensity_sharded(bmo_comm* comm, bmo_sys* sys, bmo_psf* all, in
  * bmo_spot_stats_sharded.                                                                                                     */
 int32_t bmo_pd_sweep_sharded(bmo_comm* comm, bmo_sys* sys, bmo_result* r, int32_t pd_object, int32_t n_poses, int32_t first, int32_t count,
                              double* fields, double* power, uint32_t flags);
+/* bmo_spot_stats_poses over ranks by pose range, collective: rank k passes the trace `r` of poses [first_k, first_k + count_k) of an
+ * n_poses-pose sweep, traced through a system that holds them as its poses 0 .. count_k - 1; a rank with count == 0 passes
+ * r = NULL and still takes part.  out: [n_poses] host array, counts (NULL ok): [n_poses][nz][nx] over the window, host pointer
+ * or device pointer with BMO_INPUT_DEVICE; every rank receives all n_poses statistics and histograms.  Steps, on the context's
+ * stream: (1) all-gather of each rank's verdict (bmo_spot_stats_poses' checks on its poses, with count as the result's pose
+ * count; r on another context than comm), det_object, n_poses, histogram shape and window bits, first and count; a refusal,
+ * another det_object, n_poses, histogram shape or window than rank 0's, or ranges that do not tile [0, n_poses) in rank order
+ * make every rank return the same code; (2) the rank's statistics with bmo_spot_stats_poses' code; (3) one all-gather of the
+ * statistics and one of the histograms, padded to the largest count, each rank's part then copied into pose order.  Each pose is
+ * reduced from its own entries only, so out[p] has the bits bmo_spot_stats_poses gives pose p in one sweep of all poses when the
+ * rank's trace lists the pose's entries in the same order (DESIGN §15).  With one rank there is no NCCL call.  Only arguments
+ * are agreed on, as in bmo_spot_stats_sharded.                                                                                */
+int32_t bmo_spot_stats_poses_sharded(bmo_comm* comm, bmo_result* r, int32_t det_object, int32_t n_poses, int32_t first, int32_t count,
+                                     const double* window, int32_t nx, int32_t nz, bmo_spot_info* out /* [n_poses] */,
+                                     int64_t* counts /* [n_poses][nz][nx], NULL ok */, uint32_t flags);
 int32_t bmo_comm_free(bmo_comm* comm);
 
 /* Give device memory back: the library keeps released blocks of 64 MiB and more in a per-device free list and smaller ones in
